@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Monte-Carlo network evals/s (1 eval = one (sample, frequency) point).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg5] [--dump-outputs DIR]
 
 Headline step = one pass of the hot path over one batch of synthetic input: BASELINE config 2
 (pcb/generic-filter 11th-order 0.1 dB Chebyshev LPF with ESR/SRF parasitics, +-5 % L / +-2 % C,
@@ -141,17 +141,25 @@ def workload(name, n_samples):
 
 
 def cpu_reference(rwl, n_samples, steps, warmup, nthreads):
-    """Times the oracle port (OpenMP over samples) on a bounded sample; returns (evals/s, s/step)."""
+    """Times the oracle port (OpenMP over samples) on a bounded sample; returns (evals/s, s/step, counters of the last step)."""
     from oracle import ref_workloads as RW
     times = []
     for i in range(warmup + steps):
         t0 = time.perf_counter()
-        RW.run(rwl, n_samples, sample_offset=i * n_samples, nthreads=nthreads)
+        r = RW.run(rwl, n_samples, sample_offset=i * n_samples, nthreads=nthreads)
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
     tot = sum(times)
-    return n_samples * len(rwl.f) * len(times) / tot, tot / len(times)
+    return n_samples * len(rwl.f) * len(times) / tot, tot / len(times), r
+
+
+def dump_outputs(out_dir, counters):
+    """The counters of the last timed step (what qo_mc_run returns for that sample range) as out_dir/<name>.npy in float64, exact
+    below 2**53.  The sample ranges depend on the arguments alone, so two builds run with the same arguments must write equal files."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("n_pass", "n_total", "fail_per_spec", "hist"):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(counters[name], dtype=np.float64))
 
 
 class ClockSampler:
@@ -210,7 +218,9 @@ def run_reference(args, rank, world):
     from oracle import ref_workloads as RW
     rwl = RW.get(args.workload, NF)
     n = REF_SAMPLES_PER_STEP
-    v, per_step = cpu_reference(rwl, n, args.steps, args.warmup, nthr)
+    v, per_step, last = cpu_reference(rwl, n, args.steps, args.warmup, nthr)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": per_step * 1e3, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -423,7 +433,10 @@ def main():
     ap.add_argument("--samples", type=int, default=SAMPLES_PER_GPU, help="samples per GPU per step")
     ap.add_argument("--no-extras", action="store_true", help="headline only: skip the north-star job, chain-kernel, CPU and FULL_S legs")
     ap.add_argument("--north-star-samples", type=int, default=NORTH_STAR_SAMPLES)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the counters of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else max(args.warmup, 1)
 
     rank, world, local = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("LOCAL_RANK", "0"))
@@ -515,6 +528,8 @@ def main():
         barrier()
         e2e_s = time.perf_counter() - t0
         clocks = sampler.stop() if sampler else None       # sampled over both timed regions (resident steps and end-to-end steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
 
     tm = torch.tensor([ms_total, e2e_s * 1e3, kernel_ms], dtype=torch.float64, device="cuda")
     if dist is not None:
@@ -625,8 +640,8 @@ def main():
             nthr = host_cores()
             rwl = RW.get(args.workload, NF)
             n = 40000
-            v, _ = cpu_reference(rwl, n, 2, 1, nthr)
-            v1, _ = cpu_reference(rwl, 2000, 1, 0, 1)          # the "single-threaded C loop over the same model" of north_star
+            v, _, _ = cpu_reference(rwl, n, 2, 1, nthr)
+            v1, _, _ = cpu_reference(rwl, 2000, 1, 0, 1)          # the "single-threaded C loop over the same model" of north_star
             line["cpu_baseline"] = {"value": v, "unit": UNIT, "cores": nthr, "kind": "port",
                                     "sample": "%d samples x %d freq, 2 timed passes, OpenMP over samples" % (n, nf),
                                     "single_thread": {"value": v1, "unit": UNIT, "cores": 1, "sample": "2000 samples x %d freq, 1 pass" % nf}}

@@ -106,7 +106,7 @@ def canon(branches, ports):
     return sorted(out)
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference tree not mounted (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="the upstream qo-100-tools files are not in this repository: set QO100_REFERENCE to a checkout")
 def test_netlister_reads_pa_bias_schematic(Q):
     """qo_nodal_load_qucs_sch on the reference schematic == the hand-derived netlist (up to node numbering):
     28 branches, 21 nodes, 5 ports in Pac-number order, the SPfile resolved next to the schematic."""

@@ -25,7 +25,7 @@ import sys
 import numpy as np
 import pytest
 
-from conftest import ROOT, png_curve_distance, relerr
+from conftest import REFERENCE, ROOT, png_curve_distance, relerr
 
 PNG_CASES = [("if_bpf", "util/if-bandpass-filter/schematic.svg"),
              ("gpsdo_10m", "util/gpsdo-ouput-filters/10M/schematic.svg"),
@@ -204,11 +204,11 @@ def test_preamp_bias_plot_markers_pin_the_oracle(R, golden_s2p):
     R.sblock_clear()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference tree not mounted (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="the upstream qo-100-tools files are not in this repository: set QO100_REFERENCE to a checkout")
 def test_preamp_bias_netlister_equals_hand_netlist(Q):
     """qo_nodal_load_qucs_sch on the reference's preamp schematic gives the hand-read netlist (up to node numbering), and the
     host-only plan analysis accepts the network (the 22 uF capacitor next to pF-sized ones: 8 orders of magnitude in admittance)."""
-    nd = Q.Nodal.from_qucs_sch("/root/reference/util/preamp-bias-simulation/preamp-bias-simulation.sch")
+    nd = Q.Nodal.from_qucs_sch(os.path.join(REFERENCE, "util/preamp-bias-simulation/preamp-bias-simulation.sch"))
     br, nn, ports = preamp_netlist()
     assert nd.n_nodes == nn and [z for _, z in nd.ports] == [50.0] * 5
     got = sorted((k, round(p[0] if k != NB_SBLOCK else p[2], 15)) for k, _n, p in nd.branches)

@@ -1,7 +1,6 @@
-"""Generate tests/golden/* from the reference tree (run in the build container only;
-/root/reference does not exist on the GPU box, the fixtures do).
+"""Generate tests/golden/* from a checkout of the upstream qo-100-tools tree (the tests need only the fixtures, not the tree).
 
-  python tools/make_golden.py [/root/reference]
+  python tools/make_golden.py [<qo-100-tools checkout>]      (default: $QO100_REFERENCE)
 
 Writes
   tests/golden/pa_lpf_dat.npz   -- util/pa-lpf-simulation/pa-lpf-simulation.dat:5-35017 (all 5000 points)
@@ -9,12 +8,12 @@ Writes
                                    as read by the product loader (qo_net_load_*), + .trc contents
   tests/golden/touchstone.npz   -- the three Touchstone files of the tree (util/pa-bias-simulation/11SQ39N.S2P,
                                    util/preamp-bias-simulation/06HP47N.s2p, docs/pa-driver/pa_20W_vdd_32V_idq_180mA.s2p)
-                                   parsed by an independent numpy parser (python tools/make_golden.py /root/reference touchstone)
+                                   parsed by an independent numpy parser (python tools/make_golden.py <checkout> touchstone)
   tests/golden/pa_bias_dat.npz  -- util/pa-bias-simulation/pa-bias-simulation.dat:1-85035 (5-port S entries, 5000 points)
   tests/golden/rftools_png_curves.npz -- the S21 / S11 curves of the reference's three rf-tools plots (util/if-bandpass-filter/
                                    bokeh_plot.png, util/gpsdo-ouput-filters/10M/bokeh_plot.png, docs/upconverter/
                                    upconverter-lol-filter.png) as pixel coordinates, with the axis calibration read from the
-                                   tick marks (python tools/make_golden.py /root/reference png_curves)
+                                   tick marks (python tools/make_golden.py <checkout> png_curves)
   tests/golden/appendix_b.json  -- 40-digit mpmath evaluation of the textbook ladder / coupled-line
                                    equations (SURVEY App. B) at the frequencies the survey tabulates;
                                    an implementation independent of both the oracle and the product.
@@ -30,7 +29,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "qo-100-tools_b200", "python"))
 import qo100net as Q  # noqa: E402
 
-REF = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
+REF = sys.argv[1] if len(sys.argv) > 1 else os.environ.get("QO100_REFERENCE", "")
 OUT = os.path.join(ROOT, "tests", "golden")
 
 SVGS = ["util/if-bandpass-filter/schematic.svg", "util/gpsdo-ouput-filters/10M/schematic.svg",
