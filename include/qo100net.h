@@ -312,7 +312,8 @@ int qo_chain_jit_analyze(const qo_net *net, const double *f, int nf, const qo_sp
  * ("ok", or why the job stays on the chain kernels). */
 const char *qo_plan_tf_info(const qo_plan *plan, int info[6], double *self_check_err);
 /* the host-only part of qo_plan_create (network -> program, transfer-function analysis): needs no GPU.  Same outputs as
- * qo_plan_tf_info; *seconds = host time the analysis took. */
+ * qo_plan_tf_info; *seconds = host time the analysis took.  An environment override qo_plan_create would refuse (an unknown
+ * QO100NET_KERNEL value): info[0] = QO_ERR_ARG and the reason string says why. */
 const char *qo_plan_analyze(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
                             int info[6], double *self_check_err, double *seconds);
 /* host->device bytes qo_plan_create copied for this plan (tables, masks, program), per GPU */

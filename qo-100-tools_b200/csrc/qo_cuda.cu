@@ -29,6 +29,7 @@
 #include "qo_ustrip_board.cuh"
 #include "qo_cpl_core.h"
 #include "qo_chain_jit.h"
+#include "qo_overrides.h"
 
 static int nccl_load(NcclApi *a)
 {
@@ -74,27 +75,32 @@ struct DevPlan {
     float ms;
 };
 
+/* the kernel a plan launches, in order of precedence (select_kernel); launch-time refinements: thread-per-sample inside launch_tf,
+ * the compiled chain kernel inside launch_lumped, the FULL_S transfer-function kernel ahead of them all (plan_launch_dev) */
+enum QoKern { K_BOARD, K_GENERIC, K_SPOT, K_TF, K_LADDER, K_LUMPED };
+static const char *const qo_kern_name[] = { "qo_mc_board_kernel", "qo_mc_generic_kernel", "qo_mc_spot_kernel", "qo_mc_tf_kernel",
+                                            "qo_mc_ladder_kernel", "qo_mc_lumped_kernel" };
+
 struct qo_plan {
     qo_ctx *ctx;
     DevProg hp;                /* host copy of the program */
     int nf, npairs, ncnt, precision, mode, generic;
-    int board;                                            /* microstrip yield job at <= 4 frequencies: thread-per-board kernel */
-    /* launch-time decisions of the transfer-function kernels, taken once at plan creation (environment overrides included) */
+    QoOverrides ov;                                       /* the environment overrides as they were at plan creation */
+    QoKern kern;
+    /* launch-time decisions of the transfer-function kernels, taken once at plan creation */
     int tf_cpl_matched, tf_cpl_lin, ts_ok, ts_runs_ok, ts_nruns, ts_npt;
     double tf_cpl_dw1;                                    /* angular-frequency step of one grid point on a uniformly spaced grid */
     struct { int ngroups; unsigned int any, all; } ts_runs[QO_TS_MAXRUN];
-    int ladder, lad_n, lad_first, lad_cpl, lad_variant;   /* straight-line ladder kernel (qo_ladder.cuh) */
+    int lad_n, lad_first, lad_cpl;                        /* straight-line ladder kernel (qo_ladder.cuh) */
     int cpl_fast, cpl_same;                               /* coupler block: small-angle table path, equal mode angles */
-    int spot, spot_el0, spot_nel;                         /* spot-frequency kernel (qo_spot.cuh): <= 8 points per sample */
-    int tf;                                               /* transfer-function kernel (qo_tf.cuh) selected */
-    TfPlan tfp;                                           /* its polynomial lengths, denominator form, self-check result */
+    int spot_el0, spot_nel;                               /* spot-frequency kernel (qo_spot.cuh): <= 8 points per sample */
+    TfPlan tfp;                                           /* transfer-function kernel (qo_tf.cuh): polynomial lengths, denominator form, self-check result */
     int tf_pp, tf_niter;                                  /* pairs per thread per iteration; iterations per sample */
     int fs_state;                                         /* FULL_S transfer-function path: 0 not analysed yet, 1 selected, -1 refused */
     TfPlan fsp;
     int fs_niter;
     unsigned long long h2d_bytes;                         /* host->device bytes copied by qo_plan_create, per GPU */
-    int cj_mode;                                          /* run-time compiled chain kernel (qo_chain_jit.h): 0 by job size, 1 always, -1 never */
-    int cj_debug, cj_failed[2];
+    int cj_debug, cj_failed[2];                           /* run-time compiled chain kernel (qo_chain_jit.h), used as ov.chain says */
     const void *cj[2];                                    /* its QcjEntry for the reduce-only / FULL_S flavour once this process holds it */
     std::string cj_src[2];
     unsigned long long cj_hash[2];
@@ -110,7 +116,7 @@ struct qo_plan {
     unsigned char *pinned[8];                             /* ... gathered in one page-locked buffer per device the first time they are re-sent */
 };
 
-static void tf_launch_setup(qo_plan *p);
+static void tf_launch_setup(qo_plan *p, const QoOverrides *ov);
 
 /* ---- ctx ---------------------------------------------------------------- */
 static int devctx_init(DevCtx *d, int device)
@@ -375,11 +381,10 @@ static int build_prog(const qo_net *net, const double *f, int nf, const qo_spec 
  * network that is an alternating series-inductor / shunt-capacitor ladder of 1..11 elements
  * (pcb/generic-filter), optionally behind one coupled-line block.  QO100NET_KERNEL=interp forces the
  * opcode interpreter (A/B runs, parity tests of both paths). */
-static int ladder_eligible(const DevProg *hp, int mode, int precision, int generic, int *n, int *first, int *cpl)
+static int ladder_eligible(const DevProg *hp, int mode, int precision, const QoOverrides *ov, int *n, int *first, int *cpl)
 {
-    const char *force = getenv("QO100NET_KERNEL");
-    if (force && strcmp(force, "interp") == 0) return 0;
-    if (generic || mode != QO_MODE_REDUCE_ONLY || hp->need_gd) return 0;
+    if (ov->kernel == QoOverrides::INTERP) return 0;
+    if (mode != QO_MODE_REDUCE_ONLY || hp->need_gd) return 0;
     if (precision == 32 && hp->need_s11) return 0;          /* FP32 mode: |S21| specs only on the straight-line kernel */
     if (hp->nspec > QO_LAD_NSPEC || hp->n_var > QO_MAX_VAR) return 0;
     for (int s = 0; s < hp->nspec; s++)
@@ -406,12 +411,12 @@ static int ladder_eligible(const DevProg *hp, int mode, int precision, int gener
 }
 
 /* The spot-frequency kernel (one thread per sample) serves reduce-only FP64 jobs on lumped cascades evaluated at a handful
- * of frequencies -- BASELINE config 3's harmonic-rejection yield at 2.4 / 4.8 / 7.2 GHz. */
-static int spot_eligible(const DevProg *hp, int mode, int precision, int generic, int nf, int *el0, int *nel)
+ * of frequencies -- BASELINE config 3's harmonic-rejection yield at 2.4 / 4.8 / 7.2 GHz.  Any QO100NET_KERNEL override
+ * but auto keeps jobs off it. */
+static int spot_eligible(const DevProg *hp, int mode, int precision, int nf, const QoOverrides *ov, int *el0, int *nel)
 {
-    const char *force = getenv("QO100NET_KERNEL");
-    if (force && strcmp(force, "auto") != 0 && strcmp(force, "spot") != 0) return 0;
-    if (generic || mode != QO_MODE_REDUCE_ONLY || precision != 64 || hp->need_gd) return 0;
+    if (ov->kernel != QoOverrides::AUTO) return 0;
+    if (mode != QO_MODE_REDUCE_ONLY || precision != 64 || hp->need_gd) return 0;
     if (nf > QO_SPOT_MAXF || hp->nspec < 1 || hp->nspec > QO_NSPEC_MAX) return 0;
     const int e0 = hp->op0, nl = hp->n_ops - e0;
     if (nl < 1 || nl > QO_SPOT_MAXEL) return 0;
@@ -420,6 +425,19 @@ static int spot_eligible(const DevProg *hp, int mode, int precision, int generic
         if (hp->spec_kind[s] != SK_DEN2_MAX && hp->spec_kind[s] != SK_DEN2_MIN && hp->spec_kind[s] != SK_S11_MAX) return 0;
     *el0 = e0; *nel = nl;
     return 1;
+}
+
+/* the plan's kernel (QoKern, in order of precedence) */
+static QoKern select_kernel(qo_plan *p, const double *f, int nf)
+{
+    const QoOverrides *ov = &p->ov;
+    /* analysed for every plan: qo_plan_tf_info reports the result (or why it refused) whichever kernel runs */
+    const int tf = qo_tf_plan_check(&p->hp, p->mode == QO_MODE_REDUCE_ONLY, p->precision, p->generic, f, nf, p->maskv.data(), ov, &p->tfp);
+    if (p->generic) return p->mode == QO_MODE_REDUCE_ONLY && nf <= QO_B_MAXNF && !ov->ustrip_item ? K_BOARD : K_GENERIC;
+    if (spot_eligible(&p->hp, p->mode, p->precision, nf, ov, &p->spot_el0, &p->spot_nel)) return K_SPOT;
+    if (tf) return K_TF;
+    if (ladder_eligible(&p->hp, p->mode, p->precision, ov, &p->lad_n, &p->lad_first, &p->lad_cpl)) return K_LADDER;
+    return K_LUMPED;
 }
 
 /* ---- plan ---------------------------------------------------------------- */
@@ -439,16 +457,16 @@ extern "C" void qo_plan_destroy(qo_plan *p)
     delete p;
 }
 
-extern "C" int qo_plan_create(qo_ctx *ctx, const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec,
-                              const qo_mc_cfg *cfg, qo_plan **out)
+static int plan_create(qo_ctx *ctx, const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec,
+                       const qo_mc_cfg *cfg, const QoOverrides *ov, qo_plan **out)
 {
-    qo_clear_error();
     if (!ctx || !net || !f || nf <= 0 || !out || (nspec > 0 && !spec)) { qo_set_error("bad arguments"); return QO_ERR_ARG; }
     for (int k = 0; k < nf; k++)
         if (!(f[k] > 0.0) || !isfinite(f[k])) { qo_set_error("frequency %d is not a positive finite number", k); return QO_ERR_ARG; }
     qo_plan *p = new (std::nothrow) qo_plan();
     if (!p) return QO_ERR_NOMEM;
     p->ctx = ctx;
+    p->ov = *ov;
     memset(p->pinned, 0, sizeof p->pinned);
     p->nf = nf;
     p->npairs = (nf + 1) / 2;
@@ -464,24 +482,10 @@ extern "C" int qo_plan_create(qo_ctx *ctx, const qo_net *net, const double *f, i
     if (p->hp.need_gd && p->precision == 32) { delete p; qo_set_error("group-delay specs need FP64 (the 1e-6 relative frequency step is 8 float ulps)"); return QO_ERR_UNSUPPORTED; }
     p->ncnt = 2 + nspec + p->hp.hist_bins;
     p->f.assign(f, f + nf);
-    p->ladder = ladder_eligible(&p->hp, p->mode, p->precision, p->generic, &p->lad_n, &p->lad_first, &p->lad_cpl);
-    {
-        const char *v = getenv("QO100NET_LAD_VARIANT");
-        p->lad_variant = v ? atoi(v) : 0;
-    }
-    p->tf = qo_tf_plan_check(&p->hp, p->mode == QO_MODE_REDUCE_ONLY, p->precision, p->generic, f, nf, p->maskv.data(), &p->tfp);
-    p->spot = spot_eligible(&p->hp, p->mode, p->precision, p->generic, nf, &p->spot_el0, &p->spot_nel);
-    if (p->spot) p->tf = p->ladder = 0;
-    { const char *e = getenv("QO100NET_USTRIP"); p->board = p->generic && p->mode == QO_MODE_REDUCE_ONLY && nf <= QO_B_MAXNF && !(e && !strcmp(e, "item")); }
-    {
-        /* the compiled chain kernel for what stays on the interpreter: QO100NET_CHAIN=jit always, =interp never; QO100NET_KERNEL=interp
-         * (A/B runs against the interpreter proper) also means never unless QO100NET_CHAIN=jit says otherwise */
-        const char *cj = getenv("QO100NET_CHAIN"), *fk = getenv("QO100NET_KERNEL");
-        p->cj_mode = cj && !strcmp(cj, "jit") ? 1 : cj && !strcmp(cj, "interp") ? -1 : fk && !strcmp(fk, "interp") ? -1 : 0;
-        p->cj_debug = getenv("QO100NET_CHAIN_DEBUG") != NULL;
-        p->cj[0] = p->cj[1] = NULL; p->cj_failed[0] = p->cj_failed[1] = 0; p->cj_hash[0] = p->cj_hash[1] = 0;
-    }
-    p->kernel_name = p->board ? "qo_mc_board_kernel" : p->generic ? "qo_mc_generic_kernel" : p->spot ? "qo_mc_spot_kernel" : p->tf ? "qo_mc_tf_kernel" : p->ladder ? "qo_mc_ladder_kernel" : "qo_mc_lumped_kernel";
+    p->kern = select_kernel(p, f, nf);
+    p->kernel_name = qo_kern_name[p->kern];
+    p->cj_debug = getenv("QO100NET_CHAIN_DEBUG") != NULL;
+    p->cj[0] = p->cj[1] = NULL; p->cj_failed[0] = p->cj_failed[1] = 0; p->cj_hash[0] = p->cj_hash[1] = 0;
 
     /* per-frequency tables: w = 2 pi f and 1/w (hoisted out of the kernel), padded to a pair */
     const double two_pi = 6.283185307179586476925286766559;
@@ -536,7 +540,7 @@ extern "C" int qo_plan_create(qo_ctx *ctx, const qo_net *net, const double *f, i
     std::vector<double> ctab[4];
     std::vector<float> ctabf[4];
     p->cpl_fast = p->cpl_same = 0;
-    if ((p->ladder && p->lad_cpl) || (p->tf && p->tfp.cpl_op >= 0 && p->tfp.front == 0)) {
+    if ((p->kern == K_LADDER && p->lad_cpl) || (p->kern == K_TF && p->tfp.cpl_op >= 0 && p->tfp.front == 0)) {
         const DevProg *hp = &p->hp;
         const int ec = hp->op0;                    /* the coupler op */
         double wmax = 0;
@@ -585,7 +589,7 @@ extern "C" int qo_plan_create(qo_ctx *ctx, const qo_net *net, const double *f, i
             p->cpl_same = hp->nom[ec][2] == hp->nom[ec][3] && hp->tvar[ec][2] == hp->tvar[ec][3] && hp->ttol[ec][2] == hp->ttol[ec][3] &&
                           hp->tmode[ec][2] == hp->tmode[ec][3];
         }
-        p->cpl_fast = ok && worst <= 0.1 && !getenv("QO100NET_CPL_SINCOS");
+        p->cpl_fast = ok && worst <= 0.1 && !ov->cpl_sincos;
         if (p->cpl_fast) {
             for (int t = 0; t < 4; t++) ctab[t].resize(2 * (size_t)np);
             const double ke = ke_nom, ko = ko_nom;
@@ -627,13 +631,10 @@ extern "C" int qo_plan_create(qo_ctx *ctx, const qo_net *net, const double *f, i
                     H2D(d->sdet, sdet.data(), sdet.size() * sizeof(double2));
                 }
             }
-            if (p->tf) {
+            if (p->kern == K_TF) {
                 /* tables of the transfer-function kernel, padded to whole iterations (padding repeats the last grid
                  * point and carries no spec bit, so the loop needs no bounds checks) */
                 p->tf_pp = qo_tf_default_pp(&p->tfp, np);
-#ifdef QO_TF_EXPERIMENT
-                if (getenv("QO100NET_TF_PP")) p->tf_pp = atoi(getenv("QO100NET_TF_PP"));
-#endif
                 const int ppi = 32 * p->tf_pp;
                 p->tf_niter = (np + ppi - 1) / ppi;
                 /* + one iteration of padding: the kernel requests the next iteration's y values before it is done with the current one */
@@ -689,7 +690,7 @@ extern "C" int qo_plan_create(qo_ctx *ctx, const qo_net *net, const double *f, i
                 d->tf_mb = (uint4 *)(dt + (size_t)ntab * npt);
                 d->tf_itm = (uchar2 *)((unsigned int *)d->tf_mb + 2 * npt);
             }
-            if (p->ladder || p->tf) {
+            if (p->kern == K_LADDER || p->kern == K_TF) {
                 CUP(cudaMallocAsync((void **)&d->wsq2, 2 * (size_t)np * esz, st));
                 H2D(d->wsq2, p->precision == 32 ? (const void *)wsqf.data() : (const void *)wsq.data(), 2 * (size_t)np * esz);
                 CUP(cudaMallocAsync((void **)&d->ticket, QO_TICKET_BYTES, st));      /* the sample ticket + the per-SM arrival counters of qo_ts.cuh */
@@ -709,9 +710,18 @@ extern "C" int qo_plan_create(qo_ctx *ctx, const qo_net *net, const double *f, i
         CUP(cudaMemsetAsync(d->counters, 0, (size_t)p->ncnt * sizeof(unsigned long long), st));
         CUP(cudaStreamSynchronize(st));   /* the host staging vectors die at return */
     }
-    if (p->tf) tf_launch_setup(p);
+    if (p->kern == K_TF) tf_launch_setup(p, ov);
     *out = p;
     return QO_OK;
+}
+
+extern "C" int qo_plan_create(qo_ctx *ctx, const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec,
+                              const qo_mc_cfg *cfg, qo_plan **out)
+{
+    qo_clear_error();
+    QoOverrides ov;
+    const int rc = qo_overrides_read(&ov);
+    return rc ? rc : plan_create(ctx, net, f, nf, spec, nspec, cfg, &ov, out);
 }
 
 extern "C" int qo_plan_num_counters(const qo_plan *p) { return p ? p->ncnt : QO_ERR_ARG; }
@@ -725,11 +735,14 @@ extern "C" int qo_chain_jit_analyze(const qo_net *net, const double *f, int nf, 
     qo_clear_error();
     if (!net || !f || nf <= 0 || !cfg || !info || (nspec > 0 && !spec)) return QO_ERR_ARG;
     for (int i = 0; i < 4; i++) info[i] = 0;
+    QoOverrides ov;                          /* nothing here depends on them, but a bad value is refused as everywhere else */
+    int rc = qo_overrides_read(&ov);
+    if (rc) return rc;
     DevProg hp;
     int generic = 0;
     double flops = 0.0;
     std::vector<unsigned char> maskv;
-    int rc = build_prog(net, f, nf, spec, nspec, cfg, &hp, &generic, &flops, &maskv);
+    rc = build_prog(net, f, nf, spec, nspec, cfg, &hp, &generic, &flops, &maskv);
     if (rc) return rc;
     if (generic) { qo_set_error("microstrip networks run on their own kernels"); return QO_ERR_UNSUPPORTED; }
     const std::string src = qcj_source(&hp, cfg->mode == QO_MODE_FULL_S);
@@ -743,7 +756,7 @@ extern "C" const char *qo_plan_kernel_name(const qo_plan *p) { return p ? p->ker
 extern "C" const char *qo_plan_tf_info(const qo_plan *p, int info[6], double *self_check_err)
 {
     if (!p) return "";
-    if (info) { info[0] = p->tf; info[1] = p->tfp.nn; info[2] = p->tfp.den; info[3] = p->tfp.kn; info[4] = p->tfp.kd; info[5] = p->tfp.deg; }
+    if (info) { info[0] = p->kern == K_TF; info[1] = p->tfp.nn; info[2] = p->tfp.den; info[3] = p->tfp.kn; info[4] = p->tfp.kd; info[5] = p->tfp.deg; }
     if (self_check_err) *self_check_err = p->tfp.err;
     return p->tfp.reason ? p->tfp.reason : "";
 }
@@ -755,6 +768,8 @@ extern "C" const char *qo_plan_analyze(const qo_net *net, const double *f, int n
 {
     qo_clear_error();
     if (!net || !f || nf <= 0 || !info) return "bad arguments";
+    QoOverrides ov;
+    if ((info[0] = qo_overrides_read(&ov)) != QO_OK) return qo_last_error();
     DevProg *hp = new DevProg;
     int generic = 0;
     double fl = 0;
@@ -768,7 +783,7 @@ extern "C" const char *qo_plan_analyze(const qo_net *net, const double *f, int n
     if (rc == QO_OK) {
         const int precision = cfg && cfg->precision == 32 ? 32 : 64;
         const int mode = cfg ? cfg->mode : QO_MODE_FULL_S;
-        int sel = qo_tf_plan_check(hp, mode == QO_MODE_REDUCE_ONLY, precision, generic, f, nf, maskv.data(), &tp);
+        int sel = qo_tf_plan_check(hp, mode == QO_MODE_REDUCE_ONLY, precision, generic, f, nf, maskv.data(), &ov, &tp);
         info[0] = sel; info[1] = tp.nn; info[2] = tp.den; info[3] = tp.kn; info[4] = tp.kd; info[5] = tp.deg;
         if (self_check_err) *self_check_err = tp.err;
         reason = tp.reason ? tp.reason : "";
@@ -837,17 +852,17 @@ static int launch_lumped(qo_plan *p, int g, unsigned long long off, unsigned lon
     unsigned long long blocks = (units + QO_WARPS - 1) / QO_WARPS;
     int grid = (int)(blocks < (unsigned long long)resident ? blocks : (unsigned long long)resident);
     if (grid < 1) grid = 1;
-    if (sizeof(T) == sizeof(double) && p->cj_mode >= 0 && !p->cj_failed[full_s ? 1 : 0]) {
+    if (sizeof(T) == sizeof(double) && p->ov.chain >= 0 && !p->cj_failed[full_s ? 1 : 0]) {
         /* large jobs: the element list compiled into the kernel (qo_chain_jit.h) */
         const int fs = full_s ? 1 : 0;
         const unsigned long long evals = n * (unsigned long long)p->nf;
         const QcjEntry *je = (const QcjEntry *)p->cj[fs];
-        if (!je && (p->cj_mode == 1 || evals >= QO_CJ_MIN_CACHED)) {
+        if (!je && (p->ov.chain == 1 || evals >= QO_CJ_MIN_CACHED)) {
             if (p->cj_src[fs].empty()) { p->cj_src[fs] = qcj_source(&p->hp, fs); p->cj_hash[fs] = qcj_hash(p->cj_src[fs]); }
-            je = qcj_get(p->cj_src[fs], p->cj_hash[fs], p->cj_mode == 1 || evals >= QO_CJ_MIN_EVALS, p->cj_debug != 0);
+            je = qcj_get(p->cj_src[fs], p->cj_hash[fs], p->ov.chain == 1 || evals >= QO_CJ_MIN_EVALS, p->cj_debug != 0);
             if (je && !je->ok) {
                 p->cj_failed[fs] = 1;
-                if (p->cj_mode == 1) { qo_set_error("QO100NET_CHAIN=jit: %s", je->log.substr(0, 400).c_str()); return QO_ERR_UNSUPPORTED; }
+                if (p->ov.chain == 1) { qo_set_error("QO100NET_CHAIN=jit: %s", je->log.substr(0, 400).c_str()); return QO_ERR_UNSUPPORTED; }
                 je = NULL;
             }
             p->cj[fs] = je;
@@ -906,7 +921,7 @@ static int launch_ladder(qo_plan *p, int g, unsigned long long off, unsigned lon
     P.hist_bins = hp->hist_bins;
     P.hist_spec = hp->hist_bins > 0 ? hp->hist_spec : -1;
     P.hist_kind = hp->hist_bins > 0 ? hp->spec_kind[hp->hist_spec] : 0;
-    int rc = qo_ladder_launch(p->lad_n, p->lad_first, p->lad_cpl, hp->need_s11 ? 2 : 1, p->precision, p->lad_variant, dc->sm_count, &P, dc->stream, NULL);
+    int rc = qo_ladder_launch(p->lad_n, p->lad_first, p->lad_cpl, hp->need_s11 ? 2 : 1, p->precision, dc->sm_count, &P, dc->stream);
     if (rc < 0) { qo_set_error("no ladder kernel instantiation for n=%d first=%d cpl=%d", p->lad_n, p->lad_first, p->lad_cpl); return QO_ERR_UNSUPPORTED; }
     if (rc) { qo_set_error("ladder kernel launch: %s", cudaGetErrorString((cudaError_t)rc)); return QO_ERR_CUDA; }
     return QO_OK;
@@ -915,23 +930,23 @@ static int launch_ladder(qo_plan *p, int g, unsigned long long off, unsigned lon
 /* what launch_tf needs beyond the tables, decided once per plan: the coupler block's form (matched source, uniformly spaced
  * grid), whether large launches may run thread-per-sample, and that kernel's run table (runs of point groups that see the same
  * spec bits; a group that straddles a band edge stands alone) */
-static void tf_launch_setup(qo_plan *p)
+static void tf_launch_setup(qo_plan *p, const QoOverrides *ov)
 {
     const DevProg *hp = &p->hp;
     const int cop = p->tfp.cpl_op;
     const int front = cop >= 0 ? p->tfp.front : 0;
     /* source resistance == the coupler's (unperturbed) reference impedance: the block's row vector collapses (qo_tf.cuh::tf_cpl_matched) */
-    p->tf_cpl_matched = cop >= 0 && !front && !p->tfp.s11 && hp->tvar[cop][5] < 0 && hp->nom[cop][5] == hp->rs && !getenv("QO100NET_CPL_GENERAL");
+    p->tf_cpl_matched = cop >= 0 && !front && !p->tfp.s11 && hp->tvar[cop][5] < 0 && hp->nom[cop][5] == hp->rs;
     /* uniformly spaced grid (config 5: linear 70 MHz .. 4 GHz): the coupler's mode angles advance by a constant per iteration */
     p->tf_cpl_lin = 0; p->tf_cpl_dw1 = 0.0;
-    if (cop >= 0 && !front && !p->tfp.s11 && p->nf >= 3 && !getenv("QO100NET_CPL_NO_ROT")) {
+    if (cop >= 0 && !front && !p->tfp.s11 && p->nf >= 3) {
         const double d0 = p->f[1] - p->f[0];
         int lin = d0 > 0.0;
         for (int k = 2; k < p->nf && lin; k++) if (fabs((p->f[k] - p->f[k - 1]) - d0) > 1e-9 * fabs(d0)) lin = 0;
         if (lin) { p->tf_cpl_lin = 1; p->tf_cpl_dw1 = 6.283185307179586476925286766559 * ((p->f[p->nf - 1] - p->f[0]) / (double)(p->nf - 1)); }
     }
     const bool rot_same = p->tf_cpl_lin && p->tf_cpl_matched && p->cpl_same && hp->cplms_elem < 0;
-    p->ts_ok = qo_ts_eligible(&p->tfp, hp->nspec, rot_same);
+    p->ts_ok = ov->kernel != QoOverrides::TF && qo_ts_eligible(&p->tfp, hp->nspec, rot_same);     /* KERNEL=tf: warp-per-sample only (A/B runs) */
     p->ts_nruns = 0; p->ts_runs_ok = 1; p->ts_npt = 0;
     if (p->ts_ok) {
         const int gpt = qo_ts_group_points(&p->tfp);
@@ -1005,7 +1020,7 @@ static int launch_tf(qo_plan *p, int g, unsigned long long off, unsigned long lo
             P.sample_offset = off; P.nsamples = n;
         }
     }
-    int rc = qo_tf_launch(&p->tfp, p->tf_pp, p->lad_variant, dc->sm_count, &P, dc->stream);
+    int rc = qo_tf_launch(&p->tfp, p->tf_pp, dc->sm_count, &P, dc->stream);
     if (rc < 0) { qo_set_error("no transfer-function kernel instantiation for nn=%d den=%d pp=%d", p->tfp.nn, p->tfp.den, p->tf_pp); return QO_ERR_UNSUPPORTED; }
     if (rc) { qo_set_error("transfer-function kernel launch: %s", cudaGetErrorString((cudaError_t)rc)); return QO_ERR_CUDA; }
     return QO_OK;
@@ -1081,7 +1096,7 @@ static int launch_generic(qo_plan *p, int g, unsigned long long off, unsigned lo
 {
     DevCtx *dc = &p->ctx->d[g];
     DevPlan *d = &p->d[g];
-    if (p->board) {
+    if (p->kern == K_BOARD) {
         /* yield at a handful of frequencies: one thread per board, the frequencies side by side (qo_ustrip_board.cuh) */
         const unsigned long long cap = (unsigned long long)dc->sm_count * QO_B_MINB, want = (n + QO_B_TPB - 1) / QO_B_TPB;
         const int grid = (int)(want < cap ? want : cap);
@@ -1145,14 +1160,15 @@ static int plan_launch_dev(qo_plan *p, int g, unsigned long long off, unsigned l
     }
     int rc;
     if (full_s && !p->generic && p->precision == 64 && n >= QO_FS_TF_MIN_SAMPLES && p->fs_state == 0)
-        p->fs_state = qo_tf_fs_plan_check(&p->hp, 1, p->precision, p->generic, p->f.data(), p->nf, &p->fsp) ? 1 : -1;
+        p->fs_state = qo_tf_fs_plan_check(&p->hp, 1, p->precision, p->generic, p->f.data(), p->nf, &p->ov, &p->fsp) ? 1 : -1;
     if (full_s && p->fs_state == 1 && n >= QO_FS_TF_MIN_SAMPLES) { rc = launch_tf_fs(p, g, off, n, pl); if (rc == QO_OK) p->kernel_name = "qo_fs_tf_kernel"; }
-    else if (p->generic) rc = launch_generic(p, g, off, n, cnt, pl, full_s);
-    else if (p->spot) rc = launch_spot(p, g, off, n, cnt);
-    else if (p->tf) rc = launch_tf(p, g, off, n, cnt, cplms);
-    else if (p->ladder) rc = launch_ladder(p, g, off, n, cnt, cplms);
-    else if (p->precision == 32) rc = launch_lumped<float>(p, g, off, n, cnt, pl, full_s);
-    else rc = launch_lumped<double>(p, g, off, n, cnt, pl, full_s);
+    else switch (p->kern) {
+    case K_BOARD: case K_GENERIC: rc = launch_generic(p, g, off, n, cnt, pl, full_s); break;
+    case K_SPOT: rc = launch_spot(p, g, off, n, cnt); break;
+    case K_TF: rc = launch_tf(p, g, off, n, cnt, cplms); break;
+    case K_LADDER: rc = launch_ladder(p, g, off, n, cnt, cplms); break;
+    default: rc = p->precision == 32 ? launch_lumped<float>(p, g, off, n, cnt, pl, full_s) : launch_lumped<double>(p, g, off, n, cnt, pl, full_s); break;
+    }
     if (cplms) cudaFreeAsync(cplms, p->ctx->d[g].stream);
     if (rc == QO_OK) { p->launches++; p->d[g].n_launched += n; }
     return rc;
@@ -1224,7 +1240,10 @@ extern "C" int qo_mc_run(qo_ctx *ctx, const qo_net *net, const double *f, int nf
     if (!ctx || !cfg || !res) return QO_ERR_ARG;
     if (cfg->mode == QO_MODE_FULL_S && !full_s) { qo_set_error("FULL_S needs an output buffer"); return QO_ERR_ARG; }
     if (!net || !f || nf <= 0 || (nspec > 0 && !spec) || nspec < 0) { qo_set_error("bad arguments"); return QO_ERR_ARG; }
-    /* same job as the previous call on this ctx (everything but the sample range)?  Then its plan is still good. */
+    QoOverrides ov;
+    int rc = qo_overrides_read(&ov);
+    if (rc) return rc;
+    /* same job and overrides as the previous call on this ctx (everything but the sample range)?  Then its plan is still good. */
     unsigned long long key = 1469598103934665603ull;
     {
         /* eight bytes per step (the grid alone is 32 KB: byte-wise FNV cost 45 us per call), bytes for the tail */
@@ -1240,11 +1259,9 @@ extern "C" int qo_mc_run(qo_ctx *ctx, const qo_net *net, const double *f, int nf
         if (cfg->n_tol > 0 && cfg->tol) mix(cfg->tol, (size_t)cfg->n_tol * sizeof(qo_tol));
         const long long scal[8] = { (long long)cfg->seed, cfg->dist, cfg->n_tol, cfg->mode, cfg->precision, cfg->hist_bins, cfg->hist_spec, nspec };
         mix(scal, sizeof scal); mix(&cfg->hist_lo, sizeof(double)); mix(&cfg->hist_hi, sizeof(double));
-        static const char *envs[] = { "QO100NET_KERNEL", "QO100NET_TF_TRUNC", "QO100NET_TF_TOL", "QO100NET_TF_NO_E", "QO100NET_TF_NO_FRONT", "QO100NET_CPL_GENERAL", "QO100NET_CPL_NO_ROT", "QO100NET_LAD_VARIANT", "QO100NET_CPL_SINCOS", "QO100NET_USTRIP", "QO100NET_CHAIN" };
-        for (size_t i = 0; i < sizeof envs / sizeof envs[0]; i++) { const char *v = getenv(envs[i]); mix(v ? v : "\1", v ? strlen(v) + 1 : 1); }
+        mix(&ov, sizeof ov);
     }
     qo_plan *p = NULL;
-    int rc = QO_OK;
     static const bool mc_timing = getenv("QO100NET_MC_TIMING") != NULL;
     const auto tt0 = std::chrono::steady_clock::now();
     const bool cacheable = net->nblk == 0 && !getenv("QO100NET_NO_PLAN_CACHE");      /* measured blocks are not hashed: no reuse */
@@ -1270,7 +1287,7 @@ extern "C" int qo_mc_run(qo_ctx *ctx, const qo_net *net, const double *f, int nf
         if (rc) return rc;
     } else {
         if (ctx->mc_cache) { qo_plan_destroy(ctx->mc_cache); ctx->mc_cache = NULL; }
-        rc = qo_plan_create(ctx, net, f, nf, spec, nspec, cfg, &p);
+        rc = plan_create(ctx, net, f, nf, spec, nspec, cfg, &ov, &p);
         if (rc) return rc;
         if (cacheable) { ctx->mc_cache = p; ctx->mc_cache_key = key; }
     }

@@ -36,15 +36,6 @@ template <typename T, int NROWS, int PP, int TPB, int MINB> static lad_fn lad_pi
 #undef QO_LAD_ROW
 }
 
-#ifdef QO_LAD_EXPERIMENT
-/* development builds: extra launch shapes of the 11-element series-first ladder, chosen with QO100NET_LAD_VARIANT */
-template <int PP, int TPB, int MINB> static lad_fn lad_pick11(int n, int first, int cpl)
-{
-    if (n != 11 || first) return nullptr;
-    return cpl ? lad_get<double, 11, 0, true, 1, PP, TPB, MINB>() : lad_get<double, 11, 0, false, 1, PP, TPB, MINB>();
-}
-#endif
-
 /* kernels with the |S11| row: two points per thread (the second row vector doubles the chain state) */
 #define QO_LAD2_PP 1
 #define QO_LAD2_TPB 256
@@ -53,40 +44,21 @@ template <int PP, int TPB, int MINB> static lad_fn lad_pick11(int n, int first, 
 typedef void (*lad_fn_t)(const LadParams);
 extern "C" lad_fn_t qo_ladder_pick32(int n, int first, int cpl, int *tpb, int *minb);
 
-extern "C" int qo_ladder_launch(int n, int first, int cpl, int nrows, int precision, int variant, int sm_count, const LadParams *P,
-                                cudaStream_t st, const char **shape)
+extern "C" int qo_ladder_launch(int n, int first, int cpl, int nrows, int precision, int sm_count, const LadParams *P, cudaStream_t st)
 {
-    lad_fn fn = nullptr;
-    int tpb = QO_LAD_TPB, minb = QO_LAD_MINB;
-    const char *name = "default";
-    (void)variant;
-#ifdef QO_LAD_EXPERIMENT
-    switch (variant) {
-    case 1: fn = lad_pick11<1, 256, 2>(n, first, cpl); tpb = 256; minb = 2; name = "pp1-256x2"; break;
-    case 2: fn = lad_pick11<1, 128, 5>(n, first, cpl); tpb = 128; minb = 5; name = "pp1-128x5"; break;
-    case 3: fn = lad_pick11<2, 256, 2>(n, first, cpl); tpb = 256; minb = 2; name = "pp2-256x2"; break;
-    case 4: fn = lad_pick11<1, 128, 6>(n, first, cpl); tpb = 128; minb = 6; name = "pp1-128x6"; break;
-    case 5: fn = lad_pick11<1, 256, 4>(n, first, cpl); tpb = 256; minb = 4; name = "pp1-256x4"; break;
-    case 6: fn = lad_pick11<2, 128, 4>(n, first, cpl); tpb = 128; minb = 4; name = "pp2-128x4"; break;
-    case 7: fn = lad_pick11<2, 128, 5>(n, first, cpl); tpb = 128; minb = 5; name = "pp2-128x5"; break;
-    case 8: fn = lad_pick11<2, 256, 3>(n, first, cpl); tpb = 256; minb = 3; name = "pp2-256x3"; break;
-    case 9: fn = lad_pick11<2, 64, 8>(n, first, cpl); tpb = 64; minb = 8; name = "pp2-64x8"; break;
-    default: break;
-    }
-#endif
+    lad_fn fn;
+    int tpb, minb;
     if (precision == 32) {
         if (nrows != 1) return -1;
         fn = qo_ladder_pick32(n, first, cpl, &tpb, &minb);      /* qo_ladder32.cu */
-        name = "fp32";
     } else if (nrows == 2) {
         fn = lad_pick<double, 2, QO_LAD2_PP, QO_LAD2_TPB, QO_LAD2_MINB>(n, first, cpl);
-        tpb = QO_LAD2_TPB; minb = QO_LAD2_MINB; name = "s11";
-    } else if (!fn) {
+        tpb = QO_LAD2_TPB; minb = QO_LAD2_MINB;
+    } else {
         fn = lad_pick<double, 1, QO_LAD_PP, QO_LAD_TPB, QO_LAD_MINB>(n, first, cpl);
-        tpb = QO_LAD_TPB; minb = QO_LAD_MINB; name = "default";
+        tpb = QO_LAD_TPB; minb = QO_LAD_MINB;
     }
     if (!fn) return -1;
-    if (shape) *shape = name;
     const unsigned long long warps = (unsigned long long)(tpb / 32);
     unsigned long long blocks = (P->nsamples + warps - 1) / warps;
     const unsigned long long resident = (unsigned long long)sm_count * (unsigned long long)minb;

@@ -118,15 +118,9 @@ struct QoPlanes {
 /* one element: M <- M * ABCD(op; cf) at the two points.  The interpreter calls it with the opcode read from shared memory;
  * the run-time compiled flavour (qo_chain_jit.h) calls it once per element with literal arguments, so that the switch folds away */
 template <typename T, bool TRIG, bool ROW = false>
-__device__ __forceinline__ void qo_chain_step(const int op, const T *__restrict__ cf_, const T (&w)[2], const T (&wi)[2],
+__device__ __forceinline__ void qo_chain_step(const int op, const T *__restrict__ cf, const T (&w)[2], const T (&wi)[2],
                                               const T (&w2)[2], Abcd2<T> &m, const QoPlanes &planes, int k0)
 {
-#ifdef QO_JIT_COEF_IN_LOOP      /* straight-line flavour at three blocks per SM: keep the coefficient reads in the frequency loop (shared-memory
-                                 * broadcasts) -- hoisted, a ladder's ~44 per-sample doubles do not fit into 80 registers next to the chain state */
-    const volatile T *cf = cf_;
-#else
-    const T *__restrict__ cf = cf_;
-#endif
     {
         switch (op) {
         case OP_SER_LOSSY_L: {   /* Z = (R + jwL) / (1 - w^2 L Cp + j w R Cp) */
@@ -304,7 +298,7 @@ __device__ __forceinline__ void qo_st256(double2 *p, double2 a, double2 b)
 /* Compiled ahead of time this is the opcode interpreter.  qo_chain_jit.h hands the same text to NVRTC with the job's element
  * list (QO_JIT_CHAIN), spec kinds and template arguments defined in front of it: one kernel, C linkage, no dispatch. */
 #ifdef QO_JIT_CHAIN
-extern "C" __global__ void __launch_bounds__(QO_TPB, QO_JIT_MINB)
+extern "C" __global__ void __launch_bounds__(QO_TPB, 2)
 qo_mc_chain_jit_kernel(
 #else
 template <typename T, bool FULL_S, bool TRIG, bool GD>

@@ -13,8 +13,9 @@
 #include "qo_spot.cuh"
 #include "qo_tf_fs.cuh"
 #include "qo_tf_launch.h"
+#include "qo_overrides.h"
 
-/* launch shapes (tools/tf_sweep.py, profiles/r01h_*): plain ladders run 8 points per thread (coefficient loads and loop
+/* launch shapes (profiles/r01h_*): plain ladders run 8 points per thread (coefficient loads and loop
  * overhead amortised over 8 Horner sets), the four-chain modes (coupler block, |S11| specs) 4 */
 #define QO_TF_PP 4
 #define QO_TF_TPB 128
@@ -61,45 +62,27 @@ template <int PP, int TPB, int MINB> static tf_fn tf_pick_gd(int den, int nspec)
     return nspec > 4 ? tf_pick_gd_ns<8, PP, TPB, MINB>(den) : tf_pick_gd_ns<4, PP, TPB, MINB>(den);
 }
 
-extern "C" int qo_tf_launch(const TfPlan *tp, int pp, int variant, int sm_count, const TfParams *P, cudaStream_t st)
+extern "C" int qo_tf_launch(const TfPlan *tp, int pp, int sm_count, const TfParams *P, cudaStream_t st)
 {
     tf_fn fn = nullptr;
     int tpb = QO_TF_TPB, minb = QO_TF_MINB;
     const bool rot = P->cpl_lin && P->cpl_matched;      /* coupler on a uniformly spaced grid: angles by rotation */
-    (void)variant;
-#ifdef QO_TF_EXPERIMENT
-    /* development builds: other launch shapes, chosen with QO100NET_LAD_VARIANT (and QO100NET_TF_PP) */
-    if (tp->nn == 2 && pp == 4) switch (variant) {
-        case 1: fn = tf_pick<2, 0, false, 4, 128, 3>(tp->den); tpb = 128; minb = 3; break;
-        case 2: fn = tf_pick<2, 0, false, 4, 256, 2>(tp->den); tpb = 256; minb = 2; break;
-        case 3: fn = tf_pick<2, 0, false, 4, 128, 5>(tp->den); tpb = 128; minb = 5; break;
-        default: break;
-    }
-    if (tp->cpl_op >= 0 && pp == 2) switch (variant) {
-        case 1: fn = tf_pick<4, 1, false, 2, 128, 3>(tp->den); tpb = 128; minb = 3; break;
-        case 2: fn = tf_pick<4, 1, false, 2, 256, 2>(tp->den); tpb = 256; minb = 2; break;
-        default: break;
-    }
-    if (!fn)
-#endif
-    {
-        /* a line / measured block in front, or |S11| specs behind any front block: qo_tf_front.cu (checked FIRST: the plain
-         * |S11| instantiations below know nothing about a block) */
-        if (tp->nn == 4 && tp->cpl_op >= 0 && (tp->front || tp->s11)) fn = qo_tf_pick_front(tp->front, tp->s11, pp, tp->den, P->nspec, &tpb, &minb);
-        else if (tp->nn == 2 && pp == QO_TF_PP) fn = tf_pick<2, 0, false, QO_TF_PP, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
-        else if (tp->nn == 2 && pp == 1) fn = tf_pick<2, 0, false, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
-        else if (tp->gd && pp == 1) fn = tf_pick_gd<1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
-        else if (tp->nn == 4 && tp->s11 && pp == 1) fn = tf_pick<4, 0, true, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
-        else if (tp->nn == 4 && !tp->s11 && pp == 1) fn = rot ? (P->cpl_same ? tf_pick<4, 3, false, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec) : tf_pick<4, 2, false, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec))
-                     : tf_pick<4, 1, false, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
-        else if (tp->gd && pp == QO_TF_CPL_PP) { fn = tf_pick_gd<QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec); tpb = QO_TF_CPL_TPB; minb = QO_TF_CPL_MINB; }
-        else if (tp->nn == 4 && tp->s11 && pp == QO_TF_CPL_PP) { fn = tf_pick<4, 0, true, QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec); tpb = QO_TF_CPL_TPB; minb = QO_TF_CPL_MINB; }
-        else if (tp->nn == 4 && !tp->s11 && pp == QO_TF_CPL_PP) {
-            fn = rot ? (P->cpl_same ? tf_pick<4, 3, false, QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec)
-                                    : tf_pick<4, 2, false, QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec))
-                     : tf_pick<4, 1, false, QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec);
-            tpb = QO_TF_CPL_TPB; minb = QO_TF_CPL_MINB;
-        }
+    /* a line / measured block in front, or |S11| specs behind any front block: qo_tf_front.cu (checked FIRST: the plain
+     * |S11| instantiations below know nothing about a block) */
+    if (tp->nn == 4 && tp->cpl_op >= 0 && (tp->front || tp->s11)) fn = qo_tf_pick_front(tp->front, tp->s11, pp, tp->den, P->nspec, &tpb, &minb);
+    else if (tp->nn == 2 && pp == QO_TF_PP) fn = tf_pick<2, 0, false, QO_TF_PP, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
+    else if (tp->nn == 2 && pp == 1) fn = tf_pick<2, 0, false, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
+    else if (tp->gd && pp == 1) fn = tf_pick_gd<1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
+    else if (tp->nn == 4 && tp->s11 && pp == 1) fn = tf_pick<4, 0, true, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
+    else if (tp->nn == 4 && !tp->s11 && pp == 1) fn = rot ? (P->cpl_same ? tf_pick<4, 3, false, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec) : tf_pick<4, 2, false, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec))
+                 : tf_pick<4, 1, false, 1, QO_TF_TPB, QO_TF_MINB>(tp->den, P->nspec);
+    else if (tp->gd && pp == QO_TF_CPL_PP) { fn = tf_pick_gd<QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec); tpb = QO_TF_CPL_TPB; minb = QO_TF_CPL_MINB; }
+    else if (tp->nn == 4 && tp->s11 && pp == QO_TF_CPL_PP) { fn = tf_pick<4, 0, true, QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec); tpb = QO_TF_CPL_TPB; minb = QO_TF_CPL_MINB; }
+    else if (tp->nn == 4 && !tp->s11 && pp == QO_TF_CPL_PP) {
+        fn = rot ? (P->cpl_same ? tf_pick<4, 3, false, QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec)
+                                : tf_pick<4, 2, false, QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec))
+                 : tf_pick<4, 1, false, QO_TF_CPL_PP, QO_TF_CPL_TPB, QO_TF_CPL_MINB>(tp->den, P->nspec);
+        tpb = QO_TF_CPL_TPB; minb = QO_TF_CPL_MINB;
     }
     if (!fn) return -1;
     const unsigned long long warps = (unsigned long long)(tpb / 32);
@@ -176,7 +159,7 @@ struct TfCorner {
 };
 
 static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int precision, int generic, const double *f, int nf,
-                                  const unsigned char *mask, TfPlan *out);
+                                  const unsigned char *mask, const QoOverrides *ov, TfPlan *out);
 
 /* Where in the tolerance box the analysis looks (x[v] in [-1, 1] per random variable):
  *   0 every variable at -1, 1 the nominal network, 2 every variable at +1,
@@ -208,7 +191,7 @@ static void tf_corner_vars(const DevProg *hp, int e0, int nl, int ci, double *x)
             }
 }
 
-/* The analysis is a pure function of (program, grid, masks, environment overrides); callers that run the same job
+/* The analysis is a pure function of (program, grid, masks, overrides); callers that run the same job
  * repeatedly through qo_mc_run (one plan per call) would redo ~2 ms of host work per call, so the last few results
  * are kept, keyed by a 64-bit FNV-1a hash of those inputs. */
 static unsigned long long tf_fnv(unsigned long long h, const void *p, size_t n)
@@ -223,10 +206,10 @@ static int tf_cache_next;
 static std::mutex tf_cache_mu;
 
 extern "C" int qo_tf_plan_check(const DevProg *hp, int mode_reduce_only, int precision, int generic, const double *f, int nf,
-                                const unsigned char *mask, TfPlan *out)
+                                const unsigned char *mask, const QoOverrides *ov, TfPlan *out)
 {
     /* the cheap refusals first: nominal sweeps and FULL_S jobs come through here too and must not pay for the hash */
-    if (generic || !mode_reduce_only || precision != 64) return tf_plan_check_uncached(hp, mode_reduce_only, precision, generic, f, nf, mask, out);
+    if (generic || !mode_reduce_only || precision != 64) return tf_plan_check_uncached(hp, mode_reduce_only, precision, generic, f, nf, mask, ov, out);
     unsigned long long key = 1469598103934665603ull;
     {
         /* what the analysis does not read must not split the cache: seed, distribution, histogram set-up, thresholds */
@@ -240,17 +223,13 @@ extern "C" int qo_tf_plan_check(const DevProg *hp, int mode_reduce_only, int pre
     key = tf_fnv(key, mask, (size_t)nf);
     const int scal[4] = { mode_reduce_only, precision, generic, nf };
     key = tf_fnv(key, scal, sizeof scal);
-    static const char *envs[] = { "QO100NET_KERNEL", "QO100NET_TF_TRUNC", "QO100NET_TF_TOL", "QO100NET_TF_NO_E", "QO100NET_TF_NO_FRONT" };
-    for (size_t i = 0; i < sizeof envs / sizeof envs[0]; i++) {
-        const char *v = getenv(envs[i]);
-        key = tf_fnv(key, v ? v : "\1", v ? strlen(v) + 1 : 1);
-    }
+    key = tf_fnv(key, ov, sizeof *ov);
     {
         std::lock_guard<std::mutex> lk(tf_cache_mu);
         for (int i = 0; i < 8; i++)
             if (tf_cache[i].used && tf_cache[i].key == key) { *out = tf_cache[i].plan; return tf_cache[i].sel; }
     }
-    const int sel = tf_plan_check_uncached(hp, mode_reduce_only, precision, generic, f, nf, mask, out);
+    const int sel = tf_plan_check_uncached(hp, mode_reduce_only, precision, generic, f, nf, mask, ov, out);
     {
         std::lock_guard<std::mutex> lk(tf_cache_mu);
         TfCacheEntry &e = tf_cache[tf_cache_next];
@@ -261,13 +240,12 @@ extern "C" int qo_tf_plan_check(const DevProg *hp, int mode_reduce_only, int pre
 }
 
 static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int precision, int generic, const double *f, int nf,
-                                  const unsigned char *mask, TfPlan *out)
+                                  const unsigned char *mask, const QoOverrides *ov, TfPlan *out)
 {
     memset(out, 0, sizeof *out);
     out->cpl_op = -1;
 #define QO_TF_NO(msg) do { out->reason = msg; return 0; } while (0)
-    const char *force = getenv("QO100NET_KERNEL");
-    if (force && (strcmp(force, "interp") == 0 || strcmp(force, "ladder") == 0)) QO_TF_NO("QO100NET_KERNEL override");
+    if (ov->kernel == QoOverrides::INTERP || ov->kernel == QoOverrides::LADDER) QO_TF_NO("QO100NET_KERNEL override");
     if (generic || !mode_reduce_only || precision != 64) QO_TF_NO("not a reduce-only FP64 job on a lumped cascade");
     if (hp->nspec < 1 || hp->nspec > QO_TF_NSPEC || hp->n_var > QO_MAX_VAR) QO_TF_NO("spec / variable count");
     for (int s = 0; s < hp->nspec; s++)
@@ -280,8 +258,8 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
      * measured two-port.  Its row vector [1 Rs] M_block is evaluated per point (closed form / per-frequency table) and
      * contracted with the polynomials [P; Q] of everything behind it */
     if (hp->n_ops > e0 && hp->opcode[e0] == OP_CPL) { out->cpl_op = e0; out->front = 0; e0++; }
-    else if (hp->n_ops > e0 + 1 && hp->opcode[e0] == OP_TLINE && !getenv("QO100NET_TF_NO_FRONT")) { out->cpl_op = e0; out->front = 1; e0++; }
-    else if (hp->n_ops > e0 + 1 && hp->opcode[e0] == OP_SBLOCK && !getenv("QO100NET_TF_NO_FRONT")) { out->cpl_op = e0; out->front = 2; e0++; }
+    else if (hp->n_ops > e0 + 1 && hp->opcode[e0] == OP_TLINE && !ov->tf_no_front) { out->cpl_op = e0; out->front = 1; e0++; }
+    else if (hp->n_ops > e0 + 1 && hp->opcode[e0] == OP_SBLOCK && !ov->tf_no_front) { out->cpl_op = e0; out->front = 2; e0++; }
     const int nl = hp->n_ops - e0;
     if (nl < 1 || nl > QO_TF_MAXEL) QO_TF_NO("element count");
     int deg = 0, has_d = 0;
@@ -336,9 +314,7 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
      * less than `trunc` (relative) at every grid point of all three expansions -- numerators against |P| + zn |Q|
      * (|Num| for plain ladders), D against |D|, E against E.  QO100NET_TF_TRUNC=0 keeps everything.
      * Per point the scan runs from the top coefficient down and stops at the first term that may not be dropped. */
-    double trunc = 5e-13;
-    if (getenv("QO100NET_TF_TRUNC")) trunc = atof(getenv("QO100NET_TF_TRUNC"));
-    if (gd) trunc = 0.0;                                      /* the derivative polynomials weigh the top coefficients by their index: keep all */
+    const double trunc = gd ? 0.0 : ov->tf_trunc;          /* the derivative polynomials weigh the top coefficients by their index: keep all */
     const int NE = 2 * nl + 1, NC = 2 * Kfull;
     int kn = 1, kdd = 1, ke = 1;
     std::vector<double> xg((size_t)nf), xpw((size_t)NC + 1), zpw((size_t)NE + 1);
@@ -393,11 +369,10 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
     if (!has_d) forms[nforms++] = QO_TF_DEN_NONE;
     else if (gd) forms[nforms++] = QO_TF_DEN_DD;
     else {
-        if (ke <= QO_TF_MAXKE && ke <= 2 * kdd + 3 && !getenv("QO100NET_TF_NO_E")) forms[nforms++] = QO_TF_DEN_E;
+        if (ke <= QO_TF_MAXKE && ke <= 2 * kdd + 3) forms[nforms++] = QO_TF_DEN_E;
         forms[nforms++] = QO_TF_DEN_D;
     }
-    double tol = 1e-10;
-    if (getenv("QO100NET_TF_TOL")) tol = atof(getenv("QO100NET_TF_TOL"));
+    const double tol = ov->tf_tol;
     double worst = 0.0;
     int accepted = 0;
     for (int fi = 0; fi < nforms && !accepted; fi++) {
@@ -511,13 +486,13 @@ extern "C" int qo_tf_fs_launch(int dmode, int sm_count, const TfFsParams *P, cud
 /* Can FULL_S launches of this job run on qo_fs_tf_kernel?  Lumped cascade, no coupler; polynomial lengths by the same
  * tail rule; self-check of S11, S21, S22 (complex) against the per-element ABCD chain at the nominal network (every
  * point) and both ends of the tolerance box (every 4th point). */
-extern "C" int qo_tf_fs_plan_check(const DevProg *hp, int mode_full_s, int precision, int generic, const double *f, int nf, TfPlan *out)
+extern "C" int qo_tf_fs_plan_check(const DevProg *hp, int mode_full_s, int precision, int generic, const double *f, int nf, const QoOverrides *ov,
+                                   TfPlan *out)
 {
     memset(out, 0, sizeof *out);
     out->cpl_op = -1;
 #define QO_TF_NO(msg) do { out->reason = msg; return 0; } while (0)
-    const char *force = getenv("QO100NET_KERNEL");
-    if (force && (strcmp(force, "interp") == 0 || strcmp(force, "ladder") == 0)) QO_TF_NO("QO100NET_KERNEL override");
+    if (ov->kernel == QoOverrides::INTERP || ov->kernel == QoOverrides::LADDER) QO_TF_NO("QO100NET_KERNEL override");
     if (generic || !mode_full_s || precision != 64) QO_TF_NO("not an FP64 FULL_S job on a lumped cascade");
     const int e0 = hp->op0, nl = hp->n_ops - e0;
     if (nl < 1 || nl > QO_TF_MAXEL || hp->n_var > QO_MAX_VAR) QO_TF_NO("element count");
@@ -537,9 +512,7 @@ extern "C" int qo_tf_fs_plan_check(const DevProg *hp, int mode_full_s, int preci
     const double wr = two_pi * sqrt(f_lo * f_hi);
     out->wref = wr;
     const double rs = hp->rs, rl = hp->rl, zn = sqrt(rs * rl), zni = 1.0 / zn, k21 = hp->k21;
-    double trunc = 5e-13, tol = 1e-10;
-    if (getenv("QO100NET_TF_TRUNC")) trunc = atof(getenv("QO100NET_TF_TRUNC"));
-    if (getenv("QO100NET_TF_TOL")) tol = atof(getenv("QO100NET_TF_TOL"));
+    const double trunc = ov->tf_trunc, tol = ov->tf_tol;
     const int NCORN = hp->n_var > 0 ? QO_TF_NCORNER : 2;
     std::vector<TfCorner> cs((size_t)NCORN), c2((size_t)NCORN);
     for (int ci = 0; ci < NCORN; ci++) {
@@ -606,7 +579,6 @@ extern "C" int qo_tf_fs_plan_check(const DevProg *hp, int mode_full_s, int preci
                 if (xr > xlo && xr < xhi) factored = 1;
             }
         }
-        if (getenv("QO100NET_FS_POLY_D")) factored = 0;
     }
     if (factored) { out->den = QO_TF_DEN_E + 100; out->kd = 0; }          /* marker: factored D (launch_tf_fs reads it) */
     /* self-check: S11, S21, S22 from the kept polynomials against the per-element ABCD chain */

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 struct TfParams;
 struct DevProg;
+struct QoOverrides;
 /* what the plan decided for a job that runs on the transfer-function kernel */
 struct TfPlan {
     int nn;              /* numerator chains: 2 (Num = P + Rs Q) or 4 (P and Q apart: behind a coupled-line block, or with |S11| specs) */
@@ -22,10 +23,10 @@ struct TfPlan {
  * and a numerical self-check of exactly what the device will evaluate against the per-element evaluation, at the
  * nominal network and at both ends of its tolerance box, on every grid point.  Returns 1 (plan filled) or 0. */
 extern "C" int qo_tf_plan_check(const DevProg *hp, int mode_reduce_only, int precision, int generic, const double *f, int nf,
-                                const unsigned char *mask, TfPlan *out);
+                                const unsigned char *mask, const QoOverrides *ov, TfPlan *out);
 /* pp = frequency pairs per thread per iteration the plan padded its tables for; returns 0, -1 when no
  * instantiation covers (nn, den, pp), else the cudaError_t of the launch */
-extern "C" int qo_tf_launch(const TfPlan *tp, int pp, int variant, int sm_count, const TfParams *P, cudaStream_t st);
+extern "C" int qo_tf_launch(const TfPlan *tp, int pp, int sm_count, const TfParams *P, cudaStream_t st);
 extern "C" int qo_tf_default_pp(const TfPlan *tp, int npairs);
 
 /* thread-per-sample flavour (qo_ts.cuh): eligibility, threads per wave, launch (0 or the cudaError_t) */
@@ -41,5 +42,6 @@ extern "C" int qo_spot_launch(int need_s11, int sm_count, const SpotParams *P, c
 
 /* FULL_S flavour of the transfer-function kernel (qo_tf_fs.cuh) */
 struct TfFsParams;
-extern "C" int qo_tf_fs_plan_check(const DevProg *hp, int mode_full_s, int precision, int generic, const double *f, int nf, TfPlan *out);
+extern "C" int qo_tf_fs_plan_check(const DevProg *hp, int mode_full_s, int precision, int generic, const double *f, int nf, const QoOverrides *ov,
+                                   TfPlan *out);
 extern "C" int qo_tf_fs_launch(int dmode, int sm_count, const TfFsParams *P, cudaStream_t st);   /* dmode: 0 D == 1, 1 polynomial D, 2 factored D */

@@ -5,9 +5,6 @@
  * those loop bodies only.
  */
 #include <cuda_runtime.h>
-#include <stdio.h>
-#include <stdlib.h>
-#include <string.h>
 #include "qo_ts.cuh"
 #include "qo_tf_launch.h"
 #include "qo_ts_launch.h"
@@ -17,8 +14,6 @@
  * lengths fit the register capacities; behind a coupler only the matched / uniform-grid / equal-angle form (config 5). */
 extern "C" int qo_ts_eligible(const TfPlan *tp, int nspec, int cpl_rot_same)
 {
-    const char *force = getenv("QO100NET_KERNEL");
-    if (force && strcmp(force, "tf") == 0) return 0;          /* keep everything on the warp-per-sample kernel (A/B runs) */
     if (tp->s11 || tp->gd || nspec > 4) return 0;
     if (tp->den != QO_TF_DEN_NONE && tp->den != QO_TF_DEN_E) return 0;
     if (tp->kn < 2 || (tp->den == QO_TF_DEN_E && (tp->kd < 2 || (tp->kd & 1)))) return 0;
@@ -39,7 +34,6 @@ static int ts_blocks_per_sm(const TfPlan *tp)
     int occ = 0;
     ts_fn fn = ts_pick_kernel(tp);
     if (!fn || cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, QO_TS_TPB, 0) != cudaSuccess) { cudaGetLastError(); occ = 0; }
-    if (getenv("QO100NET_TS_DEBUG")) fprintf(stderr, "qo_ts: %d blocks of %d threads resident per SM\n", occ, QO_TS_TPB);
     return occ;
 }
 

@@ -619,6 +619,8 @@ def plan_analyze(net, f, specs, tols=(), dist=DIST_UNIFORM, mode=MODE_REDUCE_ONL
     info = (C.c_int * 6)()
     err, sec = C.c_double(0.0), C.c_double(0.0)
     reason = lib().qo_plan_analyze(net._h, _dp(f), len(f), _specs(specs), len(specs), C.byref(cfg), info, C.byref(err), C.byref(sec)).decode()
+    if info[0] < 0:
+        raise QoError(info[0], reason)
     return dict(selected=bool(info[0]), numerator_chains=info[1], den_form=("none", "E", "D", "DD")[info[2]] if 0 <= info[2] <= 3 else "?",
                 kn=info[3], kd=info[4], degree=info[5], self_check_err=err.value, reason=reason, seconds=sec.value)
 

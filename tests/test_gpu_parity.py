@@ -460,7 +460,10 @@ def _ladder_workload(Q, W, order, series_first, coupler, butter=False, fc=10e6, 
     net = net.add_parasitics(fc, 60.0, 30.0, 0.1, 50.0)
     tols = Q.lc_tolerances(net, 0.05, 0.02)
     if coupler:
-        cpl = Q.Net.from_elements([(Q.CPL_THRU, [55.2771, 45.2267, 95.4225, 91.0, 4 * fc, 50.0])], 50.0, 50.0)
+        # even orders: the coupler is referenced to 60 Ohm behind the 50 Ohm source, so the block's row vector takes its general
+        # form instead of the matched one (qo_tf.cuh::tf_cpl_matched)
+        zt = 60.0 if order % 2 == 0 else 50.0
+        cpl = Q.Net.from_elements([(Q.CPL_THRU, [55.2771, 45.2267, 95.4225, 91.0, 4 * fc, zt])], 50.0, 50.0)
         net = cpl.concat(net)
         tols = [(0, 0, 0, Q.TOL_REL, 0.02), (0, 1, 1, Q.TOL_REL, 0.02), (0, 2, 2, Q.TOL_REL, 0.01), (0, 3, 2, Q.TOL_REL, 0.01)] + \
                [(e + 1, p, v + 3, m, t) for (e, p, v, m, t) in tols]

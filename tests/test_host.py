@@ -407,7 +407,7 @@ def test_transfer_function_plan_analysis(Q, W, monkeypatch):
     """Host-only part of plan creation (qo_plan_analyze, no GPU): which jobs take the transfer-function kernel, the
     polynomial lengths the grid needs, the denominator form, and the self-check of the expansion against the
     per-element evaluation (<= 1e-10 on |den|^2; north_star asks 1e-9)."""
-    for v in ("QO100NET_KERNEL", "QO100NET_TF_TOL", "QO100NET_TF_TRUNC", "QO100NET_TF_NO_E"):
+    for v in ("QO100NET_KERNEL", "QO100NET_TF_TOL", "QO100NET_TF_TRUNC", "QO100NET_TF_NO_FRONT"):
         monkeypatch.delenv(v, raising=False)
     w = W.cfg2()
     a = Q.plan_analyze(w.net, w.f, w.specs, w.tols, **w.hist)
