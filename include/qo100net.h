@@ -268,9 +268,8 @@ int qo_nodal_analyze(const qo_nodal *nd, const double *f, int nf, const qo_mc_cf
  * factorisation lives in registers), [3] = spill bytes, [4] = complex multiply-subtracts per point, [5] = reciprocals per point. */
 int qo_nodal_jit_analyze(const qo_nodal *nd, const double *f, int nf, const qo_nspec *spec, int nspec, const qo_mc_cfg *cfg, int info[6]);
 
-/* which factorisation the calling thread's last nodal call used: "qo_nodal_kernel<static,smem>" /
- * "qo_nodal_kernel<static,local>" (symbolic plan: fixed pivot order and fill pattern, verified on the host against
- * the pivoted solve; values in a thread-private array or, with QO100NET_NODAL_VALUES=smem, in shared memory), "qo_nodal_jit_kernel"
+/* which factorisation the calling thread's last nodal call used: "qo_nodal_kernel<static,local>" (symbolic plan:
+ * fixed pivot order and fill pattern, verified on the host against the pivoted solve; values in a thread-private array), "qo_nodal_jit_kernel"
  * (the same plan compiled into a kernel of its own, values in registers) or "qo_nodal_kernel<dense>" (per-point partial pivoting; QO100NET_NODAL=dense forces it) */
 const char *qo_nodal_last_kernel(void);
 /* seconds the calling thread's last nodal call spent generating + compiling its kernel (0: none needed, or taken from the process cache) */

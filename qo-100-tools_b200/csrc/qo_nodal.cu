@@ -22,9 +22,11 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <memory>
 #include <vector>
 
 #include "qo_ctx_internal.h"
+#include "qo_overrides.h"
 #include "qo_stream.h"
 
 #include "qo_nodal_prog.h"
@@ -70,14 +72,14 @@ template <int LD> struct DenseSink {
 /* ... or the compact value array of the static plan.  The order of the add() calls of nodal_stamp_all depends only on the netlist, so the host records, once per
  * job, the value index every call lands on (bit 15: first touch -> store instead of add); the kernel replays
  * that stream and never looks at (row, column) again: no index tables, no zero-fill of stamped values. */
-template <int VS> struct ReplaySink {
+struct ReplaySink {
     double2 *V;
     const uint16_t *st;
     int k;
     __host__ __device__ __forceinline__ void add(int, int, double2 v)
     {
         const unsigned int wd = st[k++];
-        const int q = (int)(wd & 0x7fffu) * VS;
+        const int q = (int)(wd & 0x7fffu);
         if (wd >> 15) V[q] = v;
         else { V[q].x += v.x; V[q].y += v.y; }
     }
@@ -147,7 +149,7 @@ __host__ __device__ __forceinline__ void nodal_stamp_all(const NodalProg *prog, 
  * partial pivoting keeps every multiplier <= 1; the fixed order does not, and a huge one means this point (this sample's
  * values at this frequency) wanted another pivot -- the caller counts such points and the host re-runs the job on the
  * pivoted dense kernel (QN_GROWTH2) */
-template <int VS> __host__ __device__ __forceinline__ double static_factor(const uint16_t *pg, int n, double2 *V)
+__host__ __device__ __forceinline__ double static_factor(const uint16_t *pg, int n, double2 *V)
 {
     double lmax2 = 0.0;
     int ip = 0;
@@ -156,15 +158,15 @@ template <int VS> __host__ __device__ __forceinline__ double static_factor(const
         const uint16_t *ucol = pg + ip + 2;          /* value indices of the pivot row's entries right of the pivot */
         const int nrows = pg[ip + 2 + nu];
         if (nrows == 0) { ip += 3 + nu; continue; }  /* nothing below the pivot */
-        const double2 inv = hd_inv(V[pg[ip] * VS]);
+        const double2 inv = hd_inv(V[pg[ip]]);
         ip += 3 + nu;
         for (int r = 0; r < nrows; r++) {
-            const int prc = pg[ip++] * VS;
+            const int prc = pg[ip++];
             const double2 l = hd_mul(V[prc], inv);
             V[prc] = l;
             const double l2 = fma(l.x, l.x, l.y * l.y);
             lmax2 = !(l2 <= lmax2) ? l2 : lmax2;                       /* NaN sticks */
-            for (int q = 0; q < nu; q++) { const int prj = pg[ip + q] * VS; V[prj] = hd_fms(V[prj], l, V[ucol[q] * VS]); }
+            for (int q = 0; q < nu; q++) { const int prj = pg[ip + q]; V[prj] = hd_fms(V[prj], l, V[ucol[q]]); }
             ip += nu;
         }
     }
@@ -179,21 +181,21 @@ template <int VS> __host__ __device__ __forceinline__ double static_factor(const
  * reach (forward) and only the rows the port unknowns depend on (backward).  Stream at `at`:
  *   n_fwd, { row i, n_terms, { q, value index } ... } ...,  n_bwd, { row i, diag index, n_terms, { q, value index } ... } ...
  * x must be zero except for the injected entry. */
-template <int VS> __host__ __device__ __forceinline__ void static_solve(const uint16_t *pg, int at, const double2 *V, double2 *x)
+__host__ __device__ __forceinline__ void static_solve(const uint16_t *pg, int at, const double2 *V, double2 *x)
 {
     int ip = at;
     const int nfwd = pg[ip++];
     for (int t = 0; t < nfwd; t++) {
         const int i = pg[ip++], nl = pg[ip++];
         double2 acc = x[i];
-        for (int q = 0; q < nl; q++) { acc = hd_fms(acc, V[pg[ip + 1] * VS], x[pg[ip]]); ip += 2; }
+        for (int q = 0; q < nl; q++) { acc = hd_fms(acc, V[pg[ip + 1]], x[pg[ip]]); ip += 2; }
         x[i] = acc;
     }
     const int nbwd = pg[ip++];
     for (int t = 0; t < nbwd; t++) {
-        const int i = pg[ip++], pii = pg[ip++] * VS, nu = pg[ip++];
+        const int i = pg[ip++], pii = pg[ip++], nu = pg[ip++];
         double2 acc = x[i];
-        for (int q = 0; q < nu; q++) { acc = hd_fms(acc, V[pg[ip + 1] * VS], x[pg[ip]]); ip += 2; }
+        for (int q = 0; q < nu; q++) { acc = hd_fms(acc, V[pg[ip + 1]], x[pg[ip]]); ip += 2; }
         x[i] = hd_mul(acc, hd_inv(V[pii]));
     }
 }
@@ -202,9 +204,7 @@ template <int VS> __host__ __device__ __forceinline__ void static_solve(const ui
  * unit u = sample * nchunks + chunk; a block works on one unit at a time: QN_TPB consecutive grid points per
  * pass.  Reduce-only jobs use nchunks == 1 (the block walks the whole grid of its sample and then reduces).
  */
-/* MODE 0: dense, per-point pivoting | 1: static plan, values in a private (local-memory) array of NNZ entries |
- * 2: static plan, values in dynamic shared memory, one column per thread (conflict-free, never spills to DRAM:
- * ncu on mode 1 showed 67 GB of DRAM traffic per launch from thrashing local arrays) */
+/* MODE 0: dense, per-point pivoting | 1: static plan, values in a private (local-memory) array of NNZ entries */
 template <int LD, int MODE, int NNZ>
 __global__ void __launch_bounds__(QN_TPB)
 qo_nodal_kernel(const NodalProg *__restrict__ prog, const NodalStatic *__restrict__ splan, const double *__restrict__ fgrid,
@@ -214,8 +214,6 @@ qo_nodal_kernel(const NodalProg *__restrict__ prog, const NodalStatic *__restric
 {
     /* static plan staged in shared memory: every thread walks the same program (broadcast reads) */
     constexpr bool STATIC = MODE != 0;
-    constexpr int VS = MODE == 2 ? QN_TPB : 1;
-    extern __shared__ double2 s_vals[];              /* MODE 2: [nnz][QN_TPB] */
     __shared__ uint8_t s_rowmap[QO_NODAL_MAX_UNK], s_colmap[QO_NODAL_MAX_UNK];
     __shared__ uint16_t s_prog[STATIC ? QN_PROG_MAX : 1];
     if (STATIC) {
@@ -257,16 +255,15 @@ qo_nodal_kernel(const NodalProg *__restrict__ prog, const NodalStatic *__restric
         for (int k = k_lo + tid; k < k_hi; k += QN_TPB) {
             const double w = 6.283185307179586476925286766559 * fgrid[k];
             const double2 *yk = yblk + (size_t)k * 4;                 /* block admittances: [block][nf][4] */
-            double2 A[MODE == 1 ? NNZ : MODE == 0 ? LD * LD : 1];
-            double2 *V = MODE == 2 ? s_vals + tid : A;
+            double2 A[STATIC ? NNZ : LD * LD];
             int perm[STATIC ? 1 : LD];
             unsigned int lmask[STATIC ? 1 : LD], umask[STATIC ? 1 : LD];
             bool singular = false;
             if (STATIC) {
-                for (int i = 0; i < splan->n_zero; i++) V[s_prog[splan->zero_at + i] * VS] = make_double2(0.0, 0.0);   /* fill-only */
-                ReplaySink<VS> S = { V, s_prog + splan->stamp_at, 0 };
+                for (int i = 0; i < splan->n_zero; i++) A[s_prog[splan->zero_at + i]] = make_double2(0.0, 0.0);   /* fill-only */
+                ReplaySink S = { A, s_prog + splan->stamp_at, 0 };
                 nodal_stamp_all(prog, s_p, w, yk, (size_t)nf * 4, S);
-                const double l2 = static_factor<VS>(s_prog, n, V);
+                const double l2 = static_factor(s_prog, n, A);
                 if (!(l2 <= growth2)) n_suspect++;
             } else {
                 for (int i = 0; i < n; i++) {
@@ -320,7 +317,7 @@ qo_nodal_kernel(const NodalProg *__restrict__ prog, const NodalStatic *__restric
                 if (STATIC) {
                     for (int i = 0; i < n; i++) x[i] = make_double2(0.0, 0.0);
                     x[s_rowmap[src]] = make_double2(1.0 / prog->port_z0[j], 0.0);
-                    static_solve<VS>(s_prog, splan->solve_at[j], V, x);
+                    static_solve(s_prog, splan->solve_at[j], A, x);
                 } else {
                     for (int i = 0; i < n; i++) x[i] = make_double2(perm[i] == src ? 1.0 / prog->port_z0[j] : 0.0, 0.0);
                     if (singular) { for (int i = 0; i < n; i++) x[i] = make_double2(nan(""), nan("")); }
@@ -494,8 +491,7 @@ static bool build_static_thr(const NodalProg *hp, const double *f, int nf, const
     for (int p = 0; p < np; p++) { if (is_port[hp->port_node[p] - 1]) return false; is_port[hp->port_node[p] - 1] = 1; }
     /* internal unknowns in greedy MINIMUM-DEGREE order on the structurally symmetrised pattern (eliminating an unknown joins
      * its neighbours): the bias networks are stars around their supply rails, and taking the leaves first leaves almost no
-     * fill -- 175 -> 60 multiply-subtracts per point on the reference network against the netlist's own numbering.
-     * QO100NET_NODAL_ORDER=natural keeps the netlist order (A/B). */
+     * fill -- 175 -> 60 multiply-subtracts per point on the reference network against the netlist's own numbering. */
     int nc = 0;
     {
         std::vector<unsigned char> raw0((size_t)LD * LD, 0);
@@ -504,8 +500,6 @@ static bool build_static_thr(const NodalProg *hp, const double *f, int nf, const
         std::vector<unsigned int> adj(n, 0);
         for (int r = 0; r < n; r++) for (int c = 0; c < n; c++) if (r != c && (raw0[r * LD + c] || raw0[c * LD + r])) adj[r] |= 1u << c;
         std::vector<int> gone(n, 0), comp(n, -1);
-        const char *ord = getenv("QO100NET_NODAL_ORDER");
-        const bool natural = ord && !strcmp(ord, "natural");
         /* unconnected sub-circuits (the reference network is two bias tees side by side) one after the other: the values of a
          * finished sub-circuit are dead before the next one is stamped, which halves the live set of the compiled kernel */
         int ncomp = 0;
@@ -524,8 +518,8 @@ static bool build_static_thr(const NodalProg *hp, const double *f, int nf, const
             int best = -1, bdeg = 1 << 30, bcomp = 1 << 30;
             for (int u = 0; u < n; u++) {
                 if (gone[u] || is_port[u]) continue;
-                const int deg = natural ? u : __builtin_popcount(adj[u]);
-                const int cu = natural ? 0 : comp[u];
+                const int deg = __builtin_popcount(adj[u]);
+                const int cu = comp[u];
                 if (cu < bcomp || (cu == bcomp && deg < bdeg)) { bcomp = cu; bdeg = deg; best = u; }
             }
             gone[best] = 1;
@@ -667,16 +661,16 @@ static bool build_static_thr(const NodalProg *hp, const double *f, int nf, const
         if (!host_dense(hp, par, f[k], yb + (size_t)k * 4, (size_t)nf * 4, NULL, &X)) return false;
         cvec V((size_t)nnz, make_double2(nan(""), nan("")));            /* poisoned: the streams must initialise every value */
         for (int i = 0; i < sp->n_zero; i++) V[sp->prog[sp->zero_at + i]] = make_double2(0.0, 0.0);
-        ReplaySink<1> S = { V.data(), sp->prog + sp->stamp_at, 0 };
+        ReplaySink S = { V.data(), sp->prog + sp->stamp_at, 0 };
         nodal_stamp_all(hp, par, 6.283185307179586476925286766559 * f[k], yb + (size_t)k * 4, (size_t)nf * 4, S);
-        const double l2 = static_factor<1>(sp->prog, n, V.data());
+        const double l2 = static_factor(sp->prog, n, V.data());
         if (getenv("QO100NET_NODAL_DEBUG") && !(l2 <= QN_GROWTH2)) fprintf(stderr, "qo_nodal: probe f=%g Hz: largest multiplier %.3g\n", f[k], sqrt(l2));
         if (!(l2 <= QN_GROWTH2)) return false;                          /* the device would flag this point: do not start on this plan */
         if (l2 > worst_l2) worst_l2 = l2;
         for (int j = 0; j < np; j++) {
             cvec x(n, make_double2(0.0, 0.0));
             x[sp->rowmap[hp->port_node[j] - 1]] = make_double2(1.0 / hp->port_z0[j], 0.0);
-            static_solve<1>(sp->prog, sp->solve_at[j], V.data(), x.data());
+            static_solve(sp->prog, sp->solve_at[j], V.data(), x.data());
             for (int p = 0; p < np; p++) {
                 const double2 a = x[sp->colmap[hp->port_node[p] - 1]], b = X[j][hp->port_node[p] - 1];
                 const double err = hypot(a.x - b.x, a.y - b.y), ref = hypot(b.x, b.y);
@@ -702,7 +696,7 @@ static bool build_static_thr(const NodalProg *hp, const double *f, int nf, const
 
 /* host-only front end: netlist + specs + tolerances -> device program, spec masks, block admittances */
 static int nodal_compile(const qo_nodal *nd, const double *f, int nf, const qo_nspec *spec, int nspec, const qo_mc_cfg *cfg, int full,
-                         NodalProg *hp, std::vector<unsigned char> &mask, std::vector<double2> &yb, int *n_unk_out)
+                         NodalProg *hp, std::vector<unsigned char> &mask, std::vector<double2> &yb)
 {
     if (!nd || !f || nf <= 0 || !cfg || nspec < 0 || nspec > QN_MAX_SPEC || (nspec && !spec)) { qo_set_error("bad arguments"); return QO_ERR_ARG; }
     if (nd->np < 1) { qo_set_error("the netlist has no ports"); return QO_ERR_ARG; }
@@ -720,7 +714,6 @@ static int nodal_compile(const qo_nodal *nd, const double *f, int nf, const qo_n
     }
     if (n_unk > QO_NODAL_MAX_UNK) { qo_set_error("%d unknowns, limit %d", n_unk, QO_NODAL_MAX_UNK); return QO_ERR_RANGE; }
     hp->n_unk = n_unk;
-    *n_unk_out = n_unk;
     for (int p = 0; p < nd->np; p++) { hp->port_node[p] = nd->port_node[p]; hp->port_z0[p] = nd->port_z0[p]; }
     int nvar = 0;
     if (cfg->n_tol < 0 || (cfg->n_tol > 0 && !cfg->tol)) return QO_ERR_ARG;
@@ -764,6 +757,27 @@ static int nodal_compile(const qo_nodal *nd, const double *f, int nf, const qo_n
     return QO_OK;
 }
 
+/* what the host prepares for a nodal job */
+struct NodalJob {
+    NodalProg prog;
+    NodalStatic plan;                   /* all zero unless use_static */
+    bool use_static;                    /* the static plan was tried and passed its self-check */
+    std::vector<unsigned char> mask;    /* per grid point: the specs that cover it (bit s) */
+    std::vector<double2> yb;            /* measured blocks' admittances [block][nf][4]; one zero entry when there is none */
+};
+
+/* the host front end of every nodal entry point (needs no GPU): compile the netlist and, if try_static, the static plan */
+static int nodal_prepare(const qo_nodal *nd, const double *f, int nf, const qo_nspec *spec, int nspec, const qo_mc_cfg *cfg, int full,
+                         bool try_static, std::unique_ptr<NodalJob> &job)
+{
+    job.reset(new NodalJob());
+    const int rc = nodal_compile(nd, f, nf, spec, nspec, cfg, full, &job->prog, job->mask, job->yb);
+    if (rc) return rc;
+    if (job->yb.empty()) job->yb.assign(4, make_double2(0.0, 0.0));
+    job->use_static = try_static && build_static(&job->prog, f, nf, job->yb.data(), &job->plan);
+    return QO_OK;
+}
+
 /* The host-only part of a nodal job (needs no GPU): compile the netlist and try the static (symbolic) factorisation plan.
  * info[0] = static plan accepted (0/1), [1] = unknowns, [2] = packed non-zeros incl. fill, [3] = program length (16-bit words);
  * *max_multiplier = largest |L| entry the plan-time probes met (per-point partial pivoting would keep it <= 1). */
@@ -771,19 +785,17 @@ extern "C" int qo_nodal_analyze(const qo_nodal *nd, const double *f, int nf, con
 {
     qo_clear_error();
     if (!info) return QO_ERR_ARG;
+    QoNodalOverrides ov;                     /* the analysis tries the static plan whatever they say, but a bad value is refused */
+    int rc = qo_nodal_overrides_read(&ov);
+    if (rc) return rc;
     qo_mc_cfg c0;
     memset(&c0, 0, sizeof c0);
-    std::vector<NodalProg> hpv(1);
-    std::vector<unsigned char> mask;
-    std::vector<double2> yb;
-    int n_unk = 0;
-    int rc = nodal_compile(nd, f, nf, NULL, 0, cfg ? cfg : &c0, 1, &hpv[0], mask, yb, &n_unk);
+    std::unique_ptr<NodalJob> job;
+    rc = nodal_prepare(nd, f, nf, NULL, 0, cfg ? cfg : &c0, 1, true, job);
     if (rc) return rc;
-    std::vector<NodalStatic> spv(1);
-    if (yb.empty()) yb.assign(4, make_double2(0.0, 0.0));
-    const bool ok = build_static(&hpv[0], f, nf, yb.data(), &spv[0]);
-    info[0] = ok; info[1] = n_unk; info[2] = ok ? spv[0].nnz : 0; info[3] = ok ? spv[0].prog_len : 0;
-    if (max_multiplier) *max_multiplier = ok ? sqrt(spv[0].worst_l2) : 0.0;
+    const bool ok = job->use_static;
+    info[0] = ok; info[1] = job->prog.n_unk; info[2] = ok ? job->plan.nnz : 0; info[3] = ok ? job->plan.prog_len : 0;
+    if (max_multiplier) *max_multiplier = ok ? sqrt(job->plan.worst_l2) : 0.0;
     return QO_OK;
 }
 
@@ -796,16 +808,14 @@ extern "C" int qo_nodal_jit_analyze(const qo_nodal *nd, const double *f, int nf,
     qo_clear_error();
     if (!info || !cfg) return QO_ERR_ARG;
     for (int i = 0; i < 6; i++) info[i] = 0;
-    std::vector<NodalProg> hpv(1);
-    std::vector<unsigned char> mask;
-    std::vector<double2> yb;
-    int n_unk = 0;
-    int rc = nodal_compile(nd, f, nf, spec, nspec, cfg, cfg->mode == QO_MODE_FULL_S, &hpv[0], mask, yb, &n_unk);
+    QoNodalOverrides ov;                     /* as in qo_nodal_analyze: read only to refuse a bad value */
+    int rc = qo_nodal_overrides_read(&ov);
     if (rc) return rc;
-    std::vector<NodalStatic> spv(1);
-    if (yb.empty()) yb.assign(4, make_double2(0.0, 0.0));
-    if (!build_static(&hpv[0], f, nf, yb.data(), &spv[0])) { qo_set_error("the static plan failed its self-check for this network"); return QO_OK; }
-    const QnJitEntry *e = qn_jit_get(&hpv[0], &spv[0], false, true);
+    std::unique_ptr<NodalJob> job;
+    rc = nodal_prepare(nd, f, nf, spec, nspec, cfg, cfg->mode == QO_MODE_FULL_S, true, job);
+    if (rc) return rc;
+    if (!job->use_static) { qo_set_error("the static plan failed its self-check for this network"); return QO_OK; }
+    const QnJitEntry *e = qn_jit_get(&job->prog, &job->plan, false, true);
     info[0] = e->ok; info[1] = e->regs; info[2] = e->stack_bytes; info[3] = e->spill_bytes; info[4] = e->n_fms; info[5] = e->n_inv;
     if (!e->ok) qo_set_error("%s", e->log.substr(0, 400).c_str());
     return QO_OK;
@@ -816,6 +826,21 @@ extern "C" int qo_nodal_jit_analyze(const qo_nodal *nd, const double *f, int nf,
 #define QN_JIT_MIN_POINTS 400000000ull
 #define QN_JIT_MIN_CACHED 1000000ull
 
+/* the interpreted kernel of a job: the static plan's instantiation by its number of values, the dense one by its unknowns */
+static const void *nodal_kernel(bool use_static, int nnz, int n_unk)
+{
+    if (use_static) {
+        if (nnz <= 64) return (const void *)qo_nodal_kernel<32, 1, 64>;
+        if (nnz <= 128) return (const void *)qo_nodal_kernel<32, 1, 128>;
+        if (nnz <= 256) return (const void *)qo_nodal_kernel<32, 1, 256>;
+        return (const void *)qo_nodal_kernel<32, 1, QN_NNZ_MAX>;
+    }
+    if (n_unk <= 8) return (const void *)qo_nodal_kernel<8, 0, 1>;
+    if (n_unk <= 16) return (const void *)qo_nodal_kernel<16, 0, 1>;
+    if (n_unk <= 24) return (const void *)qo_nodal_kernel<24, 0, 1>;
+    return (const void *)qo_nodal_kernel<32, 0, 1>;
+}
+
 static int nodal_run(qo_ctx *ctx, const qo_nodal *nd, const double *f, int nf, const qo_nspec *spec, int nspec,
                      const qo_mc_cfg *cfg, qo_mc_result *res, qo_c64 *full_s_host)
 {
@@ -824,43 +849,35 @@ static int nodal_run(qo_ctx *ctx, const qo_nodal *nd, const double *f, int nf, c
     const int full = cfg->mode == QO_MODE_FULL_S;
     if (full && !full_s_host) { qo_set_error("FULL_S needs an output buffer"); return QO_ERR_ARG; }
     if (!full && !res) return QO_ERR_ARG;
-    std::vector<NodalProg> hpv(1);
-    NodalProg *hp = &hpv[0];
-    std::vector<unsigned char> mask;
-    std::vector<double2> yb;
-    int n_unk = 0;
-    {
-        const int rcc = nodal_compile(nd, f, nf, spec, nspec, cfg, full, hp, mask, yb, &n_unk);
-        if (rcc) return rcc;
-    }
+    QoNodalOverrides ov;
+    int rc = qo_nodal_overrides_read(&ov);
+    if (rc) return rc;
     /* static (symbolic) plan unless forced off or its self-check fails */
-    std::vector<NodalStatic> spv(1);
-    const char *force = getenv("QO100NET_NODAL");
-    bool use_static = !(force && !strcmp(force, "dense"));
-    if (use_static) {
-        cvec ybs = yb;
-        if (ybs.empty()) ybs.assign(4, make_double2(0.0, 0.0));
-        use_static = build_static(hp, f, nf, ybs.data(), &spv[0]);
-    }
-    if (force && !strcmp(force, "static") && !use_static) { qo_set_error("QO100NET_NODAL=static: the static plan failed its self-check for this network"); return QO_ERR_UNSUPPORTED; }
+    std::unique_ptr<NodalJob> job;
+    rc = nodal_prepare(nd, f, nf, spec, nspec, cfg, full, ov.kernel != QoNodalOverrides::DENSE, job);
+    if (rc) return rc;
+    const NodalProg *hp = &job->prog;
+    bool use_static = job->use_static;
+    if (ov.kernel == QoNodalOverrides::STATIC && !use_static) { qo_set_error("QO100NET_NODAL=static: the static plan failed its self-check for this network"); return QO_ERR_UNSUPPORTED; }
     const int ncnt = 2 + nspec + hp->hist_bins;
     const unsigned long long N = cfg->n_samples;
     if (N == 0) { if (res) { res->n_pass = res->n_total = 0; } return QO_OK; }
     /* the plan compiled into a kernel of its own: large jobs (QO100NET_NODAL=jit: always; =static / =dense: never) */
     const QnJitEntry *jit = NULL;
-    if (use_static && !(force && !strcmp(force, "static"))) {
-        const bool forced = force && !strcmp(force, "jit");
+    if (use_static && ov.kernel != QoNodalOverrides::STATIC) {
+        const bool forced = ov.kernel == QoNodalOverrides::JIT;
         const unsigned long long npts = N * (unsigned long long)nf;
         if (forced || npts >= QN_JIT_MIN_CACHED) {
             const size_t had = g_qn_jit.size();
-            jit = qn_jit_get(hp, &spv[0], true, forced || npts >= QN_JIT_MIN_POINTS);
+            jit = qn_jit_get(hp, &job->plan, true, forced || npts >= QN_JIT_MIN_POINTS);
             if (jit && g_qn_jit.size() != had) g_last_compile_s = jit->compile_s;
             if (jit && !jit->ok) {
                 if (forced) { qo_set_error("QO100NET_NODAL=jit: %s", jit->log.substr(0, 400).c_str()); return QO_ERR_UNSUPPORTED; }
                 jit = NULL;
             }
         }
-    } else if (force && !strcmp(force, "jit")) { qo_set_error("QO100NET_NODAL=jit: the static plan failed its self-check for this network"); return QO_ERR_UNSUPPORTED; }
+    } else if (ov.kernel == QoNodalOverrides::JIT) { qo_set_error("QO100NET_NODAL=jit: the static plan failed its self-check for this network"); return QO_ERR_UNSUPPORTED; }
+    const void *kern = jit ? (const void *)jit->kern : nodal_kernel(use_static, job->plan.nnz, hp->n_unk);
 
     /* samples are independent: GPU g of the ctx takes the contiguous range [N g / G, N (g+1) / G) of the job (the Philox counter
      * carries the global sample index, so the counters do not depend on G); the host adds the u64 counters, FULL_S slabs are
@@ -872,15 +889,13 @@ static int nodal_run(qo_ctx *ctx, const qo_nodal *nd, const double *f, int nf, c
         int grid;
     } nv[8];
     memset(nv, 0, sizeof nv);
-    int rc = QO_OK;
     const int np_ = nd->np;
     std::vector<unsigned long long> h((size_t)ncnt + 1, 0ull), hg((size_t)ncnt + 1);
     float ms_max = 0.0f;
     int chunk_len = nf, nchunks = 1;
     /* FULL_S: cut the grid into QN_TPB-point chunks so that a nominal sweep fills the GPU */
     if (full) { chunk_len = QN_TPB; nchunks = (nf + chunk_len - 1) / chunk_len; }
-    double growth2 = QN_GROWTH2;
-    { const char *e = getenv("QO100NET_NODAL_GUARD2"); if (e && atof(e) > 0.0) growth2 = atof(e); }     /* tests: trip the device guard on purpose */
+    double growth2 = ov.growth2 > 0.0 ? ov.growth2 : QN_GROWTH2;
 #define CUN(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { qo_set_error("%s -> %s", #call, cudaGetErrorString(e_)); rc = e_ == cudaErrorMemoryAllocation ? QO_ERR_NOMEM : QO_ERR_CUDA; goto out; } } while (0)
     for (int g = 0; g < G; g++) {
         DevCtx *dc = &ctx->d[g];
@@ -890,100 +905,66 @@ static int nodal_run(qo_ctx *ctx, const qo_nodal *nd, const double *f, int nf, c
         CUN(cudaSetDevice(dc->device));
         CUN(cudaMallocAsync((void **)&v.dprog, sizeof(NodalProg), dc->stream));
         CUN(cudaMallocAsync((void **)&v.dsp, sizeof(NodalStatic), dc->stream));
-        CUN(cudaMemcpyAsync(v.dsp, &spv[0], sizeof(NodalStatic), cudaMemcpyHostToDevice, dc->stream));
+        CUN(cudaMemcpyAsync(v.dsp, &job->plan, sizeof(NodalStatic), cudaMemcpyHostToDevice, dc->stream));
         CUN(cudaMallocAsync((void **)&v.dfr, (size_t)nf * sizeof(double), dc->stream));
         CUN(cudaMallocAsync((void **)&v.dmask, (size_t)nf, dc->stream));
-        CUN(cudaMallocAsync((void **)&v.dy, (yb.size() ? yb.size() : 1) * sizeof(double2), dc->stream));
+        CUN(cudaMallocAsync((void **)&v.dy, job->yb.size() * sizeof(double2), dc->stream));
         CUN(cudaMallocAsync((void **)&v.dcnt, (size_t)(ncnt + 1) * sizeof(unsigned long long), dc->stream));     /* + the suspect-point counter of the static kernels */
         if (full) CUN(cudaMallocAsync((void **)&v.ds, (size_t)v.n * nf * np_ * np_ * sizeof(double2), dc->stream));
         CUN(cudaMemcpyAsync(v.dprog, hp, sizeof(NodalProg), cudaMemcpyHostToDevice, dc->stream));
         CUN(cudaMemcpyAsync(v.dfr, f, (size_t)nf * sizeof(double), cudaMemcpyHostToDevice, dc->stream));
-        CUN(cudaMemcpyAsync(v.dmask, mask.data(), (size_t)nf, cudaMemcpyHostToDevice, dc->stream));
-        if (!yb.empty()) CUN(cudaMemcpyAsync(v.dy, yb.data(), yb.size() * sizeof(double2), cudaMemcpyHostToDevice, dc->stream));
+        CUN(cudaMemcpyAsync(v.dmask, job->mask.data(), (size_t)nf, cudaMemcpyHostToDevice, dc->stream));
+        CUN(cudaMemcpyAsync(v.dy, job->yb.data(), job->yb.size() * sizeof(double2), cudaMemcpyHostToDevice, dc->stream));
         /* persistent grid = exactly the resident blocks (a larger grid runs in 1.6 waves: 4.0e8 instead of 4.4e8
          * points/s on the reference network); latency hiding matters more here than the private arrays' L2 footprint */
         int bps = 0;
-        { const char *e = getenv("QO100NET_NODAL_BPS"); if (e && atoi(e) > 0) bps = atoi(e); }
-        if (bps == 0 && jit) {
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, (const void *)jit->kern, QN_TPB, 0) != cudaSuccess || bps <= 0) {
+        if (jit) {
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, QN_TPB, 0) != cudaSuccess || bps <= 0) {
                 cudaGetLastError();
                 bps = jit->regs > 0 ? 65536 / (((jit->regs + 7) & ~7) * QN_TPB) : 4;
                 if (bps > 16) bps = 16;
             }
-        }
-        if (bps == 0) {
-            if (use_static) {
-                const int nnz = spv[0].nnz;
-                if (nnz <= 64) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, qo_nodal_kernel<32, 1, 64>, QN_TPB, 0);
-                else if (nnz <= 128) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, qo_nodal_kernel<32, 1, 128>, QN_TPB, 0);
-                else if (nnz <= 256) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, qo_nodal_kernel<32, 1, 256>, QN_TPB, 0);
-                else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, qo_nodal_kernel<32, 1, QN_NNZ_MAX>, QN_TPB, 0);
-            }
-            if (bps <= 0) bps = 8;
-        }
+        } else if (use_static) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, kern, QN_TPB, 0);
+        if (bps <= 0) bps = 8;
         const unsigned long long units = v.n * (unsigned long long)nchunks;
         const unsigned long long cap = (unsigned long long)dc->sm_count * (unsigned long long)bps;
         v.grid = (int)(units < cap ? units : cap);
     }
-  relaunch:
-    for (int g = 0; g < G; g++) {
-        DevCtx *dc = &ctx->d[g];
-        NodalDev &v = nv[g];
-        const int grid = v.grid;
-        const unsigned long long off_g = cfg->sample_offset + v.off;
-        CUN(cudaSetDevice(dc->device));
-        CUN(cudaMemsetAsync(v.dcnt, 0, (size_t)(ncnt + 1) * sizeof(unsigned long long), dc->stream));
-        cudaEventRecord(dc->ev0, dc->stream);
-#define QN_LAUNCH(LDV, MD, NZ, SM) qo_nodal_kernel<LDV, MD, NZ><<<grid, QN_TPB, SM, dc->stream>>>(v.dprog, v.dsp, v.dfr, v.dmask, v.dy, nf, chunk_len, nchunks, off_g, v.n, v.dcnt, v.ds, growth2)
-        g_last_kernel = use_static ? "qo_nodal_kernel<static,local>" : "qo_nodal_kernel<dense>";
-        if (use_static && jit) {
-            int nf_ = nf;
-            unsigned long long off_ = off_g, n_ = v.n;
-            void *args[] = { &v.dprog, &v.dfr, &v.dmask, &v.dy, &nf_, &chunk_len, &nchunks, &off_, &n_, &v.dcnt, &v.ds, &growth2 };
-            CUN(cudaLaunchKernel((const void *)jit->kern, dim3((unsigned)grid), dim3(QN_TPB), args, 0, dc->stream));
-            g_last_kernel = "qo_nodal_jit_kernel";
-        } else if (use_static) {
-            const int nnz = spv[0].nnz;
-            const size_t smem = (size_t)nnz * QN_TPB * sizeof(double2);
-            const char *loc = getenv("QO100NET_NODAL_VALUES");
-            /* shared-memory values: no DRAM traffic at all, but 1 KB per value per block leaves one 64-thread block
-             * per SM for the reference network (123 values) -- measured 2.0e8 points/s against 3.9e8 with private
-             * arrays, so it is opt-in (QO100NET_NODAL_VALUES=smem) */
-            if (smem <= 160 * 1024 && loc && !strcmp(loc, "smem")) {
-                CUN(cudaFuncSetAttribute(qo_nodal_kernel<32, 2, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                QN_LAUNCH(32, 2, 1, smem);
-                g_last_kernel = "qo_nodal_kernel<static,smem>";
-            } else if (nnz <= 64) QN_LAUNCH(32, 1, 64, 0);
-            else if (nnz <= 128) QN_LAUNCH(32, 1, 128, 0);
-            else if (nnz <= 256) QN_LAUNCH(32, 1, 256, 0);
-            else QN_LAUNCH(32, 1, QN_NNZ_MAX, 0);
-        } else if (n_unk <= 8) QN_LAUNCH(8, 0, 1, 0);
-        else if (n_unk <= 16) QN_LAUNCH(16, 0, 1, 0);
-        else if (n_unk <= 24) QN_LAUNCH(24, 0, 1, 0);
-        else QN_LAUNCH(32, 0, 1, 0);
-#undef QN_LAUNCH
-        cudaEventRecord(dc->ev1, dc->stream);
-        CUN(cudaGetLastError());
-    }
-    for (size_t i = 0; i < h.size(); i++) h[i] = 0ull;
-    ms_max = 0.0f;
-    for (int g = 0; g < G; g++) {
-        DevCtx *dc = &ctx->d[g];
-        CUN(cudaSetDevice(dc->device));
-        CUN(cudaStreamSynchronize(dc->stream));
-        CUN(cudaMemcpy(hg.data(), nv[g].dcnt, (size_t)(ncnt + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-        for (size_t i = 0; i < h.size(); i++) h[i] += hg[i];
-        float ms = 0;
-        cudaEventElapsedTime(&ms, dc->ev0, dc->ev1);
-        if (ms > ms_max) ms_max = ms;
-    }
-    if (use_static && h[ncnt] != 0) {
-        /* some (sample, frequency) point met a multiplier above QN_GROWTH2 (or a NaN) under the fixed pivot order: the whole
-         * job is redone with per-point partial pivoting */
-        if (force && !strcmp(force, "static")) { qo_set_error("QO100NET_NODAL=static: %llu points needed another pivot order", h[ncnt]); rc = QO_ERR_UNSUPPORTED; goto out; }
+    /* some (sample, frequency) point met a multiplier above the guard (or a NaN) under the static plan's fixed pivot order: the
+     * whole job is redone once with per-point partial pivoting, on the grid computed above */
+    for (int attempt = 0; attempt < 2; attempt++) {
+        g_last_kernel = jit ? "qo_nodal_jit_kernel" : use_static ? "qo_nodal_kernel<static,local>" : "qo_nodal_kernel<dense>";
+        for (int g = 0; g < G; g++) {
+            DevCtx *dc = &ctx->d[g];
+            NodalDev &v = nv[g];
+            unsigned long long off_g = cfg->sample_offset + v.off;
+            void *args[] = { &v.dprog, &v.dsp, &v.dfr, &v.dmask, &v.dy, &nf, &chunk_len, &nchunks, &off_g, &v.n, &v.dcnt, &v.ds, &growth2 };
+            void *args_jit[] = { &v.dprog, &v.dfr, &v.dmask, &v.dy, &nf, &chunk_len, &nchunks, &off_g, &v.n, &v.dcnt, &v.ds, &growth2 };   /* the plan is compiled in */
+            CUN(cudaSetDevice(dc->device));
+            CUN(cudaMemsetAsync(v.dcnt, 0, (size_t)(ncnt + 1) * sizeof(unsigned long long), dc->stream));
+            cudaEventRecord(dc->ev0, dc->stream);
+            CUN(cudaLaunchKernel(kern, dim3((unsigned)v.grid), dim3(QN_TPB), jit ? args_jit : args, 0, dc->stream));
+            cudaEventRecord(dc->ev1, dc->stream);
+            CUN(cudaGetLastError());
+        }
+        for (size_t i = 0; i < h.size(); i++) h[i] = 0ull;
+        ms_max = 0.0f;
+        for (int g = 0; g < G; g++) {
+            DevCtx *dc = &ctx->d[g];
+            CUN(cudaSetDevice(dc->device));
+            CUN(cudaStreamSynchronize(dc->stream));
+            CUN(cudaMemcpy(hg.data(), nv[g].dcnt, (size_t)(ncnt + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+            for (size_t i = 0; i < h.size(); i++) h[i] += hg[i];
+            float ms = 0;
+            cudaEventElapsedTime(&ms, dc->ev0, dc->ev1);
+            if (ms > ms_max) ms_max = ms;
+        }
+        if (!use_static || h[ncnt] == 0) break;
+        if (ov.kernel == QoNodalOverrides::STATIC) { qo_set_error("QO100NET_NODAL=static: %llu points needed another pivot order", h[ncnt]); rc = QO_ERR_UNSUPPORTED; goto out; }
         if (getenv("QO100NET_NODAL_DEBUG")) fprintf(stderr, "qo_nodal: %llu suspect points under the static plan, re-running on the dense kernel\n", h[ncnt]);
         use_static = false;
-        goto relaunch;
+        jit = NULL;
+        kern = nodal_kernel(false, 0, hp->n_unk);
     }
     if (full)
         for (int g = 0; g < G; g++) {
@@ -991,6 +972,7 @@ static int nodal_run(qo_ctx *ctx, const qo_nodal *nd, const double *f, int nf, c
             CUN(cudaMemcpy(full_s_host + (size_t)nv[g].off * nf * np_ * np_, nv[g].ds, (size_t)nv[g].n * nf * np_ * np_ * sizeof(double2), cudaMemcpyDeviceToHost));
         }
     if (res) {
+        const int n_unk = hp->n_unk;
         res->n_pass = full ? 0 : h[0];
         res->n_total = full ? N : h[1];
         if (res->fail_per_spec) for (int s = 0; s < nspec; s++) res->fail_per_spec[s] = h[2 + s];

@@ -1,10 +1,12 @@
 /*
- * qo_overrides.h -- the QO100NET_* environment overrides of the cascade (two-port) path, read in one place.
+ * qo_overrides.h -- the QO100NET_* environment overrides of the cascade (two-port) path and of the nodal (N-port) path, each
+ * read in one place.
  *
- * qo_plan_create reads them once and keeps the record in the plan; everything that chooses a kernel reads the record, never
- * the environment.  qo_mc_run keys its plan cache, and qo_tf_plan_check its analysis cache, on the record's bytes, so a new
- * override changes both keys without a list of names to keep in step.  Diagnostics and I/O switches (QO100NET_CHAIN_DEBUG,
- * _CHAIN_JIT_DUMP, _CACHE_DIR, _NVRTC, _MC_TIMING, _NO_PLAN_CACHE) are read where they act; the nodal path has its own.
+ * qo_plan_create reads the cascade overrides once and keeps the record in the plan; everything that chooses a kernel reads the
+ * record, never the environment.  qo_mc_run keys its plan cache, and qo_tf_plan_check its analysis cache, on the record's bytes,
+ * so a new override changes both keys without a list of names to keep in step.  Every nodal entry point reads the nodal record
+ * once per call.  Diagnostics and I/O switches (QO100NET_CHAIN_DEBUG, _CHAIN_JIT_DUMP, _NODAL_DEBUG, _NODAL_JIT_DUMP,
+ * _CACHE_DIR, _NVRTC, _MC_TIMING, _NO_PLAN_CACHE) are read where they act.
  */
 #pragma once
 #include <stdlib.h>
@@ -42,5 +44,25 @@ static inline int qo_overrides_read(QoOverrides *ov)
     ov->cpl_sincos = getenv("QO100NET_CPL_SINCOS") != NULL;
     const char *u = getenv("QO100NET_USTRIP");
     ov->ustrip_item = u && !strcmp(u, "item");
+    return QO_OK;
+}
+
+struct QoNodalOverrides {
+    enum Kernel { AUTO, DENSE, STATIC, JIT } kernel;      /* QO100NET_NODAL */
+    double growth2;       /* QO100NET_NODAL_GUARD2 above 0: the device's multiplier guard in place of QN_GROWTH2; else 0 */
+};
+
+/* QO_ERR_ARG (qo_last_error names the accepted values) when QO100NET_NODAL holds anything but auto, dense, static, jit */
+static inline int qo_nodal_overrides_read(QoNodalOverrides *ov)
+{
+    memset(ov, 0, sizeof *ov);
+    const char *k = getenv("QO100NET_NODAL");
+    if (!k || !*k || !strcmp(k, "auto")) ov->kernel = QoNodalOverrides::AUTO;
+    else if (!strcmp(k, "dense")) ov->kernel = QoNodalOverrides::DENSE;
+    else if (!strcmp(k, "static")) ov->kernel = QoNodalOverrides::STATIC;
+    else if (!strcmp(k, "jit")) ov->kernel = QoNodalOverrides::JIT;
+    else { qo_set_error("QO100NET_NODAL=%s: expected auto, dense, static or jit", k); return QO_ERR_ARG; }
+    const char *g = getenv("QO100NET_NODAL_GUARD2");      /* tests: trip the device guard on purpose */
+    if (g && atof(g) > 0.0) ov->growth2 = atof(g);
     return QO_OK;
 }
