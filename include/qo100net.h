@@ -307,14 +307,16 @@ int qo_chain_jit_analyze(const qo_net *net, const double *f, int nf, const qo_sp
  * [2] = denominator form (0 none, 1 truncated |D|^2 polynomial, 2 complex D, 3 D and dD/ds for group-delay jobs), [3] = coefficient pairs kept per numerator
  * polynomial, [4] = denominator coefficients (form 1) / pairs (form 2) kept, [5] = structural degree;
  * *self_check_err = worst relative disagreement on |den|^2 between the expansion and the per-element evaluation
- * (nominal network + both ends of the tolerance box, every in-band grid point).  Returns the reason string
- * ("ok", or why the job stays on the chain kernels). */
-const char *qo_plan_tf_info(const qo_plan *plan, int info[6], double *self_check_err);
+ * (nominal network + both ends of the tolerance box, every in-band grid point); *fused = bit mask of the specs whose
+ * single-spec stretches of the grid the thread-per-sample kernel walks on one fused margin polynomial, *fused_err = the worst
+ * disagreement of that margin with the unfused one, relative to |den|^2 (0 when no spec is fused).  Any output pointer may be
+ * NULL.  Returns the reason string ("ok", or why the job stays on the chain kernels). */
+const char *qo_plan_tf_info(const qo_plan *plan, int info[6], double *self_check_err, unsigned int *fused, double *fused_err);
 /* the host-only part of qo_plan_create (network -> program, transfer-function analysis): needs no GPU.  Same outputs as
  * qo_plan_tf_info; *seconds = host time the analysis took.  An environment override qo_plan_create would refuse (an unknown
  * QO100NET_KERNEL value): info[0] = QO_ERR_ARG and the reason string says why. */
 const char *qo_plan_analyze(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
-                            int info[6], double *self_check_err, double *seconds);
+                            int info[6], double *self_check_err, unsigned int *fused, double *fused_err, double *seconds);
 /* host->device bytes qo_plan_create copied for this plan (tables, masks, program), per GPU */
 uint64_t qo_plan_h2d_bytes(const qo_plan *plan);
 void qo_plan_destroy(qo_plan *plan);

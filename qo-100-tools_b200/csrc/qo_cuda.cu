@@ -88,9 +88,9 @@ struct qo_plan {
     QoOverrides ov;                                       /* the environment overrides as they were at plan creation */
     QoKern kern;
     /* launch-time decisions of the transfer-function kernels, taken once at plan creation */
-    int tf_cpl_matched, tf_cpl_lin, ts_ok, ts_runs_ok, ts_nruns, ts_npt;
+    int tf_cpl_matched, tf_cpl_lin, ts_ok, ts_runs_ok, ts_nruns, ts_nplain, ts_npt;
     double tf_cpl_dw1;                                    /* angular-frequency step of one grid point on a uniformly spaced grid */
-    struct { int ngroups; unsigned int any, all; } ts_runs[QO_TS_MAXRUN];
+    struct { int g0, ngroups; unsigned int any, all; } ts_runs[QO_TS_MAXRUN];
     int lad_n, lad_first, lad_cpl;                        /* straight-line ladder kernel (qo_ladder.cuh) */
     int cpl_fast, cpl_same;                               /* coupler block: small-angle table path, equal mode angles */
     int spot_el0, spot_nel;                               /* spot-frequency kernel (qo_spot.cuh): <= 8 points per sample */
@@ -753,18 +753,20 @@ extern "C" int qo_chain_jit_analyze(const qo_net *net, const double *f, int nf, 
 }
 
 extern "C" const char *qo_plan_kernel_name(const qo_plan *p) { return p ? p->kernel_name : ""; }
-extern "C" const char *qo_plan_tf_info(const qo_plan *p, int info[6], double *self_check_err)
+extern "C" const char *qo_plan_tf_info(const qo_plan *p, int info[6], double *self_check_err, unsigned int *fused, double *fused_err)
 {
     if (!p) return "";
     if (info) { info[0] = p->kern == K_TF; info[1] = p->tfp.nn; info[2] = p->tfp.den; info[3] = p->tfp.kn; info[4] = p->tfp.kd; info[5] = p->tfp.deg; }
     if (self_check_err) *self_check_err = p->tfp.err;
+    if (fused) *fused = p->tfp.fused;
+    if (fused_err) *fused_err = p->tfp.fused_err;
     return p->tfp.reason ? p->tfp.reason : "";
 }
 extern "C" uint64_t qo_plan_h2d_bytes(const qo_plan *p) { return p ? p->h2d_bytes : 0; }
 
 /* host-only part of qo_plan_create: compile the network, decide about the transfer-function kernel (needs no GPU) */
 extern "C" const char *qo_plan_analyze(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
-                                       int info[6], double *self_check_err, double *seconds)
+                                       int info[6], double *self_check_err, unsigned int *fused, double *fused_err, double *seconds)
 {
     qo_clear_error();
     if (!net || !f || nf <= 0 || !info) return "bad arguments";
@@ -786,6 +788,8 @@ extern "C" const char *qo_plan_analyze(const qo_net *net, const double *f, int n
         int sel = qo_tf_plan_check(hp, mode == QO_MODE_REDUCE_ONLY, precision, generic, f, nf, maskv.data(), &ov, &tp);
         info[0] = sel; info[1] = tp.nn; info[2] = tp.den; info[3] = tp.kn; info[4] = tp.kd; info[5] = tp.deg;
         if (self_check_err) *self_check_err = tp.err;
+        if (fused) *fused = tp.fused;
+        if (fused_err) *fused_err = tp.fused_err;
         reason = tp.reason ? tp.reason : "";
     }
     clock_gettime(CLOCK_MONOTONIC, &t1);
@@ -947,7 +951,7 @@ static void tf_launch_setup(qo_plan *p, const QoOverrides *ov)
     }
     const bool rot_same = p->tf_cpl_lin && p->tf_cpl_matched && p->cpl_same && hp->cplms_elem < 0;
     p->ts_ok = ov->kernel != QoOverrides::TF && qo_ts_eligible(&p->tfp, hp->nspec, rot_same);     /* KERNEL=tf: warp-per-sample only (A/B runs) */
-    p->ts_nruns = 0; p->ts_runs_ok = 1; p->ts_npt = 0;
+    p->ts_nruns = 0; p->ts_nplain = 0; p->ts_runs_ok = 1; p->ts_npt = 0;
     if (p->ts_ok) {
         const int gpt = qo_ts_group_points(&p->tfp);
         p->ts_npt = (p->nf + gpt - 1) / gpt * gpt;
@@ -956,8 +960,26 @@ static void tf_launch_setup(qo_plan *p, const QoOverrides *ov)
             for (int k = gi * gpt; k < (gi + 1) * gpt; k++) { const unsigned int mk = k < p->nf ? p->maskv[k] : 0; any |= mk; all &= mk; }
             if (p->ts_nruns > 0 && any == all && p->ts_runs[p->ts_nruns - 1].any == any && p->ts_runs[p->ts_nruns - 1].all == all) { p->ts_runs[p->ts_nruns - 1].ngroups++; continue; }
             if (p->ts_nruns == QO_TS_MAXRUN) { p->ts_runs_ok = 0; break; }       /* more band edges than the run table holds: warp-per-sample */
-            p->ts_runs[p->ts_nruns].ngroups = 1; p->ts_runs[p->ts_nruns].any = any; p->ts_runs[p->ts_nruns].all = all; p->ts_nruns++;
+            p->ts_runs[p->ts_nruns].g0 = gi; p->ts_runs[p->ts_nruns].ngroups = 1; p->ts_runs[p->ts_nruns].any = any; p->ts_runs[p->ts_nruns].all = all; p->ts_nruns++;
         }
+        /* the runs of the fused spec (one spec active, its margin a single polynomial: qo_tf_fuse) go last -- the verdict does
+         * not depend on the order, and the kernel forms the polynomial once, after the other runs, in the registers of the
+         * expansion.  One polynomial per sample: of the specs the plan accepts for it, the one that covers the most groups */
+        auto one_spec = [&](int r) -> int {
+            const unsigned int all = p->ts_runs[r].all;
+            if (p->tfp.cpl_op >= 0 || p->ts_runs[r].any != all || all == 0u || (all & (all - 1u))) return -1;
+            const int s = __builtin_ctz(all);
+            return (p->tfp.fused >> s) & 1u ? s : -1;
+        };
+        int ng[QO_TF_NSPEC] = { 0 }, fs = -1;
+        for (int r = 0; r < p->ts_nruns; r++) if (one_spec(r) >= 0) ng[one_spec(r)] += p->ts_runs[r].ngroups;
+        for (int s = 0; s < QO_TF_NSPEC; s++) if (ng[s] > 0 && (fs < 0 || ng[s] > ng[fs])) fs = s;
+        decltype(p->ts_runs) sorted;
+        int n = 0;
+        for (int r = 0; r < p->ts_nruns; r++) if (fs < 0 || one_spec(r) != fs) sorted[n++] = p->ts_runs[r];
+        p->ts_nplain = n;
+        for (int r = 0; r < p->ts_nruns; r++) if (fs >= 0 && one_spec(r) == fs) sorted[n++] = p->ts_runs[r];
+        memcpy(p->ts_runs, sorted, sizeof sorted);
     }
 }
 
@@ -1005,8 +1027,10 @@ static int launch_tf(qo_plan *p, int g, unsigned long long off, unsigned long lo
             Q.t.nsamples = nb * 32ull;
             Q.y1 = (const double *)d->tf_yt; Q.x1 = (const double *)d->tf_xt; Q.mw = (const uint2 *)d->tf_mb;
             Q.npt = p->ts_npt;
-            Q.nruns = p->ts_nruns;
-            for (int r = 0; r < p->ts_nruns; r++) { Q.runs[r].ngroups = p->ts_runs[r].ngroups; Q.runs[r].any = p->ts_runs[r].any; Q.runs[r].all = p->ts_runs[r].all; }
+            Q.nruns = p->ts_nruns; Q.nplain = p->ts_nplain;
+            for (int r = 0; r < p->ts_nruns; r++) {
+                Q.runs[r].g0 = p->ts_runs[r].g0; Q.runs[r].ngroups = p->ts_runs[r].ngroups; Q.runs[r].any = p->ts_runs[r].any; Q.runs[r].all = p->ts_runs[r].all;
+            }
             Q.nbatches = nb;
             Q.ticket = d->ticket + 1;
             Q.w0 = 6.283185307179586476925286766559 * p->f[0];

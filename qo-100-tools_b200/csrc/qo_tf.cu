@@ -161,6 +161,53 @@ struct TfCorner {
 static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int precision, int generic, const double *f, int nf,
                                   const unsigned char *mask, const QoOverrides *ov, TfPlan *out);
 
+/* Fused margins (qo_tf_fuse) for the thread-per-sample kernel.  A |S21| spec other than the histogram's is fused when, at every
+ * corner of the analysis and every grid point where it is the only spec that looks, the host twin of the device's F (same
+ * coefficients, same formation, same Horner) stays within QO_TF_FUSE_TOL of |den|^2 of the unfused margin N2 - t E evaluated
+ * from the same truncated polynomials in long double.  A stop band passes easily (~1e-13); the pass band of a ripple filter
+ * usually does not, |Num|^2 cancelling inside the ripple (~1e-11). */
+#define QO_TF_FUSE_TOL 1e-12
+static void tf_fuse_gate(const DevProg *hp, int nf, const double *xg, const unsigned char *mask, const std::vector<TfCorner> &cs,
+                         double zni, TfPlan *out)
+{
+    out->fused = 0; out->fused_err = 0.0;
+    if (out->cpl_op >= 0 || !qo_ts_eligible(out, hp->nspec, 0)) return;
+    const int kn = out->kn, ke = out->den == QO_TF_DEN_E ? out->kd : 0, nfz = 2 * kn > ke ? 2 * kn : ke;
+    const double zq0 = hp->rs * zni;
+    for (int s = 0; s < hp->nspec; s++) {
+        if (hp->spec_kind[s] != SK_DEN2_MAX && hp->spec_kind[s] != SK_DEN2_MIN) continue;
+        if (hp->hist_bins > 0 && hp->hist_spec == s) continue;
+        const bool neg = hp->spec_kind[s] == SK_DEN2_MIN;
+        const double t = hp->spec_thr[s];
+        double worst = 0.0;
+        int npts = 0;
+        for (size_t ci = 0; ci < cs.size(); ci++) {
+            double cn[2 * QO_TF_MAXK], fz[2 * QO_TF_MAXK + QO_TF_MAXKE];
+            for (int i = 0; i < 2 * kn; i++) cn[i] = fma(zq0, cs[ci].qq[i], cs[ci].pp[i]);      /* the device's numerator pairs */
+            qo_tf_fuse(kn, ke, cn, cs[ci].ee, t, neg, fz);
+            for (int k = 0; k < nf; k++) {
+                if (mask[k] != 1u << s) continue;
+                npts++;
+                const double x = xg[k], y = -(x * x);
+                double got = fz[nfz - 1];
+                for (int m = nfz - 2; m >= 0; m--) got = fma(got, y, fz[m]);
+                const long double yl = y;
+                long double r0 = cn[2 * kn - 2], r1 = cn[2 * kn - 1], e = ke > 0 ? cs[ci].ee[ke - 1] : 1.0;
+                for (int i = kn - 2; i >= 0; i--) { r0 = r0 * yl + cn[2 * i]; r1 = r1 * yl + cn[2 * i + 1]; }
+                for (int m = ke - 2; m >= 0; m--) e = e * yl + cs[ci].ee[m];
+                const long double n2 = r0 * r0 - yl * r1 * r1, ref = neg ? n2 - t * e : t * e - n2;
+                double err = (double)(fabsl((long double)got - ref) / n2);
+                if (!(err == err)) err = 1e300;
+                if (err > worst) worst = err;
+            }
+        }
+        if (npts > 0 && worst <= QO_TF_FUSE_TOL) {
+            out->fused |= 1u << s;
+            if (worst > out->fused_err) out->fused_err = worst;
+        }
+    }
+}
+
 /* Where in the tolerance box the analysis looks (x[v] in [-1, 1] per random variable):
  *   0 every variable at -1, 1 the nominal network, 2 every variable at +1,
  *   3 every variable at the end that RAISES the parameters it drives (lowest self-resonances: L, C up whatever the sign of
@@ -212,10 +259,13 @@ extern "C" int qo_tf_plan_check(const DevProg *hp, int mode_reduce_only, int pre
     if (generic || !mode_reduce_only || precision != 64) return tf_plan_check_uncached(hp, mode_reduce_only, precision, generic, f, nf, mask, ov, out);
     unsigned long long key = 1469598103934665603ull;
     {
-        /* what the analysis does not read must not split the cache: seed, distribution, histogram set-up, thresholds */
+        /* what the analysis does not read must not split the cache: seed, distribution, histogram range, user limits (the
+         * fused-margin gate reads the canonical thresholds and which spec the histogram tracks) */
         DevProg *k = new DevProg(*hp);
-        k->seed = 0; k->dist = 0; k->hist_spec = k->hist_bins = 0; k->hist_lo = k->hist_hi = 0.0;
-        for (int s = 0; s < QO_NSPEC_MAX; s++) { k->spec_thr[s] = 0.0; k->spec_limit[s] = 0.0; }
+        k->seed = 0; k->dist = 0; k->hist_lo = k->hist_hi = 0.0;
+        if (k->hist_bins <= 0) k->hist_spec = k->hist_bins = 0;
+        else k->hist_bins = 1;
+        for (int s = 0; s < QO_NSPEC_MAX; s++) k->spec_limit[s] = 0.0;
         key = tf_fnv(key, k, sizeof *k);
         delete k;
     }
@@ -462,6 +512,7 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
     }
     out->err = worst;
     if (!accepted) QO_TF_NO("polynomial expansion is too ill-conditioned on this grid");
+    tf_fuse_gate(hp, nf, xg.data(), mask, cs, zni, out);
     out->reason = "ok";
     return 1;
 #undef QO_TF_NO

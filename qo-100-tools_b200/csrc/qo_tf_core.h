@@ -49,6 +49,52 @@ QO_TF_HD int qo_tf_element(int opcode, const double *p, double wr, double *nd)
     }
 }
 
+/* Fused margin of one |S21| spec on a plain ladder (thread-per-sample kernel, qo_ts.cuh; its plan-time gate, qo_tf.cu):
+ *     F(y) = N2(y) - t E(y)   (P.neg: fail where |den|^2 < t)      or      t E(y) - N2(y)   (fail where |den|^2 > t),
+ * N2 = r0^2 - y r1^2 with r0 = sum_i cn[2i] y^i, r1 = sum_i cn[2i+1] y^i (kn pairs), E = sum_m ce[m] y^m (ke coefficients,
+ * ke = 0: E = 1).  The sign of F is the verdict at a point, and F is one polynomial of max(2 kn, ke) coefficients.
+ * Each coefficient is summed in double-double -- error-free products (fma(a, b, -a b)) and sums (two-sum), the low parts in
+ * plain double -- and rounded once, so that it carries about one rounding whatever the cancellation between its terms.
+ * Host and device run exactly this operation order (the products cannot be contracted: __dmul_rn on the device,
+ * -ffp-contract=off on the host).  A zero F(0) coefficient is +0, so that F(y) is never -0 (an exact zero passes). */
+QO_TF_HD double qo_tf_mul_rn(double a, double b)
+{
+#ifdef __CUDA_ARCH__
+    return __dmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+/* (s, c) += a b */
+QO_TF_HD void qo_tf_dd_fma(double &s, double &c, double a, double b)
+{
+    const double p = qo_tf_mul_rn(a, b), pe = fma(a, b, -p);
+    const double t = s + p, bp = t - s;
+    c += ((s - (t - bp)) + (p - bp)) + pe;
+    s = t;
+}
+QO_TF_HD void qo_tf_fuse(int kn, int ke, const double *cn, const double *ce, double t, bool neg, double *f)
+{
+    const int nf = 2 * kn > ke ? 2 * kn : ke;
+#pragma unroll
+    for (int k = 0; k < nf; k++) {
+        double s = 0.0, c = 0.0;
+#pragma unroll
+        for (int i = 0; i < kn; i++) {                        /* r0^2: a_i a_j (i + j = k), the off-diagonal pairs once, doubled */
+            const int j = k - i;
+            if (j >= i && j < kn) qo_tf_dd_fma(s, c, i == j ? cn[2 * i] : 2.0 * cn[2 * i], cn[2 * j]);
+        }
+#pragma unroll
+        for (int i = 0; i < kn; i++) {                        /* - y r1^2: b_i b_j (i + j = k - 1) */
+            const int j = k - 1 - i;
+            if (j >= i && j < kn) qo_tf_dd_fma(s, c, i == j ? -cn[2 * i + 1] : -2.0 * cn[2 * i + 1], cn[2 * j + 1]);
+        }
+        if (k < (ke > 0 ? ke : 1)) qo_tf_dd_fma(s, c, -t, ke > 0 ? ce[k] : 1.0);
+        const double v = s + c;
+        f[k] = (neg ? v : -v) + 0.0;
+    }
+}
+
 /* structural degree an element adds to the polynomials (max(deg N, deg D)); 0 = resistor, -1 = not lumped */
 static inline int qo_tf_degree(int opcode)
 {

@@ -17,6 +17,8 @@ struct TfPlan {
     int front;           /* what that block is: 0 coupled-line section, 1 transmission line (OP_TLINE), 2 measured two-port (OP_SBLOCK) */
     double wref;         /* normalising angular frequency (geometric centre of the grid) */
     double err;          /* worst relative disagreement on |den|^2 seen by the self-check */
+    unsigned int fused;  /* specs whose single-spec runs the thread-per-sample kernel walks on the fused margin (qo_tf_fuse) */
+    double fused_err;    /* worst disagreement of the fused margin with the unfused one, relative to |den|^2 (over every spec tried) */
     const char *reason;  /* "ok", or why the job stays on the chain kernels */
 };
 /* Can this job run on the transfer-function kernel?  Structural test, choice of the polynomial lengths the grid needs,

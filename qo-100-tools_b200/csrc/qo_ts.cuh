@@ -21,7 +21,13 @@
  *            the whole warp (a broadcast load per group of points, nothing per Horner step), every DFMA takes its coefficient
  *            from a register, the per-spec sign accumulators / the histogram tracker are thread-private: no shuffles, no
  *            shared memory, no warp reduction inside or after the loop.  The grid is walked as a few runs of groups that see
- *            the same spec bits, so the bookkeeping branches on loop-invariant warp-uniform predicates;
+ *            the same spec bits, so the bookkeeping branches on loop-invariant warp-uniform predicates.  Where one |S21| spec
+ *            alone looks (a stop band) only the sign of its margin N2 - t E matters, and that is one polynomial in y of
+ *            max(2 KN, KE) coefficients: the plan accepts it per spec where it stays within 1e-12 of |den|^2 of the unfused
+ *            margin (qo_tf.cu::tf_fuse_gate -- a stop band does, a ripple pass band usually not) and puts that spec's runs
+ *            last; after the other runs the thread forms the polynomial once in double-double (qo_tf_core.h::qo_tf_fuse, in the
+ *            registers of the expansion, which are dead by then) and walks the runs with one Horner chain per point:
+ *            2 KN - 1 or KE - 1 DFMA per point instead of 2 (KN - 1) + (KE - 1) + 4 (cfg2: 17 instead of 33);
  *   stage D  verdict per thread, counters by warp ballots, the histogram value (a log10) at full lane efficiency.
  *
  * Stage A costs ~4 500 instructions per sample against ~180 000 for the loop (the warp-cooperative expansion of qo_tf.cuh:
@@ -40,6 +46,8 @@
 #define QO_TS_PT2 4
 #define QO_TS_MINB2 3
 #define QO_TS_PT4 2
+#define QO_TS_FG2 3              /* fused runs of plain ladders (one Horner chain per point): groups walked at once -- 12 points in flight;
+                                    cfg2 on a B200 at its 1000 W limit: 4 points 4.97e11 evals/s, 8 points 5.32e11, 12 points 5.41e11, 16 points 5.40e11 */
 #define QO_TS_MINB4 3
 #define QO_TS_CAPN2 10           /* plain ladders (NN = 2): numerator coefficient pairs held in registers */
 #define QO_TS_CAPE2 16           /* ... and E coefficients */
@@ -53,8 +61,10 @@ struct TsParams {
     TfParams t;                          /* the job, exactly as qo_mc_tf_kernel takes it */
     const double *y1, *x1;               /* per POINT: -(w/wref)^2 and w/wref (the same tables, read as scalars) */
     const uint2 *mw;                     /* per point: byte masks of specs 0-3 (x) and 4-7 (y) */
-    struct { int ngroups; unsigned int any, all; } runs[QO_TS_MAXRUN];      /* runs of groups (PT points each) that see the same spec bits */
+    struct { int g0, ngroups; unsigned int any, all; } runs[QO_TS_MAXRUN];  /* runs of groups (PT points each) that see the same spec bits */
     int nruns;
+    int nplain;                          /* runs[0, nplain): walked on |numerator|^2 and E; runs[nplain, nruns): the runs of the one
+                                            fused spec (walked on its margin polynomial, qo_tf_fuse) */
     int npt;                             /* points to walk: the grid rounded up to a whole group (padding carries no spec bit) */
     unsigned long long nbatches;         /* 32-sample batches, handed to the warps through a ticket counter */
     unsigned long long *ticket;          /* zeroed per launch */
@@ -187,8 +197,13 @@ __device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sa
                                             looks, and beyond the last band it may well go negative (found by tools/fuzz_parity.py: it
                                             used to fail spec 0 on such samples) */
     int gi = 0;
-    for (int rn = 0; rn < Q.nruns; rn++) {
+    for (int rn = 0; rn < Q.nplain; rn++) {
         const unsigned int any = Q.runs[rn].any, all = Q.runs[rn].all;
+        if (Q.runs[rn].g0 != gi) {       /* a fused run was taken out in front of this one: the preloaded grid values are not its */
+            gi = Q.runs[rn].g0;
+#pragma unroll
+            for (int h = 0; h < PT; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + gi * PT + h)); y[h] = a.x; y[h + 1] = a.y; }
+        }
         const int g_end = gi + Q.runs[rn].ngroups;
         const int one = (any == all && all != 0u && (all & (all - 1u)) == 0u) ? __ffs((int)all) - 1 : -1;
         if (any == 0u) {
@@ -227,6 +242,46 @@ __device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sa
     }
 #undef QO_TS_VALUE
 #undef QO_TS_CORE
+    /* the fused runs (plain ladders only): one spec active, its margin sg (N2 - t E) one polynomial of NF coefficients formed
+     * once per sample (qo_tf_fuse) -- one Horner chain per point instead of three chains, |.|^2 and the margin.  cn and ce are
+     * dead from here on: the polynomial takes their registers */
+    if constexpr (NN == 2) {
+        if (Q.nplain < Q.nruns) {                        /* none for most jobs */
+            constexpr int NF = 2 * KN > KE ? 2 * KN : KE;
+            const int one = __ffs((int)Q.runs[Q.nplain].all) - 1;
+            double fz[NF];
+            qo_tf_fuse(KN, KE, cn, ce, P.thr[one], P.neg[one], fz);
+            unsigned int a1 = 0u;
+            constexpr int PF = QO_TS_FG2 * PT;
+            double yf[PF];
+            for (int rn = Q.nplain; rn < Q.nruns; rn++) {
+                gi = Q.runs[rn].g0;
+                const int g_end = gi + Q.runs[rn].ngroups;
+#pragma unroll
+                for (int h = 0; h < PF; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + gi * PT + h)); yf[h] = a.x; yf[h + 1] = a.y; }
+                for (; gi + QO_TS_FG2 <= g_end; gi += QO_TS_FG2) {
+                    double F[PF];
+                    QO_PTS_N(PF) F[p] = fma(fz[NF - 1], yf[p], fz[NF - 2]);
+#pragma unroll
+                    for (int m = NF - 3; m >= 0; m--) { QO_PTS_N(PF) F[p] = fma(F[p], yf[p], fz[m]); }
+#pragma unroll
+                    for (int h = 0; h < PF; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + (gi + QO_TS_FG2) * PT + h)); yf[h] = a.x; yf[h + 1] = a.y; }
+                    QO_PTS_N(PF) a1 |= tf_hi(F[p]);
+                }
+                for (; gi < g_end; gi++) {                /* the run's last groups: yf[0, PT) holds the next one */
+                    double F[PT];
+                    QO_PTS_N(PT) F[p] = fma(fz[NF - 1], yf[p], fz[NF - 2]);
+#pragma unroll
+                    for (int m = NF - 3; m >= 0; m--) { QO_PTS_N(PT) F[p] = fma(F[p], yf[p], fz[m]); }
+#pragma unroll
+                    for (int h = 0; h < PT; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + (gi + 1) * PT + h)); yf[h] = a.x; yf[h + 1] = a.y; }
+                    QO_PTS_N(PT) a1 |= tf_hi(F[p]);
+                }
+            }
+#pragma unroll
+            for (int sp = 0; sp < NS; sp++) if (sp == one) acc[sp] |= a1;
+        }
+    }
     if (idle >> 31) acc[0] |= idle;      /* never taken (see above); keeps the unobserved points' arithmetic alive */
 }
 

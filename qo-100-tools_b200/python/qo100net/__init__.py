@@ -149,10 +149,10 @@ def lib():
         "qo_plan_flops_per_eval": (C.c_double, [vp]),
         "qo_plan_launches": (C.c_int, [vp]),
         "qo_plan_kernel_name": (C.c_char_p, [vp]),
-        "qo_plan_tf_info": (C.c_char_p, [vp, C.POINTER(C.c_int), C.POINTER(C.c_double)]),
+        "qo_plan_tf_info": (C.c_char_p, [vp, C.POINTER(C.c_int), C.POINTER(C.c_double), C.POINTER(C.c_uint), C.POINTER(C.c_double)]),
         "qo_plan_h2d_bytes": (C.c_uint64, [vp]),
         "qo_chain_jit_analyze": (C.c_int, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_int)]),
-        "qo_plan_analyze": (C.c_char_p, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_int), C.POINTER(C.c_double), C.POINTER(C.c_double)]),
+        "qo_plan_analyze": (C.c_char_p, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_int), C.POINTER(C.c_double), C.POINTER(C.c_uint), C.POINTER(C.c_double), C.POINTER(C.c_double)]),
         "qo_s2p_load": (C.c_int, [C.c_char_p, C.POINTER(vp)]),
         "qo_s2p_from_arrays": (C.c_int, [dp, C.c_int, vp, vp, vp, vp, C.c_double, C.POINTER(vp)]),
         "qo_s2p_num_points": (C.c_int, [vp]),
@@ -617,12 +617,14 @@ def plan_analyze(net, f, specs, tols=(), dist=DIST_UNIFORM, mode=MODE_REDUCE_ONL
     f = np.ascontiguousarray(f, dtype=np.float64)
     cfg = _cfg(0, 0, list(tols), 0, dist, mode, precision, hist_bins, hist_spec, hist_lo, hist_hi)
     info = (C.c_int * 6)()
-    err, sec = C.c_double(0.0), C.c_double(0.0)
-    reason = lib().qo_plan_analyze(net._h, _dp(f), len(f), _specs(specs), len(specs), C.byref(cfg), info, C.byref(err), C.byref(sec)).decode()
+    err, sec, fused, ferr = C.c_double(0.0), C.c_double(0.0), C.c_uint(0), C.c_double(0.0)
+    reason = lib().qo_plan_analyze(net._h, _dp(f), len(f), _specs(specs), len(specs), C.byref(cfg), info, C.byref(err),
+                                   C.byref(fused), C.byref(ferr), C.byref(sec)).decode()
     if info[0] < 0:
         raise QoError(info[0], reason)
     return dict(selected=bool(info[0]), numerator_chains=info[1], den_form=("none", "E", "D", "DD")[info[2]] if 0 <= info[2] <= 3 else "?",
-                kn=info[3], kd=info[4], degree=info[5], self_check_err=err.value, reason=reason, seconds=sec.value)
+                kn=info[3], kd=info[4], degree=info[5], self_check_err=err.value, fused_specs=fused.value, fused_err=ferr.value,
+                reason=reason, seconds=sec.value)
 
 
 def chain_jit_analyze(net, f, specs=(), tols=(), mode=MODE_REDUCE_ONLY, hist_bins=0, hist_spec=0, hist_lo=0.0, hist_hi=1.0):
@@ -681,10 +683,11 @@ class Plan:
     def tf_info(self):
         """The plan's decision about the transfer-function kernel (qo_plan_tf_info)."""
         info = (C.c_int * 6)()
-        err = C.c_double(0.0)
-        reason = lib().qo_plan_tf_info(self._h, info, C.byref(err)).decode()
+        err, fused, ferr = C.c_double(0.0), C.c_uint(0), C.c_double(0.0)
+        reason = lib().qo_plan_tf_info(self._h, info, C.byref(err), C.byref(fused), C.byref(ferr)).decode()
         return dict(selected=bool(info[0]), numerator_chains=info[1], den_form=("none", "E", "D", "DD")[info[2]] if 0 <= info[2] <= 3 else "?",
-                    kn=info[3], kd=info[4], degree=info[5], self_check_err=err.value, reason=reason)
+                    kn=info[3], kd=info[4], degree=info[5], self_check_err=err.value, fused_specs=fused.value, fused_err=ferr.value,
+                    reason=reason)
 
     @property
     def h2d_bytes(self):
