@@ -807,6 +807,7 @@ def test_differential_fuzz_of_the_monte_carlo_kernels(monkeypatch):
     assert out["mismatches"] == 0, out["details"]
     assert out["compared"] >= 70 and out["oracle_checked"] >= 10
     assert {"qo_mc_tf_kernel", "qo_mc_ts_kernel", "qo_mc_spot_kernel"} <= set(out["kernels_selected"])
+    assert out["fused_runs"] >= 1                  # the batch still reaches the thread-per-sample kernel's fused margin
 
 
 def test_differential_fuzz_of_the_compiled_chain_kernel(Q, W, monkeypatch):

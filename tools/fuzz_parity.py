@@ -154,7 +154,7 @@ def main(argv=None):
     import qo100net as Q
     from oracle import refbind as R
     ctx = Q.Context(device=0)
-    kernels, mism, skipped, oracle_checked, fs_checked = {}, [], 0, 0, 0
+    kernels, mism, skipped, oracle_checked, fs_checked, fused_runs = {}, [], 0, 0, 0, 0
     big = 2 * 148 * 3 * 128 + 77          # large enough for the thread-per-sample kernel on every 7th network
     for i in range(args.nets):
         if args.only >= 0 and i != args.only:
@@ -229,6 +229,8 @@ def main(argv=None):
         plan.launch(off, n)
         got = plan.read()
         kname = plan.kernel_name
+        if kname == "qo_mc_ts_kernel" and plan.tf_info["fused_specs"]:
+            fused_runs += 1                          # the thread-per-sample kernel walked a spec on its fused margin
         plan.close()
         kernels[kname] = kernels.get(kname, 0) + 1
         os.environ["QO100NET_KERNEL"] = "interp"
@@ -268,7 +270,7 @@ def main(argv=None):
                          "specs": specs, "got": int(got["n_pass"]), "interp": int(ref["n_pass"]),
                          "got_fail": [int(v) for v in got["fail_per_spec"]], "interp_fail": [int(v) for v in ref["fail_per_spec"]]})
     out = {"networks": args.nets, "skipped": skipped, "compared": args.nets - skipped, "oracle_checked": oracle_checked, "full_s_checked": fs_checked,
-           "kernels_selected": kernels, "mismatches": len(mism), "details": mism[:10], "seed": args.seed, "samples": args.samples}
+           "fused_runs": fused_runs, "kernels_selected": kernels, "mismatches": len(mism), "details": mism[:10], "seed": args.seed, "samples": args.samples}
     print(json.dumps(out, indent=1))
     if args.out:
         open(args.out, "w").write(json.dumps(out, indent=1))
