@@ -317,7 +317,8 @@ const char *qo_plan_tf_info(const qo_plan *plan, int info[6], double *self_check
  * QO100NET_KERNEL value): info[0] = QO_ERR_ARG and the reason string says why. */
 const char *qo_plan_analyze(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
                             int info[6], double *self_check_err, unsigned int *fused, double *fused_err, double *seconds);
-/* host->device bytes qo_plan_create copied for this plan (tables, masks, program), per GPU */
+/* host->device bytes of this plan's tables per GPU, alignment padding included: the tables its kernel reads, copied by
+ * qo_plan_create and again by every qo_mc_run call that reuses the plan */
 uint64_t qo_plan_h2d_bytes(const qo_plan *plan);
 void qo_plan_destroy(qo_plan *plan);
 

@@ -39,8 +39,8 @@ struct qo_ctx {
     ncclComm_t comm[8];
     int have_nccl;
     /* the plan of the last qo_mc_run call, kept so that a caller who runs the same job again (a sweep over sample ranges, a
-     * benchmark loop) does not rebuild the program, the polynomial analysis and the device buffers; the tables are still
-     * copied host -> device on every call */
+     * benchmark loop) does not rebuild the program, the polynomial analysis and the device allocation; its tables are still
+     * copied host -> device on every call, one copy per device */
     struct qo_plan *mc_cache;
     unsigned long long mc_cache_key;
 };

@@ -53,27 +53,31 @@ static int nccl_load(NcclApi *a)
 enum { QO_NCCL_UINT64 = 5, QO_NCCL_SUM = 0 };   /* ncclUint64, ncclSum (nccl.h enum values) */
 
 #define QO_TICKET_BYTES (16 + 256 * sizeof(unsigned int))
-struct DevPlan {
-    DevProg *prog;
-    void *w2, *wi2;            /* double2 or float2 [npairs] */
-    void *wsq2;                /* double2 [npairs]: w^2, ladder kernel only */
-    /* transfer-function kernel: one blob, tables padded to whole iterations of tf_pp*32 pairs */
-    void *tf_blob;
-    double2 *tf_yt, *tf_xt, *tf_wt, *tf_ctab[4], *tf_fu2[4];
-    uint4 *tf_mb;
-    uchar2 *tf_itm;
-    void *fs_blob;             /* FULL_S flavour of the transfer-function kernel: y and x tables, padded */
-    double2 *fs_yt, *fs_xt;
-    double2 *sblk, *sdet;      /* OP_SBLOCK: ABCD per (block, grid point); product of block determinants per point */
-    void *cpl_tab[4];          /* double2 [npairs] each: sin/cos of the nominal even/odd coupler angle (ladder kernel) */
-    uchar2 *m2;
-    double *fgrid;             /* generic kernel */
-    unsigned char *mask;
-    unsigned long long *counters;
-    unsigned long long *ticket;  /* ladder kernel: dynamic sample hand-out */
-    unsigned long long n_launched;
-    float ms;
+static const size_t QO_NOTAB = ~(size_t)0;
+static size_t align256(size_t n) { return (n + 255) & ~(size_t)255; }
+
+/* A plan's device tables, built once on the host in one buffer: each table is a zeroed region at a 256-byte-aligned offset,
+ * and every device of the ctx gets the same bytes at the same offsets */
+struct QoLayout {
+    std::vector<unsigned char> buf;
+    size_t add(size_t bytes) { const size_t at = align256(buf.size()); buf.resize(at + bytes, 0); return at; }
+    template <typename T> T *host(size_t off) { return off == QO_NOTAB ? NULL : (T *)(buf.data() + off); }
 };
+
+/* Byte offsets of a plan's tables in its device allocation; QO_NOTAB (where every offset starts): the plan's kernel does not read
+ * that table.  Two grid points per entry, in the plan's precision: w2, wi2 (1/w), wsq2 (w^2), m2 (spec bits); cpl: sin/cos of the
+ * coupler's nominal even/odd mode angles, or the row vector [1 Rs] M of a measured two-port in front; sblk, sdet: measured blocks'
+ * ABCD per (block, point), product of their determinants per point.  The transfer-function kernel's tables, padded to whole
+ * iterations: yt = -(w/wref)^2, xt = w/wref, wt = w, fu2 = the second row vector [1 -Rs] M (|S11| specs), mb = per-point byte
+ * masks, itm = per-iteration (OR, AND) of the spec bits.  The counters and the ticket area follow the uploaded tables. */
+struct QoTables {
+    size_t prog, w2, wi2, wsq2, m2, cpl[4], sblk, sdet, fgrid, mask, yt, xt, wt, fu2[4], mb, itm, counters, ticket;
+    QoTables() { memset(this, 0xFF, sizeof *this); }
+};
+
+/* mem: the tables of qo_plan::lay, then the counters, then the ticket area; fs_mem: the tables of the FULL_S flavour of the
+ * transfer-function kernel (qo_plan::fs_lay) */
+struct DevPlan { unsigned char *mem, *fs_mem; };
 
 /* the kernel a plan launches, in order of precedence (select_kernel); launch-time refinements: thread-per-sample inside launch_tf,
  * the compiled chain kernel inside launch_lumped, the FULL_S transfer-function kernel ahead of them all (plan_launch_dev) */
@@ -99,7 +103,8 @@ struct qo_plan {
     int fs_state;                                         /* FULL_S transfer-function path: 0 not analysed yet, 1 selected, -1 refused */
     TfPlan fsp;
     int fs_niter;
-    unsigned long long h2d_bytes;                         /* host->device bytes copied by qo_plan_create, per GPU */
+    QoLayout fs_lay;                                      /* its tables, built at the first launch that takes it */
+    size_t fs_yt, fs_xt;
     int cj_debug, cj_failed[2];                           /* run-time compiled chain kernel (qo_chain_jit.h), used as ov.chain says */
     const void *cj[2];                                    /* its QcjEntry for the reduce-only / FULL_S flavour once this process holds it */
     std::string cj_src[2];
@@ -107,13 +112,16 @@ struct qo_plan {
     const char *kernel_name;
     double flops_per_eval;
     int launches;
-    unsigned long long n_total_launched;
+    QoLayout lay;                                         /* the tables the plan's kernel reads (qo_mc_run re-sends them on a cache hit) */
+    QoTables tab;
+    unsigned char *pinned;                                /* page-locked copy of lay, made the first time the tables are re-sent */
     DevPlan d[8];
     std::vector<double> f;
     std::vector<unsigned char> maskv;
-    struct Upload { void *dst; std::vector<unsigned char> data; size_t at; };
-    std::vector<Upload> uploads[8];                       /* what qo_plan_create copied to each device (qo_mc_run re-sends it on a cache hit) */
-    unsigned char *pinned[8];                             /* ... gathered in one page-locked buffer per device the first time they are re-sent */
+    /* device address of a table on device g; NULL when the plan's kernel does not read it */
+    template <typename T> T *dev(int g, size_t off) const { return off == QO_NOTAB ? NULL : (T *)(d[g].mem + off); }
+    unsigned long long *counters(int g) const { return dev<unsigned long long>(g, tab.counters); }
+    unsigned long long *ticket(int g) const { return dev<unsigned long long>(g, tab.ticket); }
 };
 
 static void tf_launch_setup(qo_plan *p, const QoOverrides *ov);
@@ -446,15 +454,238 @@ extern "C" void qo_plan_destroy(qo_plan *p)
     if (!p) return;
     for (int g = 0; g < p->ctx->ndev; g++) {
         cudaSetDevice(p->ctx->d[g].device);
-        DevPlan *d = &p->d[g];
         /* stream-ordered frees: back into the device's pool without a device-wide synchronisation */
         cudaStream_t st = p->ctx->d[g].stream;
-        void *ptrs[] = { d->prog, d->w2, d->wi2, d->wsq2, d->tf_blob, d->fs_blob, d->m2, d->cpl_tab[0], d->cpl_tab[1], d->cpl_tab[2], d->cpl_tab[3],
-                         d->fgrid, d->mask, d->counters, d->ticket, d->sblk, d->sdet };
-        for (size_t i = 0; i < sizeof ptrs / sizeof ptrs[0]; i++) if (ptrs[i]) cudaFreeAsync(ptrs[i], st);
-        if (p->pinned[g]) cudaFreeHost(p->pinned[g]);
+        if (p->d[g].mem) cudaFreeAsync(p->d[g].mem, st);
+        if (p->d[g].fs_mem) cudaFreeAsync(p->d[g].fs_mem, st);
     }
+    if (p->pinned) cudaFreeHost(p->pinned);
     delete p;
+}
+
+/* angular frequency of grid point k; points past the grid (padding) repeat its last one */
+static double grid_w(const double *f, int nf, size_t k) { return 6.283185307179586476925286766559 * f[k < (size_t)nf ? k : (size_t)nf - 1]; }
+
+/* Measured two-port blocks: interpolate every block at every point (Qucs SPfile "linear"), convert to ABCD at the file's reference
+ * impedance; blocks carry no tolerances, so this happens once per plan.  sblk: ABCD per (block, point) as four double2 (empty when
+ * no element uses a block); sdet: the product of the blocks' determinants per point (empty when every block is reciprocal). */
+static int block_tables(const qo_net *net, const double *f, int nf, int npts, std::vector<double2> *sblk, std::vector<double2> *sdet)
+{
+    int polar[QO_MAX_BLK];
+    for (int b = 0; b < net->nblk; b++) polar[b] = 1;
+    int used = 0;
+    for (int e = 0; e < net->n; e++)
+        if (net->e[e].kind == QO_SBLOCK) { polar[(int)net->e[e].p[0]] = net->e[e].p[1] != 0.0; used = 1; }
+    if (!used) return QO_OK;
+    int nonrecip = 0;
+    sblk->resize((size_t)net->nblk * npts * 4);
+    sdet->assign((size_t)npts, make_double2(1.0, 0.0));
+    for (int b = 0; b < net->nblk; b++)
+        for (int k = 0; k < npts; k++) {
+            qo_c64 sv[4], m[4];
+            qo_s2p_eval(net->blk[b], f[k < nf ? k : nf - 1], polar[b], sv);
+            if (!qo_s_to_abcd(sv, net->blk[b]->z0, m)) {
+                qo_set_error("S-parameter block %d has S21 = 0 at %g Hz: no chain matrix", b, f[k < nf ? k : nf - 1]);
+                return QO_ERR_RANGE;
+            }
+            for (int q = 0; q < 4; q++) (*sblk)[((size_t)b * npts + k) * 4 + q] = make_double2(m[q].re, m[q].im);
+            /* det(ABCD) = S12 / S21 */
+            const double d = sv[1].re * sv[1].re + sv[1].im * sv[1].im;
+            const double dr = (sv[2].re * sv[1].re + sv[2].im * sv[1].im) / d, di = (sv[2].im * sv[1].re - sv[2].re * sv[1].im) / d;
+            if (fabs(dr - 1.0) > 1e-12 || fabs(di) > 1e-12) nonrecip = 1;
+            const double2 o = (*sdet)[k];
+            (*sdet)[k] = make_double2(o.x * dr - o.y * di, o.x * di + o.y * dr);
+        }
+    if (!nonrecip) sdet->clear();
+    return QO_OK;
+}
+
+/* The coupler block in front of the ladder or transfer-function kernel.  Tables of sin/cos of its NOMINAL mode angles serve
+ * every sample when each sample's angles stay within 0.1 rad of nominal over the whole grid (qo_ladder.cuh::lad_cpl_first); this
+ * bounds that excursion up to wmax, the grid's largest angular frequency.  ke, ko: nominal even / odd mode angle per unit of w;
+ * same: both modes alike, nominally and in tolerance. */
+struct CplAngles { int fast, same; double ke, ko; };
+static CplAngles cpl_angles(const DevProg *hp, double wmax, const QoOverrides *ov)
+{
+    CplAngles a = { 0, 0, 0.0, 0.0 };
+    const int ec = hp->op0;                    /* the coupler op */
+    double worst = 0;
+    int ok = 1;
+    if (hp->cplms_elem == ec) {
+        /* physical element: bound the mode angles' excursion by running the analysis at every corner of the
+         * tolerance box of the parameters it reads (<= 7 of them), plus 25 % margin for the interior */
+        a.ke = hp->cplms_nom[2] / (360.0 * hp->nom[ec][4]); a.ko = hp->cplms_nom[3] / (360.0 * hp->nom[ec][4]);
+        const int es = hp->cplms_sub;
+        const int pe[7] = { ec, ec, es, es, es, ec, ec }, pk[7] = { 0, 1, 1, 2, 0, 3, 2 };      /* W S h t er ht L */
+        double lo[7], hi[7];
+        for (int q = 0; q < 7; q++) {
+            const double nomv = hp->nom[pe[q]][pk[q]], t = hp->tvar[pe[q]][pk[q]] >= 0 ? fabs(hp->ttol[pe[q]][pk[q]]) : 0.0;
+            const double dlt = hp->tmode[pe[q]][pk[q]] ? t : fabs(nomv) * t;
+            lo[q] = nomv - dlt; hi[q] = nomv + dlt;
+        }
+        ok = !(hp->tvar[ec][4] >= 0);          /* a perturbed analysis frequency: not bounded here */
+        for (int c = 0; c < 128 && ok; c++) {
+            double v[7], o[4];
+            for (int q = 0; q < 7; q++) v[q] = (c >> q) & 1 ? hi[q] : lo[q];
+            if (!(v[0] > 0 && v[1] > 0 && v[2] > 0 && v[3] >= 0 && v[4] > 1 && v[5] > 0 && v[6] > 0)) { ok = 0; break; }
+            qo_cpl_core(v[0], v[1], v[2], v[3], v[4], v[5], hp->nom[ec][4], v[6], o);
+            const double de = fabs(o[2] / (360.0 * hp->nom[ec][4]) - a.ke), dn = fabs(o[3] / (360.0 * hp->nom[ec][4]) - a.ko);
+            if (!(de == de) || !(dn == dn)) { ok = 0; break; }
+            if (1.25 * de * wmax > worst) worst = 1.25 * de * wmax;
+            if (1.25 * dn * wmax > worst) worst = 1.25 * dn * wmax;
+        }
+    } else {
+        double lo[6], hi[6];
+        for (int k = 0; k < 6; k++) {
+            const double nomv = hp->nom[ec][k], t = hp->tvar[ec][k] >= 0 ? fabs(hp->ttol[ec][k]) : 0.0;
+            const double dlt = hp->tmode[ec][k] ? t : fabs(nomv) * t;
+            lo[k] = nomv - dlt; hi[k] = nomv + dlt;
+        }
+        ok = lo[4] > 0;
+        for (int m = 0; m < 2 && ok; m++) {
+            const double kn = hp->nom[ec][2 + m] / (360.0 * hp->nom[ec][4]);
+            const double kmax = hi[2 + m] / (360.0 * lo[4]), kmin = lo[2 + m] / (360.0 * hi[4]);
+            const double dk = fmax(kmax - kn, kn - kmin);
+            if (dk * wmax > worst) worst = dk * wmax;
+        }
+        a.ke = hp->nom[ec][2] / (360.0 * hp->nom[ec][4]); a.ko = hp->nom[ec][3] / (360.0 * hp->nom[ec][4]);
+        a.same = hp->nom[ec][2] == hp->nom[ec][3] && hp->tvar[ec][2] == hp->tvar[ec][3] && hp->ttol[ec][2] == hp->ttol[ec][3] &&
+                 hp->tmode[ec][2] == hp->tmode[ec][3];
+    }
+    a.fast = ok && worst <= 0.1 && !ov->cpl_sincos;
+    return a;
+}
+
+/* tables of the ladder and lumped kernels, in the plan's precision T, one entry per grid point, padded to a whole pair */
+template <typename T>
+static void chain_tables(qo_plan *p, const double *f, const std::vector<double2> &sblk, const std::vector<double2> &sdet, const CplAngles &ca)
+{
+    QoLayout &L = p->lay; QoTables &t = p->tab;
+    const size_t npts = 2 * (size_t)p->npairs, tb = npts * sizeof(T);
+    t.w2 = L.add(tb); t.wi2 = L.add(tb); t.m2 = L.add(npts);
+    if (p->kern == K_LADDER) t.wsq2 = L.add(tb);
+    if (p->kern == K_LADDER && p->cpl_fast) for (int c = 0; c < 4; c++) t.cpl[c] = L.add(tb);
+    if (p->kern == K_LUMPED && !sblk.empty()) t.sblk = L.add(sblk.size() * sizeof(double2));
+    if (p->kern == K_LUMPED && !sdet.empty()) t.sdet = L.add(sdet.size() * sizeof(double2));
+    T *w2 = L.host<T>(t.w2), *wi2 = L.host<T>(t.wi2), *wsq2 = L.host<T>(t.wsq2), *cpl[4];
+    for (int c = 0; c < 4; c++) cpl[c] = L.host<T>(t.cpl[c]);
+    unsigned char *m2 = L.host<unsigned char>(t.m2);
+    for (size_t k = 0; k < npts; k++) {
+        const double w = grid_w(f, p->nf, k);
+        w2[k] = (T)w; wi2[k] = (T)(1.0 / w); m2[k] = k < (size_t)p->nf ? p->maskv[k] : 0;
+        if (wsq2) wsq2[k] = (T)(w * w);
+        if (cpl[0]) { cpl[0][k] = (T)sin(ca.ke * w); cpl[1][k] = (T)cos(ca.ke * w); cpl[2][k] = (T)sin(ca.ko * w); cpl[3][k] = (T)cos(ca.ko * w); }
+    }
+    if (t.sblk != QO_NOTAB) memcpy(L.host<double2>(t.sblk), sblk.data(), sblk.size() * sizeof(double2));
+    if (t.sdet != QO_NOTAB) memcpy(L.host<double2>(t.sdet), sdet.data(), sdet.size() * sizeof(double2));
+}
+
+/* tables of the transfer-function kernel, padded to whole iterations (padding repeats the last grid point and carries no spec
+ * bit, so the loop needs no bounds checks) */
+static void tf_tables(qo_plan *p, const double *f, const std::vector<double2> &sblk, const CplAngles &ca)
+{
+    QoLayout &L = p->lay; QoTables &t = p->tab;
+    const int nf = p->nf, np = p->npairs;
+    p->tf_pp = qo_tf_default_pp(&p->tfp, np);
+    const int ppi = 32 * p->tf_pp;
+    p->tf_niter = (np + ppi - 1) / ppi;
+    /* + one iteration of padding: the kernel requests the next iteration's y values before it is done with the current one */
+    const size_t npt = 2 * ((size_t)p->tf_niter + 1) * ppi, tb = npt * sizeof(double);
+    /* a measured two-port in front: its row vector [1 Rs] M(f) per grid point rides in the four coupler-table slots */
+    const bool front_blk = p->tfp.cpl_op >= 0 && p->tfp.front == 2;
+    const bool front_s11 = front_blk && p->tfp.s11;         /* + its second row vector [1 -Rs] M for |S11| specs */
+    t.yt = L.add(tb); t.xt = L.add(tb); t.wt = L.add(tb);
+    if (p->cpl_fast || front_blk) for (int c = 0; c < 4; c++) t.cpl[c] = L.add(tb);
+    if (front_s11) for (int c = 0; c < 4; c++) t.fu2[c] = L.add(tb);
+    t.mb = L.add(2 * npt * sizeof(unsigned int));
+    t.itm = L.add(((size_t)p->tf_niter * sizeof(uchar2) + 15) & ~(size_t)15);
+    double *yt = L.host<double>(t.yt), *xt = L.host<double>(t.xt), *wt = L.host<double>(t.wt), *cpl[4], *fu2[4];
+    for (int c = 0; c < 4; c++) { cpl[c] = L.host<double>(t.cpl[c]); fu2[c] = L.host<double>(t.fu2[c]); }
+    unsigned int *mb = L.host<unsigned int>(t.mb); uchar2 *itm = L.host<uchar2>(t.itm);
+    const double rs = p->hp.rs;
+    for (size_t k = 0; k < npt; k++) {
+        const size_t kc = k < (size_t)nf ? k : (size_t)nf - 1;
+        const double w = grid_w(f, nf, k), x = w / p->tfp.wref;
+        yt[k] = -(x * x); xt[k] = x; wt[k] = w;
+        if (p->cpl_fast) { cpl[0][k] = sin(ca.ke * w); cpl[1][k] = cos(ca.ke * w); cpl[2][k] = sin(ca.ko * w); cpl[3][k] = cos(ca.ko * w); }
+        if (front_blk) {
+            const int blk = (int)p->hp.nom[p->tfp.cpl_op][0];
+            const double2 *mm = &sblk[((size_t)blk * (size_t)(2 * np) + kc) * 4];
+            cpl[0][k] = mm[0].x + rs * mm[2].x; cpl[1][k] = mm[0].y + rs * mm[2].y;
+            cpl[2][k] = mm[1].x + rs * mm[3].x; cpl[3][k] = mm[1].y + rs * mm[3].y;
+            if (front_s11) {
+                fu2[0][k] = mm[0].x - rs * mm[2].x; fu2[1][k] = mm[0].y - rs * mm[2].y;
+                fu2[2][k] = mm[1].x - rs * mm[3].x; fu2[3][k] = mm[1].y - rs * mm[3].y;
+            }
+        }
+        unsigned int lo = 0, hi = 0;
+        const unsigned char mk = k < (size_t)nf ? p->maskv[k] : 0;
+        for (int sp = 0; sp < 4; sp++) {
+            if ((mk >> sp) & 1u) lo |= 0xFFu << (8 * sp);
+            if ((mk >> (sp + 4)) & 1u) hi |= 0xFFu << (8 * sp);
+        }
+        mb[2 * k] = lo; mb[2 * k + 1] = hi;
+    }
+    for (int it = 0; it < p->tf_niter; it++) {
+        unsigned char any = 0, all = 0xFF;
+        for (size_t k = (size_t)it * 2 * ppi; k < (size_t)(it + 1) * 2 * ppi; k++) {
+            const unsigned char mk = k < (size_t)nf ? p->maskv[k] : 0;
+            any |= mk; all &= mk;
+        }
+        itm[it] = make_uchar2(any, all);
+    }
+}
+
+/* the tables the plan's kernel reads, in p->lay; where they lie, in p->tab */
+static int build_tables(qo_plan *p, const qo_net *net, const double *f)
+{
+    QoLayout &L = p->lay; QoTables &t = p->tab;
+    const int nf = p->nf, npts = 2 * p->npairs;
+    t.prog = L.add(sizeof(DevProg));
+    memcpy(L.host<DevProg>(t.prog), &p->hp, sizeof(DevProg));
+    /* built for every plan with measured blocks; a transfer-function plan forms the row tables of its front block from them */
+    std::vector<double2> sblk, sdet;
+    const int rc = p->generic ? QO_OK : block_tables(net, f, nf, npts, &sblk, &sdet);
+    if (rc) return rc;
+    CplAngles ca = { 0, 0, 0.0, 0.0 };
+    if ((p->kern == K_LADDER && p->lad_cpl) || (p->kern == K_TF && p->tfp.cpl_op >= 0 && p->tfp.front == 0)) {
+        double wmax = 0;
+        for (int k = 0; k < npts; k++) if (grid_w(f, nf, k) > wmax) wmax = grid_w(f, nf, k);
+        ca = cpl_angles(&p->hp, wmax, &p->ov);
+    }
+    p->cpl_fast = ca.fast; p->cpl_same = ca.same;
+    switch (p->kern) {
+    case K_BOARD: case K_GENERIC:
+        t.fgrid = L.add((size_t)nf * sizeof(double));
+        memcpy(L.host<double>(t.fgrid), f, (size_t)nf * sizeof(double));
+        t.mask = L.add((size_t)nf);
+        memcpy(L.host<unsigned char>(t.mask), p->maskv.data(), (size_t)nf);
+        break;
+    case K_SPOT: break;                        /* its grid and spec bits travel in the kernel parameters */
+    case K_TF: tf_tables(p, f, sblk, ca); break;
+    case K_LADDER: case K_LUMPED:
+        if (p->precision == 32) chain_tables<float>(p, f, sblk, sdet, ca);
+        else chain_tables<double>(p, f, sblk, sdet, ca);
+        break;
+    }
+    return QO_OK;
+}
+
+/* one allocation per device: the tables (one copy of p->lay), the counters (zeroed), the ticket area */
+static int upload(qo_plan *p)
+{
+    const size_t cnt_bytes = (size_t)p->ncnt * sizeof(unsigned long long);
+    p->tab.counters = align256(p->lay.buf.size());
+    p->tab.ticket = align256(p->tab.counters + cnt_bytes);
+    for (int g = 0; g < p->ctx->ndev; g++) {
+        const DevCtx *dc = &p->ctx->d[g];
+        CU(cudaSetDevice(dc->device));
+        CU(cudaMallocAsync((void **)&p->d[g].mem, p->tab.ticket + QO_TICKET_BYTES, dc->stream));
+        CU(cudaMemcpyAsync(p->d[g].mem, p->lay.buf.data(), p->lay.buf.size(), cudaMemcpyHostToDevice, dc->stream));
+        CU(cudaMemsetAsync(p->counters(g), 0, cnt_bytes, dc->stream));
+        CU(cudaStreamSynchronize(dc->stream));      /* a failed copy is reported by plan creation, not by the first launch */
+    }
+    return QO_OK;
 }
 
 static int plan_create(qo_ctx *ctx, const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec,
@@ -463,253 +694,29 @@ static int plan_create(qo_ctx *ctx, const qo_net *net, const double *f, int nf, 
     if (!ctx || !net || !f || nf <= 0 || !out || (nspec > 0 && !spec)) { qo_set_error("bad arguments"); return QO_ERR_ARG; }
     for (int k = 0; k < nf; k++)
         if (!(f[k] > 0.0) || !isfinite(f[k])) { qo_set_error("frequency %d is not a positive finite number", k); return QO_ERR_ARG; }
-    qo_plan *p = new (std::nothrow) qo_plan();
+    qo_plan *p = new (std::nothrow) qo_plan();        /* value-initialised: what is not set here starts zeroed (QoTables: QO_NOTAB) */
     if (!p) return QO_ERR_NOMEM;
     p->ctx = ctx;
     p->ov = *ov;
-    memset(p->pinned, 0, sizeof p->pinned);
     p->nf = nf;
     p->npairs = (nf + 1) / 2;
     p->precision = cfg && cfg->precision == 32 ? 32 : 64;
     p->mode = cfg ? cfg->mode : QO_MODE_FULL_S;
-    p->launches = 0;
-    p->h2d_bytes = 0;
-    p->fs_state = 0;
-    memset(p->d, 0, sizeof p->d);
     int rc = build_prog(net, f, nf, spec, nspec, cfg, &p->hp, &p->generic, &p->flops_per_eval, &p->maskv);
     if (rc) { delete p; return rc; }
     if (p->generic && p->precision == 32) { delete p; qo_set_error("FP32 mode covers lumped/TL networks only"); return QO_ERR_UNSUPPORTED; }
     if (p->hp.need_gd && p->precision == 32) { delete p; qo_set_error("group-delay specs need FP64 (the 1e-6 relative frequency step is 8 float ulps)"); return QO_ERR_UNSUPPORTED; }
+    if (p->generic)
+        for (int e = 0; e < net->n; e++)
+            if (net->e[e].kind == QO_SBLOCK) { qo_set_error("S-parameter blocks cannot be mixed with microstrip elements yet"); delete p; return QO_ERR_UNSUPPORTED; }
     p->ncnt = 2 + nspec + p->hp.hist_bins;
     p->f.assign(f, f + nf);
     p->kern = select_kernel(p, f, nf);
     p->kernel_name = qo_kern_name[p->kern];
     p->cj_debug = getenv("QO100NET_CHAIN_DEBUG") != NULL;
-    p->cj[0] = p->cj[1] = NULL; p->cj_failed[0] = p->cj_failed[1] = 0; p->cj_hash[0] = p->cj_hash[1] = 0;
-
-    /* per-frequency tables: w = 2 pi f and 1/w (hoisted out of the kernel), padded to a pair */
-    const double two_pi = 6.283185307179586476925286766559;
-    const int np = p->npairs;
-    std::vector<double> w(2 * (size_t)np), wi(2 * (size_t)np), wsq(2 * (size_t)np);
-    std::vector<float> wf(2 * (size_t)np), wif(2 * (size_t)np), wsqf(2 * (size_t)np);
-    std::vector<unsigned char> m(2 * (size_t)np, 0);
-    for (int k = 0; k < 2 * np; k++) {
-        double fk = f[k < nf ? k : nf - 1];
-        w[k] = two_pi * fk; wi[k] = 1.0 / w[k]; wsq[k] = w[k] * w[k];
-        wf[k] = (float)w[k]; wif[k] = (float)wi[k]; wsqf[k] = (float)wsq[k];
-        m[k] = k < nf ? p->maskv[k] : 0;
-    }
-    /* measured two-port blocks: interpolate every block at every grid point (Qucs SPfile "linear"), convert to
-     * ABCD at the file's reference impedance; blocks carry no tolerances, so this happens once per plan */
-    std::vector<double2> sblk, sdet;
-    int nonrecip = 0;
-    if (net->nblk > 0 && !p->generic) {
-        int polar[QO_MAX_BLK];
-        for (int b = 0; b < net->nblk; b++) polar[b] = 1;
-        int used = 0;
-        for (int e = 0; e < net->n; e++)
-            if (net->e[e].kind == QO_SBLOCK) { polar[(int)net->e[e].p[0]] = net->e[e].p[1] != 0.0; used = 1; }
-        if (used) {
-            const int npts = 2 * np;
-            sblk.resize((size_t)net->nblk * npts * 4);
-            sdet.assign((size_t)npts, make_double2(1.0, 0.0));
-            for (int b = 0; b < net->nblk; b++)
-                for (int k = 0; k < npts; k++) {
-                    qo_c64 sv[4], m[4];
-                    qo_s2p_eval(net->blk[b], f[k < nf ? k : nf - 1], polar[b], sv);
-                    if (!qo_s_to_abcd(sv, net->blk[b]->z0, m)) {
-                        qo_set_error("S-parameter block %d has S21 = 0 at %g Hz: no chain matrix", b, f[k < nf ? k : nf - 1]);
-                        delete p; return QO_ERR_RANGE;
-                    }
-                    for (int q = 0; q < 4; q++) sblk[((size_t)b * npts + k) * 4 + q] = make_double2(m[q].re, m[q].im);
-                    /* det(ABCD) = S12 / S21 */
-                    const double d = sv[1].re * sv[1].re + sv[1].im * sv[1].im;
-                    const double dr = (sv[2].re * sv[1].re + sv[2].im * sv[1].im) / d, di = (sv[2].im * sv[1].re - sv[2].re * sv[1].im) / d;
-                    if (fabs(dr - 1.0) > 1e-12 || fabs(di) > 1e-12) nonrecip = 1;
-                    const double2 o = sdet[k];
-                    sdet[k] = make_double2(o.x * dr - o.y * di, o.x * di + o.y * dr);
-                }
-        }
-    }
-    if (net->nblk > 0 && p->generic) {
-        for (int e = 0; e < net->n; e++)
-            if (net->e[e].kind == QO_SBLOCK) { qo_set_error("S-parameter blocks cannot be mixed with microstrip elements yet"); delete p; return QO_ERR_UNSUPPORTED; }
-    }
-    /* coupler block of the ladder kernel: sin/cos of the NOMINAL mode angles per grid point, usable when
-     * every sample's angle stays within 0.1 rad of nominal over the whole grid (qo_ladder.cuh::lad_cpl_first) */
-    std::vector<double> ctab[4];
-    std::vector<float> ctabf[4];
-    p->cpl_fast = p->cpl_same = 0;
-    if ((p->kern == K_LADDER && p->lad_cpl) || (p->kern == K_TF && p->tfp.cpl_op >= 0 && p->tfp.front == 0)) {
-        const DevProg *hp = &p->hp;
-        const int ec = hp->op0;                    /* the coupler op */
-        double wmax = 0;
-        for (int k = 0; k < 2 * np; k++) if (w[k] > wmax) wmax = w[k];
-        double worst = 0, ke_nom, ko_nom;
-        int ok = 1;
-        if (hp->cplms_elem == ec) {
-            /* physical element: bound the mode angles' excursion by running the analysis at every corner of the
-             * tolerance box of the parameters it reads (<= 7 of them), plus 25 % margin for the interior */
-            ke_nom = hp->cplms_nom[2] / (360.0 * hp->nom[ec][4]); ko_nom = hp->cplms_nom[3] / (360.0 * hp->nom[ec][4]);
-            const int es = hp->cplms_sub;
-            const int pe[7] = { ec, ec, es, es, es, ec, ec }, pk[7] = { 0, 1, 1, 2, 0, 3, 2 };      /* W S h t er ht L */
-            double lo[7], hi[7];
-            for (int q = 0; q < 7; q++) {
-                const double nomv = hp->nom[pe[q]][pk[q]], t = hp->tvar[pe[q]][pk[q]] >= 0 ? fabs(hp->ttol[pe[q]][pk[q]]) : 0.0;
-                const double dlt = hp->tmode[pe[q]][pk[q]] ? t : fabs(nomv) * t;
-                lo[q] = nomv - dlt; hi[q] = nomv + dlt;
-            }
-            ok = !(hp->tvar[ec][4] >= 0);          /* a perturbed analysis frequency: not bounded here */
-            for (int c = 0; c < 128 && ok; c++) {
-                double v[7], o[4];
-                for (int q = 0; q < 7; q++) v[q] = (c >> q) & 1 ? hi[q] : lo[q];
-                if (!(v[0] > 0 && v[1] > 0 && v[2] > 0 && v[3] >= 0 && v[4] > 1 && v[5] > 0 && v[6] > 0)) { ok = 0; break; }
-                qo_cpl_core(v[0], v[1], v[2], v[3], v[4], v[5], hp->nom[ec][4], v[6], o);
-                const double de = fabs(o[2] / (360.0 * hp->nom[ec][4]) - ke_nom), dn = fabs(o[3] / (360.0 * hp->nom[ec][4]) - ko_nom);
-                if (!(de == de) || !(dn == dn)) { ok = 0; break; }
-                if (1.25 * de * wmax > worst) worst = 1.25 * de * wmax;
-                if (1.25 * dn * wmax > worst) worst = 1.25 * dn * wmax;
-            }
-            p->cpl_same = 0;
-        } else {
-            double lo[6], hi[6];
-            for (int k = 0; k < 6; k++) {
-                const double nomv = hp->nom[ec][k], t = hp->tvar[ec][k] >= 0 ? fabs(hp->ttol[ec][k]) : 0.0;
-                const double dlt = hp->tmode[ec][k] ? t : fabs(nomv) * t;
-                lo[k] = nomv - dlt; hi[k] = nomv + dlt;
-            }
-            ok = lo[4] > 0;
-            for (int m = 0; m < 2 && ok; m++) {
-                const double kn = hp->nom[ec][2 + m] / (360.0 * hp->nom[ec][4]);
-                const double kmax = hi[2 + m] / (360.0 * lo[4]), kmin = lo[2 + m] / (360.0 * hi[4]);
-                const double dk = fmax(kmax - kn, kn - kmin);
-                if (dk * wmax > worst) worst = dk * wmax;
-            }
-            ke_nom = hp->nom[ec][2] / (360.0 * hp->nom[ec][4]); ko_nom = hp->nom[ec][3] / (360.0 * hp->nom[ec][4]);
-            p->cpl_same = hp->nom[ec][2] == hp->nom[ec][3] && hp->tvar[ec][2] == hp->tvar[ec][3] && hp->ttol[ec][2] == hp->ttol[ec][3] &&
-                          hp->tmode[ec][2] == hp->tmode[ec][3];
-        }
-        p->cpl_fast = ok && worst <= 0.1 && !ov->cpl_sincos;
-        if (p->cpl_fast) {
-            for (int t = 0; t < 4; t++) ctab[t].resize(2 * (size_t)np);
-            const double ke = ke_nom, ko = ko_nom;
-            for (int k = 0; k < 2 * np; k++) {
-                ctab[0][k] = sin(ke * w[k]); ctab[1][k] = cos(ke * w[k]);
-                ctab[2][k] = sin(ko * w[k]); ctab[3][k] = cos(ko * w[k]);
-            }
-            for (int t = 0; t < 4; t++) { ctabf[t].resize(2 * (size_t)np); for (int k = 0; k < 2 * np; k++) ctabf[t][k] = (float)ctab[t][k]; }
-        }
-    }
-    for (int g = 0; g < ctx->ndev; g++) {
-        DevPlan *d = &p->d[g];
-        rc = QO_ERR_CUDA;
-#define H2D(DST_, SRC_, NB_) do { CUP(cudaMemcpyAsync((DST_), (SRC_), (NB_), cudaMemcpyHostToDevice, st)); if (g == 0) p->h2d_bytes += (NB_); \
-                                  qo_plan::Upload u_; u_.dst = (DST_); u_.at = 0; u_.data.assign((const unsigned char *)(SRC_), (const unsigned char *)(SRC_) + (NB_)); p->uploads[g].push_back(std::move(u_)); } while (0)
-#define CUP(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { qo_set_error("%s -> %s", #call, cudaGetErrorString(e_)); qo_plan_destroy(p); return QO_ERR_CUDA; } } while (0)
-        CUP(cudaSetDevice(ctx->d[g].device));
-        cudaStream_t st = ctx->d[g].stream;
-        CUP(cudaMallocAsync((void **)&d->prog, sizeof(DevProg), st));
-        H2D(d->prog, &p->hp, sizeof(DevProg));
-        if (!p->generic) {
-            size_t esz = p->precision == 32 ? sizeof(float) : sizeof(double);
-            CUP(cudaMallocAsync((void **)&d->w2, 2 * (size_t)np * esz, st));
-            CUP(cudaMallocAsync((void **)&d->wi2, 2 * (size_t)np * esz, st));
-            CUP(cudaMallocAsync((void **)&d->m2, 2 * (size_t)np, st));
-            if (p->precision == 32) {
-                H2D(d->w2, wf.data(), 2 * (size_t)np * esz);
-                H2D(d->wi2, wif.data(), 2 * (size_t)np * esz);
-            } else {
-                H2D(d->w2, w.data(), 2 * (size_t)np * esz);
-                H2D(d->wi2, wi.data(), 2 * (size_t)np * esz);
-            }
-            H2D(d->m2, m.data(), 2 * (size_t)np);
-            if (!sblk.empty()) {
-                CUP(cudaMallocAsync((void **)&d->sblk, sblk.size() * sizeof(double2), st));
-                H2D(d->sblk, sblk.data(), sblk.size() * sizeof(double2));
-                if (nonrecip) {
-                    CUP(cudaMallocAsync((void **)&d->sdet, sdet.size() * sizeof(double2), st));
-                    H2D(d->sdet, sdet.data(), sdet.size() * sizeof(double2));
-                }
-            }
-            if (p->kern == K_TF) {
-                /* tables of the transfer-function kernel, padded to whole iterations (padding repeats the last grid
-                 * point and carries no spec bit, so the loop needs no bounds checks) */
-                p->tf_pp = qo_tf_default_pp(&p->tfp, np);
-                const int ppi = 32 * p->tf_pp;
-                p->tf_niter = (np + ppi - 1) / ppi;
-                /* + one iteration of padding: the kernel requests the next iteration's y values before it is done with the current one */
-                const size_t npad = ((size_t)p->tf_niter + 1) * ppi, npt = 2 * npad;
-                /* a measured two-port in front: its row vector [1 Rs] M(f) per grid point rides in the four coupler-table slots */
-                const bool front_blk = p->tfp.cpl_op >= 0 && p->tfp.front == 2;
-                const bool front_s11 = front_blk && p->tfp.s11;         /* + its second row vector [1 -Rs] M for |S11| specs */
-                const int ntab = 3 + (p->cpl_fast || front_blk ? 4 : 0) + (front_s11 ? 4 : 0);
-                const size_t itm_bytes = ((size_t)p->tf_niter * sizeof(uchar2) + 15) & ~(size_t)15;
-                const size_t bytes = (size_t)ntab * npt * sizeof(double) + 2 * npt * sizeof(unsigned int) + itm_bytes;
-                std::vector<unsigned char> blob(bytes);
-                double *tab = (double *)blob.data();
-                unsigned int *mb = (unsigned int *)(tab + (size_t)ntab * npt);
-                uchar2 *itm = (uchar2 *)(mb + 2 * npt);
-                for (size_t k = 0; k < npt; k++) {
-                    const size_t kc = k < (size_t)nf ? k : (size_t)nf - 1;
-                    const double x = w[kc] / p->tfp.wref;
-                    tab[k] = -(x * x); tab[npt + k] = x; tab[2 * npt + k] = w[kc];
-                    if (p->cpl_fast) for (int t = 0; t < 4; t++) tab[(3 + t) * npt + k] = ctab[t][kc];
-                    if (front_blk) {
-                        const int blk = (int)p->hp.nom[p->tfp.cpl_op][0];
-                        const double2 *mm = &sblk[((size_t)blk * (size_t)(2 * np) + kc) * 4];
-                        tab[3 * npt + k] = mm[0].x + p->hp.rs * mm[2].x; tab[4 * npt + k] = mm[0].y + p->hp.rs * mm[2].y;
-                        tab[5 * npt + k] = mm[1].x + p->hp.rs * mm[3].x; tab[6 * npt + k] = mm[1].y + p->hp.rs * mm[3].y;
-                        if (front_s11) {
-                            tab[7 * npt + k] = mm[0].x - p->hp.rs * mm[2].x; tab[8 * npt + k] = mm[0].y - p->hp.rs * mm[2].y;
-                            tab[9 * npt + k] = mm[1].x - p->hp.rs * mm[3].x; tab[10 * npt + k] = mm[1].y - p->hp.rs * mm[3].y;
-                        }
-                    }
-                    unsigned int lo = 0, hi = 0;
-                    const unsigned char mk = k < (size_t)nf ? p->maskv[k] : 0;
-                    for (int sp = 0; sp < 4; sp++) {
-                        if ((mk >> sp) & 1u) lo |= 0xFFu << (8 * sp);
-                        if ((mk >> (sp + 4)) & 1u) hi |= 0xFFu << (8 * sp);
-                    }
-                    mb[2 * k] = lo; mb[2 * k + 1] = hi;
-                }
-                for (int it = 0; it < p->tf_niter; it++) {
-                    unsigned char any = 0, all = 0xFF;
-                    for (size_t k = (size_t)it * 2 * ppi; k < (size_t)(it + 1) * 2 * ppi; k++) {
-                        const unsigned char mk = k < (size_t)nf ? p->maskv[k] : 0;
-                        any |= mk; all &= mk;
-                    }
-                    itm[it] = make_uchar2(any, all);
-                }
-                CUP(cudaMallocAsync((void **)&d->tf_blob, bytes, st));
-                H2D(d->tf_blob, blob.data(), bytes);
-                CUP(cudaStreamSynchronize(st));
-                double *dt = (double *)d->tf_blob;
-                d->tf_yt = (double2 *)dt; d->tf_xt = (double2 *)(dt + npt); d->tf_wt = (double2 *)(dt + 2 * npt);
-                for (int t = 0; t < 4; t++) d->tf_ctab[t] = (p->cpl_fast || front_blk) ? (double2 *)(dt + (3 + t) * npt) : NULL;
-                for (int t = 0; t < 4; t++) d->tf_fu2[t] = front_s11 ? (double2 *)(dt + (7 + t) * npt) : NULL;
-                d->tf_mb = (uint4 *)(dt + (size_t)ntab * npt);
-                d->tf_itm = (uchar2 *)((unsigned int *)d->tf_mb + 2 * npt);
-            }
-            if (p->kern == K_LADDER || p->kern == K_TF) {
-                CUP(cudaMallocAsync((void **)&d->wsq2, 2 * (size_t)np * esz, st));
-                H2D(d->wsq2, p->precision == 32 ? (const void *)wsqf.data() : (const void *)wsq.data(), 2 * (size_t)np * esz);
-                CUP(cudaMallocAsync((void **)&d->ticket, QO_TICKET_BYTES, st));      /* the sample ticket + the per-SM arrival counters of qo_ts.cuh */
-                if (p->cpl_fast)
-                    for (int t = 0; t < 4; t++) {
-                        CUP(cudaMallocAsync((void **)&d->cpl_tab[t], 2 * (size_t)np * esz, st));
-                        H2D(d->cpl_tab[t], p->precision == 32 ? (const void *)ctabf[t].data() : (const void *)ctab[t].data(), 2 * (size_t)np * esz);
-                    }
-            }
-        } else {
-            CUP(cudaMallocAsync((void **)&d->fgrid, (size_t)nf * sizeof(double), st));
-            CUP(cudaMallocAsync((void **)&d->mask, (size_t)nf, st));
-            H2D(d->fgrid, f, (size_t)nf * sizeof(double));
-            H2D(d->mask, p->maskv.data(), (size_t)nf);
-        }
-        CUP(cudaMallocAsync((void **)&d->counters, (size_t)p->ncnt * sizeof(unsigned long long), st));
-        CUP(cudaMemsetAsync(d->counters, 0, (size_t)p->ncnt * sizeof(unsigned long long), st));
-        CUP(cudaStreamSynchronize(st));   /* the host staging vectors die at return */
-    }
+    rc = build_tables(p, net, f);
+    if (rc == QO_OK) rc = upload(p);
+    if (rc) { qo_plan_destroy(p); return rc; }
     if (p->kern == K_TF) tf_launch_setup(p, ov);
     *out = p;
     return QO_OK;
@@ -762,7 +769,7 @@ extern "C" const char *qo_plan_tf_info(const qo_plan *p, int info[6], double *se
     if (fused_err) *fused_err = p->tfp.fused_err;
     return p->tfp.reason ? p->tfp.reason : "";
 }
-extern "C" uint64_t qo_plan_h2d_bytes(const qo_plan *p) { return p ? p->h2d_bytes : 0; }
+extern "C" uint64_t qo_plan_h2d_bytes(const qo_plan *p) { return p ? p->lay.buf.size() : 0; }
 
 /* host-only part of qo_plan_create: compile the network, decide about the transfer-function kernel (needs no GPU) */
 extern "C" const char *qo_plan_analyze(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
@@ -803,10 +810,8 @@ extern "C" int qo_plan_reset(qo_plan *p)
     if (!p) return QO_ERR_ARG;
     for (int g = 0; g < p->ctx->ndev; g++) {
         CU(cudaSetDevice(p->ctx->d[g].device));
-        CU(cudaMemsetAsync(p->d[g].counters, 0, (size_t)p->ncnt * sizeof(unsigned long long), p->ctx->d[g].stream));
-        p->d[g].n_launched = 0;
+        CU(cudaMemsetAsync(p->counters(g), 0, (size_t)p->ncnt * sizeof(unsigned long long), p->ctx->d[g].stream));
     }
-    p->n_total_launched = 0;
     return QO_OK;
 }
 
@@ -838,8 +843,9 @@ template <typename T>
 static int launch_lumped(qo_plan *p, int g, unsigned long long off, unsigned long long n, unsigned long long *cnt, QoPlanes pl, int full_s)
 {
     DevCtx *dc = &p->ctx->d[g];
-    DevPlan *d = &p->d[g];
     typedef typename QoVec2<T>::type V2;
+    const DevProg *prog = p->dev<DevProg>(g, p->tab.prog);
+    const V2 *w2 = p->dev<V2>(g, p->tab.w2), *wi2 = p->dev<V2>(g, p->tab.wi2); const uchar2 *m2 = p->dev<uchar2>(g, p->tab.m2);
     const int resident = dc->sm_count * 2;                  /* __launch_bounds__(256, 2) */
     const unsigned long long warps_resident = (unsigned long long)resident * QO_WARPS;
     /* split the frequency axis only when there are too few samples to fill the GPU (sweeps) */
@@ -877,10 +883,8 @@ static int launch_lumped(qo_plan *p, int g, unsigned long long off, unsigned lon
                 grid = (int)(blocks < (unsigned long long)res2 ? blocks : (unsigned long long)res2);
                 if (grid < 1) grid = 1;
             }
-            const DevProg *a_prog = d->prog;
-            const void *a_w2 = d->w2, *a_wi2 = d->wi2, *a_m2 = d->m2;
             int a_nf = p->nf, a_np = p->npairs;
-            void *args[] = { &a_prog, &a_w2, &a_wi2, &a_m2, &a_nf, &a_np, &ppc, &nchunks, &off, &n, &cnt, &pl };
+            void *args[] = { &prog, &w2, &wi2, &m2, &a_nf, &a_np, &ppc, &nchunks, &off, &n, &cnt, &pl };
             CU(cudaLaunchKernel((const void *)je->kern, dim3((unsigned)grid), dim3(QO_TPB), args, 0, dc->stream));
             p->kernel_name = "qo_mc_chain_jit_kernel";
             return QO_OK;
@@ -888,8 +892,7 @@ static int launch_lumped(qo_plan *p, int g, unsigned long long off, unsigned lon
     }
     p->kernel_name = "qo_mc_lumped_kernel";
 #define QO_LAUNCH(FS, TR, GD)                                                                                       \
-    qo_mc_lumped_kernel<T, FS, TR, GD><<<grid, QO_TPB, 0, dc->stream>>>(d->prog, (const V2 *)d->w2, (const V2 *)d->wi2, \
-                                                                         d->m2, p->nf, p->npairs, ppc, nchunks, off, n, cnt, pl)
+    qo_mc_lumped_kernel<T, FS, TR, GD><<<grid, QO_TPB, 0, dc->stream>>>(prog, w2, wi2, m2, p->nf, p->npairs, ppc, nchunks, off, n, cnt, pl)
     if (full_s) { if (p->hp.has_trig) QO_LAUNCH(true, true, false); else QO_LAUNCH(true, false, false); }
     else if (p->hp.need_gd) { if (p->hp.has_trig) QO_LAUNCH(false, true, true); else QO_LAUNCH(false, false, true); }
     else { if (p->hp.has_trig) QO_LAUNCH(false, true, false); else QO_LAUNCH(false, false, false); }
@@ -901,18 +904,18 @@ static int launch_lumped(qo_plan *p, int g, unsigned long long off, unsigned lon
 static int launch_ladder(qo_plan *p, int g, unsigned long long off, unsigned long long n, unsigned long long *cnt, const double *cplms)
 {
     DevCtx *dc = &p->ctx->d[g];
-    DevPlan *d = &p->d[g];
     const DevProg *hp = &p->hp;
+    const QoTables &t = p->tab;
     LadParams P;
     memset(&P, 0, sizeof P);
-    P.prog = d->prog;
-    P.wt = d->w2; P.wit = d->wi2; P.wsqt = d->wsq2; P.m2 = d->m2;
+    P.prog = p->dev<DevProg>(g, t.prog);
+    P.wt = p->dev<void>(g, t.w2); P.wit = p->dev<void>(g, t.wi2); P.wsqt = p->dev<void>(g, t.wsq2); P.m2 = p->dev<uchar2>(g, t.m2);
     P.counters = cnt;
-    P.cse = d->cpl_tab[0]; P.cce = d->cpl_tab[1]; P.cso = d->cpl_tab[2]; P.cco = d->cpl_tab[3];
+    P.cse = p->dev<void>(g, t.cpl[0]); P.cce = p->dev<void>(g, t.cpl[1]); P.cso = p->dev<void>(g, t.cpl[2]); P.cco = p->dev<void>(g, t.cpl[3]);
     P.cpl_fast = p->cpl_fast; P.cpl_same = p->cpl_same;
     P.cplms = cplms; P.op0 = hp->op0;
-    P.ticket = d->ticket;
-    CU(cudaMemsetAsync(d->ticket, 0, sizeof(unsigned long long), dc->stream));
+    P.ticket = p->ticket(g);
+    CU(cudaMemsetAsync(P.ticket, 0, sizeof(unsigned long long), dc->stream));
     P.sample_offset = off; P.nsamples = n; P.seed = hp->seed;
     P.rs = hp->rs; P.rl = hp->rl; P.k21 = hp->k21; P.hist_lo = hp->hist_lo; P.hist_hi = hp->hist_hi;
     for (int s = 0; s < QO_LAD_NSPEC; s++) {
@@ -986,22 +989,23 @@ static void tf_launch_setup(qo_plan *p, const QoOverrides *ov)
 static int launch_tf(qo_plan *p, int g, unsigned long long off, unsigned long long n, unsigned long long *cnt, const double *cplms)
 {
     DevCtx *dc = &p->ctx->d[g];
-    DevPlan *d = &p->d[g];
     const DevProg *hp = &p->hp;
+    const QoTables &t = p->tab;
     TfParams P;
     memset(&P, 0, sizeof P);
-    P.prog = d->prog;
-    P.yt = d->tf_yt; P.xt = d->tf_xt; P.wt = d->tf_wt; P.mb = d->tf_mb; P.itm = d->tf_itm;
-    P.cse = d->tf_ctab[0]; P.cce = d->tf_ctab[1]; P.cso = d->tf_ctab[2]; P.cco = d->tf_ctab[3];
+    P.prog = p->dev<DevProg>(g, t.prog);
+    P.yt = p->dev<double2>(g, t.yt); P.xt = p->dev<double2>(g, t.xt); P.wt = p->dev<double2>(g, t.wt);
+    P.mb = p->dev<uint4>(g, t.mb); P.itm = p->dev<uchar2>(g, t.itm);
+    P.cse = p->dev<double2>(g, t.cpl[0]); P.cce = p->dev<double2>(g, t.cpl[1]); P.cso = p->dev<double2>(g, t.cpl[2]); P.cco = p->dev<double2>(g, t.cpl[3]);
     P.cpl_fast = p->cpl_fast; P.cpl_same = p->cpl_same; P.cpl_op = p->tfp.cpl_op;
     /* source resistance == the coupler's (unperturbed) reference impedance: the block's row vector collapses (qo_tf.cuh::tf_cpl_matched) */
     P.front = p->tfp.cpl_op >= 0 ? p->tfp.front : 0;
-    for (int t = 0; t < 4; t++) P.fu2[t] = d->tf_fu2[t];
+    for (int c = 0; c < 4; c++) P.fu2[c] = p->dev<double2>(g, t.fu2[c]);
     P.cpl_matched = p->tf_cpl_matched;
     P.cpl_lin = p->tf_cpl_lin; P.cpl_dw = p->tf_cpl_dw1 * (double)(64 * p->tf_pp);
     P.cplms = cplms;
-    P.counters = cnt; P.ticket = d->ticket;
-    CU(cudaMemsetAsync(d->ticket, 0, QO_TICKET_BYTES, dc->stream));
+    P.counters = cnt; P.ticket = p->ticket(g);
+    CU(cudaMemsetAsync(P.ticket, 0, QO_TICKET_BYTES, dc->stream));
     P.sample_offset = off; P.nsamples = n; P.seed = hp->seed;
     P.rs = hp->rs; P.rl = hp->rl; P.k21 = hp->k21; P.hist_lo = hp->hist_lo; P.hist_hi = hp->hist_hi;
     P.wref = p->tfp.wref; P.zn = sqrt(hp->rs * hp->rl); P.zni = 1.0 / P.zn;
@@ -1025,14 +1029,14 @@ static int launch_tf(qo_plan *p, int g, unsigned long long off, unsigned long lo
             memset(&Q, 0, sizeof Q);
             Q.t = P;
             Q.t.nsamples = nb * 32ull;
-            Q.y1 = (const double *)d->tf_yt; Q.x1 = (const double *)d->tf_xt; Q.mw = (const uint2 *)d->tf_mb;
+            Q.y1 = p->dev<double>(g, t.yt); Q.x1 = p->dev<double>(g, t.xt); Q.mw = p->dev<uint2>(g, t.mb);
             Q.npt = p->ts_npt;
             Q.nruns = p->ts_nruns; Q.nplain = p->ts_nplain;
             for (int r = 0; r < p->ts_nruns; r++) {
                 Q.runs[r].g0 = p->ts_runs[r].g0; Q.runs[r].ngroups = p->ts_runs[r].ngroups; Q.runs[r].any = p->ts_runs[r].any; Q.runs[r].all = p->ts_runs[r].all;
             }
             Q.nbatches = nb;
-            Q.ticket = d->ticket + 1;
+            Q.ticket = P.ticket + 1;
             Q.w0 = 6.283185307179586476925286766559 * p->f[0];
             Q.dw = p->nf > 1 ? 6.283185307179586476925286766559 * ((p->f[p->nf - 1] - p->f[0]) / (double)(p->nf - 1)) : 0.0;
             int rts = qo_ts_launch(&p->tfp, dc->sm_count, &Q, dc->stream);
@@ -1056,11 +1060,10 @@ static int launch_spot(qo_plan *p, int g, unsigned long long off, unsigned long 
     const DevProg *hp = &p->hp;
     SpotParams P;
     memset(&P, 0, sizeof P);
-    P.prog = p->d[g].prog; P.counters = cnt;
+    P.prog = p->dev<DevProg>(g, p->tab.prog); P.counters = cnt;
     P.sample_offset = off; P.nsamples = n; P.seed = hp->seed;
     P.rs = hp->rs; P.rl = hp->rl; P.k21 = hp->k21; P.hist_lo = hp->hist_lo; P.hist_hi = hp->hist_hi;
-    const double two_pi = 6.283185307179586476925286766559;
-    for (int k = 0; k < p->nf; k++) { P.w[k] = two_pi * p->f[k]; P.mask[k] = p->maskv[k]; }
+    for (int k = 0; k < p->nf; k++) { P.w[k] = grid_w(p->f.data(), p->nf, k); P.mask[k] = p->maskv[k]; }
     for (int s = 0; s < hp->nspec; s++) { P.thr[s] = hp->spec_thr[s]; P.kind[s] = hp->spec_kind[s]; }
     P.nf = p->nf; P.n_el = p->spot_nel; P.el0 = p->spot_el0; P.nspec = hp->nspec; P.dist = hp->dist;
     P.hist_bins = hp->hist_bins;
@@ -1078,29 +1081,30 @@ static int launch_tf_fs(qo_plan *p, int g, unsigned long long off, unsigned long
     DevCtx *dc = &p->ctx->d[g];
     DevPlan *d = &p->d[g];
     const DevProg *hp = &p->hp;
-    if (!d->fs_blob) {
+    QoLayout &L = p->fs_lay;
+    if (L.buf.empty()) {
         const int ppi = 32 * 2;
         p->fs_niter = (p->npairs + ppi - 1) / ppi;
         const size_t npt = 2 * (size_t)p->fs_niter * ppi;
-        std::vector<double> tab(2 * npt);
-        const double two_pi = 6.283185307179586476925286766559;
+        p->fs_yt = L.add(npt * sizeof(double)); p->fs_xt = L.add(npt * sizeof(double));
+        double *yt = L.host<double>(p->fs_yt), *xt = L.host<double>(p->fs_xt);
         for (size_t k = 0; k < npt; k++) {
-            const double x = two_pi * p->f[k < (size_t)p->nf ? k : (size_t)p->nf - 1] / p->fsp.wref;
-            tab[k] = -(x * x); tab[npt + k] = x;
+            const double x = grid_w(p->f.data(), p->nf, k) / p->fsp.wref;
+            yt[k] = -(x * x); xt[k] = x;
         }
-        CU(cudaMallocAsync((void **)&d->fs_blob, 2 * npt * sizeof(double), dc->stream));
-        CU(cudaMemcpyAsync(d->fs_blob, tab.data(), 2 * npt * sizeof(double), cudaMemcpyHostToDevice, dc->stream));
+    }
+    if (!d->fs_mem) {
+        CU(cudaMallocAsync((void **)&d->fs_mem, L.buf.size(), dc->stream));
+        CU(cudaMemcpyAsync(d->fs_mem, L.buf.data(), L.buf.size(), cudaMemcpyHostToDevice, dc->stream));
         CU(cudaStreamSynchronize(dc->stream));
-        d->fs_yt = (double2 *)d->fs_blob; d->fs_xt = (double2 *)((double *)d->fs_blob + npt);
-        if (!d->ticket) CU(cudaMallocAsync((void **)&d->ticket, sizeof(unsigned long long), dc->stream));
     }
     TfFsParams P;
     memset(&P, 0, sizeof P);
-    P.prog = d->prog; P.yt = d->fs_yt; P.xt = d->fs_xt;
+    P.prog = p->dev<DevProg>(g, p->tab.prog); P.yt = (const double2 *)(d->fs_mem + p->fs_yt); P.xt = (const double2 *)(d->fs_mem + p->fs_xt);
     P.s11 = pl.s11; P.s21 = pl.s21; P.s12 = pl.s12; P.s22 = pl.s22;
     P.planes_al32 = ((((size_t)pl.s11) | ((size_t)pl.s21) | ((size_t)pl.s12) | ((size_t)pl.s22)) & 31) == 0;
-    P.ticket = d->ticket;
-    CU(cudaMemsetAsync(d->ticket, 0, sizeof(unsigned long long), dc->stream));
+    P.ticket = p->ticket(g);
+    CU(cudaMemsetAsync(P.ticket, 0, sizeof(unsigned long long), dc->stream));
     P.sample_offset = off; P.nsamples = n; P.seed = hp->seed;
     P.rs = hp->rs; P.rl = hp->rl; P.k21 = hp->k21; P.wref = p->fsp.wref; P.zn = sqrt(hp->rs * hp->rl); P.zni = 1.0 / P.zn;
     P.nf = p->nf; P.niter = p->fs_niter; P.kn = p->fsp.kn; P.kd = p->fsp.kd; P.n_var = hp->n_var; P.n_el = p->fsp.n_el; P.el0 = p->fsp.el0; P.dist = hp->dist;
@@ -1119,16 +1123,17 @@ static int launch_tf_fs(qo_plan *p, int g, unsigned long long off, unsigned long
 static int launch_generic(qo_plan *p, int g, unsigned long long off, unsigned long long n, unsigned long long *cnt, QoPlanes pl, int full_s)
 {
     DevCtx *dc = &p->ctx->d[g];
-    DevPlan *d = &p->d[g];
+    const DevProg *prog = p->dev<DevProg>(g, p->tab.prog);
+    const double *fgrid = p->dev<double>(g, p->tab.fgrid); const unsigned char *mask = p->dev<unsigned char>(g, p->tab.mask);
     if (p->kern == K_BOARD) {
         /* yield at a handful of frequencies: one thread per board, the frequencies side by side (qo_ustrip_board.cuh) */
         const unsigned long long cap = (unsigned long long)dc->sm_count * QO_B_MINB, want = (n + QO_B_TPB - 1) / QO_B_TPB;
         const int grid = (int)(want < cap ? want : cap);
         switch (p->nf) {
-        case 1: qo_mc_board_kernel<1><<<grid, QO_B_TPB, 0, dc->stream>>>(d->prog, d->fgrid, d->mask, off, n, cnt); break;
-        case 2: qo_mc_board_kernel<2><<<grid, QO_B_TPB, 0, dc->stream>>>(d->prog, d->fgrid, d->mask, off, n, cnt); break;
-        case 3: qo_mc_board_kernel<3><<<grid, QO_B_TPB, 0, dc->stream>>>(d->prog, d->fgrid, d->mask, off, n, cnt); break;
-        default: qo_mc_board_kernel<4><<<grid, QO_B_TPB, 0, dc->stream>>>(d->prog, d->fgrid, d->mask, off, n, cnt); break;
+        case 1: qo_mc_board_kernel<1><<<grid, QO_B_TPB, 0, dc->stream>>>(prog, fgrid, mask, off, n, cnt); break;
+        case 2: qo_mc_board_kernel<2><<<grid, QO_B_TPB, 0, dc->stream>>>(prog, fgrid, mask, off, n, cnt); break;
+        case 3: qo_mc_board_kernel<3><<<grid, QO_B_TPB, 0, dc->stream>>>(prog, fgrid, mask, off, n, cnt); break;
+        default: qo_mc_board_kernel<4><<<grid, QO_B_TPB, 0, dc->stream>>>(prog, fgrid, mask, off, n, cnt); break;
         }
         CU(cudaGetLastError());
         return QO_OK;
@@ -1155,7 +1160,7 @@ static int launch_generic(qo_plan *p, int g, unsigned long long off, unsigned lo
     unsigned long long cap = (unsigned long long)dc->sm_count * 8;
     int grid = (int)(tiles < cap ? tiles : cap);
     if (grid < 1) grid = 1;
-    qo_mc_generic_kernel<<<grid, QO_G_TPB, 0, dc->stream>>>(d->prog, d->fgrid, d->mask, p->nf, f_chunk, n_fchunks, sb, off, n, cnt, pl, full_s);
+    qo_mc_generic_kernel<<<grid, QO_G_TPB, 0, dc->stream>>>(prog, fgrid, mask, p->nf, f_chunk, n_fchunks, sb, off, n, cnt, pl, full_s);
     CU(cudaGetLastError());
     return QO_OK;
 }
@@ -1166,12 +1171,12 @@ static int plan_launch_dev(qo_plan *p, int g, unsigned long long off, unsigned l
     if (n == 0) return QO_OK;
     CU(cudaSetDevice(p->ctx->d[g].device));
     int full_s = p->mode == QO_MODE_FULL_S;
-    QoPlanes pl = { NULL, NULL, NULL, NULL, p->d[g].sblk, p->d[g].sdet, 2 * p->npairs, NULL };
+    QoPlanes pl = { NULL, NULL, NULL, NULL, p->dev<double2>(g, p->tab.sblk), p->dev<double2>(g, p->tab.sdet), 2 * p->npairs, NULL };
     double *cplms = NULL;
     if (p->hp.cplms_elem >= 0) {
         DevCtx *dc = &p->ctx->d[g];
         CU(cudaMallocAsync((void **)&cplms, (size_t)n * 4 * sizeof(double), dc->stream));
-        qo_cplms_kernel<<<(unsigned)((n + 127) / 128), 128, 0, dc->stream>>>(p->d[g].prog, off, n, cplms);
+        qo_cplms_kernel<<<(unsigned)((n + 127) / 128), 128, 0, dc->stream>>>(p->dev<DevProg>(g, p->tab.prog), off, n, cplms);
         { cudaError_t e_ = cudaGetLastError(); if (e_ != cudaSuccess) { cudaFreeAsync(cplms, dc->stream); qo_set_error("qo_cplms_kernel launch -> %s", cudaGetErrorString(e_)); return QO_ERR_CUDA; } }
         pl.cplms = cplms;
         p->launches++;
@@ -1194,7 +1199,7 @@ static int plan_launch_dev(qo_plan *p, int g, unsigned long long off, unsigned l
     default: rc = p->precision == 32 ? launch_lumped<float>(p, g, off, n, cnt, pl, full_s) : launch_lumped<double>(p, g, off, n, cnt, pl, full_s); break;
     }
     if (cplms) cudaFreeAsync(cplms, p->ctx->d[g].stream);
-    if (rc == QO_OK) { p->launches++; p->d[g].n_launched += n; }
+    if (rc == QO_OK) p->launches++;
     return rc;
 }
 
@@ -1204,19 +1209,16 @@ extern "C" int qo_plan_launch(qo_plan *p, uint64_t sample_offset, uint64_t n_sam
     if (!p) return QO_ERR_ARG;
     qo_ctx *c = p->ctx;
     if (c->ndev == 1) {
-        unsigned long long *cnt = counters_dev ? (unsigned long long *)counters_dev : p->d[0].counters;
-        int rc = plan_launch_dev(p, 0, sample_offset, n_samples, cnt, full_s_dev, n_samples, 0);
-        if (rc == QO_OK) p->n_total_launched += n_samples;
-        return rc;
+        unsigned long long *cnt = counters_dev ? (unsigned long long *)counters_dev : p->counters(0);
+        return plan_launch_dev(p, 0, sample_offset, n_samples, cnt, full_s_dev, n_samples, 0);
     }
     if (counters_dev || full_s_dev) { qo_set_error("caller-owned device buffers need a single-device ctx"); return QO_ERR_ARG; }
     /* shard the contiguous global sample range; Philox counters carry the GLOBAL index */
     for (int g = 0; g < c->ndev; g++) {
         unsigned long long a = n_samples * (unsigned long long)g / c->ndev, b = n_samples * (unsigned long long)(g + 1) / c->ndev;
-        int rc = plan_launch_dev(p, g, sample_offset + a, b - a, p->d[g].counters, NULL, 0, 0);
+        int rc = plan_launch_dev(p, g, sample_offset + a, b - a, p->counters(g), NULL, 0, 0);
         if (rc) return rc;
     }
-    p->n_total_launched += n_samples;
     return QO_OK;
 }
 
@@ -1231,20 +1233,20 @@ extern "C" int qo_plan_read(qo_plan *p, qo_mc_result *res)
         c->nccl.GroupStart();
         for (int g = 0; g < c->ndev; g++) {
             cudaSetDevice(c->d[g].device);
-            int r = c->nccl.AllReduce(p->d[g].counters, p->d[g].counters, (size_t)p->ncnt, QO_NCCL_UINT64, QO_NCCL_SUM, c->comm[g], c->d[g].stream);
+            int r = c->nccl.AllReduce(p->counters(g), p->counters(g), (size_t)p->ncnt, QO_NCCL_UINT64, QO_NCCL_SUM, c->comm[g], c->d[g].stream);
             if (r) { c->nccl.GroupEnd(); qo_set_error("ncclAllReduce failed (%d)", r); return QO_ERR_NCCL; }
         }
         if (c->nccl.GroupEnd()) { qo_set_error("ncclGroupEnd failed"); return QO_ERR_NCCL; }
         for (int g = 0; g < c->ndev; g++) { CU(cudaSetDevice(c->d[g].device)); CU(cudaStreamSynchronize(c->d[g].stream)); }
         CU(cudaSetDevice(c->d[0].device));
-        CU(cudaMemcpy(h.data(), p->d[0].counters, (size_t)p->ncnt * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(h.data(), p->counters(0), (size_t)p->ncnt * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
         /* counters now hold the global sum on every device: keep only device 0's copy as the accumulator */
-        for (int g = 1; g < c->ndev; g++) { CU(cudaSetDevice(c->d[g].device)); CU(cudaMemset(p->d[g].counters, 0, (size_t)p->ncnt * sizeof(unsigned long long))); }
+        for (int g = 1; g < c->ndev; g++) { CU(cudaSetDevice(c->d[g].device)); CU(cudaMemset(p->counters(g), 0, (size_t)p->ncnt * sizeof(unsigned long long))); }
     } else {
         for (int g = 0; g < c->ndev; g++) {
             CU(cudaSetDevice(c->d[g].device));
             CU(cudaStreamSynchronize(c->d[g].stream));
-            CU(cudaMemcpy(tmp.data(), p->d[g].counters, (size_t)p->ncnt * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(tmp.data(), p->counters(g), (size_t)p->ncnt * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
             for (int i = 0; i < p->ncnt; i++) h[i] += tmp[i];
         }
     }
@@ -1291,21 +1293,16 @@ extern "C" int qo_mc_run(qo_ctx *ctx, const qo_net *net, const double *f, int nf
     const bool cacheable = net->nblk == 0 && !getenv("QO100NET_NO_PLAN_CACHE");      /* measured blocks are not hashed: no reuse */
     if (cacheable && ctx->mc_cache && ctx->mc_cache_key == key && ctx->mc_cache->nf == nf) {
         p = ctx->mc_cache;
-        for (int g = 0; g < ctx->ndev; g++) {                 /* the call's inputs travel host -> device every time */
+        /* the call's inputs travel host -> device every time.  Copies from pageable memory are staged by the driver (~12 us
+         * each): the tables go from one page-locked copy, and the re-sends are then truly asynchronous */
+        const size_t nb = p->lay.buf.size();
+        if (!p->pinned) {
+            if (cudaHostAlloc((void **)&p->pinned, nb, cudaHostAllocDefault) == cudaSuccess) memcpy(p->pinned, p->lay.buf.data(), nb);
+            else { cudaGetLastError(); p->pinned = NULL; }
+        }
+        for (int g = 0; g < ctx->ndev; g++) {
             CU(cudaSetDevice(ctx->d[g].device));
-            if (!p->pinned[g]) {
-                /* copies from pageable memory are staged by the driver one by one (~12 us each, eight of them per call): gather
-                 * the plan's tables in one page-locked buffer, the re-sends are then truly asynchronous */
-                size_t tot = 0;
-                for (auto &u : p->uploads[g]) { u.at = tot; tot += (u.data.size() + 255) & ~(size_t)255; }
-                if (tot && cudaHostAlloc((void **)&p->pinned[g], tot, cudaHostAllocDefault) == cudaSuccess) {
-                    for (auto &u : p->uploads[g]) { memcpy(p->pinned[g] + u.at, u.data.data(), u.data.size()); }
-                } else { cudaGetLastError(); p->pinned[g] = NULL; }
-            }
-            for (size_t i = 0; i < p->uploads[g].size(); i++) {
-                const qo_plan::Upload &u = p->uploads[g][i];
-                CU(cudaMemcpyAsync(u.dst, p->pinned[g] ? (const void *)(p->pinned[g] + u.at) : (const void *)u.data.data(), u.data.size(), cudaMemcpyHostToDevice, ctx->d[g].stream));
-            }
+            CU(cudaMemcpyAsync(p->d[g].mem, p->pinned ? (const void *)p->pinned : (const void *)p->lay.buf.data(), nb, cudaMemcpyHostToDevice, ctx->d[g].stream));
         }
         rc = qo_plan_reset(p);
         if (rc) return rc;
@@ -1328,7 +1325,7 @@ extern "C" int qo_mc_run(qo_ctx *ctx, const qo_net *net, const double *f, int nf
         if (fs && n) {
             if (cudaMalloc(&dbuf[g], 4 * (size_t)n * nf * sizeof(qo_c64)) != cudaSuccess) { cudaGetLastError(); qo_set_error("cannot allocate %zu bytes for FULL_S output", 4 * (size_t)n * nf * sizeof(qo_c64)); rc = QO_ERR_NOMEM; break; }
         }
-        rc = plan_launch_dev(p, g, cfg->sample_offset + a[g], n, p->d[g].counters, dbuf[g], n, 0);
+        rc = plan_launch_dev(p, g, cfg->sample_offset + a[g], n, p->counters(g), dbuf[g], n, 0);
         cudaEventRecord(ctx->d[g].ev1, ctx->d[g].stream);
     }
     const auto tt2 = std::chrono::steady_clock::now();
@@ -1413,7 +1410,7 @@ extern "C" int qo_sweep(qo_ctx *ctx, const qo_net *net, const double *f, int nf,
     cudaSetDevice(dc->device);
     do {
         if (cudaMallocAsync((void **)&buf, 4 * (size_t)nft * sizeof(double2), dc->stream) != cudaSuccess) { rc = QO_ERR_NOMEM; break; }
-        rc = plan_launch_dev(p, 0, 0, 1, p->d[0].counters, (qo_c64 *)buf, 1, 0);
+        rc = plan_launch_dev(p, 0, 0, 1, p->counters(0), (qo_c64 *)buf, 1, 0);
         if (rc) break;
         if (gd) {
             if (cudaMallocAsync((void **)&dgd, (size_t)nf * sizeof(double), dc->stream) != cudaSuccess ||

@@ -691,7 +691,8 @@ class Plan:
 
     @property
     def h2d_bytes(self):
-        """Host->device bytes qo_plan_create copied (per GPU)."""
+        """Host->device bytes of the plan's tables per GPU, alignment padding included: copied at creation, and again by every
+        Context.mc_run call that reuses the plan."""
         return int(lib().qo_plan_h2d_bytes(self._h))
 
     def reset(self):
