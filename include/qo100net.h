@@ -317,6 +317,13 @@ const char *qo_plan_tf_info(const qo_plan *plan, int info[6], double *self_check
  * QO100NET_KERNEL value): info[0] = QO_ERR_ARG and the reason string says why. */
 const char *qo_plan_analyze(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
                             int info[6], double *self_check_err, unsigned int *fused, double *fused_err, double *seconds);
+/* the thread-per-sample kernel's run table: 7 ints per run (first group of points, groups, spec bits seen by some point of the
+ * run, by every point, numerator pairs, E coefficients and fused-margin coefficients the run walks), up to cap runs.  Returns
+ * the number of runs (0: the job does not run thread-per-sample), meta[0] = runs walked on |numerator|^2 and E (the fused
+ * spec's runs follow), meta[1] = points per group.  The _analyze form needs no GPU, like qo_plan_analyze. */
+int qo_plan_ts_runs(const qo_plan *plan, int *runs, int cap, int meta[2]);
+int qo_plan_analyze_ts_runs(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
+                            int *runs, int cap, int meta[2]);
 /* host->device bytes of this plan's tables per GPU, alignment padding included: the tables its kernel reads, copied by
  * qo_plan_create and again by every qo_mc_run call that reuses the plan */
 uint64_t qo_plan_h2d_bytes(const qo_plan *plan);

@@ -92,9 +92,8 @@ struct qo_plan {
     QoOverrides ov;                                       /* the environment overrides as they were at plan creation */
     QoKern kern;
     /* launch-time decisions of the transfer-function kernels, taken once at plan creation */
-    int tf_cpl_matched, tf_cpl_lin, ts_ok, ts_runs_ok, ts_nruns, ts_nplain, ts_npt;
+    int tf_cpl_matched, tf_cpl_lin, ts_ok;
     double tf_cpl_dw1;                                    /* angular-frequency step of one grid point on a uniformly spaced grid */
-    struct { int g0, ngroups; unsigned int any, all; } ts_runs[QO_TS_MAXRUN];
     int lad_n, lad_first, lad_cpl;                        /* straight-line ladder kernel (qo_ladder.cuh) */
     int cpl_fast, cpl_same;                               /* coupler block: small-angle table path, equal mode angles */
     int spot_el0, spot_nel;                               /* spot-frequency kernel (qo_spot.cuh): <= 8 points per sample */
@@ -771,14 +770,17 @@ extern "C" const char *qo_plan_tf_info(const qo_plan *p, int info[6], double *se
 }
 extern "C" uint64_t qo_plan_h2d_bytes(const qo_plan *p) { return p ? p->lay.buf.size() : 0; }
 
-/* host-only part of qo_plan_create: compile the network, decide about the transfer-function kernel (needs no GPU) */
-extern "C" const char *qo_plan_analyze(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
-                                       int info[6], double *self_check_err, unsigned int *fused, double *fused_err, double *seconds)
+/* host-only part of qo_plan_create: compile the network, decide about the transfer-function kernel (needs no GPU).
+ * Returns the reason (or the error), *sel = 1 when the job takes the transfer-function kernel, < 0 on an error */
+static const char *plan_analyze(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
+                                TfPlan *tp, int *sel, double *seconds)
 {
     qo_clear_error();
-    if (!net || !f || nf <= 0 || !info) return "bad arguments";
+    memset(tp, 0, sizeof *tp);
+    *sel = 0;
+    if (!net || !f || nf <= 0) { *sel = QO_ERR_ARG; return "bad arguments"; }
     QoOverrides ov;
-    if ((info[0] = qo_overrides_read(&ov)) != QO_OK) return qo_last_error();
+    if ((*sel = qo_overrides_read(&ov)) != QO_OK) return qo_last_error();
     DevProg *hp = new DevProg;
     int generic = 0;
     double fl = 0;
@@ -786,23 +788,64 @@ extern "C" const char *qo_plan_analyze(const qo_net *net, const double *f, int n
     struct timespec t0, t1;
     clock_gettime(CLOCK_MONOTONIC, &t0);
     int rc = build_prog(net, f, nf, spec, nspec, cfg, hp, &generic, &fl, &maskv);
-    TfPlan tp;
-    memset(&tp, 0, sizeof tp);
     const char *reason = "network does not compile";
     if (rc == QO_OK) {
         const int precision = cfg && cfg->precision == 32 ? 32 : 64;
         const int mode = cfg ? cfg->mode : QO_MODE_FULL_S;
-        int sel = qo_tf_plan_check(hp, mode == QO_MODE_REDUCE_ONLY, precision, generic, f, nf, maskv.data(), &ov, &tp);
-        info[0] = sel; info[1] = tp.nn; info[2] = tp.den; info[3] = tp.kn; info[4] = tp.kd; info[5] = tp.deg;
-        if (self_check_err) *self_check_err = tp.err;
-        if (fused) *fused = tp.fused;
-        if (fused_err) *fused_err = tp.fused_err;
-        reason = tp.reason ? tp.reason : "";
+        *sel = qo_tf_plan_check(hp, mode == QO_MODE_REDUCE_ONLY, precision, generic, f, nf, maskv.data(), &ov, tp);
+        reason = tp->reason ? tp->reason : "";
     }
     clock_gettime(CLOCK_MONOTONIC, &t1);
     if (seconds) *seconds = (double)(t1.tv_sec - t0.tv_sec) + 1e-9 * (double)(t1.tv_nsec - t0.tv_nsec);
     delete hp;
     return reason;
+}
+
+extern "C" const char *qo_plan_analyze(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
+                                       int info[6], double *self_check_err, unsigned int *fused, double *fused_err, double *seconds)
+{
+    if (!net || !f || nf <= 0 || !info) return "bad arguments";
+    TfPlan tp;
+    const char *reason = plan_analyze(net, f, nf, spec, nspec, cfg, &tp, &info[0], seconds);
+    if (info[0] < 0) return reason;
+    info[1] = tp.nn; info[2] = tp.den; info[3] = tp.kn; info[4] = tp.kd; info[5] = tp.deg;
+    if (self_check_err) *self_check_err = tp.err;
+    if (fused) *fused = tp.fused;
+    if (fused_err) *fused_err = tp.fused_err;
+    return reason;
+}
+
+#define QO_TS_RUN_INTS 7
+/* the thread-per-sample kernel's run table, QO_TS_RUN_INTS ints per run (first group, groups, spec bits seen by some point, by
+ * every point, numerator pairs, E coefficients, fused-margin coefficients); returns the number of runs (0 when the job cannot run
+ * thread-per-sample), meta = { plain runs (the fused spec's follow), points per group } */
+static int ts_runs_out(const TfPlan *tp, int *runs, int cap, int meta[2])
+{
+    if (!tp->ts_runs_ok) { if (meta) meta[0] = meta[1] = 0; return 0; }
+    if (meta) { meta[0] = tp->ts_nplain; meta[1] = qo_ts_group_points(tp); }
+    for (int r = 0; r < tp->ts_nruns && r < cap; r++) {
+        const TsRun &u = tp->runs[r];
+        int *o = runs + QO_TS_RUN_INTS * r;
+        o[0] = u.g0; o[1] = u.ngroups; o[2] = (int)u.any; o[3] = (int)u.all; o[4] = u.kn; o[5] = u.ke; o[6] = u.kf;
+    }
+    return tp->ts_nruns;
+}
+
+extern "C" int qo_plan_ts_runs(const qo_plan *p, int *runs, int cap, int meta[2])
+{
+    if (!p || (cap > 0 && !runs)) return QO_ERR_ARG;
+    return ts_runs_out(&p->tfp, runs, cap, meta);
+}
+
+extern "C" int qo_plan_analyze_ts_runs(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
+                                       int *runs, int cap, int meta[2])
+{
+    if (cap > 0 && !runs) return QO_ERR_ARG;
+    TfPlan tp;
+    int sel;
+    plan_analyze(net, f, nf, spec, nspec, cfg, &tp, &sel, NULL);
+    if (sel < 0) return sel;
+    return ts_runs_out(&tp, runs, cap, meta);
 }
 
 extern "C" int qo_plan_reset(qo_plan *p)
@@ -935,8 +978,7 @@ static int launch_ladder(qo_plan *p, int g, unsigned long long off, unsigned lon
 }
 
 /* what launch_tf needs beyond the tables, decided once per plan: the coupler block's form (matched source, uniformly spaced
- * grid), whether large launches may run thread-per-sample, and that kernel's run table (runs of point groups that see the same
- * spec bits; a group that straddles a band edge stands alone) */
+ * grid) and whether large launches may run thread-per-sample (on the run table the analysis built: qo_tf.cu::tf_ts_runs) */
 static void tf_launch_setup(qo_plan *p, const QoOverrides *ov)
 {
     const DevProg *hp = &p->hp;
@@ -954,36 +996,6 @@ static void tf_launch_setup(qo_plan *p, const QoOverrides *ov)
     }
     const bool rot_same = p->tf_cpl_lin && p->tf_cpl_matched && p->cpl_same && hp->cplms_elem < 0;
     p->ts_ok = ov->kernel != QoOverrides::TF && qo_ts_eligible(&p->tfp, hp->nspec, rot_same);     /* KERNEL=tf: warp-per-sample only (A/B runs) */
-    p->ts_nruns = 0; p->ts_nplain = 0; p->ts_runs_ok = 1; p->ts_npt = 0;
-    if (p->ts_ok) {
-        const int gpt = qo_ts_group_points(&p->tfp);
-        p->ts_npt = (p->nf + gpt - 1) / gpt * gpt;
-        for (int gi = 0; gi < p->ts_npt / gpt; gi++) {
-            unsigned int any = 0, all = 0xFF;
-            for (int k = gi * gpt; k < (gi + 1) * gpt; k++) { const unsigned int mk = k < p->nf ? p->maskv[k] : 0; any |= mk; all &= mk; }
-            if (p->ts_nruns > 0 && any == all && p->ts_runs[p->ts_nruns - 1].any == any && p->ts_runs[p->ts_nruns - 1].all == all) { p->ts_runs[p->ts_nruns - 1].ngroups++; continue; }
-            if (p->ts_nruns == QO_TS_MAXRUN) { p->ts_runs_ok = 0; break; }       /* more band edges than the run table holds: warp-per-sample */
-            p->ts_runs[p->ts_nruns].g0 = gi; p->ts_runs[p->ts_nruns].ngroups = 1; p->ts_runs[p->ts_nruns].any = any; p->ts_runs[p->ts_nruns].all = all; p->ts_nruns++;
-        }
-        /* the runs of the fused spec (one spec active, its margin a single polynomial: qo_tf_fuse) go last -- the verdict does
-         * not depend on the order, and the kernel forms the polynomial once, after the other runs, in the registers of the
-         * expansion.  One polynomial per sample: of the specs the plan accepts for it, the one that covers the most groups */
-        auto one_spec = [&](int r) -> int {
-            const unsigned int all = p->ts_runs[r].all;
-            if (p->tfp.cpl_op >= 0 || p->ts_runs[r].any != all || all == 0u || (all & (all - 1u))) return -1;
-            const int s = __builtin_ctz(all);
-            return (p->tfp.fused >> s) & 1u ? s : -1;
-        };
-        int ng[QO_TF_NSPEC] = { 0 }, fs = -1;
-        for (int r = 0; r < p->ts_nruns; r++) if (one_spec(r) >= 0) ng[one_spec(r)] += p->ts_runs[r].ngroups;
-        for (int s = 0; s < QO_TF_NSPEC; s++) if (ng[s] > 0 && (fs < 0 || ng[s] > ng[fs])) fs = s;
-        decltype(p->ts_runs) sorted;
-        int n = 0;
-        for (int r = 0; r < p->ts_nruns; r++) if (fs < 0 || one_spec(r) != fs) sorted[n++] = p->ts_runs[r];
-        p->ts_nplain = n;
-        for (int r = 0; r < p->ts_nruns; r++) if (fs >= 0 && one_spec(r) == fs) sorted[n++] = p->ts_runs[r];
-        memcpy(p->ts_runs, sorted, sizeof sorted);
-    }
 }
 
 static int launch_tf(qo_plan *p, int g, unsigned long long off, unsigned long long n, unsigned long long *cnt, const double *cplms)
@@ -1020,7 +1032,7 @@ static int launch_tf(qo_plan *p, int g, unsigned long long off, unsigned long lo
     P.hist_spec = hp->hist_bins > 0 ? hp->hist_spec : -1;
     /* the bulk of a large launch runs thread-per-sample (qo_ts.cuh): whole rounds of one sample per resident thread, dealt
      * statically; what is left over (less than one wave) stays on the warp-per-sample kernel below */
-    if (p->ts_ok && p->ts_runs_ok) {
+    if (p->ts_ok && p->tfp.ts_runs_ok) {
         /* worth it from a few batches per resident warp on (one wave = every resident thread one sample) */
         const unsigned long long wave = (unsigned long long)qo_ts_wave_threads(&p->tfp, dc->sm_count);
         const unsigned long long nb = wave && n >= 2 * wave ? n / 32ull : 0;
@@ -1030,11 +1042,9 @@ static int launch_tf(qo_plan *p, int g, unsigned long long off, unsigned long lo
             Q.t = P;
             Q.t.nsamples = nb * 32ull;
             Q.y1 = p->dev<double>(g, t.yt); Q.x1 = p->dev<double>(g, t.xt); Q.mw = p->dev<uint2>(g, t.mb);
-            Q.npt = p->ts_npt;
-            Q.nruns = p->ts_nruns; Q.nplain = p->ts_nplain;
-            for (int r = 0; r < p->ts_nruns; r++) {
-                Q.runs[r].g0 = p->ts_runs[r].g0; Q.runs[r].ngroups = p->ts_runs[r].ngroups; Q.runs[r].any = p->ts_runs[r].any; Q.runs[r].all = p->ts_runs[r].all;
-            }
+            Q.npt = p->tfp.ts_npt;
+            Q.nruns = p->tfp.ts_nruns; Q.nplain = p->tfp.ts_nplain;
+            memcpy(Q.runs, p->tfp.runs, sizeof Q.runs);
             Q.nbatches = nb;
             Q.ticket = P.ticket + 1;
             Q.w0 = 6.283185307179586476925286766559 * p->f[0];

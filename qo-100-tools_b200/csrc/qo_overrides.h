@@ -21,6 +21,7 @@ struct QoOverrides {
     int tf_no_front;      /* QO100NET_TF_NO_FRONT set: no line / measured two-port in front of the transfer-function kernel */
     int cpl_sincos;       /* QO100NET_CPL_SINCOS set: coupler angles by sincos per point, no table of nominal angles */
     int ustrip_item;      /* QO100NET_USTRIP=item: microstrip yield jobs on the item kernel, not thread-per-board */
+    int ts_full_len;      /* QO100NET_TS_FULL_LENGTHS set: every run of the thread-per-sample kernel walks the plan's full polynomial lengths */
 };
 
 /* QO_ERR_ARG (qo_last_error names the accepted values) when QO100NET_KERNEL holds anything but auto, spot, tf, ladder, interp */
@@ -44,6 +45,7 @@ static inline int qo_overrides_read(QoOverrides *ov)
     ov->cpl_sincos = getenv("QO100NET_CPL_SINCOS") != NULL;
     const char *u = getenv("QO100NET_USTRIP");
     ov->ustrip_item = u && !strcmp(u, "item");
+    ov->ts_full_len = getenv("QO100NET_TS_FULL_LENGTHS") != NULL;
     return QO_OK;
 }
 

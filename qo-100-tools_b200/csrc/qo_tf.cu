@@ -167,6 +167,21 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
  * from the same truncated polynomials in long double.  A stop band passes easily (~1e-13); the pass band of a ripple filter
  * usually does not, |Num|^2 cancelling inside the ripple (~1e-11). */
 #define QO_TF_FUSE_TOL 1e-12
+/* the device's F of nfz coefficients (its Horner in double) against the unfused margin from the same truncated polynomials in
+ * long double at x, relative to |Num|^2 */
+static double tf_fuse_point_err(const double *cn, const double *ee, int kn, int ke, const double *fz, int nfz, double t, bool neg, double x)
+{
+    const double y = -(x * x);
+    double got = fz[nfz - 1];
+    for (int m = nfz - 2; m >= 0; m--) got = fma(got, y, fz[m]);
+    const long double yl = y;
+    long double r0 = cn[2 * kn - 2], r1 = cn[2 * kn - 1], e = ke > 0 ? ee[ke - 1] : 1.0;
+    for (int i = kn - 2; i >= 0; i--) { r0 = r0 * yl + cn[2 * i]; r1 = r1 * yl + cn[2 * i + 1]; }
+    for (int m = ke - 2; m >= 0; m--) e = e * yl + ee[m];
+    const long double n2 = r0 * r0 - yl * r1 * r1, ref = neg ? n2 - t * e : t * e - n2;
+    const double err = (double)(fabsl((long double)got - ref) / n2);
+    return err == err ? err : 1e300;
+}
 static void tf_fuse_gate(const DevProg *hp, int nf, const double *xg, const unsigned char *mask, const std::vector<TfCorner> &cs,
                          double zni, TfPlan *out)
 {
@@ -188,16 +203,7 @@ static void tf_fuse_gate(const DevProg *hp, int nf, const double *xg, const unsi
             for (int k = 0; k < nf; k++) {
                 if (mask[k] != 1u << s) continue;
                 npts++;
-                const double x = xg[k], y = -(x * x);
-                double got = fz[nfz - 1];
-                for (int m = nfz - 2; m >= 0; m--) got = fma(got, y, fz[m]);
-                const long double yl = y;
-                long double r0 = cn[2 * kn - 2], r1 = cn[2 * kn - 1], e = ke > 0 ? cs[ci].ee[ke - 1] : 1.0;
-                for (int i = kn - 2; i >= 0; i--) { r0 = r0 * yl + cn[2 * i]; r1 = r1 * yl + cn[2 * i + 1]; }
-                for (int m = ke - 2; m >= 0; m--) e = e * yl + cs[ci].ee[m];
-                const long double n2 = r0 * r0 - yl * r1 * r1, ref = neg ? n2 - t * e : t * e - n2;
-                double err = (double)(fabsl((long double)got - ref) / n2);
-                if (!(err == err)) err = 1e300;
+                const double err = tf_fuse_point_err(cn, cs[ci].ee, kn, ke, fz, nfz, t, neg, xg[k]);
                 if (err > worst) worst = err;
             }
         }
@@ -289,6 +295,163 @@ extern "C" int qo_tf_plan_check(const DevProg *hp, int mode_reduce_only, int pre
     return sel;
 }
 
+/* The thread-per-sample kernel's run table (qo_ts.cuh): runs of groups of points that see the same spec bits (a group that
+ * straddles a band edge stands alone), the fused spec's runs last, and per run the polynomial lengths its own points need.
+ * The plan's lengths are what the top of the grid needs -- the top coefficients come from the parasitics' self-resonances far
+ * above the band -- and lower down they drop out.  Per run, the plan's rule on the run's points only (need_n / need_e: the
+ * same corners and bound, whole pairs, an even E, at least two rows); on the fused spec's runs, F's top coefficients while
+ * what they add stays below `trunc` of |Num|^2.  A run splits where the lengths its groups need step (a stretch shorter than
+ * QO_TS_MINSPLIT groups joins a neighbour; each split of a fused run costs one reload of the grid values).  A run whose
+ * shorter lengths fail the self-check (check_point) or the fused-margin gate walks the plan's lengths. */
+#define QO_TS_MINSPLIT 16
+template <class CHECK>
+static void tf_ts_runs(const DevProg *hp, int nf, const unsigned char *mask, const double *xg, const std::vector<TfCorner> &cs, double zni,
+                       const int *need_n, const int *need_e, double trunc, double tol, int full_len, CHECK check_point, TfPlan *out)
+{
+    out->ts_nruns = out->ts_nplain = out->ts_npt = out->ts_runs_ok = 0;
+    if (!qo_ts_eligible(out, hp->nspec, 1)) return;
+    const int gpt = qo_ts_group_points(out), ngr = (nf + gpt - 1) / gpt;
+    const int KN = out->kn, KE = out->den == QO_TF_DEN_E ? out->kd : 0, NF = 2 * KN > KE ? 2 * KN : KE, NN = out->nn;
+    out->ts_npt = ngr * gpt;
+    std::vector<TsRun> raw;
+    for (int gi = 0; gi < ngr; gi++) {
+        unsigned int any = 0, all = 0xFF;
+        for (int k = gi * gpt; k < (gi + 1) * gpt; k++) { const unsigned int mk = k < nf ? mask[k] : 0; any |= mk; all &= mk; }
+        if (!raw.empty() && any == all && raw.back().any == any && raw.back().all == all) { raw.back().ngroups++; continue; }
+        raw.push_back(TsRun{ gi, 1, any, all, KN, KE, 0 });
+    }
+    /* the fused spec: of the specs the gate accepted, the one whose single-spec runs cover the most groups */
+    auto one_spec = [&](const TsRun &r) -> int {
+        if (out->cpl_op >= 0 || r.any != r.all || r.all == 0u || (r.all & (r.all - 1u))) return -1;
+        const int s = __builtin_ctz(r.all);
+        return (out->fused >> s) & 1u ? s : -1;
+    };
+    int ng[QO_TF_NSPEC] = { 0 }, fs = -1;
+    for (const TsRun &r : raw) if (one_spec(r) >= 0) ng[one_spec(r)] += r.ngroups;
+    for (int s = 0; s < QO_TF_NSPEC; s++) if (ng[s] > 0 && (fs < 0 || ng[s] > ng[fs])) fs = s;
+    const double tfs = fs >= 0 ? hp->spec_thr[fs] : 0.0;
+    const bool nfs = fs >= 0 && hp->spec_kind[fs] == SK_DEN2_MIN;
+    const double zq0 = hp->rs * zni;
+    /* the fused margin per corner, formed as the device forms it (global lengths) */
+    std::vector<double> cnv(cs.size() * 2 * QO_TF_MAXK), fzv(cs.size() * (2 * QO_TF_MAXK + QO_TF_MAXKE));
+    if (fs >= 0)
+        for (size_t ci = 0; ci < cs.size(); ci++) {
+            double *cn = &cnv[ci * 2 * QO_TF_MAXK];
+            for (int i = 0; i < 2 * KN; i++) cn[i] = fma(zq0, cs[ci].qq[i], cs[ci].pp[i]);
+            qo_tf_fuse(KN, KE, cn, cs[ci].ee, tfs, nfs, &fzv[ci * (2 * QO_TF_MAXK + QO_TF_MAXKE)]);
+        }
+    /* the lengths group gi needs: (numerator pairs, E coefficients) on a plain run, (F coefficients, 0) on a fused one */
+    auto group_need = [&](int gi, bool fused, int *a, int *b) {
+        int rn = 2, re = 2, rf = 2;
+        for (int k = gi * gpt; k < (gi + 1) * gpt && k < nf; k++) {
+            if (need_n[k] > rn) rn = need_n[k];
+            if (need_e[k] > re) re = need_e[k];
+            if (!fused) continue;
+            const double x = xg[k], y = -(x * x), ay = fabs(y);
+            for (size_t ci = 0; ci < cs.size(); ci++) {
+                const double *cn = &cnv[ci * 2 * QO_TF_MAXK], *fz = &fzv[ci * (2 * QO_TF_MAXK + QO_TF_MAXKE)];
+                double r0 = cn[2 * KN - 2], r1 = cn[2 * KN - 1];
+                for (int i = KN - 2; i >= 0; i--) { r0 = r0 * y + cn[2 * i]; r1 = r1 * y + cn[2 * i + 1]; }
+                const double bound = trunc * (r0 * r0 - y * r1 * r1);
+                double acc = 0.0, pw = 1.0;
+                for (int m = 0; m < NF - 1; m++) pw *= ay;
+                int K = NF;
+                while (K > rf) { acc += fabs(fz[K - 1]) * pw; if (!(acc <= bound)) break; pw /= ay; K--; }
+                if (K > rf) rf = K;
+            }
+        }
+        re = (re + 1) & ~1;
+        if (fused) { *a = rf < NF ? rf : NF; *b = 0; }
+        else { *a = rn < KN ? rn : KN; *b = KE == 0 ? 0 : re < KE ? re : KE; }
+    };
+    auto cost = [&](bool fused, int a, int b) -> long { return fused ? a - 1 : NN * (a - 1) + (b > 0 ? b - 1 : 0); };
+    /* split every run with one set of spec bits over several groups at the steps of its groups' lengths */
+    struct Seg { TsRun r; int origin; bool fused; };
+    std::vector<Seg> segs;
+    for (size_t ri = 0; ri < raw.size(); ri++) {
+        const TsRun &r = raw[ri];
+        const bool fused = fs >= 0 && one_spec(r) == fs;
+        if (fused) { Seg sg = { r, (int)ri, true }; sg.r.kn = KN; sg.r.ke = KE; sg.r.kf = NF; segs.push_back(sg); }
+        else segs.push_back(Seg{ r, (int)ri, false });
+        if (full_len || r.any != r.all) continue;
+        const size_t first = segs.size() - 1;
+        segs.pop_back();
+        for (int gi = r.g0; gi < r.g0 + r.ngroups; gi++) {
+            int a, b;
+            group_need(gi, fused, &a, &b);
+            Seg sg = { r, (int)ri, fused };
+            sg.r.g0 = gi; sg.r.ngroups = 1;
+            if (fused) sg.r.kf = a; else { sg.r.kn = a; sg.r.ke = b; }
+            Seg &last = segs.back();
+            if (segs.size() > first && (fused ? last.r.kf == a : last.r.kn == a && last.r.ke == b)) last.r.ngroups++;
+            else segs.push_back(sg);
+        }
+        /* merge the stretches that are too short into the neighbour that costs the fewest extra instructions */
+        for (;;) {
+            size_t best = 0; long bestc = -1; bool found = false;
+            for (size_t i = first; i + 1 < segs.size(); i++) {
+                if (segs[i].r.ngroups >= QO_TS_MINSPLIT && segs[i + 1].r.ngroups >= QO_TS_MINSPLIT) continue;
+                const TsRun &u = segs[i].r, &v = segs[i + 1].r;
+                const int a = fused ? (u.kf > v.kf ? u.kf : v.kf) : (u.kn > v.kn ? u.kn : v.kn), b = fused ? 0 : (u.ke > v.ke ? u.ke : v.ke);
+                const long c = (long)(u.ngroups + v.ngroups) * cost(fused, a, b) - (long)u.ngroups * cost(fused, fused ? u.kf : u.kn, fused ? 0 : u.ke)
+                             - (long)v.ngroups * cost(fused, fused ? v.kf : v.kn, fused ? 0 : v.ke);
+                if (!found || c < bestc) { found = true; bestc = c; best = i; }
+            }
+            if (!found) break;
+            TsRun &u = segs[best].r; const TsRun &v = segs[best + 1].r;
+            u.ngroups += v.ngroups;
+            if (v.kn > u.kn) u.kn = v.kn;
+            if (v.ke > u.ke) u.ke = v.ke;
+            if (v.kf > u.kf) u.kf = v.kf;
+            segs.erase(segs.begin() + (long)best + 1);
+        }
+    }
+    if (segs.size() > QO_TS_MAXRUN) {
+        /* more runs than the table holds: back to one run per set of spec bits, every run at the plan's lengths */
+        segs.clear();
+        for (size_t ri = 0; ri < raw.size(); ri++) {
+            Seg sg = { raw[ri], (int)ri, fs >= 0 && one_spec(raw[ri]) == fs };
+            if (sg.fused) sg.r.kf = NF;
+            segs.push_back(sg);
+        }
+        if (segs.size() > QO_TS_MAXRUN) return;                       /* warp-per-sample */
+    }
+    /* the self-check on exactly what each shortened run evaluates */
+    for (Seg &sg : segs) {
+        TsRun &r = sg.r;
+        const int k0 = r.g0 * gpt, k1 = (r.g0 + r.ngroups) * gpt < nf ? (r.g0 + r.ngroups) * gpt : nf;
+        if (sg.fused) {
+            if (r.kf >= NF) continue;
+            double worst = 0.0;
+            for (size_t ci = 0; ci < cs.size(); ci++)
+                for (int k = k0; k < k1; k++) {
+                    const double err = tf_fuse_point_err(&cnv[ci * 2 * QO_TF_MAXK], cs[ci].ee, KN, KE, &fzv[ci * (2 * QO_TF_MAXK + QO_TF_MAXKE)], r.kf, tfs, nfs, xg[k]);
+                    if (err > worst) worst = err;
+                }
+            if (worst <= QO_TF_FUSE_TOL) { if (worst > out->fused_err) out->fused_err = worst; }
+            else r.kf = NF;
+        } else {
+            if (r.kn >= KN && r.ke >= KE) continue;
+            double worst = 0.0;
+            bool ok = true;
+            for (size_t ci = 0; ci < cs.size() && ok; ci++)
+                for (int k = k0; k < k1; k++) {
+                    const double rel = check_point((int)ci, k, r.kn, KE > 0 ? r.ke : out->kd);
+                    if (rel == HUGE_VAL || rel > tol) { ok = false; break; }
+                    if (rel > worst) worst = rel;
+                }
+            if (ok) { if (worst > out->err) out->err = worst; }
+            else { r.kn = KN; r.ke = KE; }
+        }
+    }
+    int n = 0;
+    for (const Seg &sg : segs) if (!sg.fused) out->runs[n++] = sg.r;
+    out->ts_nplain = n;
+    for (const Seg &sg : segs) if (sg.fused) out->runs[n++] = sg.r;
+    out->ts_nruns = n;
+    out->ts_runs_ok = 1;
+}
+
 static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int precision, int generic, const double *f, int nf,
                                   const unsigned char *mask, const QoOverrides *ov, TfPlan *out)
 {
@@ -367,6 +530,9 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
     const double trunc = gd ? 0.0 : ov->tf_trunc;          /* the derivative polynomials weigh the top coefficients by their index: keep all */
     const int NE = 2 * nl + 1, NC = 2 * Kfull;
     int kn = 1, kdd = 1, ke = 1;
+    /* per grid point, over the corners: the numerator pairs and E coefficients that point needs (the thread-per-sample
+     * kernel's runs take the lengths of their own points: tf_ts_runs) */
+    std::vector<int> need_n((size_t)nf, 1), need_e((size_t)nf, 1);
     std::vector<double> xg((size_t)nf), xpw((size_t)NC + 1), zpw((size_t)NE + 1);
     for (int k = 0; k < nf; k++) xg[k] = two_pi * f[k] / wr;
     /* |coefficient| tables of the three expansions (numerator entry: what the device's Num / [P; Q] pair carries) */
@@ -393,8 +559,8 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
             /* numerators: drop whole pairs (2K, 2K+1) from the top while their sum stays below the bound */
             double acc = 0.0;
             int K = Kfull;
-            while (K > kn) { acc += pn[2 * K - 1] * xpw[2 * K - 1] + pn[2 * K - 2] * xpw[2 * K - 2]; if (acc > nref) break; K--; }
-            if (K > kn) kn = K;
+            while (K > need_n[k]) { acc += pn[2 * K - 1] * xpw[2 * K - 1] + pn[2 * K - 2] * xpw[2 * K - 2]; if (acc > nref) break; K--; }
+            if (K > need_n[k]) need_n[k] = K;
             if (has_d) {
                 acc = 0.0; K = Kfull;
                 while (K > kdd) { acc += pd[2 * K - 1] * xpw[2 * K - 1] + pd[2 * K - 2] * xpw[2 * K - 2]; if (acc > dref) break; K--; }
@@ -403,10 +569,12 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
                 for (int m = 0; m < NE; m++) full += c.ee[m] * (m & 1 ? -zpw[m] : zpw[m]);
                 const double eref = trunc * full;
                 acc = 0.0; K = NE;
-                while (K > ke) { acc += pe[K - 1] * zpw[K - 1]; if (!(acc <= eref)) break; K--; }
-                if (K > ke) ke = K;
+                while (K > need_e[k]) { acc += pe[K - 1] * zpw[K - 1]; if (!(acc <= eref)) break; K--; }
+                if (K > need_e[k]) need_e[k] = K;
             }
         }
+        if (need_n[k] > kn) kn = need_n[k];
+        if (need_e[k] > ke) ke = need_e[k];
     }
     ke = (ke + 1) & ~1;                                       /* the kernel loads E two coefficients at a time */
     if (ke < 2) ke = 2;
@@ -423,6 +591,84 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
         forms[nforms++] = QO_TF_DEN_D;
     }
     const double tol = ov->tf_tol;
+    /* self-check of grid point k at corner ci, evaluated exactly as the device does with kn_ numerator pairs and kd_ denominator
+     * coefficients of the form out->den: -1 where the point is not looked at, HUGE_VAL where the denominator leaves the range of
+     * the batched reciprocal, else the relative error */
+    auto check_point = [&](int ci, int k, int kn_, int kd_) -> double {
+        const TfCorner &c = cs[ci];
+        const double x = xg[k], y = -x * x;
+        if (ci > 2 && (k & 3) && k > 0 && k + 1 < nf && mask[k - 1] == mask[k] && mask[k + 1] == mask[k]) return -1.0;
+        double d2 = 1.0;
+        if (out->den == QO_TF_DEN_E) { d2 = c.ee[kd_ - 1]; for (int m = kd_ - 2; m >= 0; m--) d2 = d2 * y + c.ee[m]; }
+        else if (out->den == QO_TF_DEN_D || out->den == QO_TF_DEN_DD) d2 = std::norm(tf_horner_host(c.dd, kd_, x));
+        if (!(d2 > 1e-70 && d2 < 1e70)) return HUGE_VAL;      /* the batched reciprocal multiplies four of them */
+        /* value check: every in-band point of the nominal network; every other point of the box on every 4th point and
+         * around the band edges (their job is to catch a tolerance-driven loss of conditioning, which is smooth in x) */
+        if (!mask[k]) return -1.0;
+        if (ci != QO_TF_NOMINAL && (k & 3) && k > 0 && k + 1 < nf && mask[k - 1] == mask[k] && mask[k + 1] == mask[k]) return -1.0;
+        const cplx P_ = tf_horner_host(c.pp, kn_, x), Q_ = tf_horner_host(c.qq, kn_, x) * zni;
+        /* per-element evaluation, column vector from the load end: imm = N(jx) / D(jx) */
+        double ar = hp->rl, ai = 0.0, br = 1.0, bi = 0.0, dref = 1.0;
+        for (int e = nl - 1; e >= 0; e--) {
+            const double *nd = c.nd[e];
+            const double nr = nd[2] * y + nd[0], ni = nd[1] * x, dr = nd[5] * y + nd[3], di = nd[4] * x;
+            const double dn = dr * dr + di * di, inv = 1.0 / dn;
+            const double ir = (nr * dr + ni * di) * inv, ii = (ni * dr - nr * di) * inv;
+            if (c.ser[e]) { const double tr = ir * br - ii * bi, ti = ir * bi + ii * br; ar += tr; ai += ti; }
+            else { const double tr = ir * ar - ii * ai, ti = ir * ai + ii * ar; br += tr; bi += ti; }
+            dref *= dn;
+        }
+        const cplx a(ar, ai), b(br, bi);
+        double rel;
+        if (cpl) {
+            /* P/D and Q/D as complex numbers (the coupler's row vector mixes them), plus the kernel's |D|^2 against the true one */
+            const cplx Dc = tf_horner_host(c.dd, Kfull, x);
+            rel = 2.0 * (std::abs(P_ / Dc - a) + zn * std::abs(Q_ / Dc - b)) / (std::abs(a) + zn * std::abs(b)) + (need_s21 ? fabs(d2 / dref - 1.0) : 0.0);   /* |S11|-only jobs: D cancels in the ratio */
+        } else {
+            const double got = std::norm(P_ + hp->rs * Q_) / d2, ref = std::norm(a + hp->rs * b);
+            rel = need_s21 ? fabs(got - ref) / ref : 0.0;
+            if (gd) {
+                /* group delay: the derivative polynomials against the central difference of the per-element chain's phase
+                 * over x (1 +- 1e-6) -- the definition the sweep API and the oracle use */
+                cplx Np(0, 0), Dp(0, 0);
+                const cplx sj1(0.0, x);
+                cplx pw(1.0, 0.0);
+                for (int i = 1; i < 2 * kn_; i++) { Np += (double)i * (c.pp[i] + hp->rs * zni * c.qq[i]) * pw; pw *= sj1; }
+                pw = cplx(1.0, 0.0);
+                for (int i = 1; i < 2 * kd_ && out->den == QO_TF_DEN_DD; i++) { Dp += (double)i * c.dd[i] * pw; pw *= sj1; }
+                const cplx Nn = P_ + hp->rs * Q_;
+                double tau = (Np / Nn).real();
+                if (out->den == QO_TF_DEN_DD) tau -= (Dp / tf_horner_host(c.dd, kd_, x)).real();
+                cplx dv[2];
+                for (int sgn = 0; sgn < 2; sgn++) {
+                    const double xq = x * (sgn ? 1.0 - 1e-6 : 1.0 + 1e-6), yq = -xq * xq;
+                    double ar2 = hp->rl, ai2 = 0.0, br2 = 1.0, bi2 = 0.0;
+                    for (int e = nl - 1; e >= 0; e--) {
+                        const double *nd = c.nd[e];
+                        const double nr = nd[2] * yq + nd[0], ni = nd[1] * xq, dr = nd[5] * yq + nd[3], di = nd[4] * xq;
+                        const double inv = 1.0 / (dr * dr + di * di);
+                        const double ir = (nr * dr + ni * di) * inv, ii = (ni * dr - nr * di) * inv;
+                        if (c.ser[e]) { const double tr = ir * br2 - ii * bi2, ti = ir * bi2 + ii * br2; ar2 += tr; ai2 += ti; }
+                        else { const double tr = ir * ar2 - ii * ai2, ti = ir * ai2 + ii * ar2; br2 += tr; bi2 += ti; }
+                    }
+                    dv[sgn] = cplx(ar2 + hp->rs * br2, ai2 + hp->rs * bi2);
+                }
+                const cplx cr = dv[0] * std::conj(dv[1]);
+                const double tau_fd = atan2(cr.imag(), cr.real()) / (2e-6 * x);
+                /* the finite difference itself carries ~1e-10 of rounding noise relative to the largest delay; 1e-7 is far below any spec resolution */
+                const double egd = 1e-3 * fabs(tau - tau_fd) / (fabs(tau_fd) > 1e-3 ? fabs(tau_fd) : 1e-3);
+                if (egd > rel) rel = egd;
+            }
+            if (s11) {
+                /* |S11|^2, relative with an absolute floor of -40 dB (return-loss nulls are not thresholds) */
+                const double g11 = std::norm(P_ - hp->rs * Q_) / std::norm(P_ + hp->rs * Q_), r11 = std::norm(a - hp->rs * b) / ref;
+                const double e11 = fabs(g11 - r11) / (r11 > 1e-4 ? r11 : 1e-4);
+                if (e11 > rel) rel = e11;
+            }
+        }
+        if (!(rel == rel)) rel = 1e300;
+        return rel;
+    };
     double worst = 0.0;
     int accepted = 0;
     for (int fi = 0; fi < nforms && !accepted; fi++) {
@@ -432,79 +678,9 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
         worst = 0.0;
         int range_ok = 1;
         for (int ci = 0; ci < NCORN && range_ok; ci++) {
-            const TfCorner &c = cs[ci];
             for (int k = 0; k < nf; k++) {
-                const double x = xg[k], y = -x * x;
-                if (ci > 2 && (k & 3) && k > 0 && k + 1 < nf && mask[k - 1] == mask[k] && mask[k + 1] == mask[k]) continue;
-                double d2 = 1.0;
-                if (out->den == QO_TF_DEN_E) { d2 = c.ee[out->kd - 1]; for (int m = out->kd - 2; m >= 0; m--) d2 = d2 * y + c.ee[m]; }
-                else if (out->den == QO_TF_DEN_D || out->den == QO_TF_DEN_DD) d2 = std::norm(tf_horner_host(c.dd, out->kd, x));
-                if (!(d2 > 1e-70 && d2 < 1e70)) { range_ok = 0; break; }      /* the batched reciprocal multiplies four of them */
-                /* value check: every in-band point of the nominal network; every other point of the box on every 4th point and
-                 * around the band edges (their job is to catch a tolerance-driven loss of conditioning, which is smooth in x) */
-                if (!mask[k]) continue;
-                if (ci != QO_TF_NOMINAL && (k & 3) && k > 0 && k + 1 < nf && mask[k - 1] == mask[k] && mask[k + 1] == mask[k]) continue;
-                const cplx P_ = tf_horner_host(c.pp, kn, x), Q_ = tf_horner_host(c.qq, kn, x) * zni;
-                /* per-element evaluation, column vector from the load end: imm = N(jx) / D(jx) */
-                double ar = hp->rl, ai = 0.0, br = 1.0, bi = 0.0, dref = 1.0;
-                for (int e = nl - 1; e >= 0; e--) {
-                    const double *nd = c.nd[e];
-                    const double nr = nd[2] * y + nd[0], ni = nd[1] * x, dr = nd[5] * y + nd[3], di = nd[4] * x;
-                    const double dn = dr * dr + di * di, inv = 1.0 / dn;
-                    const double ir = (nr * dr + ni * di) * inv, ii = (ni * dr - nr * di) * inv;
-                    if (c.ser[e]) { const double tr = ir * br - ii * bi, ti = ir * bi + ii * br; ar += tr; ai += ti; }
-                    else { const double tr = ir * ar - ii * ai, ti = ir * ai + ii * ar; br += tr; bi += ti; }
-                    dref *= dn;
-                }
-                const cplx a(ar, ai), b(br, bi);
-                double rel;
-                if (cpl) {
-                    /* P/D and Q/D as complex numbers (the coupler's row vector mixes them), plus the kernel's |D|^2 against the true one */
-                    const cplx Dc = tf_horner_host(c.dd, Kfull, x);
-                    rel = 2.0 * (std::abs(P_ / Dc - a) + zn * std::abs(Q_ / Dc - b)) / (std::abs(a) + zn * std::abs(b)) + (need_s21 ? fabs(d2 / dref - 1.0) : 0.0);   /* |S11|-only jobs: D cancels in the ratio */
-                } else {
-                    const double got = std::norm(P_ + hp->rs * Q_) / d2, ref = std::norm(a + hp->rs * b);
-                    rel = need_s21 ? fabs(got - ref) / ref : 0.0;
-                    if (gd) {
-                        /* group delay: the derivative polynomials against the central difference of the per-element chain's phase
-                         * over x (1 +- 1e-6) -- the definition the sweep API and the oracle use */
-                        cplx Np(0, 0), Dp(0, 0);
-                        const cplx sj1(0.0, x);
-                        cplx pw(1.0, 0.0);
-                        for (int i = 1; i < 2 * kn; i++) { Np += (double)i * (c.pp[i] + hp->rs * zni * c.qq[i]) * pw; pw *= sj1; }
-                        pw = cplx(1.0, 0.0);
-                        for (int i = 1; i < 2 * out->kd && out->den == QO_TF_DEN_DD; i++) { Dp += (double)i * c.dd[i] * pw; pw *= sj1; }
-                        const cplx Nn = P_ + hp->rs * Q_;
-                        double tau = (Np / Nn).real();
-                        if (out->den == QO_TF_DEN_DD) tau -= (Dp / tf_horner_host(c.dd, out->kd, x)).real();
-                        cplx dv[2];
-                        for (int sgn = 0; sgn < 2; sgn++) {
-                            const double xq = x * (sgn ? 1.0 - 1e-6 : 1.0 + 1e-6), yq = -xq * xq;
-                            double ar2 = hp->rl, ai2 = 0.0, br2 = 1.0, bi2 = 0.0;
-                            for (int e = nl - 1; e >= 0; e--) {
-                                const double *nd = c.nd[e];
-                                const double nr = nd[2] * yq + nd[0], ni = nd[1] * xq, dr = nd[5] * yq + nd[3], di = nd[4] * xq;
-                                const double inv = 1.0 / (dr * dr + di * di);
-                                const double ir = (nr * dr + ni * di) * inv, ii = (ni * dr - nr * di) * inv;
-                                if (c.ser[e]) { const double tr = ir * br2 - ii * bi2, ti = ir * bi2 + ii * br2; ar2 += tr; ai2 += ti; }
-                                else { const double tr = ir * ar2 - ii * ai2, ti = ir * ai2 + ii * ar2; br2 += tr; bi2 += ti; }
-                            }
-                            dv[sgn] = cplx(ar2 + hp->rs * br2, ai2 + hp->rs * bi2);
-                        }
-                        const cplx cr = dv[0] * std::conj(dv[1]);
-                        const double tau_fd = atan2(cr.imag(), cr.real()) / (2e-6 * x);
-                        /* the finite difference itself carries ~1e-10 of rounding noise relative to the largest delay; 1e-7 is far below any spec resolution */
-                        const double egd = 1e-3 * fabs(tau - tau_fd) / (fabs(tau_fd) > 1e-3 ? fabs(tau_fd) : 1e-3);
-                        if (egd > rel) rel = egd;
-                    }
-                    if (s11) {
-                        /* |S11|^2, relative with an absolute floor of -40 dB (return-loss nulls are not thresholds) */
-                        const double g11 = std::norm(P_ - hp->rs * Q_) / std::norm(P_ + hp->rs * Q_), r11 = std::norm(a - hp->rs * b) / ref;
-                        const double e11 = fabs(g11 - r11) / (r11 > 1e-4 ? r11 : 1e-4);
-                        if (e11 > rel) rel = e11;
-                    }
-                }
-                if (!(rel == rel)) rel = 1e300;
+                const double rel = check_point(ci, k, kn, out->kd);
+                if (rel == HUGE_VAL) { range_ok = 0; break; }
                 if (rel > worst) worst = rel;
             }
         }
@@ -513,6 +689,7 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
     out->err = worst;
     if (!accepted) QO_TF_NO("polynomial expansion is too ill-conditioned on this grid");
     tf_fuse_gate(hp, nf, xg.data(), mask, cs, zni, out);
+    tf_ts_runs(hp, nf, mask, xg.data(), cs, zni, need_n.data(), need_e.data(), trunc, tol, ov->ts_full_len, check_point, out);
     out->reason = "ok";
     return 1;
 #undef QO_TF_NO

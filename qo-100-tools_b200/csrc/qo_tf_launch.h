@@ -4,6 +4,15 @@
 struct TfParams;
 struct DevProg;
 struct QoOverrides;
+/* One run of the thread-per-sample kernel (qo_ts.cuh): consecutive groups of points that see the same spec bits, walked with
+ * the polynomial lengths its own points need (never above the plan's kn / kd, the kernel's static capacities) */
+#define QO_TS_MAXRUN 40          /* <= 4 band edges per spec, each at most one straddling group, plus the splits at length steps */
+struct TsRun {
+    int g0, ngroups;             /* first group, groups */
+    unsigned int any, all;       /* spec bits seen by some / by every point of the run */
+    int kn, ke;                  /* |numerator|^2 and E runs: numerator pairs and E coefficients walked (ke 0 without E) */
+    int kf;                      /* runs of the fused spec: margin coefficients walked (0 on the other runs) */
+};
 /* what the plan decided for a job that runs on the transfer-function kernel */
 struct TfPlan {
     int nn;              /* numerator chains: 2 (Num = P + Rs Q) or 4 (P and Q apart: behind a coupled-line block, or with |S11| specs) */
@@ -20,6 +29,11 @@ struct TfPlan {
     unsigned int fused;  /* specs whose single-spec runs the thread-per-sample kernel walks on the fused margin (qo_tf_fuse) */
     double fused_err;    /* worst disagreement of the fused margin with the unfused one, relative to |den|^2 (over every spec tried) */
     const char *reason;  /* "ok", or why the job stays on the chain kernels */
+    /* the thread-per-sample kernel's run table (filled when qo_ts_eligible admits the job in some form): runs[0, ts_nplain) are
+     * walked on |numerator|^2 and E, runs[ts_nplain, ts_nruns) are the fused spec's; ts_npt = the grid rounded up to whole
+     * groups; ts_runs_ok = 0 when the band edges need more runs than the table holds */
+    TsRun runs[QO_TS_MAXRUN];
+    int ts_nruns, ts_nplain, ts_npt, ts_runs_ok;
 };
 /* Can this job run on the transfer-function kernel?  Structural test, choice of the polynomial lengths the grid needs,
  * and a numerical self-check of exactly what the device will evaluate against the per-element evaluation, at the

@@ -37,6 +37,7 @@
  */
 #pragma once
 #include "qo_tf.cuh"
+#include "qo_tf_launch.h"
 
 #define QO_TS_TPB 128
 /* points in flight per thread / resident blocks per SM (both at 168 registers, 12 warps per SM): plain ladders hold <= 36
@@ -54,14 +55,13 @@
 #define QO_TS_CAPN4 8            /* behind a coupled-line block (NN = 4: P and Q apart) */
 #define QO_TS_CAPE4 8
 
-#define QO_TS_MAXRUN 40          /* <= 4 band edges per spec, each at most one straddling group */
 #define QO_PTS_N(n) _Pragma("unroll") for (int p = 0; p < (n); p++)
 
 struct TsParams {
     TfParams t;                          /* the job, exactly as qo_mc_tf_kernel takes it */
     const double *y1, *x1;               /* per POINT: -(w/wref)^2 and w/wref (the same tables, read as scalars) */
     const uint2 *mw;                     /* per point: byte masks of specs 0-3 (x) and 4-7 (y) */
-    struct { int g0, ngroups; unsigned int any, all; } runs[QO_TS_MAXRUN];  /* runs of groups (PT points each) that see the same spec bits */
+    TsRun runs[QO_TS_MAXRUN];            /* runs of groups (PT points each) that see the same spec bits, with their lengths (qo_tf_launch.h) */
     int nruns;
     int nplain;                          /* runs[0, nplain): walked on |numerator|^2 and E; runs[nplain, nruns): the runs of the one
                                             fused spec (walked on its margin polynomial, qo_tf_fuse) */
@@ -70,6 +70,65 @@ struct TsParams {
     unsigned long long *ticket;          /* zeroed per launch */
     double w0, dw;                       /* coupler on a uniform grid: first angular frequency and step */
 };
+
+/* NC interleaved Horner chains of PT points each, entered at a run-time length L (warp-uniform, 2 <= L <= K, K <= 20):
+ * r[c][p] = sum_{m < L} coef[NC m + c] y[p]^m.  The coefficients stay in registers with static indices: a jump table enters the
+ * unrolled steps at the run's top row -- fma(coef[L-1], y, coef[L-2]) -- and falls through the steps fma(r, y, coef[m]) down to
+ * row 0.  With L == K that is the DFMA sequence of a chain of static length K, operand for operand. */
+#pragma nv_diagnostic push
+#pragma nv_diag_suppress 177                 /* the rows above K - 3 keep their labels and are never entered */
+template <int NC, int K, int PT>
+__device__ __forceinline__ void ts_horner(double (&r)[NC][PT], const double (&coef)[NC * K], const double (&y)[PT], int L)
+{
+    static_assert(K >= 2 && K <= 20, "entry rows 2 .. 20");
+#define QO_TS_HINIT(t) _Pragma("unroll") for (int c = 0; c < NC; c++) { QO_PTS_N(PT) r[c][p] = fma(coef[NC * (t) + c], y[p], coef[NC * ((t) - 1) + c]); }
+#define QO_TS_HROW(m) _Pragma("unroll") for (int c = 0; c < NC; c++) { QO_PTS_N(PT) r[c][p] = fma(r[c][p], y[p], coef[NC * (m) + c]); }
+    switch (L) {
+    case 20: if constexpr (K >= 20) { QO_TS_HINIT(19) goto hr17; } else __builtin_unreachable();
+    case 19: if constexpr (K >= 19) { QO_TS_HINIT(18) goto hr16; } else __builtin_unreachable();
+    case 18: if constexpr (K >= 18) { QO_TS_HINIT(17) goto hr15; } else __builtin_unreachable();
+    case 17: if constexpr (K >= 17) { QO_TS_HINIT(16) goto hr14; } else __builtin_unreachable();
+    case 16: if constexpr (K >= 16) { QO_TS_HINIT(15) goto hr13; } else __builtin_unreachable();
+    case 15: if constexpr (K >= 15) { QO_TS_HINIT(14) goto hr12; } else __builtin_unreachable();
+    case 14: if constexpr (K >= 14) { QO_TS_HINIT(13) goto hr11; } else __builtin_unreachable();
+    case 13: if constexpr (K >= 13) { QO_TS_HINIT(12) goto hr10; } else __builtin_unreachable();
+    case 12: if constexpr (K >= 12) { QO_TS_HINIT(11) goto hr9; } else __builtin_unreachable();
+    case 11: if constexpr (K >= 11) { QO_TS_HINIT(10) goto hr8; } else __builtin_unreachable();
+    case 10: if constexpr (K >= 10) { QO_TS_HINIT(9) goto hr7; } else __builtin_unreachable();
+    case 9: if constexpr (K >= 9) { QO_TS_HINIT(8) goto hr6; } else __builtin_unreachable();
+    case 8: if constexpr (K >= 8) { QO_TS_HINIT(7) goto hr5; } else __builtin_unreachable();
+    case 7: if constexpr (K >= 7) { QO_TS_HINIT(6) goto hr4; } else __builtin_unreachable();
+    case 6: if constexpr (K >= 6) { QO_TS_HINIT(5) goto hr3; } else __builtin_unreachable();
+    case 5: if constexpr (K >= 5) { QO_TS_HINIT(4) goto hr2; } else __builtin_unreachable();
+    case 4: if constexpr (K >= 4) { QO_TS_HINIT(3) goto hr1; } else __builtin_unreachable();
+    case 3: if constexpr (K >= 3) { QO_TS_HINIT(2) goto hr0; } else __builtin_unreachable();
+    case 2: if constexpr (K >= 2) { QO_TS_HINIT(1) goto hdone; } else __builtin_unreachable();
+    default: __builtin_unreachable();
+    }
+hr17: if constexpr (17 <= K - 3) { QO_TS_HROW(17) }
+hr16: if constexpr (16 <= K - 3) { QO_TS_HROW(16) }
+hr15: if constexpr (15 <= K - 3) { QO_TS_HROW(15) }
+hr14: if constexpr (14 <= K - 3) { QO_TS_HROW(14) }
+hr13: if constexpr (13 <= K - 3) { QO_TS_HROW(13) }
+hr12: if constexpr (12 <= K - 3) { QO_TS_HROW(12) }
+hr11: if constexpr (11 <= K - 3) { QO_TS_HROW(11) }
+hr10: if constexpr (10 <= K - 3) { QO_TS_HROW(10) }
+hr9: if constexpr (9 <= K - 3) { QO_TS_HROW(9) }
+hr8: if constexpr (8 <= K - 3) { QO_TS_HROW(8) }
+hr7: if constexpr (7 <= K - 3) { QO_TS_HROW(7) }
+hr6: if constexpr (6 <= K - 3) { QO_TS_HROW(6) }
+hr5: if constexpr (5 <= K - 3) { QO_TS_HROW(5) }
+hr4: if constexpr (4 <= K - 3) { QO_TS_HROW(4) }
+hr3: if constexpr (3 <= K - 3) { QO_TS_HROW(3) }
+hr2: if constexpr (2 <= K - 3) { QO_TS_HROW(2) }
+hr1: if constexpr (1 <= K - 3) { QO_TS_HROW(1) }
+hr0: if constexpr (0 <= K - 3) { QO_TS_HROW(0) }
+hdone:
+    return;
+#undef QO_TS_HROW
+#undef QO_TS_HINIT
+}
+#pragma nv_diagnostic pop
 
 /* stage C for one (KN, KE): everything in registers.
  * The grid is walked as a few RUNS of groups (PT points each) that see the same spec bits (TsParams::runs, built by the
@@ -156,15 +215,9 @@ __device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sa
 #define QO_TS_CORE                                                                                                   \
         const int j = gi * PT;                                                                                       \
         double r[NN][PT], dd[PT], n2[PT];                                                                            \
-        _Pragma("unroll") for (int c = 0; c < NN; c++) { QO_PTS_N(PT) r[c][p] = fma(cn[NN * (KN - 1) + c], y[p], cn[NN * (KN - 2) + c]); } \
-        if (KE >= 2) { QO_PTS_N(PT) dd[p] = fma(ce[KE - 1], y[p], ce[KE - 2]); }                                     \
+        ts_horner<NN, KN, PT>(r, cn, y, rkn);                                                                        \
+        if constexpr (KE >= 2) { double e_[1][PT]; ts_horner<1, KE, PT>(e_, ce, y, rke); QO_PTS_N(PT) dd[p] = e_[0][p]; } \
         else { QO_PTS_N(PT) dd[p] = 1.0; }                                                                           \
-        _Pragma("unroll") for (int s_ = 0; s_ < (KN - 2 > KE - 2 ? KN - 2 : KE - 2); s_++) {                         \
-            if (s_ < KN - 2) {                                                                                       \
-                _Pragma("unroll") for (int c = 0; c < NN; c++) { QO_PTS_N(PT) r[c][p] = fma(r[c][p], y[p], cn[NN * (KN - 3 - s_) + c]); } \
-            }                                                                                                        \
-            if (s_ < KE - 2) { QO_PTS_N(PT) dd[p] = fma(dd[p], y[p], ce[KE - 3 - s_]); }                             \
-        }                                                                                                            \
         if (!CPL) {                                                                                                  \
             QO_PTS_N(PT) { const double t_ = r[1][p] * r[1][p]; n2[p] = fma(-y[p], t_, r[0][p] * r[0][p]); }         \
         } else {                                                                                                     \
@@ -205,6 +258,7 @@ __device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sa
             for (int h = 0; h < PT; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + gi * PT + h)); y[h] = a.x; y[h + 1] = a.y; }
         }
         const int g_end = gi + Q.runs[rn].ngroups;
+        const int rkn = Q.runs[rn].kn, rke = Q.runs[rn].ke;      /* this run's lengths (<= KN, KE) */
         const int one = (any == all && all != 0u && (all & (all - 1u)) == 0u) ? __ffs((int)all) - 1 : -1;
         if (any == 0u) {
             for (; gi < g_end; gi++) { QO_TS_CORE QO_PTS_N(PT) idle |= tf_hi(n2[p]) | (tf_hi(dd[p]) & 0x7fffffffu); }
@@ -256,26 +310,23 @@ __device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sa
             double yf[PF];
             for (int rn = Q.nplain; rn < Q.nruns; rn++) {
                 gi = Q.runs[rn].g0;
-                const int g_end = gi + Q.runs[rn].ngroups;
+                const int g_end = gi + Q.runs[rn].ngroups, rkf = Q.runs[rn].kf;      /* this run's margin coefficients (<= NF) */
 #pragma unroll
                 for (int h = 0; h < PF; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + gi * PT + h)); yf[h] = a.x; yf[h + 1] = a.y; }
                 for (; gi + QO_TS_FG2 <= g_end; gi += QO_TS_FG2) {
-                    double F[PF];
-                    QO_PTS_N(PF) F[p] = fma(fz[NF - 1], yf[p], fz[NF - 2]);
-#pragma unroll
-                    for (int m = NF - 3; m >= 0; m--) { QO_PTS_N(PF) F[p] = fma(F[p], yf[p], fz[m]); }
+                    double F[1][PF];
+                    ts_horner<1, NF, PF>(F, fz, yf, rkf);
 #pragma unroll
                     for (int h = 0; h < PF; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + (gi + QO_TS_FG2) * PT + h)); yf[h] = a.x; yf[h + 1] = a.y; }
-                    QO_PTS_N(PF) a1 |= tf_hi(F[p]);
+                    QO_PTS_N(PF) a1 |= tf_hi(F[0][p]);
                 }
                 for (; gi < g_end; gi++) {                /* the run's last groups: yf[0, PT) holds the next one */
-                    double F[PT];
-                    QO_PTS_N(PT) F[p] = fma(fz[NF - 1], yf[p], fz[NF - 2]);
-#pragma unroll
-                    for (int m = NF - 3; m >= 0; m--) { QO_PTS_N(PT) F[p] = fma(F[p], yf[p], fz[m]); }
+                    double F[1][PT], yt[PT];
+                    QO_PTS_N(PT) yt[p] = yf[p];
+                    ts_horner<1, NF, PT>(F, fz, yt, rkf);
 #pragma unroll
                     for (int h = 0; h < PT; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + (gi + 1) * PT + h)); yf[h] = a.x; yf[h + 1] = a.y; }
-                    QO_PTS_N(PT) a1 |= tf_hi(F[p]);
+                    QO_PTS_N(PT) a1 |= tf_hi(F[0][p]);
                 }
             }
 #pragma unroll

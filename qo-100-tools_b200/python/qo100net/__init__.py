@@ -93,6 +93,7 @@ EXPORTS = [
     "qo_ctx_num_devices", "qo_ctx_destroy", "qo_sweep", "qo_mc_run", "qo_plan_create", "qo_plan_num_counters",
     "qo_plan_reset", "qo_plan_launch", "qo_plan_read", "qo_plan_flops_per_eval", "qo_plan_launches",
     "qo_plan_kernel_name", "qo_plan_tf_info", "qo_plan_h2d_bytes", "qo_plan_analyze", "qo_chain_jit_analyze",
+    "qo_plan_ts_runs", "qo_plan_analyze_ts_runs",
     "qo_s2p_load", "qo_s2p_from_arrays", "qo_s2p_num_points", "qo_s2p_z0", "qo_s2p_get", "qo_s2p_interp",
     "qo_s2p_fit_inductor", "qo_s2p_free", "qo_net_from_sblock",
     "qo_nodal_create", "qo_nodal_add_branch", "qo_nodal_add_port", "qo_nodal_add_sblock", "qo_nodal_load_qucs_sch",
@@ -151,6 +152,8 @@ def lib():
         "qo_plan_kernel_name": (C.c_char_p, [vp]),
         "qo_plan_tf_info": (C.c_char_p, [vp, C.POINTER(C.c_int), C.POINTER(C.c_double), C.POINTER(C.c_uint), C.POINTER(C.c_double)]),
         "qo_plan_h2d_bytes": (C.c_uint64, [vp]),
+        "qo_plan_ts_runs": (C.c_int, [vp, C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_int)]),
+        "qo_plan_analyze_ts_runs": (C.c_int, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_int)]),
         "qo_chain_jit_analyze": (C.c_int, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_int)]),
         "qo_plan_analyze": (C.c_char_p, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_int), C.POINTER(C.c_double), C.POINTER(C.c_uint), C.POINTER(C.c_double), C.POINTER(C.c_double)]),
         "qo_s2p_load": (C.c_int, [C.c_char_p, C.POINTER(vp)]),
@@ -610,6 +613,37 @@ def _res_dict(res, fps, hist, nspec, hist_bins):
                 flops_per_eval=res.flops_per_eval)
 
 
+TS_MAXRUN = 40
+
+
+def _ts_runs(fn, *args):
+    """The thread-per-sample kernel's run table (qo_plan_ts_runs / qo_plan_analyze_ts_runs) as a list of dicts: first point and
+    points of the run, the spec bits its points see (some / every point), whether it is walked on the fused margin, and the
+    polynomial lengths it walks (numerator pairs kn and E coefficients ke, or the fused margin's coefficients kf)."""
+    buf = (C.c_int * (7 * TS_MAXRUN))()
+    meta = (C.c_int * 2)()
+    n = fn(*args, buf, TS_MAXRUN, meta)
+    if n < 0:
+        raise QoError(n, lib().qo_last_error().decode())
+    gpt = meta[1]
+    out = []
+    for r in range(n):
+        g0, ng, any_, all_, kn, ke, kf = buf[7 * r: 7 * r + 7]
+        fused = r >= meta[0]
+        out.append(dict(point=g0 * gpt, points=ng * gpt, any=any_ & 0xFF, all=all_ & 0xFF, fused=fused,
+                        kn=None if fused else kn, ke=None if fused else ke, kf=kf if fused else None))
+    return out
+
+
+def plan_ts_runs(net, f, specs, tols=(), dist=DIST_UNIFORM, mode=MODE_REDUCE_ONLY, precision=64,
+                 hist_bins=0, hist_spec=0, hist_lo=0.0, hist_hi=1.0):
+    """Host-only (qo_plan_analyze_ts_runs): the run table the thread-per-sample kernel would walk, with each run's
+    polynomial lengths (see _ts_runs); empty when the job does not run thread-per-sample."""
+    f = np.ascontiguousarray(f, dtype=np.float64)
+    cfg = _cfg(0, 0, list(tols), 0, dist, mode, precision, hist_bins, hist_spec, hist_lo, hist_hi)
+    return _ts_runs(lib().qo_plan_analyze_ts_runs, net._h, _dp(f), len(f), _specs(specs), len(specs), C.byref(cfg))
+
+
 def plan_analyze(net, f, specs, tols=(), dist=DIST_UNIFORM, mode=MODE_REDUCE_ONLY, precision=64,
                  hist_bins=0, hist_spec=0, hist_lo=0.0, hist_hi=1.0):
     """Host-only part of plan creation (qo_plan_analyze, no GPU needed): which kernel family the job would take and the
@@ -685,9 +719,15 @@ class Plan:
         info = (C.c_int * 6)()
         err, fused, ferr = C.c_double(0.0), C.c_uint(0), C.c_double(0.0)
         reason = lib().qo_plan_tf_info(self._h, info, C.byref(err), C.byref(fused), C.byref(ferr)).decode()
+        runs = [(r["point"], r["points"], r["kf"] if r["fused"] else (r["kn"], r["ke"])) for r in self.ts_runs]
         return dict(selected=bool(info[0]), numerator_chains=info[1], den_form=("none", "E", "D", "DD")[info[2]] if 0 <= info[2] <= 3 else "?",
                     kn=info[3], kd=info[4], degree=info[5], self_check_err=err.value, fused_specs=fused.value, fused_err=ferr.value,
-                    reason=reason)
+                    reason=reason, ts_runs=runs)
+
+    @property
+    def ts_runs(self):
+        """The thread-per-sample kernel's run table with each run's polynomial lengths (qo_plan_ts_runs; see _ts_runs)."""
+        return _ts_runs(lib().qo_plan_ts_runs, self._h)
 
     @property
     def h2d_bytes(self):
