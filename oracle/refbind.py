@@ -100,6 +100,7 @@ def lib():
         L.ref_cpl_analyze.argtypes = [C.c_double] * 8 + [dp] * 4
         L.ref_sblock_register.argtypes = [C.c_int, dp, dp, C.c_int, C.c_double]
         L.ref_sblock_clear.argtypes = []
+        L.ref_sblock_s.argtypes = [C.c_int, C.c_double, C.c_int, dp]
         ip = C.POINTER(C.c_int)
         L.ref_nodal_sweep.argtypes = [C.POINTER(Branch), C.c_int, C.c_int, ip, dp, C.c_int, dp, C.c_int, dp]
         L.ref_nodal_mc_run.argtypes = [C.POINTER(Branch), C.c_int, C.c_int, ip, dp, C.c_int, dp, C.c_int,
@@ -191,6 +192,15 @@ def sblock_register(idx, f, s11, s21, s12, s22, z0=50.0):
 
 def sblock_clear():
     lib().ref_sblock_clear()
+
+
+def sblock_s(idx, f, polar=True):
+    """The oracle's interpolated S of measured block idx at one frequency -> (s11, s21, s12, s22), complex."""
+    s = np.empty(8)
+    rc = lib().ref_sblock_s(int(idx), float(f), int(bool(polar)), _dp(s))
+    if rc:
+        raise RuntimeError("ref_sblock_s failed: %d" % rc)
+    return tuple(complex(s[2 * j], s[2 * j + 1]) for j in range(4))
 
 
 def elems_to_list(arr, n=None):

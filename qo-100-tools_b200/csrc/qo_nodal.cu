@@ -60,6 +60,7 @@ struct NodalStatic {
     int16_t pos[QO_NODAL_MAX_UNK * QO_NODAL_MAX_UNK];   /* (pivot-order row, permuted column) -> value index, -1 = structural zero */
     uint8_t rowmap[QO_NODAL_MAX_UNK];                   /* original row (equation) -> pivot-order row */
     uint8_t colmap[QO_NODAL_MAX_UNK];                   /* original unknown -> permuted column (port unknowns last) */
+    uint8_t szero[QO_NODAL_MAX_PORTS];                  /* port j driven: bit k = V at port k is zero for any stamp values */
     uint16_t prog[QN_PROG_MAX];
     double worst_l2;                                    /* largest |multiplier|^2 the plan-time probes met */
 };
@@ -336,7 +337,8 @@ qo_nodal_kernel(const NodalProg *__restrict__ prog, const NodalStatic *__restric
                 }
                 for (int kk = 0; kk < np; kk++) {
                     const double sc = 2.0 * sqrt(prog->port_z0[j] / prog->port_z0[kk]);
-                    const double2 v = x[STATIC ? s_colmap[prog->port_node[kk] - 1] : prog->port_node[kk] - 1];
+                    const double2 v = STATIC && ((splan->szero[j] >> kk) & 1u) ? make_double2(0.0, 0.0)
+                                                                                : x[STATIC ? s_colmap[prog->port_node[kk] - 1] : prog->port_node[kk] - 1];
                     const double2 sv = make_double2(sc * v.x - (kk == j ? 1.0 : 0.0), sc * v.y);
                     if (full) s_out[obase + (size_t)kk * np + j] = sv;
 #pragma unroll
@@ -467,6 +469,30 @@ struct MarkSink {
     void add(int r, int c, double2) { m[r * QO_NODAL_MAX_UNK + c] = 1; }
 };
 
+/* does A without row drop_r and column drop_c (structural pattern raw) have a perfect matching?  If not, the cofactor -- and so
+ * the entry (drop_c, drop_r) of A^-1 -- is zero whatever values the stamps take (augmenting paths, n <= 32) */
+static bool match_aug(const std::vector<unsigned int> &adj, int r, unsigned int &seen, std::vector<int> &row_of)
+{
+    for (unsigned int m = adj[r] & ~seen; m; m &= m - 1) {
+        const int c = __builtin_ctz(m);
+        seen |= 1u << c;
+        if (row_of[c] < 0 || match_aug(adj, row_of[c], seen, row_of)) { row_of[c] = r; return true; }
+    }
+    return false;
+}
+static bool minor_matches(const unsigned char *raw, int n, int drop_r, int drop_c)
+{
+    std::vector<unsigned int> adj(n, 0);
+    for (int r = 0; r < n; r++)
+        for (int c = 0; c < n; c++) if (r != drop_r && c != drop_c && raw[r * QO_NODAL_MAX_UNK + c]) adj[r] |= 1u << c;
+    std::vector<int> row_of(n, -1);
+    for (int r = 0; r < n; r++) {
+        unsigned int seen = 0;
+        if (r != drop_r && !match_aug(adj, r, seen, row_of)) return false;
+    }
+    return true;
+}
+
 /* Build the static plan; verify it at several grid points.  Returns false when the job should use the dense
  * kernel.  Unknowns are re-ordered so that the port nodes come LAST and, while the internal unknowns are being
  * eliminated, pivots are taken from the internal equations whenever one is close to the column maximum
@@ -563,6 +589,11 @@ static bool build_static_thr(const NodalProg *hp, const double *f, int nf, const
     MarkSink M = { raw.data() };
     nodal_stamp_all(hp, hp->nom, 1.0, yb, (size_t)nf * 4, M);
     for (int r = 0; r < n; r++) for (int c = 0; c < n; c++) if (raw[r * LD + c]) pat[sp->rowmap[r] * LD + sp->colmap[c]] = 1;
+    /* port voltages that vanish structurally (the reverse isolation of an ideal buffer): per-point pivoting cancels them to ~1e-16,
+     * the fixed order through the stiff stamps to ~1e-11, so the plan writes them as exact zeros */
+    for (int j = 0; j < np; j++)
+        for (int k = 0; k < np; k++)
+            if (!minor_matches(raw.data(), n, hp->port_node[j] - 1, hp->port_node[k] - 1)) sp->szero[j] |= (uint8_t)(1u << k);
     for (int c = 0; c < n; c++) {
         if (!pat[c * LD + c]) return false;                                 /* structurally zero pivot */
         for (int r = c + 1; r < n; r++)
@@ -672,12 +703,11 @@ static bool build_static_thr(const NodalProg *hp, const double *f, int nf, const
             x[sp->rowmap[hp->port_node[j] - 1]] = make_double2(1.0 / hp->port_z0[j], 0.0);
             static_solve(sp->prog, sp->solve_at[j], V.data(), x.data());
             for (int p = 0; p < np; p++) {
-                const double2 a = x[sp->colmap[hp->port_node[p] - 1]], b = X[j][hp->port_node[p] - 1];
+                const double2 a = ((sp->szero[j] >> p) & 1u) ? make_double2(0.0, 0.0) : x[sp->colmap[hp->port_node[p] - 1]], b = X[j][hp->port_node[p] - 1];
                 const double err = hypot(a.x - b.x, a.y - b.y), ref = hypot(b.x, b.y);
-                /* port voltages are O(1) (1/Z0 injected into ~Z0).  Entries that are exactly zero under per-point
-                 * pivoting (reverse isolation of an ideal buffer) come out as ~1e-11 residues when the stiff
-                 * reference network (100 uF next to 1.2 pF) is eliminated in the fixed ports-last order; 5e-11 on V
-                 * = 1e-10 on S keeps the plan inside the 1e-9 parity bar, anything worse takes the dense kernel */
+                /* port voltages are O(1) (1/Z0 injected into ~Z0); structurally zero ones (szero) are exact zeros on both
+                 * sides.  5e-11 on V = 1e-10 on S keeps the plan inside the 1e-9 parity bar, anything worse takes the
+                 * dense kernel */
                 if (!(err <= 1e-9 * ref + 5e-11)) {                                    /* NaN fails too */
                     if (getenv("QO100NET_NODAL_DEBUG")) fprintf(stderr, "qo_nodal: static plan rejected at f=%g Hz (%s), port %d<-%d: err %.3e ref %.3e\n", f[k], vert < 0 ? "nominal" : "tolerance-box vertex", p, j, err, ref);
                     return false;
