@@ -2,6 +2,15 @@
 #pragma once
 #include <cuda_runtime.h>
 #include "qo_internal.h"
+#include "qo_tally.cuh"
+
+/* a histogram request (cfg->hist_bins > 0) of a job with nspec specs: fits the counters, names one of the specs, has a window */
+static inline bool qo_hist_cfg_ok(const qo_mc_cfg *cfg, int nspec)
+{
+    if (cfg->hist_bins <= QO_MAX_HIST && cfg->hist_spec >= 0 && cfg->hist_spec < nspec && cfg->hist_hi > cfg->hist_lo) return true;
+    qo_set_error("bad histogram configuration");
+    return false;
+}
 
 #define CU(call)                                                                                      \
     do {                                                                                              \

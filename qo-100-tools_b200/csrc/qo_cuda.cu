@@ -378,7 +378,7 @@ static int build_prog(const qo_net *net, const double *f, int nf, const qo_spec 
         if (cfg && cfg->hist_bins > 0 && cfg->hist_spec == s && hits == 0) { qo_set_error("histogram spec %d covers no grid frequency", s); return QO_ERR_ARG; }
     }
     if (cfg && cfg->hist_bins > 0) {
-        if (cfg->hist_bins > QO_MAX_HIST || cfg->hist_spec < 0 || cfg->hist_spec >= nspec || !(cfg->hist_hi > cfg->hist_lo)) { qo_set_error("bad histogram configuration"); return QO_ERR_ARG; }
+        if (!qo_hist_cfg_ok(cfg, nspec)) return QO_ERR_ARG;
         hp->hist_bins = cfg->hist_bins; hp->hist_spec = cfg->hist_spec; hp->hist_lo = cfg->hist_lo; hp->hist_hi = cfg->hist_hi;
     }
     return QO_OK;
@@ -708,7 +708,7 @@ static int plan_create(qo_ctx *ctx, const qo_net *net, const double *f, int nf, 
     if (p->generic)
         for (int e = 0; e < net->n; e++)
             if (net->e[e].kind == QO_SBLOCK) { qo_set_error("S-parameter blocks cannot be mixed with microstrip elements yet"); delete p; return QO_ERR_UNSUPPORTED; }
-    p->ncnt = 2 + nspec + p->hp.hist_bins;
+    p->ncnt = qo_ncnt(nspec, p->hp.hist_bins);
     p->f.assign(f, f + nf);
     p->kern = select_kernel(p, f, nf);
     p->kernel_name = qo_kern_name[p->kern];

@@ -10,12 +10,11 @@
  */
 #pragma once
 #include <stdint.h>
+#include "qo_tally.cuh"      /* QO_NSPEC_MAX, QO_MAX_HIST */
 
 #define QO_MAX_OPS 96
 #define QO_MAX_VAR 64
 #define QO_MAX_COEF 256      /* doubles per per-sample coefficient table */
-#define QO_MAX_HIST 1024
-#define QO_NSPEC_MAX 8
 
 enum {
     OP_NOP = 0,

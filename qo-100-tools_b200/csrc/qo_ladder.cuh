@@ -319,11 +319,11 @@ __global__ void __launch_bounds__(TPB, MINB) qo_mc_ladder_kernel(const __grid_co
     constexpr int NREC = (CPL ? QO_LAD_CPL : 0) + N * QO_LAD_STRIDE;
     __shared__ __align__(16) T s_coef[WARPS][NREC];
     __shared__ double s_x[WARPS][QO_MAX_VAR];
-    __shared__ unsigned int s_cnt[2 + QO_NSPEC_MAX + QO_MAX_HIST];
+    __shared__ unsigned int s_cnt[QO_NCNT_MAX];
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int ncnt = 2 + P.nspec + (P.hist_bins > 0 ? P.hist_bins : 0);
-    for (int i = threadIdx.x; i < ncnt; i += TPB) s_cnt[i] = 0;
+    const int ncnt = qo_ncnt(P.nspec, P.hist_bins);
+    qo_tally_zero<TPB>(s_cnt, ncnt);
     __syncthreads();
 
     T *coefw = s_coef[warp];
@@ -465,27 +465,18 @@ __global__ void __launch_bounds__(TPB, MINB) qo_mc_ladder_kernel(const __grid_co
             }
         }
         if (lane == 0) {
-            atomicAdd(&s_cnt[0], fail == 0 ? 1u : 0u);
-            atomicAdd(&s_cnt[1], 1u);
-            for (int sp = 0; sp < P.nspec; sp++)
-                if ((fail >> sp) & 1u) atomicAdd(&s_cnt[2 + sp], 1u);
+            qo_tally_one(s_cnt, P.nspec, fail);
             if (P.hist_spec >= 0) {
                 double worst = 0.0;      /* |den|^2 (or |S11|^2) extreme of the histogram spec's band */
 #pragma unroll
                 for (int sp = 0; sp < QO_LAD_NSPEC; sp++) if (sp == P.hist_spec) worst = fabs((double)trk[sp]);
                 const double k21 = P.k21;
                 const double lin = P.hist_kind == SK_S11_MAX ? worst : P.hist_kind == SK_DEN2_MAX ? k21 * k21 / worst : k21 * k21 * (1.0 / worst);
-                const double v = 10.0 * log10(lin);
-                const double xb = (v - P.hist_lo) / (P.hist_hi - P.hist_lo) * (double)P.hist_bins;
-                long long b = (long long)floor(xb);
-                if (!(xb >= 0.0)) b = 0;
-                if (b >= P.hist_bins) b = P.hist_bins - 1;
-                atomicAdd(&s_cnt[2 + P.nspec + (int)b], 1u);
+                qo_tally_hist(s_cnt, P.nspec, qo_hist_bin(10.0 * log10(lin), P.hist_lo, P.hist_hi, P.hist_bins));
             }
         }
         s = __shfl_sync(0xffffffffu, s_next, 0);
     }
     __syncthreads();
-    for (int i = threadIdx.x; i < ncnt; i += TPB)
-        if (s_cnt[i]) atomicAdd(&P.counters[i], (unsigned long long)s_cnt[i]);
+    qo_tally_flush<TPB>(s_cnt, ncnt, P.counters);
 }

@@ -313,7 +313,7 @@ qo_mc_lumped_kernel(
     __shared__ int s_op[QO_MAX_OPS], s_coff[QO_MAX_OPS];
     __shared__ __align__(16) T s_coef[QO_WARPS][QO_MAX_COEF];
     __shared__ double s_x[QO_WARPS][QO_MAX_VAR];
-    __shared__ unsigned int s_cnt[2 + QO_NSPEC_MAX + QO_MAX_HIST];
+    __shared__ unsigned int s_cnt[QO_NCNT_MAX];
     __shared__ T s_thr[QO_NSPEC_MAX];
     __shared__ int s_sk[QO_NSPEC_MAX];
     __shared__ double s_gdthr[QO_NSPEC_MAX];
@@ -330,10 +330,10 @@ qo_mc_lumped_kernel(
     const bool need_s11 = FULL_S || prog->need_s11;
 #define QO_SK(sp) s_sk[sp]
 #endif
-    const int ncnt = 2 + nspec + (prog->hist_bins > 0 ? prog->hist_bins : 0);
+    const int ncnt = qo_ncnt(nspec, prog->hist_bins);
     const bool planes_al32 = ((((size_t)planes.s11) | ((size_t)planes.s21) | ((size_t)planes.s12) | ((size_t)planes.s22)) & 31) == 0;
     for (int i = threadIdx.x; i < n_ops; i += QO_TPB) { s_op[i] = prog->opcode[i]; s_coff[i] = prog->coff[i]; }
-    for (int i = threadIdx.x; i < ncnt; i += QO_TPB) s_cnt[i] = 0;
+    qo_tally_zero<QO_TPB>(s_cnt, ncnt);
     if (threadIdx.x < QO_NSPEC_MAX) {
         s_thr[threadIdx.x] = T(prog->spec_thr[threadIdx.x]); s_sk[threadIdx.x] = prog->spec_kind[threadIdx.x];
         s_gdthr[threadIdx.x] = prog->spec_thr[threadIdx.x];
@@ -498,21 +498,14 @@ qo_mc_lumped_kernel(
                 }
             }
             if (lane == 0) {
-                atomicAdd(&s_cnt[0], fail == 0 ? 1u : 0u);
-                atomicAdd(&s_cnt[1], 1u);
-                for (int sp = 0; sp < nspec; sp++)
-                    if ((fail >> sp) & 1u) atomicAdd(&s_cnt[2 + sp], 1u);
+                qo_tally_one(s_cnt, nspec, fail);
                 if (hist_spec >= 0) {
                     double ratio = (double)wn / (double)wd;
                     double lin = hist_kind == SK_S11_MAX ? ratio
                                : hist_kind == SK_DEN2_MAX ? (double)k21 * (double)k21 / ratio
                                                           : (double)k21 * (double)k21 * ratio;
                     double v = hist_kind == SK_GD_MAX ? gd_worst : 10.0 * log10(lin);
-                    double xb = (v - prog->hist_lo) / (prog->hist_hi - prog->hist_lo) * (double)prog->hist_bins;
-                    long long b = (long long)floor(xb);
-                    if (!(xb >= 0.0)) b = 0;
-                    if (b >= prog->hist_bins) b = prog->hist_bins - 1;
-                    atomicAdd(&s_cnt[2 + nspec + (int)b], 1u);
+                    qo_tally_hist(s_cnt, nspec, qo_hist_bin(v, prog->hist_lo, prog->hist_hi, prog->hist_bins));
                 }
             }
         }
@@ -520,8 +513,7 @@ qo_mc_lumped_kernel(
     }
     if (!FULL_S) {
         __syncthreads();
-        for (int i = threadIdx.x; i < ncnt; i += QO_TPB)
-            if (s_cnt[i]) atomicAdd(&counters[i], (unsigned long long)s_cnt[i]);
+        qo_tally_flush<QO_TPB>(s_cnt, ncnt, counters);
     }
 }
 #undef QO_SK

@@ -28,8 +28,10 @@
 #include "qo_ctx_internal.h"
 #include "qo_overrides.h"
 #include "qo_stream.h"
+#include "qo_tally.cuh"
 
 #include "qo_nodal_prog.h"
+static_assert(QN_MAX_SPEC == QO_NSPEC_MAX, "the nodal kernels' counters take the cascade kernels' layout (qo_tally.cuh)");
 
 __device__ __forceinline__ double2 c_mul(double2 a, double2 b) { return make_double2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
 __device__ __forceinline__ double2 c_sub(double2 a, double2 b) { return make_double2(a.x - b.x, a.y - b.y); }
@@ -224,12 +226,12 @@ qo_nodal_kernel(const NodalProg *__restrict__ prog, const NodalStatic *__restric
     __shared__ double s_p[QO_NODAL_MAX_BR][4];
     __shared__ double s_x[QN_MAX_VAR];
     __shared__ double s_trk[QN_MAX_SPEC][QN_TPB / 32];
-    __shared__ unsigned int s_cnt[2 + QN_MAX_SPEC + 1024];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    __shared__ unsigned int s_cnt[QO_NCNT_MAX];
+    const int tid = threadIdx.x;
     const int n = prog->n_unk, np = prog->np, nb = prog->nb, nspec = prog->nspec, n_nodes = prog->n_nodes;
     const int full = prog->full;
-    const int ncnt = 2 + nspec + (prog->hist_bins > 0 ? prog->hist_bins : 0);
-    for (int i = tid; i < ncnt; i += QN_TPB) s_cnt[i] = 0;
+    const int ncnt = qo_ncnt(nspec, prog->hist_bins);
+    qo_tally_zero<QN_TPB>(s_cnt, ncnt);
     unsigned int n_suspect = 0;                      /* points whose fixed pivot order met a huge multiplier (static plan) */
     __syncthreads();
 
@@ -351,48 +353,10 @@ qo_nodal_kernel(const NodalProg *__restrict__ prog, const NodalStatic *__restric
                 }
             }
         }
-        if (!full) {
-            /* per-sample verdict: block max of every tracker */
-#pragma unroll
-            for (int sp = 0; sp < QN_MAX_SPEC; sp++) {
-                if (sp < nspec) {
-                    double v = trk[sp];
-#pragma unroll
-                    for (int off = 16; off > 0; off >>= 1) { const double o = __shfl_xor_sync(0xffffffffu, v, off); v = o > v ? o : v; }
-                    if (lane == 0) s_trk[sp][warp] = v;
-                }
-            }
-            __syncthreads();
-            if (tid == 0) {
-                unsigned int fail = 0;
-                double hist_worst = 0.0;
-                for (int sp = 0; sp < nspec; sp++) {
-                    double v = s_trk[sp][0];
-                    for (int q = 1; q < QN_TPB / 32; q++) v = s_trk[sp][q] > v ? s_trk[sp][q] : v;
-                    if (v == -1e300) continue;                          /* the spec covers no grid point */
-                    const double thr = prog->spec_min[sp] ? -prog->spec_thr[sp] : prog->spec_thr[sp];
-                    if (v > thr) fail |= 1u << sp;
-                    if (sp == prog->hist_spec) hist_worst = fabs(v);
-                }
-                atomicAdd(&s_cnt[0], fail == 0 ? 1u : 0u);
-                atomicAdd(&s_cnt[1], 1u);
-                for (int sp = 0; sp < nspec; sp++) if ((fail >> sp) & 1u) atomicAdd(&s_cnt[2 + sp], 1u);
-                if (prog->hist_bins > 0) {
-                    const double v = 10.0 * log10(hist_worst);
-                    const double xb = (v - prog->hist_lo) / (prog->hist_hi - prog->hist_lo) * (double)prog->hist_bins;
-                    long long b = (long long)floor(xb);
-                    if (!(xb >= 0.0)) b = 0;
-                    if (b >= prog->hist_bins) b = prog->hist_bins - 1;
-                    atomicAdd(&s_cnt[2 + nspec + (int)b], 1u);
-                }
-            }
-        }
+        if (!full) qn_verdict(prog, nspec, trk, s_trk, s_cnt);
         __syncthreads();
     }
-    if (!full) {
-        for (int i = tid; i < ncnt; i += QN_TPB)
-            if (s_cnt[i]) atomicAdd(&counters[i], (unsigned long long)s_cnt[i]);
-    }
+    if (!full) qo_tally_flush<QN_TPB>(s_cnt, ncnt, counters);
     if (STATIC && n_suspect) atomicAdd(&counters[ncnt], (unsigned long long)n_suspect);     /* one slot past the job's counters */
 }
 
@@ -767,7 +731,7 @@ static int nodal_compile(const qo_nodal *nd, const double *f, int nf, const qo_n
     }
     hp->hist_bins = 0; hp->hist_spec = -1;
     if (!full && cfg->hist_bins > 0) {
-        if (cfg->hist_bins > 1024 || cfg->hist_spec < 0 || cfg->hist_spec >= nspec || !(cfg->hist_hi > cfg->hist_lo)) { qo_set_error("bad histogram configuration"); return QO_ERR_ARG; }
+        if (!qo_hist_cfg_ok(cfg, nspec)) return QO_ERR_ARG;
         hp->hist_bins = cfg->hist_bins; hp->hist_spec = cfg->hist_spec; hp->hist_lo = cfg->hist_lo; hp->hist_hi = cfg->hist_hi;
     }
     /* measured blocks: admittance per (block branch, grid point), in branch order */
@@ -889,7 +853,7 @@ static int nodal_run(qo_ctx *ctx, const qo_nodal *nd, const double *f, int nf, c
     const NodalProg *hp = &job->prog;
     bool use_static = job->use_static;
     if (ov.kernel == QoNodalOverrides::STATIC && !use_static) { qo_set_error("QO100NET_NODAL=static: the static plan failed its self-check for this network"); return QO_ERR_UNSUPPORTED; }
-    const int ncnt = 2 + nspec + hp->hist_bins;
+    const int ncnt = qo_ncnt(nspec, hp->hist_bins);
     const unsigned long long N = cfg->n_samples;
     if (N == 0) { if (res) { res->n_pass = res->n_total = 0; } return QO_OK; }
     /* the plan compiled into a kernel of its own: large jobs (QO100NET_NODAL=jit: always; =static / =dense: never) */

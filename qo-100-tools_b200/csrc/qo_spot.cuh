@@ -39,9 +39,9 @@ __global__ void __launch_bounds__(QO_SPOT_TPB, 4) qo_mc_spot_kernel(const __grid
     __shared__ short s_var[QO_SPOT_MAXEL][6];
     __shared__ unsigned char s_mode[QO_SPOT_MAXEL][6];
     __shared__ int s_op[QO_SPOT_MAXEL];
-    __shared__ unsigned int s_cnt[2 + QO_NSPEC_MAX + QO_MAX_HIST];
-    const int ncnt = 2 + P.nspec + (P.hist_bins > 0 ? P.hist_bins : 0);
-    for (int i = threadIdx.x; i < ncnt; i += QO_SPOT_TPB) s_cnt[i] = 0;
+    __shared__ unsigned int s_cnt[QO_NCNT_MAX];
+    const int ncnt = qo_ncnt(P.nspec, P.hist_bins);
+    qo_tally_zero<QO_SPOT_TPB>(s_cnt, ncnt);
     for (int i = threadIdx.x; i < P.n_el * 6; i += QO_SPOT_TPB) {
         const int e = i / 6, k = i - 6 * e;
         s_nom[e][k] = P.prog->nom[P.el0 + e][k]; s_tol[e][k] = P.prog->ttol[P.el0 + e][k];
@@ -129,26 +129,14 @@ __global__ void __launch_bounds__(QO_SPOT_TPB, 4) qo_mc_spot_kernel(const __grid
                 }
             }
         }
-        /* warp-aggregated counters */
-        const unsigned int vm = __ballot_sync(0xffffffffu, valid), pm = __ballot_sync(0xffffffffu, valid && fail == 0);
-        if (lane == 0) { atomicAdd(&s_cnt[0], (unsigned int)__popc(pm)); atomicAdd(&s_cnt[1], (unsigned int)__popc(vm)); }
-        for (int sp = 0; sp < P.nspec; sp++) {
-            const unsigned int fm = __ballot_sync(0xffffffffu, valid && ((fail >> sp) & 1u));
-            if (lane == 0 && fm) atomicAdd(&s_cnt[2 + sp], (unsigned int)__popc(fm));
-        }
+        qo_tally_warp(s_cnt, P.nspec, fail, __ballot_sync(0xffffffffu, valid));
         if (valid && P.hist_spec >= 0) {
             const int sk = P.kind[P.hist_spec];
             const double k21 = P.k21;
             const double lin = sk == SK_S11_MAX ? worst : sk == SK_DEN2_MAX ? k21 * k21 / worst : k21 * k21 * (1.0 / worst);
-            const double v = 10.0 * log10(lin);
-            const double xb = (v - P.hist_lo) / (P.hist_hi - P.hist_lo) * (double)P.hist_bins;
-            long long b = (long long)floor(xb);
-            if (!(xb >= 0.0)) b = 0;
-            if (b >= P.hist_bins) b = P.hist_bins - 1;
-            atomicAdd(&s_cnt[2 + P.nspec + (int)b], 1u);
+            qo_tally_hist(s_cnt, P.nspec, qo_hist_bin(10.0 * log10(lin), P.hist_lo, P.hist_hi, P.hist_bins));
         }
     }
     __syncthreads();
-    for (int i = threadIdx.x; i < ncnt; i += QO_SPOT_TPB)
-        if (s_cnt[i]) atomicAdd(&P.counters[i], (unsigned long long)s_cnt[i]);
+    qo_tally_flush<QO_SPOT_TPB>(s_cnt, ncnt, P.counters);
 }

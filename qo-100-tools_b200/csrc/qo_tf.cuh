@@ -315,11 +315,11 @@ __global__ void __launch_bounds__(TPB, MINB) qo_mc_tf_kernel(const __grid_consta
     __shared__ __align__(16) double s_el[WARPS][QO_TF_MAXEL * QO_TF_REC];
     __shared__ __align__(16) double s_cpl[WARPS][CPL ? QO_LAD_CPL + 8 : 2];     /* + the equal-angle constants of tf_cpl_matched_same */
     __shared__ double s_x[WARPS][QO_MAX_VAR];
-    __shared__ unsigned int s_cnt[2 + QO_NSPEC_MAX + QO_MAX_HIST];
+    __shared__ unsigned int s_cnt[QO_NCNT_MAX];
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int ncnt = 2 + P.nspec + (P.hist_bins > 0 ? P.hist_bins : 0);
-    for (int i = threadIdx.x; i < ncnt; i += TPB) s_cnt[i] = 0;
+    const int ncnt = qo_ncnt(P.nspec, P.hist_bins);
+    qo_tally_zero<TPB>(s_cnt, ncnt);
     __syncthreads();
     double *numw = s_num[warp] + 2 * NN, *denw = s_den[warp] + (DEN == QO_TF_DEN_NONE ? 0 : 4), *elw = s_el[warp], *xw = s_x[warp];
     const unsigned int nums = (unsigned int)__cvta_generic_to_shared(numw), dens = (unsigned int)__cvta_generic_to_shared(denw);
@@ -665,24 +665,16 @@ __global__ void __launch_bounds__(TPB, MINB) qo_mc_tf_kernel(const __grid_consta
             if (hneg ? trkv < t : trkv > t) fail |= 1u << hs;
         }
         if (lane == 0) {
-            atomicAdd(&s_cnt[0], fail == 0 ? 1u : 0u);
-            atomicAdd(&s_cnt[1], 1u);
-            for (int sp = 0; sp < P.nspec; sp++)
-                if ((fail >> sp) & 1u) atomicAdd(&s_cnt[2 + sp], 1u);
+            qo_tally_one(s_cnt, P.nspec, fail);
             if (hs >= 0) {
                 const double k21 = P.k21;
                 const double lin = (S11 && P.s11[hs & (QO_TF_NSPEC - 1)]) ? trkv : hneg ? k21 * k21 * (1.0 / trkv) : k21 * k21 / trkv;
                 const double v = (GD && P.gd[hs & (QO_TF_NSPEC - 1)]) ? trkv / P.wref : 10.0 * log10(lin);      /* seconds, or dB */
-                const double xb = (v - P.hist_lo) / (P.hist_hi - P.hist_lo) * (double)P.hist_bins;
-                long long b = (long long)floor(xb);
-                if (!(xb >= 0.0)) b = 0;
-                if (b >= P.hist_bins) b = P.hist_bins - 1;
-                atomicAdd(&s_cnt[2 + P.nspec + (int)b], 1u);
+                qo_tally_hist(s_cnt, P.nspec, qo_hist_bin(v, P.hist_lo, P.hist_hi, P.hist_bins));
             }
         }
         s = __shfl_sync(0xffffffffu, s_next, 0);
     }
     __syncthreads();
-    for (int i = threadIdx.x; i < ncnt; i += TPB)
-        if (s_cnt[i]) atomicAdd(&P.counters[i], (unsigned long long)s_cnt[i]);
+    qo_tally_flush<TPB>(s_cnt, ncnt, P.counters);
 }

@@ -368,10 +368,10 @@ __global__ void __launch_bounds__(QO_TS_TPB, MINB) qo_mc_ts_kernel(const __grid_
     static_assert(NN == 2 || NN == 4, "two or four numerator chains");
     static_assert(CPL == (NN == 4), "P and Q stay apart exactly when a coupled-line block is in front");
     const TfParams &P = Q.t;
-    __shared__ unsigned int s_cnt[2 + QO_NSPEC_MAX + QO_MAX_HIST];
+    __shared__ unsigned int s_cnt[QO_NCNT_MAX];
     const int lane = threadIdx.x & 31;
-    const int ncnt = 2 + P.nspec + (P.hist_bins > 0 ? P.hist_bins : 0);
-    for (int i = threadIdx.x; i < ncnt; i += QO_TS_TPB) s_cnt[i] = 0;
+    const int ncnt = qo_ncnt(P.nspec, P.hist_bins);
+    qo_tally_zero<QO_TS_TPB>(s_cnt, ncnt);
     __syncthreads();
     const int hs = P.hist_spec;
     const bool hneg = hs >= 0 && P.neg[hs & (QO_TF_NSPEC - 1)];
@@ -398,25 +398,14 @@ __global__ void __launch_bounds__(QO_TS_TPB, MINB) qo_mc_ts_kernel(const __grid_
             const double t = P.thr[hs & (QO_TF_NSPEC - 1)];
             if (hneg ? trkv < t : trkv > t) fail |= 1u << hs;
         }
-        const unsigned int okm = __ballot_sync(0xffffffffu, fail == 0u);
-        if (lane == 0) { atomicAdd(&s_cnt[0], (unsigned int)__popc(okm)); atomicAdd(&s_cnt[1], 32u); }
-        for (int sp = 0; sp < P.nspec; sp++) {
-            const unsigned int m = __ballot_sync(0xffffffffu, (fail >> sp) & 1u);
-            if (lane == 0 && m) atomicAdd(&s_cnt[2 + sp], (unsigned int)__popc(m));
-        }
+        qo_tally_warp(s_cnt, P.nspec, fail, 0xffffffffu);
         if (hs >= 0) {
             const double k21 = P.k21;
             const double lin = hneg ? k21 * k21 * (1.0 / trkv) : k21 * k21 / trkv;
-            const double v = 10.0 * log10(lin);
-            const double xb = (v - P.hist_lo) / (P.hist_hi - P.hist_lo) * (double)P.hist_bins;
-            long long bin = (long long)floor(xb);
-            if (!(xb >= 0.0)) bin = 0;
-            if (bin >= P.hist_bins) bin = P.hist_bins - 1;
-            atomicAdd(&s_cnt[2 + P.nspec + (int)bin], 1u);
+            qo_tally_hist(s_cnt, P.nspec, qo_hist_bin(10.0 * log10(lin), P.hist_lo, P.hist_hi, P.hist_bins));
         }
         batch = __shfl_sync(0xffffffffu, next, 0);
     }
     __syncthreads();
-    for (int i = threadIdx.x; i < ncnt; i += QO_TS_TPB)
-        if (s_cnt[i]) atomicAdd(&P.counters[i], (unsigned long long)s_cnt[i]);
+    qo_tally_flush<QO_TS_TPB>(s_cnt, ncnt, P.counters);
 }
