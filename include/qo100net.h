@@ -207,7 +207,9 @@ void qo_ctx_destroy(qo_ctx *ctx);
 int qo_sweep(qo_ctx *ctx, const qo_net *net, const double *f, int nf, int precision,
              qo_c64 *s11, qo_c64 *s21, qo_c64 *s12, qo_c64 *s22, double *gd);
 
-typedef enum { QO_SPEC_S21_MIN_DB = 1, QO_SPEC_S21_MAX_DB = 2, QO_SPEC_S11_MAX_DB = 3, QO_SPEC_GD_MAX = 4 } qo_spec_kind;
+/* a point fails when |S21| dB < limit (MIN), |S21| dB > limit (MAX), |S11| dB > limit, group delay [s] > limit, |S22| dB > limit
+ * (return loss at the output port; cascades only: qo_nodal_mc_run addresses S[row][col] itself) */
+typedef enum { QO_SPEC_S21_MIN_DB = 1, QO_SPEC_S21_MAX_DB = 2, QO_SPEC_S11_MAX_DB = 3, QO_SPEC_GD_MAX = 4, QO_SPEC_S22_MAX_DB = 5 } qo_spec_kind;
 typedef struct { int32_t kind; int32_t pad; double f_lo, f_hi, limit; } qo_spec; /* applies to grid f in [f_lo,f_hi] */
 #define QO_MAX_SPEC 8
 
@@ -297,7 +299,13 @@ int qo_plan_launches(const qo_plan *plan);            /* kernels launched so far
  * (util/pa-bias-simulation/pa-bias-simulation.sch:39), FULL_S behind a coupled line (util/directional-couplers/
  * dir_cpl_2.4g_20dB.trc:18-20) -- runs, from 2e10 evals per launch on (5e7 once this process or QO100NET_CACHE_DIR holds the
  * kernel; QO100NET_CHAIN=jit always, =interp never), on the interpreter's own source compiled at run time with the element
- * list, spec kinds and mode as constants (NVRTC, sm_100a): same arithmetic, no dispatch.  The name follows the last launch. */
+ * list, spec kinds and mode as constants (NVRTC, sm_100a): same arithmetic, no dispatch.  The name follows the last launch.
+ * |S22| jobs (QO_SPEC_S22_MAX_DB) without an |S11| spec, reduce-only FP64, on cascades of lumped branches and QO_TLINE lines run
+ * as the |S11| job on the reversed cascade (element e at n-1-e with its tolerances, Rs and Rl swapped: the same samples, S22 of
+ * the network = S11 of the reversal) when the spot, transfer-function or ladder kernel takes that job -- one of those three names
+ * therefore means the reversed route ran, as none of them takes |S22| otherwise.  Every other |S22| job (a coupled line or measured
+ * block in the cascade, |S11| next to it, FP32, QO100NET_KERNEL=interp) evaluates S22 directly on the interpreter or the compiled
+ * chain kernel; microstrip jobs on their own kernels. */
 const char *qo_plan_kernel_name(const qo_plan *plan);
 /* The host-only part of that (NVRTC compiles without a GPU): fold this job's element list into the chain kernel and compile it.
  * info[0] = compiled (0: libnvrtc missing or a compilation error, see qo_last_error), [1] = registers per thread, [2] = spill

@@ -364,6 +364,7 @@ static int build_prog(const qo_net *net, const double *f, int nf, const qo_spec 
         case QO_SPEC_S21_MIN_DB: hp->spec_kind[s] = SK_DEN2_MAX; hp->spec_thr[s] = ustrip ? lin : hp->k21 * hp->k21 / lin; break;
         case QO_SPEC_S21_MAX_DB: hp->spec_kind[s] = SK_DEN2_MIN; hp->spec_thr[s] = ustrip ? lin : hp->k21 * hp->k21 / lin; break;
         case QO_SPEC_S11_MAX_DB: hp->spec_kind[s] = SK_S11_MAX; hp->spec_thr[s] = lin; hp->need_s11 = 1; break;
+        case QO_SPEC_S22_MAX_DB: hp->spec_kind[s] = SK_S22_MAX; hp->spec_thr[s] = lin; hp->need_s22 = 1; break;
         case QO_SPEC_GD_MAX:        /* limit in seconds; evaluated in-kernel by the central difference of arg S21 */
             if (ustrip) { qo_set_error("QO_SPEC_GD_MAX is not available for microstrip networks"); return QO_ERR_UNSUPPORTED; }
             for (int e = 0; e < net->n; e++)
@@ -432,6 +433,43 @@ static int spot_eligible(const DevProg *hp, int mode, int precision, int nf, con
         if (hp->spec_kind[s] != SK_DEN2_MAX && hp->spec_kind[s] != SK_DEN2_MIN && hp->spec_kind[s] != SK_S11_MAX) return 0;
     *el0 = e0; *nel = nl;
     return 1;
+}
+
+/* |S22| jobs on the polynomial and ladder kernels.  Every lumped branch and every lossless line is a symmetric, reciprocal two-port,
+ * so S22 of a cascade N between (Rs, Rl) is exactly S11 of the reversed cascade between (Rl, Rs), and S21 is unchanged.  Each
+ * element's draw depends on (sample, var) and its own parameters only, so the reversed job -- element e at n-1-e, terminations
+ * swapped, |S22| specs turned into |S11| specs in the same order -- draws the same samples and runs on the |S11| instantiations
+ * those kernels already have.  Builds the reversed network and program (rnet, rhp, rmask: the grid mask is the same) and returns
+ * NULL when the spot, transfer-function or ladder kernel takes it (rtp, *rtf: its transfer-function analysis), else why not; the
+ * job then runs on the interpreter or the compiled chain kernel, which evaluate S22 directly. */
+static const char *s22_reversed(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
+                                const DevProg *hp, int generic, const QoOverrides *ov, qo_net *rnet, DevProg *rhp,
+                                std::vector<unsigned char> *rmask, TfPlan *rtp, int *rtf)
+{
+    const int mode = cfg ? cfg->mode : QO_MODE_FULL_S, precision = cfg && cfg->precision == 32 ? 32 : 64;
+    if (generic || mode != QO_MODE_REDUCE_ONLY || precision != 64) return "not a reduce-only FP64 job on a lumped cascade";
+    if (hp->need_s11) return "|S11| and |S22| specs in one job";
+    /* a coupled line is symmetric too, but the kernels take it in front only; a measured block may be non-reciprocal */
+    for (int e = 0; e < hp->n_ops; e++)
+        if (qo_tf_degree(hp->opcode[e]) < 0 && hp->opcode[e] != OP_TLINE) return "|S22| needs a cascade of lumped branches and lines";
+    const int n = net->n;
+    memset(rnet, 0, sizeof *rnet);
+    rnet->n = n; rnet->rs = net->rl; rnet->rl = net->rs;
+    for (int e = 0; e < n; e++) rnet->e[e] = net->e[n - 1 - e];
+    std::vector<qo_spec> rspec(spec, spec + nspec);
+    for (qo_spec &s : rspec) if (s.kind == QO_SPEC_S22_MAX_DB) s.kind = QO_SPEC_S11_MAX_DB;
+    std::vector<qo_tol> rtol;
+    if (cfg->n_tol > 0) rtol.assign(cfg->tol, cfg->tol + cfg->n_tol);
+    for (qo_tol &t : rtol) t.elem = n - 1 - t.elem;
+    qo_mc_cfg rcfg = *cfg;
+    rcfg.tol = rtol.data();
+    int rgen = 0;
+    double rfl = 0.0;
+    if (build_prog(rnet, f, nf, rspec.data(), nspec, &rcfg, rhp, &rgen, &rfl, rmask) != QO_OK) return "reversed cascade does not compile";
+    *rtf = qo_tf_plan_check(rhp, 1, precision, 0, f, nf, rmask->data(), ov, rtp);
+    int a, b, c;
+    if (*rtf || spot_eligible(rhp, mode, precision, nf, ov, &a, &b) || ladder_eligible(rhp, mode, precision, ov, &a, &b, &c)) return NULL;
+    return rtp->reason;
 }
 
 /* the plan's kernel (QoKern, in order of precedence) */
@@ -710,10 +748,24 @@ static int plan_create(qo_ctx *ctx, const qo_net *net, const double *f, int nf, 
             if (net->e[e].kind == QO_SBLOCK) { qo_set_error("S-parameter blocks cannot be mixed with microstrip elements yet"); delete p; return QO_ERR_UNSUPPORTED; }
     p->ncnt = qo_ncnt(nspec, p->hp.hist_bins);
     p->f.assign(f, f + nf);
+    const char *s22_why = NULL;
+    qo_net *rnet = NULL;
+    if (p->hp.need_s22) {
+        rnet = new qo_net;
+        DevProg *rhp = new DevProg;
+        std::vector<unsigned char> rmask;
+        TfPlan rtp;
+        int rtf;
+        s22_why = s22_reversed(net, f, nf, spec, nspec, cfg, &p->hp, p->generic, ov, rnet, rhp, &rmask, &rtp, &rtf);
+        if (!s22_why) { p->hp = *rhp; p->maskv.swap(rmask); net = rnet; }
+        delete rhp;
+    }
     p->kern = select_kernel(p, f, nf);
+    if (s22_why) p->tfp.reason = s22_why;
     p->kernel_name = qo_kern_name[p->kern];
     p->cj_debug = getenv("QO100NET_CHAIN_DEBUG") != NULL;
     rc = build_tables(p, net, f);
+    delete rnet;
     if (rc == QO_OK) rc = upload(p);
     if (rc) { qo_plan_destroy(p); return rc; }
     if (p->kern == K_TF) tf_launch_setup(p, ov);
@@ -793,6 +845,17 @@ static const char *plan_analyze(const qo_net *net, const double *f, int nf, cons
         const int precision = cfg && cfg->precision == 32 ? 32 : 64;
         const int mode = cfg ? cfg->mode : QO_MODE_FULL_S;
         *sel = qo_tf_plan_check(hp, mode == QO_MODE_REDUCE_ONLY, precision, generic, f, nf, maskv.data(), &ov, tp);
+        if (hp->need_s22) {             /* the analysis of the program that runs: the reversed cascade's when it is taken */
+            qo_net *rnet = new qo_net;
+            DevProg *rhp = new DevProg;
+            std::vector<unsigned char> rmask;
+            TfPlan *rtp = new TfPlan;
+            int rtf = 0;
+            const char *why = s22_reversed(net, f, nf, spec, nspec, cfg, hp, generic, &ov, rnet, rhp, &rmask, rtp, &rtf);
+            if (why) tp->reason = why;
+            else { *tp = *rtp; *sel = rtf; }
+            delete rtp; delete rhp; delete rnet;
+        }
         reason = tp->reason ? tp->reason : "";
     }
     clock_gettime(CLOCK_MONOTONIC, &t1);
@@ -934,11 +997,15 @@ static int launch_lumped(qo_plan *p, int g, unsigned long long off, unsigned lon
         }
     }
     p->kernel_name = "qo_mc_lumped_kernel";
-#define QO_LAUNCH(FS, TR, GD)                                                                                       \
-    qo_mc_lumped_kernel<T, FS, TR, GD><<<grid, QO_TPB, 0, dc->stream>>>(prog, w2, wi2, m2, p->nf, p->npairs, ppc, nchunks, off, n, cnt, pl)
-    if (full_s) { if (p->hp.has_trig) QO_LAUNCH(true, true, false); else QO_LAUNCH(true, false, false); }
-    else if (p->hp.need_gd) { if (p->hp.has_trig) QO_LAUNCH(false, true, true); else QO_LAUNCH(false, false, true); }
-    else { if (p->hp.has_trig) QO_LAUNCH(false, true, false); else QO_LAUNCH(false, false, false); }
+#define QO_LAUNCH(FS, TR, GD, S22)                                                                                  \
+    qo_mc_lumped_kernel<T, FS, TR, GD, S22><<<grid, QO_TPB, 0, dc->stream>>>(prog, w2, wi2, m2, p->nf, p->npairs, ppc, nchunks, off, n, cnt, pl)
+#define QO_LAUNCH_TR(FS, GD, S22) do { if (p->hp.has_trig) QO_LAUNCH(FS, true, GD, S22); else QO_LAUNCH(FS, false, GD, S22); } while (0)
+    /* |S22| jobs have instantiations of their own: the others' machine code stays as it was */
+    if (full_s) QO_LAUNCH_TR(true, false, false);
+    else if (p->hp.need_s22) { if (p->hp.need_gd) QO_LAUNCH_TR(false, true, true); else QO_LAUNCH_TR(false, false, true); }
+    else if (p->hp.need_gd) QO_LAUNCH_TR(false, true, false);
+    else QO_LAUNCH_TR(false, false, false);
+#undef QO_LAUNCH_TR
 #undef QO_LAUNCH
     CU(cudaGetLastError());
     return QO_OK;

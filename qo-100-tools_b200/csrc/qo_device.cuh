@@ -34,13 +34,14 @@ enum {
 
 /* canonical spec forms: a point FAILS when q > thr */
 enum { SK_DEN2_MAX = 1 /* S21_MIN_DB: |den|^2 <= thr */, SK_DEN2_MIN = 2 /* S21_MAX_DB: |den|^2 >= thr */,
-       SK_S11_MAX = 3 /* |n11|^2 <= thr*|den|^2 */, SK_GD_MAX = 4 };
+       SK_S11_MAX = 3 /* |n11|^2 <= thr*|den|^2 */, SK_GD_MAX = 4, SK_S22_MAX = 5 /* |n22|^2 <= thr*|den|^2 */ };
 
 struct DevProg {
     int32_t n_ops, n_var, n_coef, dist;
     int32_t nspec, hist_spec, hist_bins, need_s11;
     int32_t has_trig, has_ustrip, need_gd, op0;     /* op0: first op that is not an OP_NOP (a SUBST that only serves a QO_CPL_MS) */
-    int32_t cplms_elem, cplms_sub, pad1, pad2;      /* physical coupled-line element and its substrate element, -1 = none */
+    int32_t cplms_elem, cplms_sub;                  /* physical coupled-line element and its substrate element, -1 = none */
+    int32_t need_s22, pad2;                         /* need_s22 sits where a pad was: every other field keeps its offset */
     double cplms_nom[4];                            /* its nominal Z0e, Z0o, theta_e, theta_o [deg] */
     uint64_t seed;
     double rs, rl, rsrl, k21;                /* k21 = 2*sqrt(rs*rl) */

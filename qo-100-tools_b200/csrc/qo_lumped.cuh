@@ -301,7 +301,7 @@ __device__ __forceinline__ void qo_st256(double2 *p, double2 a, double2 b)
 extern "C" __global__ void __launch_bounds__(QO_TPB, 2)
 qo_mc_chain_jit_kernel(
 #else
-template <typename T, bool FULL_S, bool TRIG, bool GD>
+template <typename T, bool FULL_S, bool TRIG, bool GD, bool S22>
 __global__ void __launch_bounds__(QO_TPB, 2)
 qo_mc_lumped_kernel(
 #endif
@@ -383,7 +383,7 @@ qo_mc_lumped_kernel(
             double2 o11[2], o21[2], o22[2];
             QO_P2 {
                 /* den = A Rl + B + C Rs Rl + D Rs ; n11 = A Rl + B - C Rs Rl - D Rs */
-                T den_r, den_i, n_r = T(0), n_i = T(0), num2 = T(0);
+                T den_r, den_i, n_r = T(0), n_i = T(0), num2 = T(0), num22 = T(0);
                 if (need_s11) {
                     T pr = qfma(m.ar[p], rl, m.br[p]), pi_ = qfma(m.ai[p], rl, m.bi[p]);
                     T qr = qfma(m.cr[p], rsrl, m.dr[p] * rs), qi = qfma(m.ci[p], rsrl, m.di[p] * rs);
@@ -396,6 +396,16 @@ qo_mc_lumped_kernel(
                     den_i = qfma(m.di[p], rs, qfma(m.ci[p], rsrl, qfma(m.ai[p], rl, m.bi[p])));
                 }
                 const T den2 = qfma(den_r, den_r, den_i * den_i);
+                if (S22 && !FULL_S) {
+                    /* n22 = -A Rl + B - C Rs Rl + D Rs; on the row vector (a, b) = [1 Rs] M that is -a Rl + b */
+                    T xr, xi;
+                    if (QO_ROW) { xr = qfma(-m.ar[p], rl, m.br[p]); xi = qfma(-m.ai[p], rl, m.bi[p]); }
+                    else {
+                        xr = qfma(-m.ar[p], rl, m.br[p]) + qfma(-m.cr[p], rsrl, m.dr[p] * rs);
+                        xi = qfma(-m.ai[p], rl, m.bi[p]) + qfma(-m.ci[p], rsrl, m.di[p] * rs);
+                    }
+                    num22 = qfma(xr, xr, xi * xi);
+                }
                 if (FULL_S) {
                     const T r = qrcp(den2);
                     const T ir = den_r * r, ii = -den_i * r;
@@ -436,14 +446,15 @@ qo_mc_lumped_kernel(
                             const int sk = QO_SK(sp);
                             const T thr = s_thr[sp];
                             bool bad = sk == SK_DEN2_MAX ? (den2 > thr) : sk == SK_DEN2_MIN ? (den2 < thr)
-                                     : sk == SK_S11_MAX ? (num2 > thr * den2) : (gdv > s_gdthr[sp]);
+                                     : sk == SK_S11_MAX ? (num2 > thr * den2) : (S22 && sk == SK_S22_MAX) ? (num22 > thr * den2)
+                                     : (gdv > s_gdthr[sp]);
                             if (bad && ((mb >> sp) & 1u)) fail |= 1u << sp;
                         }
                     }
                     if (GD && hist_kind == SK_GD_MAX && hist_spec >= 0 && ((mb >> hist_spec) & 1u) && gdv > gd_worst) gd_worst = gdv;
                     if (hist_spec >= 0 && hist_kind != SK_GD_MAX && ((mb >> hist_spec) & 1u)) {
                         /* track the worst value as a ratio a/b ("larger is worse") without dividing */
-                        T a = hist_kind == SK_DEN2_MAX ? den2 : hist_kind == SK_DEN2_MIN ? T(1) : num2;
+                        T a = hist_kind == SK_DEN2_MAX ? den2 : hist_kind == SK_DEN2_MIN ? T(1) : (S22 && hist_kind == SK_S22_MAX) ? num22 : num2;
                         T b = hist_kind == SK_DEN2_MAX ? T(1) : den2;
                         if (a * wd > wn * b) { wn = a; wd = b; }
                     }
@@ -501,7 +512,7 @@ qo_mc_lumped_kernel(
                 qo_tally_one(s_cnt, nspec, fail);
                 if (hist_spec >= 0) {
                     double ratio = (double)wn / (double)wd;
-                    double lin = hist_kind == SK_S11_MAX ? ratio
+                    double lin = hist_kind == SK_S11_MAX || (S22 && hist_kind == SK_S22_MAX) ? ratio
                                : hist_kind == SK_DEN2_MAX ? (double)k21 * (double)k21 / ratio
                                                           : (double)k21 * (double)k21 * ratio;
                     double v = hist_kind == SK_GD_MAX ? gd_worst : 10.0 * log10(lin);

@@ -376,14 +376,16 @@ qo_mc_board_kernel(const DevProg *__restrict__ prog, const double *__restrict__ 
             cd s11, s21, s12, s22;
             qo_generic_s(prog, M[k], s11, s21, s12, s22);
             const double p21 = s21.re * s21.re + s21.im * s21.im, p11 = s11.re * s11.re + s11.im * s11.im;
+            const double p22 = s22.re * s22.re + s22.im * s22.im;
             for (int sp = 0; sp < nspec; sp++) {
                 if (!((mb[k] >> sp) & 1u)) continue;
                 const int uk = prog->spec_user_kind[sp];
                 const double lim = prog->spec_thr[sp];      /* linear power limit in this kernel */
-                const bool bad = uk == 1 ? (p21 < lim) : uk == 2 ? (p21 > lim) : (p11 > lim);
+                const double v = uk == 3 ? p11 : uk == 5 ? p22 : p21;      /* qo_spec_kind: |S11|, |S22|, else |S21| */
+                const bool bad = uk == 1 ? (v < lim) : (v > lim);
                 if (bad) fail |= 1u << sp;
                 if (sp == hist_spec) {
-                    const unsigned long long key = d2key(uk == 3 ? p11 : p21);
+                    const unsigned long long key = d2key(v);
                     worst = hist_min ? (key < worst ? key : worst) : (key > worst ? key : worst);
                 }
             }

@@ -3,7 +3,7 @@
 
 For each of --nets random networks -- 3..14 branches drawn from all ten lumped branch kinds (with and without parasitics),
 optionally behind a front block (coupled line, transmission line), random terminations, random tolerances, log or linear
-grid of random length, 1..4 specs on |S21| / |S11| placed at quantiles of a FULL_S pre-run so that the yield is never
+grid of random length, 1..4 specs on |S21| / |S11| (and |S22| with --s22) placed at quantiles of a FULL_S pre-run so that the yield is never
 degenerate, optional histogram -- the job runs
    (a) on the kernel the plan selects (thread-per-sample / warp-per-sample transfer-function kernel, spot kernel, chain kernel),
    (b) on the opcode interpreter (QO100NET_KERNEL=interp),
@@ -37,6 +37,48 @@ def _block(Q):
         R.sblock_clear()
         R.sblock_register(0, fd, sd[:, 0], sd[:, 1], sd[:, 2], sd[:, 3], z0)
     return _BLK["blk"]
+
+
+SPEC_S21_MIN_DB, SPEC_S11_MAX_DB, SPEC_GD_MAX, SPEC_S22_MAX_DB = 1, 3, 4, 5     # qo_spec_kind
+_PLANE = {1: 1, 2: 1, 3: 0, 5: 3}                                                # spec kind -> FULL_S plane (S11, S21, S12, S22)
+
+
+def oracle_counters(R, net, f, specs, cfg, nthreads=None, chunk=256):
+    """The CPU oracle's counters of a cascade job.  Its own reduction (ref_mc_run) knows |S21|, |S11| and group-delay specs; a job
+    with |S22| specs is reduced here from the oracle's FULL_S planes of the same samples, the way ref_mc_run reduces the others:
+    per spec the worst in-band 10 log10 |S|^2 (smallest for an |S21| minimum, else largest), a fail when it is beyond the limit,
+    the histogram bin floor((worst - lo) / (hi - lo) * bins) clamped to the window."""
+    nthreads = nthreads or R.max_threads()
+    rs, rl = net.terminations
+    el = R.make_elems(net.elements)
+    f = np.ascontiguousarray(f, dtype=np.float64)
+    if not any(s[0] == SPEC_S22_MAX_DB for s in specs):
+        return R.mc_run(el, rs, rl, f, specs, cfg, nthreads=nthreads)
+    if any(s[0] not in _PLANE for s in specs):
+        raise ValueError("group-delay specs next to |S22| specs are not reduced from FULL_S planes")
+    n, nspec = int(cfg.n_samples), len(specs)
+    bands = [(f >= s[1]) & (f <= s[2]) for s in specs]
+    worst = np.zeros((nspec, n))
+    for a in range(0, n, chunk):
+        c = type(cfg).from_buffer_copy(cfg)              # same seed, tolerances (the pointer stays valid), distribution
+        c.sample_offset, c.n_samples, c.hist_bins = cfg.sample_offset + a, min(chunk, n - a), 0
+        planes = R.mc_run(el, rs, rl, f, [], c, full_s=True, nthreads=nthreads)["s"]
+        for i, s in enumerate(specs):
+            if not bands[i].any():
+                continue
+            p = planes[_PLANE[s[0]]][:, bands[i]]
+            v = 10.0 * np.log10(p.real * p.real + p.imag * p.imag)
+            worst[i, a:a + c.n_samples] = v.min(axis=1) if s[0] == SPEC_S21_MIN_DB else v.max(axis=1)
+    fails = np.zeros((nspec, n), dtype=bool)
+    for i, s in enumerate(specs):
+        if bands[i].any():
+            fails[i] = ~(worst[i] >= s[3]) if s[0] == SPEC_S21_MIN_DB else ~(worst[i] <= s[3])
+    hb = int(cfg.hist_bins)
+    hist = np.zeros(max(hb, 0), dtype=np.uint64)
+    if hb > 0 and 0 <= cfg.hist_spec < nspec and bands[cfg.hist_spec].any():
+        x = (worst[cfg.hist_spec] - cfg.hist_lo) / (cfg.hist_hi - cfg.hist_lo) * hb
+        np.add.at(hist, np.clip(np.floor(x), 0, hb - 1).astype(np.int64), 1)
+    return dict(n_pass=int((~fails.any(axis=0)).sum()), n_total=n, fail_per_spec=fails.sum(axis=1).astype(np.uint64), hist=hist)
 
 
 def random_ladder(Q, rng):
@@ -148,13 +190,15 @@ def main(argv=None):
     ap.add_argument("--gd", action="store_true", help="add a group-delay spec (limit around the nominal network's worst in-band delay) to networks without a front block")
     ap.add_argument("--chain-jit", action="store_true", help="the selected run is the run-time compiled chain kernel (QO100NET_KERNEL=interp QO100NET_CHAIN=jit) against the "
                     "interpreter proper; 60 %% of the networks get a perturbed line BEHIND the cascade and 30 %% the measured two-port behind that -- what no polynomial kernel takes")
+    ap.add_argument("--s22", action="store_true", help="|S22| specs in the random spec mix: the reversed cascade on the polynomial / ladder kernels, "
+                    "or the interpreter's direct S22 (next to |S11|, behind a front block)")
     ap.add_argument("--only", type=int, default=-1, help="run just this network (each network has its own random stream) and dump it")
     ap.add_argument("--out", default=None)
     args = ap.parse_args(argv)
     import qo100net as Q
     from oracle import refbind as R
     ctx = Q.Context(device=0)
-    kernels, mism, skipped, oracle_checked, fs_checked, fused_runs = {}, [], 0, 0, 0, 0
+    kernels, mism, skipped, oracle_checked, fs_checked, fused_runs, s22_jobs = {}, [], 0, 0, 0, 0, 0
     big = 2 * 148 * 3 * 128 + 77          # large enough for the thread-per-sample kernel on every 7th network
     for i in range(args.nets):
         if args.only >= 0 and i != args.only:
@@ -179,7 +223,8 @@ def main(argv=None):
             continue
         a21 = 20 * np.log10(np.maximum(np.abs(fs[1]), 1e-300))
         a11 = 20 * np.log10(np.maximum(np.abs(fs[0]), 1e-300))
-        if not (np.all(np.isfinite(a21)) and np.all(np.isfinite(a11))):
+        a22 = 20 * np.log10(np.maximum(np.abs(fs[3]), 1e-300))
+        if not (np.all(np.isfinite(a21)) and np.all(np.isfinite(a11)) and (not args.s22 or np.all(np.isfinite(a22)))):
             skipped += 1
             continue
         specs = []
@@ -190,12 +235,14 @@ def main(argv=None):
             band = (f >= lo) & (f <= hi)
             if not band.any():
                 continue
-            kind = int(rng.choice([Q.SPEC_S21_MIN_DB, Q.SPEC_S21_MAX_DB, Q.SPEC_S11_MAX_DB]))
+            kind = int(rng.choice([Q.SPEC_S21_MIN_DB, Q.SPEC_S21_MAX_DB, Q.SPEC_S11_MAX_DB] + ([Q.SPEC_S22_MAX_DB] * 2 if args.s22 else [])))
             q = float(rng.uniform(0.2, 0.8))
             if kind == Q.SPEC_S21_MIN_DB:
                 v, qq = a21[:, band].min(axis=1), 1 - q
             elif kind == Q.SPEC_S21_MAX_DB:
                 v, qq = a21[:, band].max(axis=1), q
+            elif kind == Q.SPEC_S22_MAX_DB:
+                v, qq = a22[:, band].max(axis=1), q
             else:
                 v, qq = a11[:, band].max(axis=1), q
             # no knife-edge specs: a quantity the tolerances barely move (all samples within 0.01 dB: any threshold inside that
@@ -203,7 +250,7 @@ def main(argv=None):
             if np.quantile(v, 0.9) - np.quantile(v, 0.1) < 0.01 or v.min() < -140.0:
                 continue
             specs.append((kind, float(lo), float(hi), float(np.quantile(v, qq))))
-        if args.gd and net.elements[0][0] not in (Q.CPL_THRU, Q.TLINE, Q.SBLOCK) and all(k_ != Q.SBLOCK for k_, _p in net.elements) and len(specs) < 8 and not any(s_[0] == Q.SPEC_S11_MAX_DB for s_ in specs):
+        if args.gd and net.elements[0][0] not in (Q.CPL_THRU, Q.TLINE, Q.SBLOCK) and all(k_ != Q.SBLOCK for k_, _p in net.elements) and len(specs) < 8 and not any(s_[0] in (Q.SPEC_S11_MAX_DB, Q.SPEC_S22_MAX_DB) for s_ in specs):
             gdn = ctx.sweep(net, f, gd=True)[4]
             lo, hi = sorted(rng.uniform(f[0], f[-1], 2))
             band = (f >= lo) & (f <= hi)
@@ -214,6 +261,7 @@ def main(argv=None):
         if not specs:
             skipped += 1
             continue
+        s22_jobs += any(s_[0] == Q.SPEC_S22_MAX_DB for s_ in specs)
         hist = {}
         if rng.random() < 0.6:
             hs = int(rng.integers(0, len(specs)))
@@ -243,8 +291,7 @@ def main(argv=None):
         os.environ.pop("QO100NET_KERNEL", None)
         same = got["n_pass"] == ref["n_pass"] and np.array_equal(got["fail_per_spec"], ref["fail_per_spec"]) and np.array_equal(got["hist"], ref["hist"])
         if same and i % args.oracle_every == 0 and n <= args.samples:
-            rs, rl = net.terminations
-            o = R.mc_run(R.make_elems(net.elements), rs, rl, f, specs, R.mc_cfg(1000 + i, n, tols, sample_offset=off, dist=dist, **hist), nthreads=R.max_threads())
+            o = oracle_counters(R, net, f, specs, R.mc_cfg(1000 + i, n, tols, sample_offset=off, dist=dist, **hist))
             oracle_checked += 1
             same = got["n_pass"] == o["n_pass"] and np.array_equal(got["fail_per_spec"], o["fail_per_spec"]) and np.array_equal(got["hist"], o["hist"])
         if same and i % 4 == 1:
@@ -270,7 +317,7 @@ def main(argv=None):
                          "specs": specs, "got": int(got["n_pass"]), "interp": int(ref["n_pass"]),
                          "got_fail": [int(v) for v in got["fail_per_spec"]], "interp_fail": [int(v) for v in ref["fail_per_spec"]]})
     out = {"networks": args.nets, "skipped": skipped, "compared": args.nets - skipped, "oracle_checked": oracle_checked, "full_s_checked": fs_checked,
-           "fused_runs": fused_runs, "kernels_selected": kernels, "mismatches": len(mism), "details": mism[:10], "seed": args.seed, "samples": args.samples}
+           "fused_runs": fused_runs, "s22_jobs": s22_jobs, "kernels_selected": kernels, "mismatches": len(mism), "details": mism[:10], "seed": args.seed, "samples": args.samples}
     print(json.dumps(out, indent=1))
     if args.out:
         open(args.out, "w").write(json.dumps(out, indent=1))
