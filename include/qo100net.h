@@ -208,8 +208,16 @@ int qo_sweep(qo_ctx *ctx, const qo_net *net, const double *f, int nf, int precis
              qo_c64 *s11, qo_c64 *s21, qo_c64 *s12, qo_c64 *s22, double *gd);
 
 /* a point fails when |S21| dB < limit (MIN), |S21| dB > limit (MAX), |S11| dB > limit, group delay [s] > limit, |S22| dB > limit
- * (return loss at the output port; cascades only: qo_nodal_mc_run addresses S[row][col] itself) */
-typedef enum { QO_SPEC_S21_MIN_DB = 1, QO_SPEC_S21_MAX_DB = 2, QO_SPEC_S11_MAX_DB = 3, QO_SPEC_GD_MAX = 4, QO_SPEC_S22_MAX_DB = 5 } qo_spec_kind;
+ * (return loss at the output port; cascades only: qo_nodal_mc_run addresses S[row][col] itself), or !(mu >= limit) (MU_MIN).
+ * QO_SPEC_MU_MIN: the Edwards-Sinsky load-side stability factor of the power-wave S w.r.t. (Rs, Rl) that qo_sweep returns,
+ *   mu = (1 - |S11|^2) / (|S22 - Delta conj(S11)| + |S12 S21|), Delta = S11 S22 - S12 S21; limit dimensionless (e.g. 1.0 or 1.05).
+ *   mu > 1 alone is necessary and sufficient for unconditional stability.  A NaN point fails.  With hist_spec on a mu spec the
+ *   histogram bins each sample's in-band MINIMUM of mu, linear (not dB).  Cascades with a measured block (QO_SBLOCK) only: every
+ *   other element is passive (mu >= 1 by construction), so a cascade without one is refused (QO_ERR_ARG); FP32 and microstrip
+ *   networks are refused (QO_ERR_UNSUPPORTED), and qo_nodal_mc_run refuses the kind.  Runs on the interpreter or the compiled
+ *   chain kernel (qo_plan_kernel_name). */
+typedef enum { QO_SPEC_S21_MIN_DB = 1, QO_SPEC_S21_MAX_DB = 2, QO_SPEC_S11_MAX_DB = 3, QO_SPEC_GD_MAX = 4, QO_SPEC_S22_MAX_DB = 5,
+               QO_SPEC_MU_MIN = 6 } qo_spec_kind;
 typedef struct { int32_t kind; int32_t pad; double f_lo, f_hi, limit; } qo_spec; /* applies to grid f in [f_lo,f_hi] */
 #define QO_MAX_SPEC 8
 

@@ -365,6 +365,15 @@ static int build_prog(const qo_net *net, const double *f, int nf, const qo_spec 
         case QO_SPEC_S21_MAX_DB: hp->spec_kind[s] = SK_DEN2_MIN; hp->spec_thr[s] = ustrip ? lin : hp->k21 * hp->k21 / lin; break;
         case QO_SPEC_S11_MAX_DB: hp->spec_kind[s] = SK_S11_MAX; hp->spec_thr[s] = lin; hp->need_s11 = 1; break;
         case QO_SPEC_S22_MAX_DB: hp->spec_kind[s] = SK_S22_MAX; hp->spec_thr[s] = lin; hp->need_s22 = 1; break;
+        case QO_SPEC_MU_MIN: {      /* limit dimensionless; mu from all four S-parameters, so the 2x2 product (need_s11) */
+            if (ustrip) { qo_set_error("QO_SPEC_MU_MIN is not available for microstrip networks"); return QO_ERR_UNSUPPORTED; }
+            if (cfg && cfg->precision == 32) { qo_set_error("QO_SPEC_MU_MIN needs FP64 (1 - |S11|^2 near |S11| = 1)"); return QO_ERR_UNSUPPORTED; }
+            int blk = 0;
+            for (int e = 0; e < net->n; e++) blk |= net->e[e].kind == QO_SBLOCK;
+            if (!blk) { qo_set_error("QO_SPEC_MU_MIN needs a measured two-port (QO_SBLOCK): every other element is passive, mu >= 1"); return QO_ERR_ARG; }
+            hp->spec_kind[s] = SK_MU_MIN; hp->spec_thr[s] = sp->limit; hp->need_s11 = 1;
+            break;
+        }
         case QO_SPEC_GD_MAX:        /* limit in seconds; evaluated in-kernel by the central difference of arg S21 */
             if (ustrip) { qo_set_error("QO_SPEC_GD_MAX is not available for microstrip networks"); return QO_ERR_UNSUPPORTED; }
             for (int e = 0; e < net->n; e++)
@@ -435,6 +444,16 @@ static int spot_eligible(const DevProg *hp, int mode, int precision, int nf, con
     return 1;
 }
 
+/* Stability specs (SK_MU_MIN) need S11, S21, S12 and S22 of each point: only the interpreter and the compiled chain kernel form
+ * them all.  The spot, transfer-function and ladder selectors refuse the spec kind; this gives qo_plan_tf_info and
+ * qo_plan_analyze the reason. */
+static const char *const qo_mu_reason = "stability spec needs all four S-parameters";
+static int prog_has_mu(const DevProg *hp)
+{
+    for (int s = 0; s < hp->nspec; s++) if (hp->spec_kind[s] == SK_MU_MIN) return 1;
+    return 0;
+}
+
 /* |S22| jobs on the polynomial and ladder kernels.  Every lumped branch and every lossless line is a symmetric, reciprocal two-port,
  * so S22 of a cascade N between (Rs, Rl) is exactly S11 of the reversed cascade between (Rl, Rs), and S21 is unchanged.  Each
  * element's draw depends on (sample, var) and its own parameters only, so the reversed job -- element e at n-1-e, terminations
@@ -448,6 +467,7 @@ static const char *s22_reversed(const qo_net *net, const double *f, int nf, cons
 {
     const int mode = cfg ? cfg->mode : QO_MODE_FULL_S, precision = cfg && cfg->precision == 32 ? 32 : 64;
     if (generic || mode != QO_MODE_REDUCE_ONLY || precision != 64) return "not a reduce-only FP64 job on a lumped cascade";
+    if (prog_has_mu(hp)) return qo_mu_reason;
     if (hp->need_s11) return "|S11| and |S22| specs in one job";
     /* a coupled line is symmetric too, but the kernels take it in front only; a measured block may be non-reciprocal */
     for (int e = 0; e < hp->n_ops; e++)
@@ -478,6 +498,7 @@ static QoKern select_kernel(qo_plan *p, const double *f, int nf)
     const QoOverrides *ov = &p->ov;
     /* analysed for every plan: qo_plan_tf_info reports the result (or why it refused) whichever kernel runs */
     const int tf = qo_tf_plan_check(&p->hp, p->mode == QO_MODE_REDUCE_ONLY, p->precision, p->generic, f, nf, p->maskv.data(), ov, &p->tfp);
+    if (!p->generic && p->mode == QO_MODE_REDUCE_ONLY && prog_has_mu(&p->hp)) { p->tfp.reason = qo_mu_reason; return K_LUMPED; }
     if (p->generic) return p->mode == QO_MODE_REDUCE_ONLY && nf <= QO_B_MAXNF && !ov->ustrip_item ? K_BOARD : K_GENERIC;
     if (spot_eligible(&p->hp, p->mode, p->precision, nf, ov, &p->spot_el0, &p->spot_nel)) return K_SPOT;
     if (tf) return K_TF;
@@ -845,6 +866,7 @@ static const char *plan_analyze(const qo_net *net, const double *f, int nf, cons
         const int precision = cfg && cfg->precision == 32 ? 32 : 64;
         const int mode = cfg ? cfg->mode : QO_MODE_FULL_S;
         *sel = qo_tf_plan_check(hp, mode == QO_MODE_REDUCE_ONLY, precision, generic, f, nf, maskv.data(), &ov, tp);
+        if (!generic && mode == QO_MODE_REDUCE_ONLY && prog_has_mu(hp)) { *sel = 0; tp->reason = qo_mu_reason; }
         if (hp->need_s22) {             /* the analysis of the program that runs: the reversed cascade's when it is taken */
             qo_net *rnet = new qo_net;
             DevProg *rhp = new DevProg;
@@ -997,11 +1019,13 @@ static int launch_lumped(qo_plan *p, int g, unsigned long long off, unsigned lon
         }
     }
     p->kernel_name = "qo_mc_lumped_kernel";
-#define QO_LAUNCH(FS, TR, GD, S22)                                                                                  \
-    qo_mc_lumped_kernel<T, FS, TR, GD, S22><<<grid, QO_TPB, 0, dc->stream>>>(prog, w2, wi2, m2, p->nf, p->npairs, ppc, nchunks, off, n, cnt, pl)
-#define QO_LAUNCH_TR(FS, GD, S22) do { if (p->hp.has_trig) QO_LAUNCH(FS, true, GD, S22); else QO_LAUNCH(FS, false, GD, S22); } while (0)
-    /* |S22| jobs have instantiations of their own: the others' machine code stays as it was */
+#define QO_LAUNCH(FS, TR, GD, S22, MU)                                                                              \
+    qo_mc_lumped_kernel<T, FS, TR, GD, S22, MU><<<grid, QO_TPB, 0, dc->stream>>>(prog, w2, wi2, m2, p->nf, p->npairs, ppc, nchunks, off, n, cnt, pl)
+#define QO_LAUNCH_TR(FS, GD, S22) do { if (p->hp.has_trig) QO_LAUNCH(FS, true, GD, S22, false); else QO_LAUNCH(FS, false, GD, S22, false); } while (0)
+    /* |S22| and stability jobs have instantiations of their own: the others' machine code stays as it was.  A stability job is
+     * FP64 and has a measured block, hence TRIG, and never group delay (build_prog); its one instantiation serves |S22| too. */
     if (full_s) QO_LAUNCH_TR(true, false, false);
+    else if (prog_has_mu(&p->hp)) { if constexpr (sizeof(T) == sizeof(double)) QO_LAUNCH(false, true, false, true, true); }
     else if (p->hp.need_s22) { if (p->hp.need_gd) QO_LAUNCH_TR(false, true, true); else QO_LAUNCH_TR(false, false, true); }
     else if (p->hp.need_gd) QO_LAUNCH_TR(false, true, false);
     else QO_LAUNCH_TR(false, false, false);

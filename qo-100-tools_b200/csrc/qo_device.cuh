@@ -35,6 +35,9 @@ enum {
 /* canonical spec forms: a point FAILS when q > thr */
 enum { SK_DEN2_MAX = 1 /* S21_MIN_DB: |den|^2 <= thr */, SK_DEN2_MIN = 2 /* S21_MAX_DB: |den|^2 >= thr */,
        SK_S11_MAX = 3 /* |n11|^2 <= thr*|den|^2 */, SK_GD_MAX = 4, SK_S22_MAX = 5 /* |n22|^2 <= thr*|den|^2 */ };
+//@mu{ lines between these markers reach the run-time compiled chain kernel's source only for jobs with a stability spec
+enum { SK_MU_MIN = 6 /* Edwards-Sinsky mu = num / den with den >= 0: a point fails when !(num >= thr*den) */ };
+//@mu}
 
 struct DevProg {
     int32_t n_ops, n_var, n_coef, dist;

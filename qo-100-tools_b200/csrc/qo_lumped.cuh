@@ -301,7 +301,14 @@ __device__ __forceinline__ void qo_st256(double2 *p, double2 a, double2 b)
 extern "C" __global__ void __launch_bounds__(QO_TPB, 2)
 qo_mc_chain_jit_kernel(
 #else
+//@mu{ MU: the stability spec (SK_MU_MIN) on the full 2x2 product; the chain kernel of every other job keeps the head below
+template <typename T, bool FULL_S, bool TRIG, bool GD, bool S22, bool MU>
+#if 0
+//@mu}
 template <typename T, bool FULL_S, bool TRIG, bool GD, bool S22>
+//@mu{
+#endif
+//@mu}
 __global__ void __launch_bounds__(QO_TPB, 2)
 qo_mc_lumped_kernel(
 #endif
@@ -365,6 +372,9 @@ qo_mc_lumped_kernel(
         /* 3. frequency loop: two points per lane per iteration */
         unsigned int fail = 0;
         T wn = T(0), wd = T(1);
+//@mu{
+        if (MU && hist_kind == SK_MU_MIN) { wn = T(-1); wd = T(0); }    /* -mu = -infinity: the first in-band point replaces it */
+//@mu}
         double gd_worst = -1e300;        /* largest group delay seen in the histogram spec's band (GD specs) */
         const int lo = chunk * pairs_per_chunk;
         const int hi = min(npairs, lo + pairs_per_chunk);
@@ -406,6 +416,24 @@ qo_mc_lumped_kernel(
                     }
                     num22 = qfma(xr, xr, xi * xi);
                 }
+//@mu{
+                /* Edwards-Sinsky mu = (1 - |S11|^2) / (|S22 - Delta conj(S11)| + |S12 S21|), Delta = S11 S22 - S12 S21, with
+                 * S11 = n11/D, S22 = n22/D, S21 = k21/D, S12 = k21 det/D (det: the blocks' product of AD - BC, 1 when every block
+                 * is reciprocal).  Multiplied through by |D|^3: mu = mu_n / mu_d, mu_n = (|D|^2 - |n11|^2) |D|,
+                 * mu_d = |X| + k21^2 |det| |D|, X = n22 (|D|^2 - |n11|^2) + k21^2 det conj(n11).  mu_d >= 0, so the verdict
+                 * needs no division and the worst-value tracker below orders -mu = -mu_n / mu_d correctly though mu may be < 0. */
+                T mu_n = T(0), mu_d = T(1);
+                if (MU && !FULL_S) {
+                    const T ur = qfma(-m.ar[p], rl, m.br[p]) + qfma(-m.cr[p], rsrl, m.dr[p] * rs);
+                    const T ui = qfma(-m.ai[p], rl, m.bi[p]) + qfma(-m.ci[p], rsrl, m.di[p] * rs);
+                    T dtr = T(1), dti = T(0);
+                    if (planes.sdet) { const double2 dt = planes.sdet[min(2 * j + p, planes.npts - 1)]; dtr = T(dt.x); dti = T(dt.y); }
+                    const T g = den2 - num2, kk = k21 * k21, aden = sqrt(den2);
+                    const T xr = qfma(ur, g, kk * qfma(dtr, n_r, dti * n_i)), xi = qfma(ui, g, kk * qfma(dti, n_r, -dtr * n_i));
+                    mu_n = g * aden;
+                    mu_d = qfma(kk * sqrt(qfma(dtr, dtr, dti * dti)), aden, sqrt(qfma(xr, xr, xi * xi)));
+                }
+//@mu}
                 if (FULL_S) {
                     const T r = qrcp(den2);
                     const T ir = den_r * r, ii = -den_i * r;
@@ -448,6 +476,9 @@ qo_mc_lumped_kernel(
                             bool bad = sk == SK_DEN2_MAX ? (den2 > thr) : sk == SK_DEN2_MIN ? (den2 < thr)
                                      : sk == SK_S11_MAX ? (num2 > thr * den2) : (S22 && sk == SK_S22_MAX) ? (num22 > thr * den2)
                                      : (gdv > s_gdthr[sp]);
+//@mu{
+                            if (MU && sk == SK_MU_MIN) bad = !(mu_n >= thr * mu_d);     /* !(mu >= limit): NaN fails */
+//@mu}
                             if (bad && ((mb >> sp) & 1u)) fail |= 1u << sp;
                         }
                     }
@@ -456,6 +487,9 @@ qo_mc_lumped_kernel(
                         /* track the worst value as a ratio a/b ("larger is worse") without dividing */
                         T a = hist_kind == SK_DEN2_MAX ? den2 : hist_kind == SK_DEN2_MIN ? T(1) : (S22 && hist_kind == SK_S22_MAX) ? num22 : num2;
                         T b = hist_kind == SK_DEN2_MAX ? T(1) : den2;
+//@mu{
+                        if (MU && hist_kind == SK_MU_MIN) { a = -mu_n; b = mu_d; }
+//@mu}
                         if (a * wd > wn * b) { wn = a; wd = b; }
                     }
                 }
@@ -516,6 +550,9 @@ qo_mc_lumped_kernel(
                                : hist_kind == SK_DEN2_MAX ? (double)k21 * (double)k21 / ratio
                                                           : (double)k21 * (double)k21 * ratio;
                     double v = hist_kind == SK_GD_MAX ? gd_worst : 10.0 * log10(lin);
+//@mu{
+                    if (MU && hist_kind == SK_MU_MIN) v = -ratio;               /* the in-band minimum of mu, linear */
+//@mu}
                     qo_tally_hist(s_cnt, nspec, qo_hist_bin(v, prog->hist_lo, prog->hist_hi, prog->hist_bins));
                 }
             }

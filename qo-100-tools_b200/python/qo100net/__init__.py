@@ -21,7 +21,7 @@ OK, ERR_ARG, ERR_IO, ERR_PARSE, ERR_UNSUPPORTED, ERR_NOMEM, ERR_NO_DEVICE, ERR_C
 SER_R, SHUNT_R, SER_L, SHUNT_L, SER_C, SHUNT_C = 1, 2, 3, 4, 5, 6
 SER_LC_SER, SER_LC_PAR, SHUNT_LC_SER, SHUNT_LC_PAR = 7, 8, 9, 10
 TLINE, CPL_THRU, SUBST, MLIN, MCORN, MTEE, MOPEN, SBLOCK, CPL_MS = 11, 12, 13, 14, 15, 16, 17, 18, 19
-SPEC_S21_MIN_DB, SPEC_S21_MAX_DB, SPEC_S11_MAX_DB, SPEC_GD_MAX, SPEC_S22_MAX_DB = 1, 2, 3, 4, 5
+SPEC_S21_MIN_DB, SPEC_S21_MAX_DB, SPEC_S11_MAX_DB, SPEC_GD_MAX, SPEC_S22_MAX_DB, SPEC_MU_MIN = 1, 2, 3, 4, 5, 6
 DIST_UNIFORM, DIST_GAUSS3S = 0, 1
 TOL_REL, TOL_ABS = 0, 1
 MODE_REDUCE_ONLY, MODE_FULL_S = 0, 1

@@ -3,7 +3,7 @@
 
 For each of --nets random networks -- 3..14 branches drawn from all ten lumped branch kinds (with and without parasitics),
 optionally behind a front block (coupled line, transmission line), random terminations, random tolerances, log or linear
-grid of random length, 1..4 specs on |S21| / |S11| (and |S22| with --s22) placed at quantiles of a FULL_S pre-run so that the yield is never
+grid of random length, 1..4 specs on |S21| / |S11| (and |S22| with --s22, a stability factor mu with --mu) placed at quantiles of a FULL_S pre-run so that the yield is never
 degenerate, optional histogram -- the job runs
    (a) on the kernel the plan selects (thread-per-sample / warp-per-sample transfer-function kernel, spot kernel, chain kernel),
    (b) on the opcode interpreter (QO100NET_KERNEL=interp),
@@ -27,9 +27,28 @@ sys.path.insert(0, ROOT)
 _BLK = {}
 
 
+def _register(R, names):
+    """hand the oracle the golden two-ports in the order the network holds them (block i = names[i])"""
+    g = np.load(os.path.join(ROOT, "tests", "golden", "touchstone.npz"))
+    R.sblock_clear()
+    for i, nm in enumerate(names):
+        sd = g[nm + "_s"]
+        R.sblock_register(i, g[nm + "_f"], sd[:, 0], sd[:, 1], sd[:, 2], sd[:, 3], float(g[nm + "_z0"]))
+
+
+def _driver(Q):
+    """The reference's 20 W driver (docs/pa-driver/pa_20W_vdd_32V_idq_180mA.s2p, tests/golden/touchstone.npz): active and
+    non-reciprocal."""
+    if "drv" not in _BLK:
+        g = np.load(os.path.join(ROOT, "tests", "golden", "touchstone.npz"))
+        sd = g["pa_20W_s"]
+        _BLK["drv"] = Q.SBlock.from_arrays(g["pa_20W_f"], sd[:, 0], sd[:, 1], sd[:, 2], sd[:, 3], float(g["pa_20W_z0"]))
+    return _BLK["drv"]
+
+
 def _block(Q):
     """The measured inductor of pa-bias-simulation.sch:39 (tests/golden/touchstone.npz), registered with the oracle as block 0."""
-    if not _BLK:
+    if "blk" not in _BLK:
         from oracle import refbind as R
         g = np.load(os.path.join(ROOT, "tests", "golden", "touchstone.npz"))
         fd, sd, z0 = g["11SQ39N_f"], g["11SQ39N_s"], float(g["11SQ39N_z0"])
@@ -39,26 +58,35 @@ def _block(Q):
     return _BLK["blk"]
 
 
-SPEC_S21_MIN_DB, SPEC_S11_MAX_DB, SPEC_GD_MAX, SPEC_S22_MAX_DB = 1, 3, 4, 5     # qo_spec_kind
+SPEC_S21_MIN_DB, SPEC_S11_MAX_DB, SPEC_GD_MAX, SPEC_S22_MAX_DB, SPEC_MU_MIN = 1, 3, 4, 5, 6     # qo_spec_kind
 _PLANE = {1: 1, 2: 1, 3: 0, 5: 3}                                                # spec kind -> FULL_S plane (S11, S21, S12, S22)
+
+
+def mu_factor(s11, s21, s12, s22):
+    """Edwards-Sinsky load-side stability factor: mu > 1 <=> unconditionally stable"""
+    d = s11 * s22 - s12 * s21
+    return (1.0 - np.abs(s11) ** 2) / (np.abs(s22 - d * np.conj(s11)) + np.abs(s12 * s21))
 
 
 def oracle_counters(R, net, f, specs, cfg, nthreads=None, chunk=256):
     """The CPU oracle's counters of a cascade job.  Its own reduction (ref_mc_run) knows |S21|, |S11| and group-delay specs; a job
-    with |S22| specs is reduced here from the oracle's FULL_S planes of the same samples, the way ref_mc_run reduces the others:
-    per spec the worst in-band 10 log10 |S|^2 (smallest for an |S21| minimum, else largest), a fail when it is beyond the limit,
-    the histogram bin floor((worst - lo) / (hi - lo) * bins) clamped to the window."""
+    with |S22| or stability (mu) specs is reduced here from the oracle's FULL_S planes of the same samples, the way ref_mc_run
+    reduces the others: per spec the worst in-band 10 log10 |S|^2 (smallest for an |S21| minimum, else largest), a fail when it is
+    beyond the limit, the histogram bin floor((worst - lo) / (hi - lo) * bins) clamped to the window.  A mu spec takes mu of each
+    point from all four planes (S12 carries the blocks' determinant); it fails when some in-band point has !(mu >= limit), NaN
+    included, and its histogram value is the smallest in-band mu that is not NaN (+inf when there is none), linear."""
     nthreads = nthreads or R.max_threads()
     rs, rl = net.terminations
     el = R.make_elems(net.elements)
     f = np.ascontiguousarray(f, dtype=np.float64)
-    if not any(s[0] == SPEC_S22_MAX_DB for s in specs):
+    if not any(s[0] in (SPEC_S22_MAX_DB, SPEC_MU_MIN) for s in specs):
         return R.mc_run(el, rs, rl, f, specs, cfg, nthreads=nthreads)
-    if any(s[0] not in _PLANE for s in specs):
-        raise ValueError("group-delay specs next to |S22| specs are not reduced from FULL_S planes")
+    if any(s[0] not in _PLANE and s[0] != SPEC_MU_MIN for s in specs):
+        raise ValueError("group-delay specs next to |S22| or mu specs are not reduced from FULL_S planes")
     n, nspec = int(cfg.n_samples), len(specs)
     bands = [(f >= s[1]) & (f <= s[2]) for s in specs]
     worst = np.zeros((nspec, n))
+    fails = np.zeros((nspec, n), dtype=bool)
     for a in range(0, n, chunk):
         c = type(cfg).from_buffer_copy(cfg)              # same seed, tolerances (the pointer stays valid), distribution
         c.sample_offset, c.n_samples, c.hist_bins = cfg.sample_offset + a, min(chunk, n - a), 0
@@ -66,12 +94,16 @@ def oracle_counters(R, net, f, specs, cfg, nthreads=None, chunk=256):
         for i, s in enumerate(specs):
             if not bands[i].any():
                 continue
+            if s[0] == SPEC_MU_MIN:
+                mu = mu_factor(*(planes[q][:, bands[i]] for q in range(4)))
+                worst[i, a:a + c.n_samples] = np.where(np.isnan(mu), np.inf, mu).min(axis=1)
+                fails[i, a:a + c.n_samples] = ~(mu >= s[3]).all(axis=1)
+                continue
             p = planes[_PLANE[s[0]]][:, bands[i]]
             v = 10.0 * np.log10(p.real * p.real + p.imag * p.imag)
             worst[i, a:a + c.n_samples] = v.min(axis=1) if s[0] == SPEC_S21_MIN_DB else v.max(axis=1)
-    fails = np.zeros((nspec, n), dtype=bool)
     for i, s in enumerate(specs):
-        if bands[i].any():
+        if bands[i].any() and s[0] != SPEC_MU_MIN:
             fails[i] = ~(worst[i] >= s[3]) if s[0] == SPEC_S21_MIN_DB else ~(worst[i] <= s[3])
     hb = int(cfg.hist_bins)
     hist = np.zeros(max(hb, 0), dtype=np.uint64)
@@ -192,13 +224,16 @@ def main(argv=None):
                     "interpreter proper; 60 %% of the networks get a perturbed line BEHIND the cascade and 30 %% the measured two-port behind that -- what no polynomial kernel takes")
     ap.add_argument("--s22", action="store_true", help="|S22| specs in the random spec mix: the reversed cascade on the polynomial / ladder kernels, "
                     "or the interpreter's direct S22 (next to |S11|, behind a front block)")
+    ap.add_argument("--mu", action="store_true", help="the 20 W driver (active, non-reciprocal) in front of or behind each random cascade, a "
+                    "stability spec mu >= limit in every job, the selected run on the compiled chain kernel against the interpreter")
     ap.add_argument("--only", type=int, default=-1, help="run just this network (each network has its own random stream) and dump it")
     ap.add_argument("--out", default=None)
     args = ap.parse_args(argv)
     import qo100net as Q
     from oracle import refbind as R
     ctx = Q.Context(device=0)
-    kernels, mism, skipped, oracle_checked, fs_checked, fused_runs, s22_jobs = {}, [], 0, 0, 0, 0, 0
+    kernels, mism, skipped, oracle_checked, fs_checked, fused_runs, s22_jobs, mu_jobs = {}, [], 0, 0, 0, 0, 0, 0
+    jit = args.chain_jit or args.mu
     big = 2 * 148 * 3 * 128 + 77          # large enough for the thread-per-sample kernel on every 7th network
     for i in range(args.nets):
         if args.only >= 0 and i != args.only:
@@ -214,6 +249,19 @@ def main(argv=None):
                 tols = list(tols) + [(ne, 0, nv, Q.TOL_REL, 0.05), (ne, 1, nv + 1, Q.TOL_REL, 0.03)]
             if rng.random() < 0.3 and fc < 2e9 and net.elements[0][0] != Q.SBLOCK:
                 net = net.concat(_block(Q).as_net(True, rs_, rl_))
+        if args.mu:
+            # the driver's data covers 10 MHz - 10 GHz: keep the grid inside it
+            f = f[(f >= 1e7) & (f <= 1e10)]
+            rs_, rl_ = net.terminations
+            drv = _driver(Q).as_net(bool(rng.integers(0, 2)), rs_, rl_)
+            ind = ["11SQ39N"] if any(k_ == Q.SBLOCK for k_, _p in net.elements) else []
+            if rng.random() < 0.5:
+                net = drv.concat(net)
+                tols = [(e + 1, p, v, m_, t) for (e, p, v, m_, t) in tols]
+                _register(R, ["pa_20W"] + ind)
+            else:
+                net = net.concat(drv)
+                _register(R, ind + ["pa_20W"])
         n = big if i % args.big_every == args.big_every - 1 else args.samples
         dist = Q.DIST_GAUSS3S if rng.random() < 0.3 else Q.DIST_UNIFORM
         try:
@@ -224,11 +272,22 @@ def main(argv=None):
         a21 = 20 * np.log10(np.maximum(np.abs(fs[1]), 1e-300))
         a11 = 20 * np.log10(np.maximum(np.abs(fs[0]), 1e-300))
         a22 = 20 * np.log10(np.maximum(np.abs(fs[3]), 1e-300))
-        if not (np.all(np.isfinite(a21)) and np.all(np.isfinite(a11)) and (not args.s22 or np.all(np.isfinite(a22)))):
+        if len(f) == 0 or not (np.all(np.isfinite(a21)) and np.all(np.isfinite(a11)) and (not args.s22 or np.all(np.isfinite(a22)))):
             skipped += 1
             continue
         specs = []
-        for _ in range(int(rng.choice([1, 2, 3, 4, 4, 6, 8]))):
+        if args.mu:
+            lo, hi = sorted(rng.uniform(f[0], f[-1], 2))
+            band = (f >= lo) & (f <= hi)
+            if band.any():
+                mu = mu_factor(*(np.asarray(fs[q])[:, band] for q in range(4))).min(axis=1)
+                # not a knife edge: the limit inside a real spread of the samples' smallest mu
+                if np.all(np.isfinite(mu)) and np.quantile(mu, 0.9) - np.quantile(mu, 0.1) > 1e-4 * max(1.0, abs(np.median(mu))):
+                    specs.append((Q.SPEC_MU_MIN, float(lo), float(hi), float(np.quantile(mu, rng.uniform(0.2, 0.8)))))
+            if not specs:
+                skipped += 1
+                continue
+        for _ in range(int(rng.choice([1, 2, 3, 4, 4, 6, 8])) - len(specs)):
             lo, hi = sorted(rng.uniform(f[0], f[-1], 2))
             if rng.random() < 0.3:
                 lo = hi = float(f[int(rng.integers(0, len(f)))])
@@ -262,6 +321,7 @@ def main(argv=None):
             skipped += 1
             continue
         s22_jobs += any(s_[0] == Q.SPEC_S22_MAX_DB for s_ in specs)
+        mu_jobs += any(s_[0] == Q.SPEC_MU_MIN for s_ in specs)
         hist = {}
         if rng.random() < 0.6:
             hs = int(rng.integers(0, len(specs)))
@@ -269,7 +329,7 @@ def main(argv=None):
         os.environ.pop("QO100NET_KERNEL", None)
         if args.ladders:
             os.environ["QO100NET_KERNEL"] = "ladder"
-        if args.chain_jit:
+        if jit:
             os.environ["QO100NET_KERNEL"] = "interp"
             os.environ["QO100NET_CHAIN"] = "jit"
         plan = Q.Plan(ctx, net, f, specs, seed=1000 + i, tols=tols, dist=dist, **hist)
@@ -296,7 +356,7 @@ def main(argv=None):
             same = got["n_pass"] == o["n_pass"] and np.array_equal(got["fail_per_spec"], o["fail_per_spec"]) and np.array_equal(got["hist"], o["hist"])
         if same and i % 4 == 1:
             # FULL_S: a launch large enough for qo_fs_tf_kernel against the interpreter's planes of the same samples
-            if args.chain_jit:
+            if jit:
                 os.environ["QO100NET_KERNEL"] = "interp"
                 os.environ["QO100NET_CHAIN"] = "jit"
             a = ctx.mc_run(net, f, [], 1000 + i, 1536, tols, sample_offset=off, mode=Q.MODE_FULL_S, dist=dist)["s"]
@@ -317,7 +377,7 @@ def main(argv=None):
                          "specs": specs, "got": int(got["n_pass"]), "interp": int(ref["n_pass"]),
                          "got_fail": [int(v) for v in got["fail_per_spec"]], "interp_fail": [int(v) for v in ref["fail_per_spec"]]})
     out = {"networks": args.nets, "skipped": skipped, "compared": args.nets - skipped, "oracle_checked": oracle_checked, "full_s_checked": fs_checked,
-           "fused_runs": fused_runs, "s22_jobs": s22_jobs, "kernels_selected": kernels, "mismatches": len(mism), "details": mism[:10], "seed": args.seed, "samples": args.samples}
+           "fused_runs": fused_runs, "s22_jobs": s22_jobs, "mu_jobs": mu_jobs, "kernels_selected": kernels, "mismatches": len(mism), "details": mism[:10], "seed": args.seed, "samples": args.samples}
     print(json.dumps(out, indent=1))
     if args.out:
         open(args.out, "w").write(json.dumps(out, indent=1))
