@@ -340,6 +340,14 @@ const char *qo_plan_analyze(const qo_net *net, const double *f, int nf, const qo
 int qo_plan_ts_runs(const qo_plan *plan, int *runs, int cap, int meta[2]);
 int qo_plan_analyze_ts_runs(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
                             int *runs, int cap, int meta[2]);
+/* The thread-per-sample kernel's histogram screen: "ok" when the histogram spec's runs are walked behind it, else why not;
+ * info = { relative margin eps, smallest and largest tracker value it covers, worst error bound / (eps / 8) }, meta = { seed runs
+ * (the first runs of the table), screened runs, 1 when the plan's last thread-per-sample launch ran the screen's kernel
+ * qo_mc_ts_screen_kernel (qo_plan_kernel_name names the family, "qo_mc_ts_kernel") }.  The analyze form needs no GPU (meta[2] = 0);
+ * on an error meta holds the error code.  QO100NET_TS_HIST_SEEDS=low keeps only the band's lowest group as a seed (tests). */
+const char *qo_plan_ts_screen(const qo_plan *plan, double info[4], int meta[3]);
+const char *qo_plan_analyze_ts_screen(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
+                                      double info[4], int meta[3]);
 /* host->device bytes of this plan's tables per GPU, alignment padding included: the tables its kernel reads, copied by
  * qo_plan_create and again by every qo_mc_run call that reuses the plan */
 uint64_t qo_plan_h2d_bytes(const qo_plan *plan);

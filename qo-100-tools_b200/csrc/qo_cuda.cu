@@ -93,6 +93,7 @@ struct qo_plan {
     QoKern kern;
     /* launch-time decisions of the transfer-function kernels, taken once at plan creation */
     int tf_cpl_matched, tf_cpl_lin, ts_ok;
+    int ts_screen_ran;                                    /* the last thread-per-sample launch was qo_mc_ts_screen_kernel */
     double tf_cpl_dw1;                                    /* angular-frequency step of one grid point on a uniformly spaced grid */
     int lad_n, lad_first, lad_cpl;                        /* straight-line ladder kernel (qo_ladder.cuh) */
     int cpl_fast, cpl_same;                               /* coupler block: small-angle table path, equal mode angles */
@@ -933,6 +934,36 @@ extern "C" int qo_plan_analyze_ts_runs(const qo_net *net, const double *f, int n
     return ts_runs_out(&tp, runs, cap, meta);
 }
 
+/* the histogram screen of the thread-per-sample kernel: "ok" or why the plan declined it; info = { eps, smallest and largest
+ * threshold covered, worst error bound over eps/8 }; meta = { seed runs (the first ones of the run table), screened runs,
+ * whether the plan's last thread-per-sample launch ran qo_mc_ts_screen_kernel (0 before a launch and for the analyze form) } */
+static const char *ts_screen_out(const TfPlan *tp, double info[4], int meta[3])
+{
+    int n = 0;
+    for (int r = 0; r < tp->ts_nplain && tp->ts_screen_reason && !strcmp(tp->ts_screen_reason, "ok"); r++) n += tp->runs[r].kf > 0;
+    if (info) { info[0] = tp->ts_screen_eps; info[1] = tp->ts_screen_mlo; info[2] = tp->ts_screen_mhi; info[3] = tp->ts_screen_bound; }
+    if (meta) { meta[0] = tp->ts_nseed; meta[1] = n; meta[2] = 0; }
+    return tp->ts_screen_reason ? tp->ts_screen_reason : tp->reason && strcmp(tp->reason, "ok") ? tp->reason : "the job does not run thread-per-sample";
+}
+
+extern "C" const char *qo_plan_ts_screen(const qo_plan *p, double info[4], int meta[3])
+{
+    if (!p) return "";
+    const char *r = ts_screen_out(&p->tfp, info, meta);
+    if (meta) meta[2] = p->ts_screen_ran;
+    return r;
+}
+
+extern "C" const char *qo_plan_analyze_ts_screen(const qo_net *net, const double *f, int nf, const qo_spec *spec, int nspec, const qo_mc_cfg *cfg,
+                                                 double info[4], int meta[3])
+{
+    TfPlan tp;
+    int sel;
+    const char *reason = plan_analyze(net, f, nf, spec, nspec, cfg, &tp, &sel, NULL);
+    if (sel < 0) { if (meta) meta[0] = meta[1] = meta[2] = sel; return reason; }
+    return ts_screen_out(&tp, info, meta);
+}
+
 extern "C" int qo_plan_reset(qo_plan *p)
 {
     if (!p) return QO_ERR_ARG;
@@ -1140,9 +1171,11 @@ static int launch_tf(qo_plan *p, int g, unsigned long long off, unsigned long lo
             Q.ticket = P.ticket + 1;
             Q.w0 = 6.283185307179586476925286766559 * p->f[0];
             Q.dw = p->nf > 1 ? 6.283185307179586476925286766559 * ((p->f[p->nf - 1] - p->f[0]) / (double)(p->nf - 1)) : 0.0;
+            Q.screen_eps = p->tfp.ts_screen_eps; Q.screen_mlo = p->tfp.ts_screen_mlo; Q.screen_mhi = p->tfp.ts_screen_mhi;
             int rts = qo_ts_launch(&p->tfp, dc->sm_count, &Q, dc->stream);
             if (rts) { qo_set_error("thread-per-sample kernel launch: %s", cudaGetErrorString((cudaError_t)rts)); return QO_ERR_CUDA; }
-            p->kernel_name = "qo_mc_ts_kernel";
+            p->kernel_name = "qo_mc_ts_kernel";                   /* the family: qo_plan_ts_screen says whether its screen flavour ran */
+            p->ts_screen_ran = p->tfp.ts_nseed > 0;
             p->launches++;
             off += nb * 32ull; n -= nb * 32ull;
             if (n == 0) return QO_OK;

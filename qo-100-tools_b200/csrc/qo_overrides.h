@@ -22,6 +22,9 @@ struct QoOverrides {
     int cpl_sincos;       /* QO100NET_CPL_SINCOS set: coupler angles by sincos per point, no table of nominal angles */
     int ustrip_item;      /* QO100NET_USTRIP=item: microstrip yield jobs on the item kernel, not thread-per-board */
     int ts_full_len;      /* QO100NET_TS_FULL_LENGTHS set: every run of the thread-per-sample kernel walks the plan's full polynomial lengths */
+    int ts_no_screen;     /* QO100NET_TS_HIST_SCREEN=0: the thread-per-sample kernel walks the histogram band without its screen */
+    int ts_low_seed;      /* QO100NET_TS_HIST_SEEDS=low: the band's lowest group is the screen's only seed (tests: the tracker then rises
+                             after the seed, and the exact path moves the screen polynomial) */
 };
 
 /* QO_ERR_ARG (qo_last_error names the accepted values) when QO100NET_KERNEL holds anything but auto, spot, tf, ladder, interp */
@@ -46,6 +49,10 @@ static inline int qo_overrides_read(QoOverrides *ov)
     const char *u = getenv("QO100NET_USTRIP");
     ov->ustrip_item = u && !strcmp(u, "item");
     ov->ts_full_len = getenv("QO100NET_TS_FULL_LENGTHS") != NULL;
+    const char *hsc = getenv("QO100NET_TS_HIST_SCREEN");
+    ov->ts_no_screen = hsc && !strcmp(hsc, "0");
+    const char *hsd = getenv("QO100NET_TS_HIST_SEEDS");
+    ov->ts_low_seed = hsd && !strcmp(hsd, "low");
     return QO_OK;
 }
 

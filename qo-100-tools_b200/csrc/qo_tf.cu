@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 #include <complex>
 #include <vector>
+#include <algorithm>
 #include <mutex>
 #include <math.h>
 #include <stdlib.h>
@@ -452,6 +453,128 @@ static void tf_ts_runs(const DevProg *hp, int nf, const unsigned char *mask, con
     out->ts_runs_ok = 1;
 }
 
+/* The histogram screen of the thread-per-sample kernel (qo_ts.cuh).  The histogram spec needs only each sample's extreme of
+ * v = N2 / E over its band, and all but a few points of a ripple pass band are far from it.  Where that spec looks alone, the
+ * kernel walks the sign of S = +-(N2 - m E), m the extreme so far moved by eps to the conservative side, and evaluates a group
+ * exactly (today's operations) only where some lane's S is not certainly negative.  A point it skips has a computed v below
+ * the tracker, so the tracker, the bin and the verdict stay bit for bit what the full walk gives, provided that
+ *   - S's error (its Horner rounding, the formation and up to QO_TS_SCREEN_CAP updates in place, the coefficients above the
+ *     run's kf it leaves out) stays below eps/8 of m E, for every m in [mlo, mhi], and
+ *   - the computed v stays within eps/8 of the network's (the plan's self-check: out->err).
+ * The first bound is taken a priori from |coefficient| sums at every corner of the analysis and every point of the screened
+ * runs; mlo / mhi are half / twice the corners' extremes, and a lane outside them walks exactly.  Seeds: the groups of the
+ * nominal network's local extremes of v over the band and of the band's ends, walked exactly first (their runs are
+ * duplicates of groups of the band: walking a point twice leaves an extreme unchanged), so that m starts near the sample's
+ * extreme.  Sets ts_screen_reason to "ok" or why not. */
+static void tf_hist_screen(const DevProg *hp, int nf, const double *xg, const std::vector<TfCorner> &cs, double zni, int off, int low_seed,
+                           TfPlan *out)
+{
+    out->ts_nseed = 0; out->ts_screen_eps = QO_TS_SCREEN_EPS; out->ts_screen_mlo = out->ts_screen_mhi = out->ts_screen_bound = 0.0;
+#define QO_TS_SCREEN_NO(msg) do { out->ts_screen_reason = msg; return; } while (0)
+    if (!out->ts_runs_ok) QO_TS_SCREEN_NO("the job does not run thread-per-sample");
+    if (off) QO_TS_SCREEN_NO("QO100NET_TS_HIST_SCREEN=0");
+    if (hp->hist_bins <= 0) QO_TS_SCREEN_NO("no histogram");
+    if (out->nn != 2) QO_TS_SCREEN_NO("numerator polynomials kept apart (coupled-line block in front)");
+    const int hs = hp->hist_spec;
+    const unsigned int hb = 1u << hs;
+    std::vector<int> band;                                            /* runs where the histogram spec looks alone */
+    for (int r = 0; r < out->ts_nplain; r++) if (out->runs[r].any == hb && out->runs[r].all == hb) band.push_back(r);
+    if (band.empty()) QO_TS_SCREEN_NO("the histogram spec shares every run with another spec");
+    const bool hneg = hp->spec_kind[hs] == SK_DEN2_MIN;
+    const int gpt = qo_ts_group_points(out), KN = out->kn, KE = out->den == QO_TF_DEN_E ? out->kd : 0, NSG = 2 * KN > KE ? 2 * KN : KE;
+    const double eps = QO_TS_SCREEN_EPS, u = 0x1p-53, gam = NSG * u / (1.0 - NSG * u);
+    const double zq0 = hp->rs * zni;
+    /* per corner: |N2| coefficient bounds, |E|, and v at the band's points; the corner's extreme */
+    struct Pt { int k, run; };
+    std::vector<Pt> pts;
+    for (int r : band)
+        for (int k = out->runs[r].g0 * gpt; k < (out->runs[r].g0 + out->runs[r].ngroups) * gpt && k < nf; k++) pts.push_back(Pt{ k, r });
+    const size_t nc = cs.size(), np = pts.size();
+    std::vector<double> v(nc * np), ext(nc);
+    std::vector<double> an2(nc * NSG), ae(nc * NSG);
+    for (size_t ci = 0; ci < nc; ci++) {
+        double cn[2 * QO_TF_MAXK];
+        for (int i = 0; i < 2 * KN; i++) cn[i] = fma(zq0, cs[ci].qq[i], cs[ci].pp[i]);
+        double *a = &an2[ci * NSG], *e = &ae[ci * NSG];
+        for (int k = 0; k < NSG; k++) {
+            a[k] = 0.0;
+            for (int i = 0; i < KN; i++) {
+                if (k - i >= 0 && k - i < KN) a[k] += fabs(cn[2 * i] * cn[2 * (k - i)]);
+                if (k - 1 - i >= 0 && k - 1 - i < KN) a[k] += fabs(cn[2 * i + 1] * cn[2 * (k - 1 - i) + 1]);
+            }
+            e[k] = KE > 0 ? (k < KE ? fabs(cs[ci].ee[k]) : 0.0) : (k == 0 ? 1.0 : 0.0);
+        }
+        ext[ci] = hneg ? HUGE_VAL : -HUGE_VAL;
+        for (size_t j = 0; j < np; j++) {
+            const long double yl = -(xg[pts[j].k] * xg[pts[j].k]);
+            long double r0 = cn[2 * KN - 2], r1 = cn[2 * KN - 1], el = KE > 0 ? cs[ci].ee[KE - 1] : 1.0;
+            for (int i = KN - 2; i >= 0; i--) { r0 = r0 * yl + cn[2 * i]; r1 = r1 * yl + cn[2 * i + 1]; }
+            for (int m = KE - 2; m >= 0; m--) el = el * yl + cs[ci].ee[m];
+            const double vv = (double)((r0 * r0 - yl * r1 * r1) / el);
+            v[ci * np + j] = vv;
+            if (!(el > 0.0L) || !(vv > 0.0)) QO_TS_SCREEN_NO("E or |numerator|^2 not positive in the band");
+            if (hneg ? vv < ext[ci] : vv > ext[ci]) ext[ci] = vv;
+        }
+    }
+    double mlo = HUGE_VAL, mhi = 0.0;
+    for (size_t ci = 0; ci < nc; ci++) { if (ext[ci] < mlo) mlo = ext[ci]; if (ext[ci] > mhi) mhi = ext[ci]; }
+    mlo *= 0.5; mhi *= 2.0;
+    /* the a priori bound on S relative to m E at every corner and point, each screened run walking kf = max(2 kn, ke) of its own */
+    double worst = 0.0;
+    for (size_t ci = 0; ci < nc; ci++)
+        for (size_t j = 0; j < np; j++) {
+            const TsRun &r = out->runs[pts[j].run];
+            const int ks = 2 * r.kn > r.ke ? 2 * r.kn : r.ke;
+            const double ay = xg[pts[j].k] * xg[pts[j].k];
+            double ns = 0.0, es = 0.0, nt = 0.0, et = 0.0, pw = 1.0;
+            for (int k = 0; k < NSG; k++) {
+                const double a = an2[ci * NSG + k] * pw, e = ae[ci * NSG + k] * pw;
+                ns += a; es += e;
+                if (k >= ks) { nt += a; et += e; }
+                pw *= ay;
+            }
+            long double el = KE > 0 ? cs[ci].ee[KE - 1] : 1.0;
+            for (int m = KE - 2; m >= 0; m--) el = el * (long double)(-ay) + cs[ci].ee[m];
+            const double ev = (double)el;
+            const double b = (gam * ns + (3 + 2 * QO_TS_SCREEN_CAP) * u * (ns + mhi * es) + nt) / (mlo * ev) + (gam * es + et) / ev;
+            if (!(b <= worst)) worst = b == b ? b : HUGE_VAL;
+        }
+    out->ts_screen_bound = worst / (eps / 8.0);
+    if (!(worst <= eps / 8.0)) QO_TS_SCREEN_NO("the screen's error bound exceeds eps/8");
+    if (!(out->err <= eps / 8.0)) QO_TS_SCREEN_NO("the self-check error exceeds eps/8");
+    /* seeds: the nominal network's local extremes of v over the band, and the band's two ends, most extreme first */
+    const size_t nom = nc > 1 ? QO_TF_NOMINAL : 0;
+    std::vector<std::pair<double, int>> cand;                       /* (extremeness, point index into pts) */
+    for (size_t j = 0; j < np; j++) {
+        const double w = v[nom * np + j], sgn = hneg ? -1.0 : 1.0;
+        const bool edge = j == 0 || j + 1 == np || pts[j - 1].k + 1 != pts[j].k || pts[j + 1].k != pts[j].k + 1;
+        const bool peak = !edge && sgn * w >= sgn * v[nom * np + j - 1] && sgn * w >= sgn * v[nom * np + j + 1];
+        if (edge || peak) cand.push_back(std::make_pair(sgn * w, (int)j));
+    }
+    std::sort(cand.begin(), cand.end(), [](const std::pair<double, int> &a, const std::pair<double, int> &b) { return a.first > b.first; });
+    if (low_seed) cand.assign(1, std::make_pair(0.0, 0));             /* QO100NET_TS_HIST_SEEDS=low: the band's lowest group alone */
+    TsRun seeds[QO_TS_NSEED];
+    int ns = 0;
+    for (const auto &c : cand) {
+        if (ns >= QO_TS_NSEED || out->ts_nruns + ns >= QO_TS_MAXRUN) break;
+        const int g = pts[c.second].k / gpt;
+        bool dup = false;
+        for (int i = 0; i < ns; i++) dup |= seeds[i].g0 == g;
+        if (dup) continue;
+        seeds[ns] = out->runs[pts[c.second].run];
+        seeds[ns].g0 = g; seeds[ns].ngroups = 1; seeds[ns].kf = 0;
+        ns++;
+    }
+    if (ns == 0) QO_TS_SCREEN_NO("no room in the run table for a seed");
+    for (int r : band) { const TsRun &b = out->runs[r]; out->runs[r].kf = 2 * b.kn > b.ke ? 2 * b.kn : b.ke; }
+    memmove(&out->runs[ns], &out->runs[0], sizeof(TsRun) * (size_t)out->ts_nruns);
+    memcpy(&out->runs[0], seeds, sizeof(TsRun) * (size_t)ns);
+    out->ts_nruns += ns; out->ts_nplain += ns; out->ts_nseed = ns;
+    out->ts_screen_mlo = mlo; out->ts_screen_mhi = mhi;
+    out->ts_screen_reason = "ok";
+#undef QO_TS_SCREEN_NO
+}
+
 static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int precision, int generic, const double *f, int nf,
                                   const unsigned char *mask, const QoOverrides *ov, TfPlan *out)
 {
@@ -690,6 +813,7 @@ static int tf_plan_check_uncached(const DevProg *hp, int mode_reduce_only, int p
     if (!accepted) QO_TF_NO("polynomial expansion is too ill-conditioned on this grid");
     tf_fuse_gate(hp, nf, xg.data(), mask, cs, zni, out);
     tf_ts_runs(hp, nf, mask, xg.data(), cs, zni, need_n.data(), need_e.data(), trunc, tol, ov->ts_full_len, check_point, out);
+    tf_hist_screen(hp, nf, xg.data(), cs, zni, ov->ts_no_screen, ov->ts_low_seed, out);
     out->reason = "ok";
     return 1;
 #undef QO_TF_NO

@@ -73,26 +73,29 @@ QO_TF_HD void qo_tf_dd_fma(double &s, double &c, double a, double b)
     c += ((s - (t - bp)) + (p - bp)) + pe;
     s = t;
 }
+/* coefficient k of F (the histogram screen of qo_ts.cuh forms them one at a time) */
+QO_TF_HD double qo_tf_fuse_coef(int k, int kn, int ke, const double *cn, const double *ce, double t, bool neg)
+{
+    double s = 0.0, c = 0.0;
+#pragma unroll
+    for (int i = 0; i < kn; i++) {                        /* r0^2: a_i a_j (i + j = k), the off-diagonal pairs once, doubled */
+        const int j = k - i;
+        if (j >= i && j < kn) qo_tf_dd_fma(s, c, i == j ? cn[2 * i] : 2.0 * cn[2 * i], cn[2 * j]);
+    }
+#pragma unroll
+    for (int i = 0; i < kn; i++) {                        /* - y r1^2: b_i b_j (i + j = k - 1) */
+        const int j = k - 1 - i;
+        if (j >= i && j < kn) qo_tf_dd_fma(s, c, i == j ? -cn[2 * i + 1] : -2.0 * cn[2 * i + 1], cn[2 * j + 1]);
+    }
+    if (k < (ke > 0 ? ke : 1)) qo_tf_dd_fma(s, c, -t, ke > 0 ? ce[k] : 1.0);
+    const double v = s + c;
+    return (neg ? v : -v) + 0.0;
+}
 QO_TF_HD void qo_tf_fuse(int kn, int ke, const double *cn, const double *ce, double t, bool neg, double *f)
 {
     const int nf = 2 * kn > ke ? 2 * kn : ke;
 #pragma unroll
-    for (int k = 0; k < nf; k++) {
-        double s = 0.0, c = 0.0;
-#pragma unroll
-        for (int i = 0; i < kn; i++) {                        /* r0^2: a_i a_j (i + j = k), the off-diagonal pairs once, doubled */
-            const int j = k - i;
-            if (j >= i && j < kn) qo_tf_dd_fma(s, c, i == j ? cn[2 * i] : 2.0 * cn[2 * i], cn[2 * j]);
-        }
-#pragma unroll
-        for (int i = 0; i < kn; i++) {                        /* - y r1^2: b_i b_j (i + j = k - 1) */
-            const int j = k - 1 - i;
-            if (j >= i && j < kn) qo_tf_dd_fma(s, c, i == j ? -cn[2 * i + 1] : -2.0 * cn[2 * i + 1], cn[2 * j + 1]);
-        }
-        if (k < (ke > 0 ? ke : 1)) qo_tf_dd_fma(s, c, -t, ke > 0 ? ce[k] : 1.0);
-        const double v = s + c;
-        f[k] = (neg ? v : -v) + 0.0;
-    }
+    for (int k = 0; k < nf; k++) f[k] = qo_tf_fuse_coef(k, kn, ke, cn, ce, t, neg);
 }
 
 /* structural degree an element adds to the polynomials (max(deg N, deg D)); 0 = resistor, -1 = not lumped */

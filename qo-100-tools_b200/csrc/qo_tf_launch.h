@@ -11,8 +11,14 @@ struct TsRun {
     int g0, ngroups;             /* first group, groups */
     unsigned int any, all;       /* spec bits seen by some / by every point of the run */
     int kn, ke;                  /* |numerator|^2 and E runs: numerator pairs and E coefficients walked (ke 0 without E) */
-    int kf;                      /* runs of the fused spec: margin coefficients walked (0 on the other runs) */
+    int kf;                      /* runs of the fused spec: margin coefficients walked; runs of the histogram spec alone: coefficients
+                                    of its screen walked (0: not screened); 0 on the other runs */
 };
+/* The histogram screen of the thread-per-sample kernel (qo_ts.cuh, plain ladders; its gate, qo_tf.cu::tf_hist_screen):
+ * updates of the screen polynomial in place per sample, the plan's relative margin and its seed runs at most */
+#define QO_TS_SCREEN_CAP 8
+#define QO_TS_SCREEN_EPS 1e-6
+#define QO_TS_NSEED 10
 /* what the plan decided for a job that runs on the transfer-function kernel */
 struct TfPlan {
     int nn;              /* numerator chains: 2 (Num = P + Rs Q) or 4 (P and Q apart: behind a coupled-line block, or with |S11| specs) */
@@ -34,6 +40,12 @@ struct TfPlan {
      * groups; ts_runs_ok = 0 when the band edges need more runs than the table holds */
     TsRun runs[QO_TS_MAXRUN];
     int ts_nruns, ts_nplain, ts_npt, ts_runs_ok;
+    /* the histogram screen (runs with kf > 0 among the plain ones): its relative margin and the thresholds it covers, the seed runs
+     * (the first ts_nseed runs: hist-band groups walked exactly before any screened one), the worst error bound the gate saw
+     * relative to the margin, and "ok" or why the plan declined it */
+    double ts_screen_eps, ts_screen_mlo, ts_screen_mhi, ts_screen_bound;
+    int ts_nseed;
+    const char *ts_screen_reason;
 };
 /* Can this job run on the transfer-function kernel?  Structural test, choice of the polynomial lengths the grid needs,
  * and a numerical self-check of exactly what the device will evaluate against the per-element evaluation, at the

@@ -1,8 +1,8 @@
 /*
  * qo_ts.cu -- instantiations and launcher of the thread-per-sample transfer-function kernel (qo_ts.cuh).
- * The kernels themselves are instantiated in qo_ts2a.cu, qo_ts2b.cu, qo_ts2c.cu and qo_ts4.cu (most of the library's compile
- * time, hence in parallel).  Development builds: -DQO_TS_DEV_KN=9 -DQO_TS_DEV_KE=14 -DQO_TS_DEV_KN2=8 -DQO_TS_DEV_KE2=8 compiles
- * those loop bodies only.
+ * The kernels themselves are instantiated in qo_ts2a.cu, qo_ts2b.cu, qo_ts2c.cu, qo_ts4.cu and, behind the histogram screen,
+ * qo_ts2sa.cu ... qo_ts2sc.cu (most of the library's compile time, hence in parallel).  Development builds:
+ * -DQO_TS_DEV_KN=9 -DQO_TS_DEV_KE=14 -DQO_TS_DEV_KN2=8 -DQO_TS_DEV_KE2=8 compiles those loop bodies only.
  */
 #include <cuda_runtime.h>
 #include "qo_ts.cuh"
@@ -24,6 +24,8 @@ extern "C" int qo_ts_eligible(const TfPlan *tp, int nspec, int cpl_rot_same)
 static ts_fn ts_pick_kernel(const TfPlan *tp)
 {
     if (tp->cpl_op >= 0) return qo_ts_kernel_4(tp->kn);
+    if (tp->ts_nseed > 0)                /* the plan screens the histogram band (tf_hist_screen) */
+        return tp->kn <= 5 ? qo_ts_screen_kernel_a(tp->kn) : tp->kn <= 8 ? qo_ts_screen_kernel_b(tp->kn) : qo_ts_screen_kernel_c(tp->kn);
     return tp->kn <= 5 ? qo_ts_kernel_2a(tp->kn) : tp->kn <= 8 ? qo_ts_kernel_2b(tp->kn) : qo_ts_kernel_2c(tp->kn);
 }
 

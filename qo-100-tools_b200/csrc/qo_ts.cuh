@@ -28,6 +28,11 @@
  *            last; after the other runs the thread forms the polynomial once in double-double (qo_tf_core.h::qo_tf_fuse, in the
  *            registers of the expansion, which are dead by then) and walks the runs with one Horner chain per point:
  *            2 KN - 1 or KE - 1 DFMA per point instead of 2 (KN - 1) + (KE - 1) + 4 (cfg2: 17 instead of 33);
+ *            Where the histogram spec alone looks (plain ladders, the plan's tf_hist_screen), qo_mc_ts_screen_kernel walks the
+ *            sign of S = +-(N2 - m E) instead, m the tracker moved by a relative eps to the conservative side, S formed once
+ *            after the plan's seed runs (single hist-band groups walked exactly first) and kept in shared memory; a batch of
+ *            QO_TS_FG2 groups goes exactly (the loop above, on every lane) only where some lane's S is not certainly negative,
+ *            which keeps the tracker bit for bit (cfg2: 15 DFMA per point instead of ~27 FP64 operations, 0.3 % exact);
  *   stage D  verdict per thread, counters by warp ballots, the histogram value (a log10) at full lane efficiency.
  *
  * Stage A costs ~4 500 instructions per sample against ~180 000 for the loop (the warp-cooperative expansion of qo_tf.cuh:
@@ -69,6 +74,11 @@ struct TsParams {
     unsigned long long nbatches;         /* 32-sample batches, handed to the warps through a ticket counter */
     unsigned long long *ticket;          /* zeroed per launch */
     double w0, dw;                       /* coupler on a uniform grid: first angular frequency and step */
+    /* the histogram screen (plain ladders): the histogram spec's runs with kf > 0 are walked behind the sign of the first kf
+     * coefficients of S = +-(N2 - m E), m the sample's extreme so far moved by the relative screen_eps to the conservative side;
+     * a lane screens, and moves m, only inside [screen_mlo, screen_mhi], the thresholds the plan's error bound covers.  Behind
+     * every field the kernels read before, so that their parameter offsets stay */
+    double screen_eps, screen_mlo, screen_mhi;
 };
 
 /* NC interleaved Horner chains of PT points each, entered at a run-time length L (warp-uniform, 2 <= L <= K, K <= 20):
@@ -135,8 +145,8 @@ hdone:
  * plan from the band edges): inside a run the spec bookkeeping branches on loop-invariant, warp-uniform predicates -- nothing
  * is loaded or decoded per group except the PT grid values themselves.  Groups that straddle a band edge are runs of their own
  * and take their per-point byte masks. */
-template <int NN, int KN, int KE, bool CPL, int NS, int PT>
-__device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sample, unsigned int (&acc)[NS], double &trkv)
+template <int NN, int KN, int KE, bool CPL, int NS, int PT, bool SCREEN>
+__device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sample, unsigned int (&acc)[NS], double &trkv, double (*sg)[QO_TS_TPB])
 {
     static_assert(PT == 2 || PT == 4, "two or four points in flight");
     constexpr int NC = 2 * KN;           /* kept coefficients per numerator polynomial */
@@ -249,6 +259,14 @@ __device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sa
                                             the sign of the TRUNCATED E(y) is masked off -- the plan validates it only where a spec
                                             looks, and beyond the last band it may well go negative (found by tools/fuzz_parity.py: it
                                             used to fail spec 0 on such samples) */
+    /* the histogram screen (qo_mc_ts_screen_kernel): sg = +-(N2 - mh E), formed once the seed runs have set the tracker,
+     * negative (strictly, not NaN) where the computed value cannot reach the tracker */
+    static_assert(!SCREEN || NN == 2, "the screen is for plain ladders");
+    constexpr int NSG = 2 * KN > KE ? 2 * KN : KE;
+    const int tc = threadIdx.x;
+    double mh = 0.0;
+    int nup = -1;                        /* updates of sg in place; -1 before it is formed */
+    bool scr = false;                    /* this lane screens: mh within the range the plan's error bound covers */
     int gi = 0;
     for (int rn = 0; rn < Q.nplain; rn++) {
         const unsigned int any = Q.runs[rn].any, all = Q.runs[rn].all;
@@ -263,6 +281,64 @@ __device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sa
         if (any == 0u) {
             for (; gi < g_end; gi++) { QO_TS_CORE QO_PTS_N(PT) idle |= tf_hi(n2[p]) | (tf_hi(dd[p]) & 0x7fffffffu); }
         } else if (one >= 0 && one == hs) {
+            if constexpr (SCREEN) {
+                if (Q.runs[rn].kf > 0) {
+                    const int rks = Q.runs[rn].kf;
+                    if (nup < 0) {
+                        nup = 0;
+                        mh = hneg ? trkv * (1.0 + Q.screen_eps) : trkv * (1.0 - Q.screen_eps);
+                        scr = mh >= Q.screen_mlo && mh <= Q.screen_mhi;
+#pragma unroll
+                        for (int k = 0; k < NSG; k++) sg[k][tc] = qo_tf_fuse_coef(k, KN, KE, cn, ce, mh, !hneg);
+                    }
+                    /* QO_TS_FG2 groups at a time: twelve independent chains (four leave the FP64 pipe waiting on latency) and one load
+                     * of a coefficient for twelve points; the groups go exactly together when some lane needs one of them */
+                    constexpr int PS = QO_TS_FG2 * PT;
+                    double ys[PS];
+#pragma unroll
+                    for (int h = 0; h < PS; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + gi * PT + h)); ys[h] = a.x; ys[h + 1] = a.y; }
+                    for (; gi < g_end;) {
+                        const int gn = g_end - gi < QO_TS_FG2 ? g_end - gi : QO_TS_FG2;
+                        bool need = !scr || gn < QO_TS_FG2;          /* the run's last groups go exactly */
+                        if (!need) {
+                            double F[PS];
+                            {
+                                const double top = sg[rks - 1][tc];
+                                QO_PTS_N(PS) F[p] = top;
+                            }
+                            for (int m = rks - 2; m >= 0; m--) { const double g = sg[m][tc]; QO_PTS_N(PS) F[p] = fma(F[p], ys[p], g); }
+#pragma unroll
+                            for (int h = 0; h < PS; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + (gi + QO_TS_FG2) * PT + h)); ys[h] = a.x; ys[h + 1] = a.y; }
+                            QO_PTS_N(PS) need |= !(F[p] < 0.0);
+                        }
+                        if (!__any_sync(0xffffffffu, need)) { gi += QO_TS_FG2; continue; }
+                        /* the groups exactly, as below: every lane, so the tree of tf_extreme sees what it always saw */
+#pragma unroll
+                        for (int h = 0; h < PT; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + gi * PT + h)); y[h] = a.x; y[h + 1] = a.y; }
+                        for (const int ge = gi + gn; gi < ge; gi++) {
+                            QO_TS_CORE
+                            QO_TS_VALUE
+                            const double t0 = trkv;
+                            trkv = hneg ? tf_extreme<PT, true>(val, trkv) : tf_extreme<PT, false>(val, trkv);
+                            const double mn = hneg ? trkv * (1.0 + Q.screen_eps) : trkv * (1.0 - Q.screen_eps);
+                            if (scr && trkv != t0 && nup < QO_TS_SCREEN_CAP && mn >= Q.screen_mlo && mn <= Q.screen_mhi) {   /* move mh behind the tracker: the E rows of sg */
+                                const double c = hneg ? mn - mh : mh - mn;
+                                if constexpr (KE > 0) {
+#pragma unroll
+                                    for (int k = 0; k < KE; k++) sg[k][tc] = fma(c, ce[k], sg[k][tc]);
+                                } else sg[0][tc] += c;
+                                mh = mn;
+                                nup++;
+                            }
+                        }
+#pragma unroll
+                        for (int h = 0; h < PS; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + gi * PT + h)); ys[h] = a.x; ys[h + 1] = a.y; }
+                    }
+#pragma unroll
+                    for (int h = 0; h < PT; h += 2) { const double2 a = __ldg((const double2 *)(Q.y1 + gi * PT + h)); y[h] = a.x; y[h + 1] = a.y; }
+                    continue;
+                }
+            }
             for (; gi < g_end; gi++) {
                 QO_TS_CORE
                 QO_TS_VALUE
@@ -345,12 +421,12 @@ __device__ __forceinline__ void ts_loop(const TsParams &Q, unsigned long long sa
 #define QO_TS_KE_OK(k) true
 #endif
 /* the loop body for this launch's kd (KN is the kernel's): one switch per sample, outside the frequency loop */
-template <int NN, int KN, bool CPL, int NS, int PT>
-__device__ __forceinline__ void ts_pick_e(const TsParams &Q, unsigned long long sample, unsigned int (&acc)[NS], double &trkv)
+template <int NN, int KN, bool CPL, int NS, int PT, bool SCREEN>
+__device__ __forceinline__ void ts_pick_e(const TsParams &Q, unsigned long long sample, unsigned int (&acc)[NS], double &trkv, double (*sg)[QO_TS_TPB])
 {
     constexpr int CAPE = NN == 2 ? QO_TS_CAPE2 : QO_TS_CAPE4;
     const int kd = Q.t.den == QO_TF_DEN_E ? Q.t.kd : 0;
-#define QO_TS_CASE(K) case K: if (K <= CAPE && QO_TS_KE_OK(K)) ts_loop<NN, KN, (K <= CAPE ? K : 0), CPL, NS, PT>(Q, sample, acc, trkv); break;
+#define QO_TS_CASE(K) case K: if (K <= CAPE && QO_TS_KE_OK(K)) ts_loop<NN, KN, (K <= CAPE ? K : 0), CPL, NS, PT, SCREEN>(Q, sample, acc, trkv, sg); break;
 #ifdef QO_TS_DEV_KN
     if (!QO_TS_KN_OK(KN) || !QO_TS_KE_OK(kd)) __trap();          /* a development build was asked for a body it does not carry */
 #endif
@@ -388,7 +464,56 @@ __global__ void __launch_bounds__(QO_TS_TPB, MINB) qo_mc_ts_kernel(const __grid_
 #pragma unroll
         for (int sp = 0; sp < NS; sp++) acc[sp] = 0u;
         double trkv = hneg ? 1.7e308 : -1.7e308;
-        ts_pick_e<NN, KN, CPL, NS, PT>(Q, sample, acc, trkv);
+        ts_pick_e<NN, KN, CPL, NS, PT, false>(Q, sample, acc, trkv, nullptr);
+        /* stage D: verdict per thread */
+        unsigned int fail = 0;
+#pragma unroll
+        for (int sp = 0; sp < NS; sp++)
+            if (sp < P.nspec && sp != hs && (acc[sp] >> 31)) fail |= 1u << sp;
+        if (hs >= 0) {
+            const double t = P.thr[hs & (QO_TF_NSPEC - 1)];
+            if (hneg ? trkv < t : trkv > t) fail |= 1u << hs;
+        }
+        qo_tally_warp(s_cnt, P.nspec, fail, 0xffffffffu);
+        if (hs >= 0) {
+            const double k21 = P.k21;
+            const double lin = hneg ? k21 * k21 * (1.0 / trkv) : k21 * k21 / trkv;
+            qo_tally_hist(s_cnt, P.nspec, qo_hist_bin(10.0 * log10(lin), P.hist_lo, P.hist_hi, P.hist_bins));
+        }
+        batch = __shfl_sync(0xffffffffu, next, 0);
+    }
+    __syncthreads();
+    qo_tally_flush<QO_TS_TPB>(s_cnt, ncnt, P.counters);
+}
+
+/* plain ladders whose plan walks the histogram band behind its screen (TsRun::kf on the histogram spec's runs): the same kernel
+ * with the screen's loop.  The screen's polynomial sits in shared memory, one column per thread: next to cn and ce it does not
+ * fit the registers (cfg2: 18 + 18 + 14 coefficients), and one load serves the points walked at once */
+template <int PT, int MINB, int KN>
+__global__ void __launch_bounds__(QO_TS_TPB, MINB) qo_mc_ts_screen_kernel(const __grid_constant__ TsParams Q)
+{
+    constexpr int NS = 4, NN = 2;
+    constexpr bool CPL = false;
+    const TfParams &P = Q.t;
+    __shared__ unsigned int s_cnt[QO_NCNT_MAX];
+    __shared__ double s_sg[2 * KN > QO_TS_CAPE2 ? 2 * KN : QO_TS_CAPE2][QO_TS_TPB];
+    const int lane = threadIdx.x & 31;
+    const int ncnt = qo_ncnt(P.nspec, P.hist_bins);
+    qo_tally_zero<QO_TS_TPB>(s_cnt, ncnt);
+    __syncthreads();
+    const int hs = P.hist_spec;
+    const bool hneg = hs >= 0 && P.neg[hs & (QO_TF_NSPEC - 1)];
+    const unsigned long long nwarps = (unsigned long long)gridDim.x * (QO_TS_TPB / 32);        /* batches by ticket, as above */
+    unsigned long long batch = (unsigned long long)blockIdx.x * (QO_TS_TPB / 32) + (threadIdx.x >> 5);
+    while (batch < Q.nbatches) {
+        unsigned long long next = 0;
+        if (lane == 0) next = nwarps + atomicAdd(Q.ticket, 1ull);
+        const unsigned long long sample = batch * 32ull + (unsigned long long)lane;
+        unsigned int acc[NS];
+#pragma unroll
+        for (int sp = 0; sp < NS; sp++) acc[sp] = 0u;
+        double trkv = hneg ? 1.7e308 : -1.7e308;
+        ts_pick_e<NN, KN, CPL, NS, PT, true>(Q, sample, acc, trkv, s_sg);
         /* stage D: verdict per thread */
         unsigned int fail = 0;
 #pragma unroll

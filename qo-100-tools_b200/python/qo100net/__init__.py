@@ -93,7 +93,7 @@ EXPORTS = [
     "qo_ctx_num_devices", "qo_ctx_destroy", "qo_sweep", "qo_mc_run", "qo_plan_create", "qo_plan_num_counters",
     "qo_plan_reset", "qo_plan_launch", "qo_plan_read", "qo_plan_flops_per_eval", "qo_plan_launches",
     "qo_plan_kernel_name", "qo_plan_tf_info", "qo_plan_h2d_bytes", "qo_plan_analyze", "qo_chain_jit_analyze",
-    "qo_plan_ts_runs", "qo_plan_analyze_ts_runs",
+    "qo_plan_ts_runs", "qo_plan_analyze_ts_runs", "qo_plan_ts_screen", "qo_plan_analyze_ts_screen",
     "qo_s2p_load", "qo_s2p_from_arrays", "qo_s2p_num_points", "qo_s2p_z0", "qo_s2p_get", "qo_s2p_interp",
     "qo_s2p_fit_inductor", "qo_s2p_free", "qo_net_from_sblock",
     "qo_nodal_create", "qo_nodal_add_branch", "qo_nodal_add_port", "qo_nodal_add_sblock", "qo_nodal_load_qucs_sch",
@@ -154,6 +154,8 @@ def lib():
         "qo_plan_h2d_bytes": (C.c_uint64, [vp]),
         "qo_plan_ts_runs": (C.c_int, [vp, C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_int)]),
         "qo_plan_analyze_ts_runs": (C.c_int, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_int), C.c_int, C.POINTER(C.c_int)]),
+        "qo_plan_ts_screen": (C.c_char_p, [vp, C.POINTER(C.c_double), C.POINTER(C.c_int)]),
+        "qo_plan_analyze_ts_screen": (C.c_char_p, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_double), C.POINTER(C.c_int)]),
         "qo_chain_jit_analyze": (C.c_int, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_int)]),
         "qo_plan_analyze": (C.c_char_p, [vp, C.POINTER(C.c_double), C.c_int, vp, C.c_int, vp, C.POINTER(C.c_int), C.POINTER(C.c_double), C.POINTER(C.c_uint), C.POINTER(C.c_double), C.POINTER(C.c_double)]),
         "qo_s2p_load": (C.c_int, [C.c_char_p, C.POINTER(vp)]),
@@ -644,6 +646,29 @@ def plan_ts_runs(net, f, specs, tols=(), dist=DIST_UNIFORM, mode=MODE_REDUCE_ONL
     return _ts_runs(lib().qo_plan_analyze_ts_runs, net._h, _dp(f), len(f), _specs(specs), len(specs), C.byref(cfg))
 
 
+def _ts_screen(fn, *args):
+    """The thread-per-sample kernel's histogram screen (qo_plan_ts_screen / qo_plan_analyze_ts_screen): reason ("ok" when the
+    histogram spec's runs are screened), eps, the tracker values it covers, the worst error bound over eps/8, and the seed and
+    screened runs' counts (the seeds are the first runs of the run table), and whether the plan's last launch ran the screen's
+    kernel qo_mc_ts_screen_kernel (Plan.kernel_name names the family, qo_mc_ts_kernel)."""
+    info = (C.c_double * 4)()
+    meta = (C.c_int * 3)()
+    reason = fn(*args, info, meta).decode()
+    if meta[0] < 0:
+        raise QoError(meta[0], reason)
+    return dict(reason=reason, screened=reason == "ok", eps=info[0], m_lo=info[1], m_hi=info[2], bound=info[3],
+                seeds=meta[0], screened_runs=meta[1], screen_kernel_ran=bool(meta[2]))
+
+
+def plan_ts_screen(net, f, specs, tols=(), dist=DIST_UNIFORM, mode=MODE_REDUCE_ONLY, precision=64,
+                   hist_bins=0, hist_spec=0, hist_lo=0.0, hist_hi=1.0):
+    """Host-only (qo_plan_analyze_ts_screen): whether the thread-per-sample kernel would walk the histogram band behind its
+    screen (see _ts_screen)."""
+    f = np.ascontiguousarray(f, dtype=np.float64)
+    cfg = _cfg(0, 0, list(tols), 0, dist, mode, precision, hist_bins, hist_spec, hist_lo, hist_hi)
+    return _ts_screen(lib().qo_plan_analyze_ts_screen, net._h, _dp(f), len(f), _specs(specs), len(specs), C.byref(cfg))
+
+
 def plan_analyze(net, f, specs, tols=(), dist=DIST_UNIFORM, mode=MODE_REDUCE_ONLY, precision=64,
                  hist_bins=0, hist_spec=0, hist_lo=0.0, hist_hi=1.0):
     """Host-only part of plan creation (qo_plan_analyze, no GPU needed): which kernel family the job would take and the
@@ -722,7 +747,7 @@ class Plan:
         runs = [(r["point"], r["points"], r["kf"] if r["fused"] else (r["kn"], r["ke"])) for r in self.ts_runs]
         return dict(selected=bool(info[0]), numerator_chains=info[1], den_form=("none", "E", "D", "DD")[info[2]] if 0 <= info[2] <= 3 else "?",
                     kn=info[3], kd=info[4], degree=info[5], self_check_err=err.value, fused_specs=fused.value, fused_err=ferr.value,
-                    reason=reason, ts_runs=runs)
+                    reason=reason, ts_runs=runs, hist_screen=_ts_screen(lib().qo_plan_ts_screen, self._h))
 
     @property
     def ts_runs(self):
